@@ -3,7 +3,7 @@
 bench.py -- BASELINE.json's headline measurement: Gcell-steps/s (and % of the HBM roofline) of the
 Fenton 4v spiral-wave fibrillation run on a 32768x32768 grid, row-sharded over N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--size S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--size S] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one run() iteration of the reference driver loop = dt_per_step = 10 explicit time
@@ -58,21 +58,6 @@ def fenton_config(size, duration, distributed=False, **kw):
 # ---------------------------------------------------------------------------------------------
 # synthetic input: a developed 512^2 spiral, mirror-tiled (SURVEY.md 8d item 5)
 # ---------------------------------------------------------------------------------------------
-def spiral_tile_gpu(device):
-    """S1-S2 protocol of fenton.py:155-185 on 512^2 (no hole) run to 400 ms on the GPU."""
-    from fib_tf_b200.fenton import Fenton4v
-    m = Fenton4v(fenton_config(TILE, 400, device=device))
-    m.define()
-    m.add_pace_op('s2', 'luq', 1.0)
-    s2 = m.millisecond_to_step(210)
-    m._ctx.step(0, s2 + 1)
-    m.fire_op('s2')
-    m._ctx.step(0, m.millisecond_to_step(400) - s2 - 1)
-    tile = {n: m._State[n].local() for n in ('U', 'V', 'W', 'S')}
-    m.close()
-    return tile
-
-
 def strips_of(tile_plane, width):
     """[512, width] strips for even / odd tile rows: alternate tiles are mirrored so that every
     tile seam is a mirror plane, i.e. a no-flux boundary of the small problem."""
@@ -237,9 +222,11 @@ def numpy_restatement_baseline(iterations=20):
 
 
 def spiral_tile_cpu():
-    """The developed 512^2 spiral WITHOUT a GPU (the reference arm must not map the product's .so):
-    the S1-S2 protocol of fenton.py:155-185 (no hole) run to 400 ms with the oracle's C/OpenMP port,
-    about 3 s on 16 cores."""
+    """The developed 512^2 spiral WITHOUT a GPU: the S1-S2 protocol of fenton.py:155-185 (no hole) run
+    to 400 ms with the oracle's C/OpenMP port, about 3 s on 16 cores.  Both arms start from it: the
+    reference arm must not map the product's .so, and our arm's input must not depend on the build
+    being measured, so that --dump-outputs of two builds can be compared cell by cell.  Every cell is
+    updated independently, so the result does not depend on the number of threads."""
     from oracle import cpu_port
     m = cpu_port.CPortModel('fenton4v', fenton_config(TILE, 400))
     m.define()
@@ -290,6 +277,35 @@ def workload_config(size, n):
             'parallelism': 'row-shard x%d' % n, 'halo': halo if n > 1 else 'none',
             'l2': 'state %.1f GiB >> 126 MB L2: no flush needed' % (size * size * 16 / 2 ** 30),
             'seed': 0}
+
+
+# ---------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed steps computed, for comparing two builds output for output
+# ---------------------------------------------------------------------------------------------
+DUMP_ROWS = 64      # full rows of every plane: 64 x 32768 x 4 planes x 4 B = 32 MiB at the default size
+
+
+def dump_rows(size):
+    """The fixed, seeded sample of global rows that --dump-outputs writes (every row of a smaller grid)."""
+    return np.sort(np.random.default_rng(0).choice(size, min(DUMP_ROWS, size), replace=False))
+
+
+def read_dump_rows(ctx, size):
+    """(global rows, {plane: [len(rows), size] float32}) for the dump rows inside this rank's shard."""
+    rows = [int(r) for r in dump_rows(size) if ctx.row0 <= r < ctx.row0 + ctx.rows]
+    return rows, {n: np.array([ctx.get_rect(n, r, r + 1, 0, size)[0] for r in rows],
+                              np.float32).reshape(len(rows), size) for n in ctx.var_names}
+
+
+def write_dump(out_dir, parts):
+    """parts: read_dump_rows of every rank -> out_dir/<plane>.npy, rows in ascending order, and
+    out_dir/rows.npy with their global indices."""
+    rows = np.concatenate([np.asarray(r, np.float64) for r, _ in parts])
+    order = np.argsort(rows)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'rows.npy'), rows[order])
+    for name in parts[0][1]:
+        np.save(os.path.join(out_dir, name + '.npy'), np.concatenate([p[name] for _, p in parts])[order])
 
 
 # ---------------------------------------------------------------------------------------------
@@ -394,9 +410,17 @@ def main():
     ap.add_argument('--size', type=int, default=32768)
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-suite', action='store_true', help='skip the per-kernel suite (N = 1)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the state after the timed steps to DIR/<plane>.npy (a fixed sample of %d '
+                         'full rows, float32; their indices in DIR/rows.npy)' % DUMP_ROWS)
     args = ap.parse_args()
     if args.impl == 'reference':
         return run_reference_arm(args)
+    if 'TORCHELASTIC_RUN_ID' in os.environ:
+        # torchrun exports OMP_NUM_THREADS=1: share the host cores among the ranks of this node for the
+        # CPU-built input instead.  Before torch is imported: it loads the libgomp the oracle port uses.
+        local_world = int(os.environ.get('LOCAL_WORLD_SIZE', 1))
+        os.environ['OMP_NUM_THREADS'] = str(max(1, (os.cpu_count() or 1) // local_world))
 
     import torch
     import torch.distributed as dist
@@ -436,7 +460,7 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
         return float(t.item())
 
-    tile = spiral_tile_gpu(local)
+    tile = spiral_tile_cpu()
     model = Fenton4v(fenton_config(size, K * 10 * 0.1, distributed=world > 1, device=local))
     model.define(s1=False)
     ctx = model._ctx
@@ -448,27 +472,17 @@ def main():
     sampler.start()
     ctx.step(0, Wm)                                     # warm-up (also instantiates the graph)
     barrier()
-    # EXACTLY K steps per timed region, bracketed by barrier + synchronize.  A region shorter than
-    # 0.5 s (8 GPUs: ~0.1 s) is repeated back to back and the MEAN of the repetitions is reported.
-    reps, ms_list, ms_dev_list, launches_rank = 1, [], [], 0
-    r = 0
-    while r < reps:
-        n0 = ctx.launch_count()
-        ctx.timer_start()
-        ctx.step(0, K)
-        ctx.timer_stop()
-        ms_dev = ctx.timer_ms()
-        barrier()
-        launches_rank = ctx.launch_count() - n0
-        ms_r = max_over_ranks(ms_dev)
-        ms_list.append(ms_r)
-        ms_dev_list.append(ms_dev)
-        if r == 0 and ms_r < 500.0:
-            reps = min(int(np.ceil(500.0 / max(ms_r, 1e-3))), 20)
-        r += 1
-    ms = float(np.mean(ms_list))
-    ms_dev = float(np.mean(ms_dev_list))
+    # EXACTLY K steps in the timed region, bracketed by barrier + synchronize
+    n0 = ctx.launch_count()
+    ctx.timer_start()
+    ctx.step(0, K)
+    ctx.timer_stop()
+    ms_dev = ctx.timer_ms()
+    barrier()
+    launches_rank = ctx.launch_count() - n0
+    ms = max_over_ranks(ms_dev)
     launches = int(sum_over_ranks(launches_rank))
+    dump = read_dump_rows(ctx, size) if args.dump_outputs else None
     cells = float(size) * size
     value = cells * K * 10 / (ms * 1e-3) / 1e9
 
@@ -538,7 +552,6 @@ def main():
         'e2e': {'value': e2e_value, 'unit': METRIC, 'h2d_bytes_per_step': sum_over_ranks(h2d) / K,
                 'd2h_bytes_per_step': sum_over_ranks(d2h) / K, 'seconds': e2e_s},
         'gpu_launches': launches, 'clocks': clocks, 'roofline': roofline,
-        'timed_regions': {'repeats': reps, 'ms_each': ms_list},
     }
     if rank == 0 and world == 1 and not args.no_suite:
         line['suite'] = run_suite(local, peak)
@@ -548,6 +561,13 @@ def main():
         line['cpu_baseline'] = info
     if rank == 0:
         emit(line)
+    if dump is not None:
+        parts = [dump]
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, dump)
+        if rank == 0:
+            write_dump(args.dump_outputs, parts)
     for p in [b for bufs in strips.values() for b in bufs] + [frame]:
         _capi.pinned_free(p)
     model.close()

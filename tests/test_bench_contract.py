@@ -7,6 +7,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 NEED = ['metric', 'value', 'unit', 'n_gpus', 'steps', 'warmup', 'ms_per_step', 'higher_is_better',
         'scaling', 'vs_baseline', 'dtype', 'data', 'config', 'e2e', 'cpu_baseline', 'impl']
@@ -44,12 +46,13 @@ import pytest  # noqa: E402
 
 
 @pytest.mark.gpu
-def test_our_arm_prints_one_contract_line(cuda_device):
+def test_our_arm_prints_one_contract_line(cuda_device, tmp_path):
     """`python bench.py` at a reduced grid (4096^2, still >> L2): one JSON line with every key of
-    the contract, the device-timed value consistent with ms_per_step, a non-trivial e2e leg and
-    kernels of this library launched inside the timed region."""
+    the contract, the device-timed value consistent with ms_per_step, a non-trivial e2e leg,
+    kernels of this library launched inside the timed region, and the --dump-outputs sample."""
     p = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--size', '4096', '--steps', '3',
-                        '--warmup', '3', '--no-cpu', '--no-suite'], capture_output=True, text=True, timeout=900, cwd=ROOT)
+                        '--warmup', '3', '--no-cpu', '--no-suite', '--dump-outputs', str(tmp_path)],
+                       capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert p.returncode == 0, p.stderr[-2000:]
     lines = [l for l in p.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -68,3 +71,9 @@ def test_our_arm_prints_one_contract_line(cuda_device):
     e = d['e2e']
     assert 0 < e['value'] < d['value'] and e['h2d_bytes_per_step'] > 0 and e['d2h_bytes_per_step'] > 0
     assert d['clocks']['sm_mhz'] > 0
+    rows = np.load(str(tmp_path / 'rows.npy'))
+    assert rows.dtype == np.float64 and len(rows) == 64 and np.all(np.diff(rows) > 0)
+    for v in ('U', 'V', 'W', 'S'):
+        a = np.load(str(tmp_path / (v + '.npy')))
+        assert a.dtype == np.float32 and a.shape == (64, 4096) and np.isfinite(a).all(), v
+    assert sum(f.stat().st_size for f in tmp_path.iterdir()) <= 64 << 20

@@ -3,6 +3,8 @@ arguments, and fails LOUDLY without a GPU (no CPU fallback).  No compute calls h
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -79,17 +81,24 @@ def test_null_arguments_are_errors_not_crashes():
     assert 'NULL' in L.fib_last_error().decode()
 
 
+NO_GPU_CHILD = '''
+import pytest
+from fib_tf_b200 import _capi
+with pytest.raises(_capi.FibError) as e:
+    _capi.Context(_capi.FENTON4V, 16, 16, 0.1, 1.0)
+assert 'cuda' in str(e.value).lower()
+from fib_tf_b200.fenton import Fenton4v
+m = Fenton4v({'width': 16, 'height': 16, 'dt': 0.1, 'diff': 1.0, 'duration': 1, 'dt_per_plot': 10})
+with pytest.raises(_capi.FibError):
+    m.define()
+'''
+
+
 def test_no_cpu_fallback_without_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip('a GPU is present')
-    with pytest.raises(_capi.FibError) as e:
-        _capi.Context(_capi.FENTON4V, 16, 16, 0.1, 1.0)
-    assert 'cuda' in str(e.value).lower()
-    from fib_tf_b200.fenton import Fenton4v
-    m = Fenton4v({'width': 16, 'height': 16, 'dt': 0.1, 'diff': 1.0, 'duration': 1, 'dt_per_plot': 10})
-    with pytest.raises(_capi.FibError):
-        m.define()
+    """In a child process that sees no GPU (on a GPU machine the devices are hidden from it)."""
+    r = subprocess.run([sys.executable, '-c', NO_GPU_CHILD], cwd=ROOT, capture_output=True, text=True,
+                       timeout=300, env=dict(os.environ, CUDA_VISIBLE_DEVICES=''))
+    assert r.returncode == 0, r.stderr[-2000:]
 
 
 def test_product_never_imports_the_oracle_or_tensorflow():

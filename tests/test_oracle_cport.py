@@ -36,6 +36,13 @@ NAMES = ('d_infinity', 'f_infinity', 'tau_w', 'tau_d', 'tau_f', 'w_infinity', 'm
          'xs_infinity', 'g_Kur', 'f_NaK', 'i_NaCaa', 'i_NaCab', 'i_K1a', 'i_Kra')
 
 
+def test_numpy_oracle_reproduces_the_reference_known_answer():
+    """The NumPy oracle's calc_inter(V = -50) against the vector above, with nothing compiled: the two
+    bars of the next test added (printing with %f, then oracle vs header)."""
+    mine = onp.court_inter(np.array([-50.0], np.float32))
+    assert np.allclose([float(mine[n][0]) for n in NAMES], KAT_M50, rtol=6e-6, atol=5e-7)
+
+
 def test_reference_header_known_answer_and_numpy_oracle_agree():
     ref = cpu_port.court_ref()
     if ref is None:
