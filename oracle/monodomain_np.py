@@ -54,13 +54,15 @@ def clip_by_value(x, lo, hi):
     return np.fmax(np.fmin(x, F32(hi)), F32(lo))
 
 
-def rush_larsen(g, g_inf, tau, dt):
-    """ionic.py:115-123 -- clip(g + (g - g_inf) * expm1(-dt / tau), 1e-5, 0.99999)."""
+def rush_larsen(g, g_inf, tau, dt, clip=True):
+    """ionic.py:115-123 -- clip(g + (g - g_inf) * expm1(-dt / tau), 1e-5, 0.99999).
+    clip=False: no clip, the rule of courtemanche.h (FIB_F_NO_CLIP)."""
     if isinstance(tau, np.ndarray):
         e = np.expm1(F32(-dt) / tau)
     else:                                   # Python-scalar tau: folded in Python, then fp32
         e = np.expm1(F32(-dt / tau))
-    return clip_by_value(g + (g - g_inf) * e, 0.00001, 0.99999)
+    g1 = g + (g - g_inf) * e
+    return clip_by_value(g1, 0.00001, 0.99999) if clip else g1
 
 
 def hole_phase(phase, height, width, x, y, radius, neg=False):
@@ -398,18 +400,64 @@ def court_inter(V, ultra=False):
     q['i_Kra'] = (Cm * g_Kr) / (1.0 + exp((V + 15.0) / 22.4))
 
     if ultra:
-        V_us, K_us = -83.0, 23.0
-        alpha_us = 3e-5 * (0.5 * (1 - np.tanh((V - V_us) / K_us)))
-        beta_us = 1e-5 * (0.5 * (1 + np.tanh((V - (V_us + 30)) / K_us)))
-        q['us_infinity'] = alpha_us / (alpha_us + beta_us)
-        q['tau_us'] = rcp(alpha_us + beta_us)
+        court_us(V, q)
     return q
 
 
-def court_solve(S, dt, diff, phase=None, multirate=True, chronic=True, ultra_slow=False):
+def court_us(V, q):
+    """court_ultra.py:445-450 -- us_infinity and tau_us into the dict q."""
+    V_us, K_us = -83.0, 23.0
+    alpha_us = 3e-5 * (0.5 * (1 - np.tanh((V - V_us) / K_us)))
+    beta_us = 1e-5 * (0.5 * (1 + np.tanh((V - (V_us + 30)) / K_us)))
+    q['us_infinity'] = alpha_us / (alpha_us + beta_us)
+    q['tau_us'] = np.reciprocal(alpha_us + beta_us)
+    return q
+
+
+# courtemanche.h:105-134 -- the 30 columns of the lookup table, in the header's order (the kernels'
+# CourtQ enum and fib_tf_b200._capi.INTER_NAMES[:30])
+COURT_LUT_COLUMNS = (
+    'd_infinity', 'f_infinity', 'tau_w', 'tau_d', 'tau_f', 'w_infinity', 'm_inf', 'h_inf', 'j_inf',
+    'tau_oa', 'tau_oi', 'tau_ua', 'tau_ui', 'tau_xr', 'tau_xs', 'tau_m', 'tau_h', 'tau_j',
+    'oa_infinity', 'oi_infinity', 'ua_infinity', 'ui_infinity', 'xr_infinity', 'xs_infinity',
+    'g_Kur', 'f_NaK', 'i_NaCaa', 'i_NaCab', 'i_K1a', 'i_Kra')
+COURT_LUT_ROWS = 150                   # V = -100 ... 49 mV, 1 mV apart (courtemanche.h:473-479)
+
+
+def court_lut_table():
+    """float32 [150, 30]: row k = court_inter(k - 100) in COURT_LUT_COLUMNS order."""
+    q = court_inter(np.arange(COURT_LUT_ROWS, dtype=np.float32) - F32(100))
+    return np.stack([np.asarray(q[n], np.float32) for n in COURT_LUT_COLUMNS], axis=1)
+
+
+def court_lut_row(V):
+    """courtemanche.h:354-356 -- row clamp(int(fp32(V) + fp32(100)), 0, 149): the sum is rounded to
+    fp32 before it is truncated towards zero (so V = -1e-6 reads row 100).  NaN reads row 0 (the
+    device's float-to-int conversion)."""
+    s = np.asarray(V, np.float32) + F32(100)
+    with np.errstate(invalid='ignore'):
+        r = np.clip(np.trunc(np.nan_to_num(s, nan=0.0)), 0, COURT_LUT_ROWS - 1)
+    return r.astype(np.intp)
+
+
+def court_lookup(V, table):
+    """The court_inter dict of the 30 tabulated columns, read from `table` [150, 30] at the row of
+    the truncating lookup (court_lut_row).  Every array has V's shape."""
+    t = np.asarray(table, np.float32)
+    if t.shape != (COURT_LUT_ROWS, len(COURT_LUT_COLUMNS)):
+        raise ValueError('court_lookup: table shape %r' % (t.shape,))
+    rows = t[court_lut_row(V)]
+    return {n: rows[..., k] for k, n in enumerate(COURT_LUT_COLUMNS)}
+
+
+def court_solve(S, dt, diff, phase=None, multirate=True, chronic=True, ultra_slow=False, table=None,
+                clip=True):
     """court.py:124-271 -- the full next-state dict S1 from the current state S.
     multirate=True (court.py:118-122): fast states (COURT_FAST) use dt, all others 10*dt.
     multirate=False (court_ultra.py:127-128): every state uses dt.
+    table: the LUT flavour -- the 30 tabulated intermediates come from court_lookup(V, table);
+    us_infinity / tau_us are still computed directly (the table has no such columns).
+    clip=False: the gates are not clipped to [1e-5, 0.99999] (FIB_F_NO_CLIP).
     The caller decides which entries of S1 are assigned (court.py:94-103)."""
     def step_of(name):
         return dt if (not multirate or name in COURT_FAST) else dt * 10
@@ -430,7 +478,12 @@ def court_solve(S, dt, diff, phase=None, multirate=True, chronic=True, ultra_slo
     chron = 1.0 if chronic else 0.0
     rcp, exp, log, power, square = np.reciprocal, np.exp, np.log, np.power, np.square
 
-    q = court_inter(V, ultra=ultra_slow)
+    if table is None:
+        q = court_inter(V, ultra=ultra_slow)
+    else:                                               # model_court.cuh:386-396
+        q = court_lookup(V, table)
+        if ultra_slow:
+            court_us(V, q)
     N = {}
     # court.py:175-186 -- note _w_ is stepped with the step of '_d_' (court.py:177)
     for g, inf, tau, clock in (
@@ -440,11 +493,11 @@ def court_solve(S, dt, diff, phase=None, multirate=True, chronic=True, ultra_slo
             ('_oa_', 'oa_infinity', 'tau_oa', '_oa_'), ('_oi_', 'oi_infinity', 'tau_oi', '_oi_'),
             ('_ua_', 'ua_infinity', 'tau_ua', '_ua_'), ('_ui_', 'ui_infinity', 'tau_ui', '_ui_'),
             ('_xr_', 'xr_infinity', 'tau_xr', '_xr_'), ('_xs_', 'xs_infinity', 'tau_xs', '_xs_')):
-        N[g] = rush_larsen(S[g], q[inf], q[tau], step_of(clock))
+        N[g] = rush_larsen(S[g], q[inf], q[tau], step_of(clock), clip=clip)
     f_Ca_inf = rcp(1.0 + S['_Ca_i_'] / 0.00035)
-    N['_f_Ca_'] = rush_larsen(S['_f_Ca_'], f_Ca_inf, tau_f_Ca, step_of('_f_Ca_'))
+    N['_f_Ca_'] = rush_larsen(S['_f_Ca_'], f_Ca_inf, tau_f_Ca, step_of('_f_Ca_'), clip=clip)
     if ultra_slow:                                      # court_ultra.py:198-199
-        N['_us_'] = rush_larsen(S['_us_'], q['us_infinity'], q['tau_us'], step_of('_us_'))
+        N['_us_'] = rush_larsen(S['_us_'], q['us_infinity'], q['tau_us'], step_of('_us_'), clip=clip)
 
     E_K = ((R * T) / F) * log(K_o / S['_K_i_'])
     i_K1 = q['i_K1a'] * (V - E_K)
@@ -484,10 +537,10 @@ def court_solve(S, dt, diff, phase=None, multirate=True, chronic=True, ultra_slo
     Fn = 1000.0 * (1.0e-15 * V_rel * i_rel - (1.0e-15 / (2.0 * F)) * (0.5 * i_Ca_L - 0.2 * i_NaCa))
     with np.errstate(over='ignore'):
         u_inf = rcp(1.0 + exp(-(Fn - 3.4175e-13) / 1.367e-15))
-        N['_u_'] = rush_larsen(S['_u_'], u_inf, tau_u, step_of('_u_'))
+        N['_u_'] = rush_larsen(S['_u_'], u_inf, tau_u, step_of('_u_'), clip=clip)
         tau_v = 1.91 + 2.09 * u_inf
         v_inf = 1.0 - rcp(1.0 + exp(-(Fn - 6.835e-14) / 1.367e-15))
-    N['_v_'] = rush_larsen(S['_v_'], v_inf, tau_v, step_of('_v_'))
+    N['_v_'] = rush_larsen(S['_v_'], v_inf, tau_v, step_of('_v_'), clip=clip)
 
     i_up = I_up_max / (1.0 + K_up / S['_Ca_i_'])
     i_up_leak = (I_up_max * S['_Ca_up_']) / Ca_up_max
@@ -649,13 +702,17 @@ class OracleModel:
 
     kind: 'fenton4v' | 'br' | 'court' | 'court_ultra'.  One iterate() == one run()
     iteration == dt_per_step time steps (10 / 5 / 1 / 1: fenton.py:135-138, br.py:96-107,
-    court.py:92)."""
+    court.py:92).
+
+    Courtemanche: config['lut'] selects the table flavour (court_lookup), with `table` [150, 30]
+    if given and court_lut_table() otherwise; config['chronic'] (default True) the chronic-AF
+    remodelling constants."""
 
     POT = {'fenton4v': 'U', 'br': 'V', 'court': 'V', 'court_ultra': 'V'}
     RANGE = {'fenton4v': (0.0, 1.0), 'br': (-90.0, 30.0), 'court': (-100.0, 50.0),
              'court_ultra': (-100.0, 50.0)}
 
-    def __init__(self, kind, config):
+    def __init__(self, kind, config, table=None):
         self.kind = kind
         self.cfg = dict(config)
         self.height, self.width = config['height'], config['width']
@@ -665,6 +722,10 @@ class OracleModel:
         self.paces = {}
         self.state = None
         self.coeffs = None
+        self.chronic = bool(self.cfg.get('chronic', True))
+        self.table = None
+        if kind in ('court', 'court_ultra') and self.cfg.get('lut'):
+            self.table = np.array(table if table is not None else court_lut_table(), dtype=np.float32)
 
     def add_hole(self, x, y, radius, neg=False):
         self.phase = hole_phase(self.phase, self.height, self.width, x, y, radius, neg)
@@ -697,7 +758,8 @@ class OracleModel:
         """court.py:103 -- assign the 17 slow states from a solve of the CURRENT state."""
         if self.kind != 'court':
             return                              # court_ultra.py:108: 'slow' is an empty group
-        new = court_solve(self.state, self.dt, self.diff, self.phase, multirate=True)
+        new = court_solve(self.state, self.dt, self.diff, self.phase, multirate=True,
+                          chronic=self.chronic, table=self.table)
         for k in new:
             if k not in COURT_FAST:
                 self.state[k] = new[k]
@@ -713,12 +775,14 @@ class OracleModel:
                 self.state = br_step(self.state, self.dt, self.diff, n, bool(c.get('cheby')),
                                      self.coeffs, self.phase)
         elif self.kind == 'court':
-            new = court_solve(self.state, self.dt, self.diff, self.phase, multirate=True)
+            new = court_solve(self.state, self.dt, self.diff, self.phase, multirate=True,
+                              chronic=self.chronic, table=self.table)
             for k in COURT_FAST:
                 self.state[k] = new[k]
         else:
             self.state = court_solve(self.state, self.dt, self.diff, self.phase, multirate=False,
-                                     ultra_slow=bool(c.get('ultra_slow')))
+                                     chronic=self.chronic, ultra_slow=bool(c.get('ultra_slow')),
+                                     table=self.table)
 
     def pot(self):
         return self.state[self.POT[self.kind]]

@@ -23,6 +23,9 @@ class CudaModel:
         cfg.update(extra)
         self.kind = kind
         self.m = CLASSES[kind](cfg)
+        if kind in ('court', 'court_ultra'):
+            # court.py sets `chronic` in __init__ (the config cannot reach it); define() reads it
+            self.m.chronic = bool(cfg.get('chronic', True))
         self.state = _StateView(self.m)
 
     def add_hole(self, x, y, radius, neg=False):

@@ -102,19 +102,30 @@ def live_tolerance(kind, cfg, var, drift=0.0):
     ('br', dict(diff=0.809, cheby=False, skip=True), 20),
     ('court', dict(diff=0.809, width=256, height=256), 100),
     ('court_ultra', dict(diff=1.5, width=256, height=256, ultra_slow=True), 100),
+    ('court', dict(diff=0.809, width=256, height=256, lut=True), 100),
+    ('court_ultra', dict(diff=1.5, width=256, height=256, lut=True, ultra_slow=True), 100),
+    ('court', dict(diff=0.809, width=256, height=256, chronic=False), 100),
 ])
 def test_100_steps_against_live_oracle(cuda, kind, cfg, iters):
-    """BASELINE configs 1-2 (512^2 with the shipped holes) and Courtemanche at 256^2: 100 time
-    steps, every state variable, against the oracle run here on the same inputs."""
+    """BASELINE configs 1-2 (512^2 with the shipped holes) and Courtemanche at 256^2 (one cell per
+    thread), also with the lookup table and without chronic-AF remodelling: 100 time steps, every
+    state variable, against the oracle run here on the same inputs (the oracle's table flavour reads
+    the table the device built)."""
+    from fib_tf_b200 import _capi
     base = {'width': 512, 'height': 512, 'dt': 0.1, 'dt_per_plot': 10, 'duration': 10,
             'timeline': False, 'timeline_name': 'x', 'save_graph': False, 'skip': False,
             'cheby': False, 'ultra_slow': False}
     base.update(cfg)
     W = base['width']
-    ref, jit, gpu = onp.OracleModel(kind, base), onp.OracleModel(kind, base), cuda.CudaModel(kind, base)
-    for m in (ref, jit, gpu):
+    gpu = cuda.CudaModel(kind, base)
+    gpu.add_hole(W // 2, W // 2, 30 * W // 512)
+    gpu.define()
+    table = gpu.m._ctx.get_table(_capi.TABLE_COURT_LUT, (150, 30)) if cfg.get('lut') else None
+    ref, jit = onp.OracleModel(kind, base, table=table), onp.OracleModel(kind, base, table=table)
+    for m in (ref, jit):
         m.add_hole(W // 2, W // 2, 30 * W // 512)
         m.define()
+    for m in (ref, jit, gpu):
         m.add_pace('s2', 'luq', 1.0 if kind == 'fenton4v' else 10.0)
     rng = np.random.default_rng(1)
     for i in range(iters):
@@ -124,6 +135,9 @@ def test_100_steps_against_live_oracle(cuda, kind, cfg, iters):
                 m.fire('slow')
             if i == iters // 2:
                 m.fire('s2')
+        if i == 0 and kind.startswith('court'):
+            last = _capi.last_kernel()
+            assert 'VEC=1' in last and ('lut' in last) == bool(cfg.get('lut')), last
         if i + 1 < iters:
             onp.ulp_jitter(jit.state, rng)
     for v in ref.state:
@@ -138,7 +152,8 @@ def test_100_steps_against_live_oracle(cuda, kind, cfg, iters):
                                         ('court', {}), ('court_ultra', {'ultra_slow': True}),
                                         # large enough for the wide kernel flavours and deeper marching
                                         ('br', {'cheby': True, 'width': 1300, 'height': 900}),
-                                        ('fenton4v', {'width': 1100, 'height': 1000})])
+                                        ('fenton4v', {'width': 1100, 'height': 1000}),
+                                        ('court', {'lut': True}), ('court_ultra', {'lut': True, 'ultra_slow': True})])
 def test_row_shards_are_bit_identical_to_the_unsharded_run(cuda, kind, extra):
     """Emulates R row shards in one process (fib_step_group, device-to-device halo rows) and
     requires BIT-IDENTICAL planes: sharding must not change arithmetic; seams are interior."""
@@ -166,6 +181,8 @@ def test_row_shards_are_bit_identical_to_the_unsharded_run(cuda, kind, extra):
         s.set_phase(m.phase, 0)
         if kind == 'br':
             s.set_table(_capi.TABLE_BR_CHEBY, m.chebyshev_table())
+        if flags & _capi.F_LUT:
+            s.build_lut()
     for it in range(6):
         c0.step(_capi.OP_ODE, 1)
         _capi.step_group(shards, _capi.OP_ODE, 1)

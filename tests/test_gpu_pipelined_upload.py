@@ -48,6 +48,7 @@ CASES = [
     ('br exact', 'BR', 0, {}, 4),
     ('courtemanche multi-rate', 'COURT', 0, {}, 12),
     ('courtemanche all-state', 'COURT_ULTRA', 'F_ULTRA_SLOW', {}, 12),
+    ('courtemanche all-state lut', 'COURT_ULTRA', 'F_LUT|F_ULTRA_SLOW', {}, 12),
 ]
 
 
@@ -75,6 +76,8 @@ def test_stepping_behind_the_upload_is_bit_identical(cuda, monkeypatch, label, m
         c.set_phase(phase, 0)
         if fl & _capi.F_CHEBY:
             c.set_table(_capi.TABLE_BR_CHEBY, table)
+        if fl & _capi.F_LUT:
+            c.build_lut()
         for v in c.var_names:                                # something else in the buffers first
             c.set_state(v, np.full((H, W), 0.5, np.float32))
         c.step(0, 1)

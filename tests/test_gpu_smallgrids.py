@@ -23,7 +23,7 @@ def test_every_flavour_on_degenerate_grids(cuda_device):
     for (H, W) in ((3, 3), (7, 5), (33, 47), (40, 130)):
         for kind, extra in (('fenton4v', {}), ('br', {}), ('br', {'cheby': True, 'skip': True}),
                             ('court', {}), ('court', {'lut': True}), ('court_ultra', {'ultra_slow': True}),
-                            ('court_ultra', {'lut': True})):
+                            ('court_ultra', {'lut': True}), ('court_ultra', {'lut': True, 'ultra_slow': True})):
             for hole in (False, True):
                 cfg = dict(base, width=W, height=H, **extra)
                 m = CudaModel(kind, cfg)

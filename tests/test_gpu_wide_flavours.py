@@ -5,13 +5,16 @@ launch_step (csrc/fib_kernels.cuh) switches to one cell per thread on grids of <
 the golden fixtures (<= 56 x 40) and the 512^2 live-oracle runs only ever see that small flavour.
 Here:
   * every BR flag combination (exact, skip, cheby, cheby+skip, cheby_strict) on 1024 x 512 and the
-    Courtemanche variants (multi-rate fast + slow ops, ultra, ultra + ultra-slow gate) on 768 x 512,
-    with a hole and a stimulus, 100 / 50 time steps against the NumPy oracle run on the same inputs;
-  * the tabulated Courtemanche flavour (two cells per thread, depth 2) against the reference's own
-    compiled courtemanche.h on a 2200-column version of the table-row experiment;
+    Courtemanche variants (multi-rate fast + slow ops, ultra, ultra + ultra-slow gate, each of them
+    with the lookup table, and chronic-AF remodelling off) on 768 x 512, with a hole and a stimulus,
+    100 / 50 time steps against the NumPy oracle run on the same inputs.  The oracle's table flavour
+    (oracle.monodomain_np.court_lookup) reads the table the device built;
+  * where oracle/_ref can be built: the tabulated flavour also against the reference's own compiled
+    courtemanche.h on a 2200-column version of the table-row experiment;
   * every golden fixture replayed with FIB_SMALL_CELLS=0 (a subprocess: the switch is read once per
     process), which forces the wide flavours onto the reference-generated data.
 Each test asserts, through fib_last_kernel, WHICH instantiation ran."""
+import contextlib
 import os
 import subprocess
 import sys
@@ -40,18 +43,22 @@ def base_config(**kw):
     return cfg
 
 
-def compare(kind, cfg, gpu, ref, jit):
+def compare(kind, cfg, gpu, ref, jit, wide=None):
     """Bar per variable: oracle.monodomain_np.tolerance (flat 1e-5 / named waivers), but never tighter than
-    3x the drift of the ulp-jittered oracle `jit` in this very scenario (see onp.ulp_jitter)."""
+    3x the drift of the ulp-jittered oracle `jit` in this very scenario (see onp.ulp_jitter), nor than 3x the
+    distance of `wide` (if given: the oracle with its V-only intermediates in float64) -- the oracle's own
+    rounding, as the fixtures' `rounding` term."""
     report = []
     for v in ref.state:
         fl = onp.var_floor(kind, v)
         e = onp.rel_err(gpu.state[v], ref.state[v], fl)
         tol = max(onp.tolerance(kind, cfg, v, *onp.model_uncertainty(METAS, kind, cfg, v)),
-                  3.0 * onp.rel_err(jit.state[v], ref.state[v], fl))
+                  3.0 * onp.rel_err(jit.state[v], ref.state[v], fl),
+                  3.0 * onp.rel_err(wide.state[v], ref.state[v], fl) if wide is not None else 0.0)
         report.append((v, e, tol))
     bad = [(v, '%.3e > %.3e' % (e, t)) for v, e, t in report if not e <= t]
-    assert not bad, (kind, {k: cfg.get(k) for k in ('cheby', 'skip', 'cheby_strict', 'lut', 'ultra_slow')}, bad)
+    assert not bad, (kind, {k: cfg.get(k) for k in ('cheby', 'skip', 'cheby_strict', 'lut', 'ultra_slow', 'chronic')},
+                     bad)
     return report
 
 
@@ -89,41 +96,83 @@ def test_beeler_reuter_wide_flavour_against_the_oracle(cuda, flags, kernels):
 
 @pytest.mark.parametrize('kind,extra,steps,kernel', [
     ('court', {}, 50, 'Courtemanche<fast>,VEC=2'),
-    ('court', {'lut': True}, 0, 'Courtemanche<fast,lut>,VEC=2,R=2'),      # flavour check only (no oracle for LUT here)
+    ('court', {'lut': True}, 50, 'Courtemanche<fast,lut>,VEC=2,R=2'),
     ('court_ultra', {}, 50, 'Courtemanche<all>'),
     ('court_ultra', {'ultra_slow': True}, 50, 'Courtemanche<all,us>'),
+    ('court_ultra', {'lut': True}, 50, 'Courtemanche<all,lut>,VEC=2,R=2'),
+    ('court_ultra', {'lut': True, 'ultra_slow': True}, 50, 'Courtemanche<all,lut,us>,VEC=2,R=2'),
+    ('court', {'chronic': False}, 50, 'Courtemanche<fast>,VEC=2'),
+    ('court_ultra', {'chronic': False}, 50, 'Courtemanche<all>,VEC=2'),
 ])
 def test_courtemanche_wide_flavours_against_the_oracle(cuda, kind, extra, steps, kernel):
     """BASELINE config 4's flavours on 768 x 512 = 384 Ki cells: the multi-rate loop ('slow' every 10th
-    iteration), the all-states variant and the ultra-slow gate; hole, S2 half way."""
+    iteration), the all-states variant, the ultra-slow gate, the lookup table and chronic-AF remodelling
+    switched off; hole, S2 half way, `steps` iterations.  The oracle's table flavour reads the table the
+    device built (test_gpu_court_lut.py tests that table on its own)."""
     from fib_tf_b200 import _capi
     cfg = base_config(width=768, height=512, diff=0.809 if kind == 'court' else 1.5, **extra)
     gpu = cuda.CudaModel(kind, cfg, graph=False)
-    ref = onp.OracleModel(kind, cfg) if steps else None
-    jit = onp.OracleModel(kind, cfg) if steps else None
-    models = [m for m in (gpu, ref, jit) if m is not None]
-    for m in models:
+    gpu.add_hole(300, 200, 40)
+    gpu.define()
+    table = gpu.m._ctx.get_table(_capi.TABLE_COURT_LUT, (150, 30)) if extra.get('lut') else None
+    ref, jit = onp.OracleModel(kind, cfg, table=table), onp.OracleModel(kind, cfg, table=table)
+    # direct flavours: the oracle's fp32 calc_inter has no correct digit right next to its removable
+    # singularities (test_gpu_parity.py::test_courtemanche_removable_singularities), which a wave crosses;
+    # `wide` measures that: measured with chronic=False, court_ultra, _xr_: 1.5e-5 away from the fp32 oracle,
+    # 8.6e-7 in the cells that never came within 0.5 mV of a singular voltage
+    wide = onp.OracleModel(kind, cfg) if table is None else None
+    oracles = [m for m in (ref, jit, wide) if m is not None]
+    for m in oracles:
         m.add_hole(300, 200, 40)
         m.define()
+    models = [gpu] + oracles
+    for m in models:
         m.add_pace('s2', 'luq', 10.0)
+
+    def step(m):
+        if m is wide:
+            with float64_intermediates():
+                return m.iterate()
+        return m.iterate()
+
     gpu.iterate()
     assert kernel in _capi.last_kernel() and 'PHASE=1' in _capi.last_kernel(), _capi.last_kernel()
-    if ref is None:
-        gpu.close()
-        return
     rng = np.random.default_rng(3)
-    ref.iterate()
-    jit.iterate()
+    for m in oracles:
+        step(m)
     for i in range(1, steps):
         onp.ulp_jitter(jit.state, rng)
         for m in models:
             if kind == 'court' and (i - 1) % 10 == 0:
-                m.fire('slow')
+                if m is wide:
+                    with float64_intermediates():
+                        m.fire('slow')
+                else:
+                    m.fire('slow')
+                if m is gpu and i == 1:
+                    slow = kernel.split(',VEC')[0].replace('<fast', '<slow')
+                    assert slow + ',VEC=2' in _capi.last_kernel(), (slow, _capi.last_kernel())
             if i == steps // 2:
                 m.fire('s2')
-            m.iterate()
-    compare(kind, cfg, gpu, ref, jit)
+            step(m)
+    compare(kind, cfg, gpu, ref, jit, wide)
     gpu.close()
+
+
+@contextlib.contextmanager
+def float64_intermediates():
+    """onp.court_inter evaluated in float64 (then rounded to fp32) inside the block."""
+    fp32 = onp.court_inter
+
+    def wide(V, ultra=False):
+        with np.errstate(all='ignore'):
+            q = fp32(np.asarray(V, np.float64), ultra)
+        return {k: np.asarray(a, np.float32) for k, a in q.items()}
+    onp.court_inter = wide
+    try:
+        yield
+    finally:
+        onp.court_inter = fp32
 
 
 def test_lut_wide_flavour_against_the_compiled_reference_header(cuda):
@@ -246,7 +295,9 @@ cfg = {'width': 200, 'height': 120, 'dt': 0.1, 'dt_per_plot': 10, 'diff': 0.809,
        'timeline_name': 'x', 'save_graph': False, 'skip': False, 'cheby': False, 'ultra_slow': False, 'graph': False}
 for tag, kind, extra in (('br_exact', 'br', {}), ('br_cheby_skip', 'br', {'cheby': True, 'skip': True}),
                          ('br_strict', 'br', {'cheby': True, 'cheby_strict': True}),
-                         ('court', 'court', {}), ('court_ultra_us', 'court_ultra', {'ultra_slow': True, 'diff': 1.5})):
+                         ('court', 'court', {}), ('court_ultra_us', 'court_ultra', {'ultra_slow': True, 'diff': 1.5}),
+                         ('court_lut', 'court', {'lut': True}),
+                         ('court_ultra_lut_us', 'court_ultra', {'lut': True, 'ultra_slow': True, 'diff': 1.5})):
     m = CudaModel(kind, dict(cfg, **extra))
     m.add_hole(90, 60, 17)
     m.define()
@@ -283,6 +334,10 @@ def test_packed_pairs_are_bit_identical_to_scalar_cells(cuda, tmp_path):
     a, b = files
     assert 'VEC=1' in str(a['br_exact/kernel']) and 'VEC=2' in str(b['br_exact/kernel'])
     assert 'VEC=2' in str(b['court_ultra_us/kernel']) and 'VEC=2' in str(b['br_strict/kernel'])
+    assert 'Courtemanche<fast,lut>,VEC=1' in str(a['court_lut/kernel'])
+    assert 'Courtemanche<fast,lut>,VEC=2' in str(b['court_lut/kernel'])
+    assert 'Courtemanche<all,lut,us>,VEC=1' in str(a['court_ultra_lut_us/kernel'])
+    assert 'Courtemanche<all,lut,us>,VEC=2' in str(b['court_ultra_lut_us/kernel'])
     for k in a.files:
         if not k.endswith('/kernel'):
             assert np.array_equal(a[k], b[k], equal_nan=True), k

@@ -30,10 +30,7 @@ KAT_M50 = [0.006693, 0.960396, 0.345409, 0.711940, 387.911591, 0.995004, 0.26825
            12.825628, 23.367565, 0.156622, 0.786152, 0.113842, 0.995673, 0.003978, 0.063673,
            0.005335, 0.720790, 0.010301, 102066.710938, 0.981871, 2.431505]
 # courtemanche.h:105-134 column order -> names used by court.py's calc_inter dict
-NAMES = ('d_infinity', 'f_infinity', 'tau_w', 'tau_d', 'tau_f', 'w_infinity', 'm_inf', 'h_inf',
-         'j_inf', 'tau_oa', 'tau_oi', 'tau_ua', 'tau_ui', 'tau_xr', 'tau_xs', 'tau_m', 'tau_h',
-         'tau_j', 'oa_infinity', 'oi_infinity', 'ua_infinity', 'ui_infinity', 'xr_infinity',
-         'xs_infinity', 'g_Kur', 'f_NaK', 'i_NaCaa', 'i_NaCab', 'i_K1a', 'i_Kra')
+NAMES = onp.COURT_LUT_COLUMNS
 
 
 def test_numpy_oracle_reproduces_the_reference_known_answer():
