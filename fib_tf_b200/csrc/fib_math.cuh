@@ -4,9 +4,11 @@
 // CUDA's IEEE division (~10 instr + slow path) and libm-grade expf/expm1f/logf/tanhf (12-35
 // instr) the BR cell costs ~700 instructions.  Two things bring that down:
 //
-//  1. Few-ulp transcendentals built on the SFU approximations (MUFU.EX2 / LG2 / RCP), each <= ~3 ulp
-//     -- the same error class as swapping one fp32 libm for another, which is what the parity
-//     bars are calibrated against (oracle/tfshim.ALT_LIBM, tests/test_gpu_parity.py).
+//  1. Few-ulp transcendentals built on the SFU approximations (MUFU.EX2 / LG2 / RCP), 1 - 4.5 ulp
+//     each (expm1 away from 0: < 13 ulp; the numbers below were measured on a B200 by
+//     tests/test_gpu_math_layer.py against float64) -- the same error class as swapping one fp32
+//     libm for another, which is what the parity bars are calibrated against
+//     (oracle/tfshim.ALT_LIBM, tests/test_gpu_parity.py).
 //     Build with -DFIB_ACCURATE_MATH=1 to get IEEE division and CUDA's libm instead (A/B checks).
 //
 //  2. Packed fp32 (sm_100: fma/mul/add.rn.f32x2 -> SASS FFMA2 / FMUL2 / FADD2): a thread that owns
@@ -70,8 +72,9 @@ FIB_F2_OP2(sub2, "sub.rn.f32x2")
 // although the scalar mul.rn / add.rn are never fused (checked in SASS; it even sees through
 // fma(a,b,-0) and fma(p,1,b) with literal constants), which would make a packed lane round differently
 // from the scalar cell.  So a * b is issued as fma(a, b, NZERO) with NZERO = -0.0f read from constant
-// memory at run time: exactly fl(a * b), signed zeros included (+0 + -0 = +0, -0 + -0 = -0), one FFMA2
-// instead of one FMUL2 -- and with no packed multiply left in the code there is nothing to contract.
+// memory at run time: exactly fl(a * b), signed zeros included (+0 + -0 = +0, -0 + -0 = -0; tested lane
+// for lane against the scalar multiply), one FFMA2 instead of one FMUL2 -- and with no packed multiply
+// left in the code there is nothing to contract.
 static __constant__ float kFibNegZero = -0.0f;
 __device__ __forceinline__ f2 mul2(f2 a, f2 b) {
   const float nz = kFibNegZero;
@@ -171,11 +174,17 @@ __device__ __forceinline__ f2 m_exp_affine(f2 x, float c, float add) {
   return f2(m_exp_affine(x.x, c, add), m_exp_affine(x.y, c, add));
 }
 #else
-template <class T> __device__ __forceinline__ T m_rcp(T x) { return sfu_rcp(x); }                 // 1 ulp
-template <class T, class U> __device__ __forceinline__ T m_div(U a, T b) { return T(a) * sfu_rcp(b); }   // 2 ulp
+// < 1 ulp (measured 0.96) / < 2 ulp (1.95); subnormal inputs and results flush to zero
+template <class T> __device__ __forceinline__ T m_rcp(T x) { return sfu_rcp(x); }
+template <class T, class U> __device__ __forceinline__ T m_div(U a, T b) { return T(a) * sfu_rcp(b); }
 
 // e^x = 2^t * 2^r, t = fl(x*log2e), r = the rounding error of that product + x*lo(log2e),
-// 2^r ~ 1 + r ln2.  ~2 ulp over the whole range; +inf / 0 on overflow / underflow like expf.
+// 2^r ~ 1 + r ln2.  < 3 ulp (measured 2.96) for |x| <= 2^24; +inf on overflow; 0 below
+// ln(FLT_MIN) = -87.34 (the SFU flushes the subnormal results that expf returns down to -103.9).
+// Beyond |x| ~ 2.3e7, |r| exceeds 1/ln2 and 1 + r ln2 can be negative: x that large gives -inf or NaN
+// (negative x: +-0), and x = +-inf gives NaN (r = inf - inf).  No call site comes near: the models'
+// exponents are within +-60 for V in [-120, 80] mV, and those of the Ca-release sigmoids (u_inf, v_inf)
+// are large only when negative, where 2^t = 0 whatever the factor.
 template <class T> __device__ __forceinline__ T m_exp(T x) {
   const float L2E_HI = 1.44269502162933349609375f, L2E_LO = 1.92596299112661746e-8f;
   const T t = x * T(L2E_HI);
@@ -209,7 +218,8 @@ template <class T> __device__ __forceinline__ T expm1_poly(T x) {
 // expm1: the polynomial for |x| < 0.125, exp(x)-1 beyond.  The polynomial side is the one that
 // matters for accuracy: |x| = dt/tau is small exactly for the slow gates, whose per-step error would
 // otherwise accumulate over hundreds of steps; for |x| >= 0.125 a gate relaxes within ~10 steps and
-// exp(x)-1 (|result| >= 0.117, so < 8 ulp) is plenty.  Both sides are computed and selected: no
+// exp(x)-1 (|result| >= 0.117, so < 13 ulp; measured 12.9) is plenty.  The polynomial side is < 1 ulp
+// (0.55).  Built on m_exp: NaN for x = +-inf.  Both sides are computed and selected: no
 // divergence.
 template <class T> __device__ __forceinline__ T m_expm1(T x) {
   const T p = expm1_poly(x);
@@ -220,18 +230,23 @@ template <class T> __device__ __forceinline__ T m_expm1(T x) {
 // expm1 for the Rush-Larsen factor, x = -dt/tau <= 0.  On the far side the exponential needs no
 // argument compensation: the uncompensated 2^(x log2e) is off by e^x (2 ulp + |x| 2^-24), i.e. an
 // ABSOLUTE error <= 1.6e-7 (|x| e^x <= 1/e), against a result of magnitude >= 0.117 -- the same
-// < 8 ulp as m_expm1, three instructions cheaper per gate.
+// < 13 ulp as m_expm1 (measured 12.9), three instructions cheaper per gate.  Negative tau (the BR
+// polynomial tau_h below -83.85 mV) feeds it x > 0, where the uncompensated product costs up to
+// x 2^-24 relative: measured < 10 ulp for 0 < x <= 1 and < 8 + x ulp beyond.  Valid for every x:
+// +inf -> +inf, -inf -> -1.
 template <class T> __device__ __forceinline__ T m_expm1_neg(T x) {
   const T p = expm1_poly(x);
   const T e = sfu_ex2(x * T(1.44269502162933349609375f)) - T(1.0f);
   return sel(lt(vabs(x), T(0.125f)), p, e);
 }
 
+// log: lg2.approx has an absolute error bound (2^-22 for x in [0.5, 2]), so through 0 near x = 1 the
+// error is absolute (measured <= 1.6e-7); < 3.5 ulp elsewhere (3.17).  sqrt: < 1 ulp (0.93).
 template <class T> __device__ __forceinline__ T m_log(T x) { return sfu_lg2(x) * T(0.693147182464599609375f); }
 template <class T> __device__ __forceinline__ T m_sqrt(T x) { return sfu_sqrt(x); }
 // 1 + e^{-2z} as ONE explicit FMA: left to the compiler, ptxas decides per kernel whether the
 // multiply and the add fuse, and two kernels that must agree bit for bit (the one- and the
-// two-steps-per-launch 4v kernels) would differ in the last place.
+// two-steps-per-launch 4v kernels) would differ in the last place.  < 4.5 ulp (4.19) for |z| <= 2^23.
 template <class T> __device__ __forceinline__ T m_half_1p_tanh(T z) {
   return sfu_rcp(m_exp_affine(T(-2.0f) * z, 1.0f, 1.0f));
 }

@@ -61,11 +61,34 @@ def test_model_level_helpers_mirror_the_reference_methods(cuda):
     g = rng.uniform(1e-3, 0.998, X.shape).astype(np.float32)
     gi = rng.uniform(0.0, 1.0, X.shape).astype(np.float32)
     tau = rng.uniform(0.05, 500.0, X.shape).astype(np.float32)
-    want = onp.rush_larsen(g, gi, tau, 0.1)
-    assert onp.rel_err(m.rush_larsen(g, gi, tau, 0.1), want, 1e-3) <= 2e-6
+    # the edges of x = -dt/tau (rl_edge_inputs): tau < 0, tau -> 0+, +-0, +-inf, very large tau, |dt/tau|
+    # straddling the 0.125 switch of the expm1 polynomial, g == g_inf with an infinite exponent (0 * inf
+    # = NaN, which the clip turns into its upper bound)
+    from test_gpu_math_layer import rl_edge_inputs
+    n = g.size
+    g, gi, tau = (np.concatenate([a.ravel(), b]) for a, b in zip((g, gi, tau), rl_edge_inputs()))
+    with np.errstate(all='ignore'):
+        want = onp.rush_larsen(g, gi, tau, 0.1)
+        want64 = onp.rush_larsen(g.astype(np.float64), gi.astype(np.float64), tau.astype(np.float64), 0.1)
+        e32 = np.expm1(np.float32(-0.1) / tau)
+    got = m.rush_larsen(g, gi, tau, 0.1)
+    assert onp.rel_err(got[:n], want64[:n], 1e-3) <= 2e-6
+    # the edges: where e = expm1(-dt/tau) overflows fp32 (0 * inf = NaN for g == g_inf, which the clip
+    # turns into its upper bound) the fp32 oracle is the reference; elsewhere float64, with the error of
+    # m_expm1_neg (fib_math.cuh: < 13 ulp, < 8 + x ulp for x = -dt/tau > 1) carried by |g - g_inf|
+    inf = ~np.isfinite(e32[n:])
+    assert onp.rel_err(got[n:][inf], want[n:][inf], 1e-3) == 0.0
+    x = -0.1 / tau[n:][~inf].astype(np.float64)
+    bar = (2e-6 * np.maximum(np.abs(want64[n:][~inf]), 1e-3) + np.abs(g - gi)[n:][~inf].astype(np.float64) *
+           np.where(x > 1, 8 + x, 13) * np.spacing(np.abs(e32[n:][~inf])))
+    assert np.all(np.abs(got[n:][~inf] - want64[n:][~inf]) <= bar)
     from fib_tf_b200 import _capi
     strict = _capi.op_rush_larsen(g, gi, tau, 0.1, strict=True)
-    assert np.all(np.abs(strict.astype(np.float64) - want) <= 2 * np.spacing(np.abs(want)))   # expm1f: 1 ulp
+    assert np.all(np.abs(strict[:n].astype(np.float64) - want[:n]) <= 2 * np.spacing(np.abs(want[:n])))   # expm1f: 1 ulp
+    # at the edges that ulp of e is carried by |g - g_inf|, which can exceed the result (cancellation)
+    ulp_e = np.nan_to_num(np.spacing(np.abs(e32[n:])), nan=0.0)
+    assert np.all(np.abs(strict[n:].astype(np.float64) - want[n:]) <=
+                  2 * np.spacing(np.abs(want[n:])) + np.abs(g - gi)[n:].astype(np.float64) * ulp_e)
     m.close()
 
 
