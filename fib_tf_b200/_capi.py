@@ -20,7 +20,8 @@ F_CHEBY_STRICT, F_NO_PERSIST = 0x80, 0x100
 PROBE_RING = 4096
 OP_ODE, OP_SLOW = 0, 1
 TABLE_BR_CHEBY, TABLE_COURT_LUT = 0, 1
-ABI_VERSION = 2
+ACT_FIRST, ACT_LAST, ACT_PREV, ACT_REPOL, ACT_COUNT = 0, 1, 2, 3, 4
+ABI_VERSION = 3
 INTER_COLS = 32
 
 # courtemanche.h:105-134 column order (+ the two court_ultra.py:445-450 extras)
@@ -68,6 +69,9 @@ _SIGNATURES = {
     'fib_last_kernel': (C.c_int, [C.c_char_p, C.c_size_t]),
     'fib_probe_watch': (C.c_int, [_P, C.c_int, C.c_int, C.c_int]),
     'fib_probe_fetch': (C.c_int, [_P, _P, C.c_size_t, C.POINTER(C.c_size_t)]),
+    'fib_activation_watch': (C.c_int, [_P, C.c_float, C.c_float]),
+    'fib_activation_stop': (C.c_int, [_P]),
+    'fib_activation_get': (C.c_int, [_P, C.c_int, _P, C.c_size_t]),
     'fib_count_below': (C.c_int, [_P, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float,
                                   C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     'fib_op_enforce_boundary': (C.c_int, [C.c_int, _P, C.c_int, C.c_int, _P]),
@@ -288,6 +292,19 @@ class Context:
         n = C.c_size_t()
         check(lib().fib_probe_fetch(self._h, out.ctypes.data_as(_P), max_values, C.byref(n)))
         return out[:n.value]
+
+    def activation_watch(self, up, down):
+        """Arm (or re-arm) the activation maps of the diffusing variable at levels up / down."""
+        check(lib().fib_activation_watch(self._h, up, down))
+
+    def activation_stop(self):
+        check(lib().fib_activation_stop(self._h))
+
+    def activation_get(self, which):
+        """[rows, W] float32 map ACT_* of this shard, times in iterations since arming."""
+        out = np.empty((self.rows, self.width), dtype=np.float32)
+        check(lib().fib_activation_get(self._h, which, out.ctypes.data_as(_P), out.size))
+        return out
 
     def count_below(self, var, sub, div, cutoff, w_min):
         a, b = C.c_uint64(), C.c_uint64()

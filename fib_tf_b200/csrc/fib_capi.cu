@@ -9,6 +9,7 @@
 #include <string.h>
 
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/fib_b200.h"
@@ -143,6 +144,12 @@ struct fib_ctx {
   unsigned long long ring_ev_total[kRingEvents] = {0, 0, 0, 0};
   int ring_ev_next = 0;
   int watch_var = -1, watch_row = -1, watch_col = -1;
+  // activation maps (fib_activation_watch, fib_activation.cuh): armed iff act_maps != nullptr
+  float* act_prev = nullptr;          // the last sample of the diffusing variable, [rows][pitch]
+  float* act_maps = nullptr;          // kActMaps planes [rows][pitch]
+  unsigned long long* act_iter = nullptr;   // device: samples taken since arming (= k - 1 of the next one)
+  unsigned long long act_n = 0;       // host mirror of *act_iter (iterations enqueued since arming)
+  float act_up = 0.f, act_down = 0.f;
   float* weights[4] = {nullptr, nullptr, nullptr, nullptr};   // user masks, halo layout like phase
   // persistent on-chip kernel (fib_persist.cuh): small unsharded 4v / BR grids
   int persist = -1;                   // -1 not decided yet, 0 no, 1 yes
@@ -540,6 +547,9 @@ extern "C" int fib_destroy(fib_ctx* c) {
   for (auto& e : c->ring_ev)
     if (e) cudaEventDestroy(e);
   cudaFree(c->ring_count);
+  cudaFree(c->act_prev);
+  cudaFree(c->act_maps);
+  cudaFree(c->act_iter);
   cudaFree(c->pmail);
   if (c->perr) cudaFreeHost(c->perr);
   if (c->ptimeline) cudaFreeHost(c->ptimeline);
@@ -744,7 +754,7 @@ static int set_rect_impl(fib_ctx* c, int var, int r0, int r1, int c0, int c1, co
     // On an NCCL shard the block order may also run bottom to top (odd ranks do, so that both shards of a seam
     // either begin or end there: fib_step_behind_upload).
     const bool eligible = (c->comm ? c->pipeline_nccl : c->g.rows == c->g.H) && c0 == 0 && c1 == c->g.W &&
-                          c->watch_var < 0 && (long long)c->g.rows * c->g.W >= c->pipeline_min_cells;
+                          c->watch_var < 0 && !c->act_maps && (long long)c->g.rows * c->g.W >= c->pipeline_min_cells;
     const int row_end = c->g.row0 + c->g.rows;
     const int dir = c->up_session ? c->up_dir : (r0 == c->g.row0 ? +1 : (r1 == row_end && c->comm ? -1 : 0));
     const int dlo = dir > 0 ? r0 - c->g.row0 : row_end - r1, dhi = dir > 0 ? r1 - c->g.row0 : row_end - r0;
@@ -1146,13 +1156,13 @@ static bool make_tile_map(CUtensorMap* m, float* base, int W, int rows, int pitc
          CUDA_SUCCESS;
 }
 
-template <class MS, class MF, int TH, bool PHASE>
+template <class MS, class MF, int TH, bool PHASE, bool ACT>
 static cudaError_t launch_persist_t(fib_ctx* c, const PersistArgs<MS, MF>& a) {
   PersistMaps<MS::NS> maps;
   maps.x[0] = c->pmap_x[0];
   maps.x[1] = c->pmap_x[1];
   for (int k = 0; k < MS::NS; ++k) maps.s[k] = c->pmap_s[k];
-  auto kern = persist_kernel<MS, MF, TH, PHASE>;
+  auto kern = persist_kernel<MS, MF, TH, PHASE, ACT>;
   constexpr size_t smem = persist_smem_bytes<MS::NS, TH>();
   static bool attr_set = false;           // per instantiation
   if (!attr_set) {
@@ -1172,7 +1182,8 @@ static cudaError_t launch_persist_t(fib_ctx* c, const PersistArgs<MS, MF>& a) {
   // FIB_PERSIST_COOP=0 (experiments only): a plain launch; co-residency then rests on tiles <= SMs alone
   static const bool coop = !(getenv("FIB_PERSIST_COOP") && atoi(getenv("FIB_PERSIST_COOP")) == 0);
   cfg.numAttrs = coop ? 1 : 0;
-  snprintf(last_kernel_name(), 160, "persist_kernel<%s,TH=%d,PHASE=%d>", MS::name(), TH, PHASE ? 1 : 0);
+  snprintf(last_kernel_name(), 160, "persist_kernel<%s,TH=%d,PHASE=%d%s>", MS::name(), TH, PHASE ? 1 : 0,
+           ACT ? ",ACT=1" : "");
   return cudaLaunchKernelEx(&cfg, kern, maps, c->g, a);
 }
 
@@ -1196,14 +1207,25 @@ static cudaError_t launch_persist_m(fib_ctx* c, PersistArgs<MS, MF>& a, int max_
   a.probe_var = c->watch_var;
   a.probe_row = c->watch_row;
   a.probe_col = c->watch_col;
-  const bool ph = c->phase != nullptr;
+  a.act_prev = c->act_prev;
+  a.act_maps = c->act_maps;
+  a.act_plane = c->plane_floats();
+  a.act_iter = c->act_iter;
+  a.act_k0 = c->act_n;
+  a.act_up = c->act_up;
+  a.act_down = c->act_down;
+  const bool ph = c->phase != nullptr, act = c->act_maps != nullptr;
   (void)max_th;
+  auto go = [&](auto th) {
+    constexpr int TH = decltype(th)::value;
+    if (act) return ph ? launch_persist_t<MS, MF, TH, true, true>(c, a) : launch_persist_t<MS, MF, TH, false, true>(c, a);
+    return ph ? launch_persist_t<MS, MF, TH, true, false>(c, a) : launch_persist_t<MS, MF, TH, false, false>(c, a);
+  };
   switch (c->persist_th) {
-    case 2: return ph ? launch_persist_t<MS, MF, 2, true>(c, a) : launch_persist_t<MS, MF, 2, false>(c, a);
-    case 4: return ph ? launch_persist_t<MS, MF, 4, true>(c, a) : launch_persist_t<MS, MF, 4, false>(c, a);
+    case 2: return go(std::integral_constant<int, 2>());
+    case 4: return go(std::integral_constant<int, 4>());
     case 8:
-      if constexpr (MS::NS <= 3)
-        return ph ? launch_persist_t<MS, MF, 8, true>(c, a) : launch_persist_t<MS, MF, 8, false>(c, a);
+      if constexpr (MS::NS <= 3) return go(std::integral_constant<int, 8>());
     default: return cudaErrorInvalidValue;
   }
 }
@@ -1297,6 +1319,7 @@ static int run_iteration_persist(fib_ctx* c, int iters) {
     return 1;           // caller retries on the plain path
   }
   c->launches++;
+  if (c->act_maps) c->act_n += (unsigned)iters;
   if (c->watch_var >= 0) {
     c->ring_total += (unsigned)iters;
     const int k = c->ring_ev_next;
@@ -1339,6 +1362,28 @@ static int record_probe(fib_ctx* c, int op) {
   return 0;
 }
 
+// fib_activation_watch: after an ODE iteration, sample the diffusing variable of the CURRENT buffers into
+// the maps, then advance the iteration index (two nodes of the iteration graph)
+static int record_activation(fib_ctx* c, int op) {
+  if (!c->act_maps || op != FIB_OP_ODE) return 0;
+  const size_t n4 = c->plane_floats() / 4;
+  const int grid = (int)min((n4 + 255) / 256, (size_t)c->sms * 32);
+  activation_update_kernel<<<grid, 256, 0, c->stream>>>(reinterpret_cast<const float4*>(owned_rows(c, 0)),
+                                                        reinterpret_cast<float4*>(c->act_prev), c->act_maps, n4,
+                                                        c->plane_floats(), c->act_iter, c->act_up, c->act_down);
+  activation_advance_kernel<<<1, 1, 0, c->stream>>>(c->act_iter);
+  CU(cudaGetLastError());
+  c->launches += 2;
+  c->act_n++;
+  return 0;
+}
+
+// the observers that sample the state at the end of an ODE iteration
+static int record_observers(fib_ctx* c, int op) {
+  const int r = record_activation(c, op);
+  return r ? r : record_probe(c, op);
+}
+
 static int run_iteration_plain(fib_ctx* c, int op) {
   const int ns = substeps_of(c, op);
   for (int s = 0; s < ns; s += c->fuse) {
@@ -1346,7 +1391,7 @@ static int run_iteration_plain(fib_ctx* c, int op) {
     if (r) return r;
     if (op_writes_x(c, op)) c->cur ^= 1;
   }
-  return record_probe(c, op);
+  return record_observers(c, op);
 }
 
 // boundary rows first, halo exchange on the side stream overlapped with the interior rows
@@ -1380,7 +1425,7 @@ static int run_iteration_nccl(fib_ctx* c, int op) {
     }
     c->cur ^= 1;
   }
-  return record_probe(c, op);
+  return record_observers(c, op);
 }
 
 // Every rank must take part in an exchange, but a host write (fib_set_state / fib_set_rect /
@@ -1435,13 +1480,14 @@ static int step_now(fib_ctx* c, int op, int n_iter) {
       cudaGraph_t graph = nullptr;
       CU(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
       const uint64_t l0 = c->launches;
-      const unsigned long long rt0 = c->ring_total;
+      const unsigned long long rt0 = c->ring_total, an0 = c->act_n;
       pdl_enabled() = false;               // plain kernel nodes replay faster (see fib_kernels.cuh)
       int r = run_iteration_plain(c, op);
       pdl_enabled() = true;
       cudaError_t ce = cudaStreamEndCapture(c->stream, &graph);
       c->launches = l0;
       c->ring_total = rt0;
+      c->act_n = an0;
       c->cur = cur0;
       if (r) { if (graph) cudaGraphDestroy(graph); return r; }
       if (ce != cudaSuccess) return fail(FIB_E_CUDA, "graph capture failed: %s", cudaGetErrorString(ce));
@@ -1452,8 +1498,10 @@ static int step_now(fib_ctx* c, int op, int n_iter) {
     CU(cudaGraphLaunch(exec, c->stream));
     const int nl = substeps_of(c, op) / c->fuse;      // step launches per iteration
     const int rec = (c->watch_var >= 0 && op == FIB_OP_ODE) ? 1 : 0;
-    c->launches += nl + rec;
+    const int act = (c->act_maps && op == FIB_OP_ODE) ? 1 : 0;
+    c->launches += nl + rec + 2 * act;
     c->ring_total += rec;
+    c->act_n += act;
     if (op_writes_x(c, op) && (nl & 1)) c->cur ^= 1;
   }
   return 0;
@@ -1700,7 +1748,7 @@ extern "C" int fib_step_group(fib_ctx** cs, int n, int op, int n_iter) {
     }
     for (int i = 0; i < n; ++i) {
       DevGuard dg(cs[i]->cfg.device);
-      if ((r = record_probe(cs[i], op))) return r;
+      if ((r = record_observers(cs[i], op))) return r;
     }
   }
   return 0;
@@ -1880,6 +1928,63 @@ extern "C" int fib_probe_fetch(fib_ctx* c, float* out, size_t max, size_t* n) {
   c->ring_fetched = first + take;
   *n = (size_t)take;
   return 0;
+}
+
+// Activation maps: the sample s[0] is the current plane; the update runs after every ODE iteration from
+// here on (record_activation, or inside the persistent kernel).  The iteration graphs are rebuilt with or
+// without the update nodes.
+extern "C" int fib_activation_watch(fib_ctx* c, float up, float down) {
+  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
+  if (!isfinite(up) || !isfinite(down)) return fail(FIB_E_ARG, "activation levels must be finite (up %g, down %g)", up, down);
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  CU(wait_comm(c));
+  CU(cudaStreamSynchronize(c->stream));
+  drop_graphs(c);
+  const size_t plane = c->plane_floats();
+  if (!c->act_iter) CU(cudaMalloc(&c->act_iter, sizeof(unsigned long long)));
+  if (!c->act_prev) CU(cudaMalloc(&c->act_prev, plane * sizeof(float)));
+  if (!c->act_maps) CU(cudaMalloc(&c->act_maps, kActMaps * plane * sizeof(float)));   // last: armed from here
+  CU(cudaMemcpyAsync(c->act_prev, owned_rows(c, 0), plane * sizeof(float), cudaMemcpyDeviceToDevice, c->stream));
+  activation_reset_kernel<<<c->sms * 4, 256, 0, c->stream>>>(c->act_maps, plane);
+  CU(cudaGetLastError());
+  c->launches++;
+  CU(cudaMemsetAsync(c->act_iter, 0, sizeof(unsigned long long), c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  c->act_n = 0;
+  c->act_up = up;
+  c->act_down = down;
+  return 0;
+}
+
+extern "C" int fib_activation_stop(fib_ctx* c) {
+  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  CU(cudaStreamSynchronize(c->stream));
+  drop_graphs(c);
+  CU(cudaFree(c->act_maps));
+  CU(cudaFree(c->act_prev));
+  CU(cudaFree(c->act_iter));
+  c->act_maps = c->act_prev = nullptr;
+  c->act_iter = nullptr;
+  c->act_n = 0;
+  return check_persist_error(c);
+}
+
+extern "C" int fib_activation_get(fib_ctx* c, int map, float* host, size_t n) {
+  if (!c || !host) return fail(FIB_E_ARG, "ctx/host is NULL");
+  if (map < 0 || map >= kActMaps) return fail(FIB_E_ARG, "unknown activation map %d", map);
+  if (n != (size_t)c->g.rows * c->g.W)
+    return fail(FIB_E_ARG, "fib_activation_get: n=%zu, expected rows*width=%zu", n, (size_t)c->g.rows * c->g.W);
+  if (!c->act_maps) return fail(FIB_E_STATE, "no activation map is armed (fib_activation_watch)");
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  CU(cudaMemcpy2DAsync(host, c->g.W * sizeof(float), c->act_maps + (size_t)map * c->plane_floats(),
+                       c->g.pitch * sizeof(float), c->g.W * sizeof(float), c->g.rows, cudaMemcpyDeviceToHost,
+                       c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return check_persist_error(c);
 }
 
 extern "C" int fib_count_below(fib_ctx* c, int var, float sub, float div, float cutoff, float w_min,

@@ -32,6 +32,7 @@
 #pragma once
 #include <cuda.h>
 
+#include "fib_activation.cuh"
 #include "model_br.cuh"
 #include "model_fenton.cuh"
 
@@ -125,11 +126,22 @@ struct PersistArgs {
   int probe_var, probe_row, probe_col;
   typename MS::Params ps;      // parameters of the MS steps
   typename MF::Params pf;      // parameters of the MF steps
+  // fib_activation_watch (ACT instantiations only): the thread owning a cell samples it at the end of every
+  // iteration against its last sample in act_prev (global, L2-resident at these sizes: the register file
+  // is full), exactly what activation_update_kernel does between the launches of the plain path.  Iteration
+  // it of this launch has k - 1 = act_k0 + it; the launch leaves act_k0 + iterations in *act_iter.
+  float* act_prev;             // [rows][pitch]
+  float* act_maps;             // kActMaps planes of act_plane floats
+  size_t act_plane;
+  unsigned long long* act_iter;
+  unsigned long long act_k0;
+  float act_up, act_down;
 };
 
 // ---- the kernel ----------------------------------------------------------------------------------
 // MS / MF: the cell types of the "slow" and "fast" steps of a schedule (Fenton4v twice; BeelerReuter<C,true>
-// and <C,false> for br.py's skip schedule).  TH: rows per tile.  PHASE: phase field present.
+// and <C,false> for br.py's skip schedule).  TH: rows per tile.  PHASE: phase field present.  ACT: an
+// activation map is armed (fib_activation.cuh).
 //
 // Where the state lives between the steps of a launch:
 //   * a thread owns ONE column of its tile: its TH cells of every plane, the diffusing variable included
@@ -143,7 +155,7 @@ struct PersistArgs {
 //     and the rows of a column are read once per step (marching reuse in registers);
 //   * the rows of the neighbour tiles arrive through the mailbox and are written into the ring rows by
 //     the thread that will read them (each thread writes the three columns it reads: no barrier).
-template <class MS, class MF, int TH, bool PHASE>
+template <class MS, class MF, int TH, bool PHASE, bool ACT>
 __global__ void __launch_bounds__(kPersistThreads, 1)
 persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, const PersistArgs<MS, MF> a) {
   constexpr int NS = MS::NS;
@@ -291,6 +303,7 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
   const bool probe_me = a.ring && active && c == a.probe_col && a.probe_row >= r0 && a.probe_row < r0 + nrows;
   unsigned long long probe_n = probe_me ? *a.ring_count : 0ull;
   int sub = 0;                                               // time step within the current iteration
+  unsigned long long act_k = a.act_k0;                       // ACT: k - 1 of the current iteration
   for (int step = 0; step < a.nsteps; ++step) {
     const int p = step & 1;                                  // shared buffer holding the state this step reads
     const bool slow = !a.slow_first_only || sub == 0;
@@ -454,11 +467,28 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
         a.ring[probe_n % FIB_PROBE_RING] = v;
         ++probe_n;
       }
+      if constexpr (ACT) {
+        if (active) {
+          const float k1 = (float)act_k;
+#pragma unroll
+          for (int i = 0; i < TH; ++i)
+            if (i < nrows) {
+              const size_t idx = (size_t)(r0 + i) * pitch + c;
+              const float pv = a.act_prev[idx];
+              a.act_prev[idx] = u[i];
+              act_cell(pv, u[i], k1, a.act_up, a.act_down, a.act_maps + idx, a.act_plane);
+            }
+        }
+        ++act_k;
+      }
     }
     __syncthreads();            // shared tile of the next step complete, the old one free for reuse
     now(2 + step);
   }
   if (probe_me) *a.ring_count = probe_n;
+  if constexpr (ACT) {
+    if (tile == 0 && t == 0) *a.act_iter = act_k;
+  }
 
   // ---- TMA out: registers -> staging, then tile stores (rows beyond the grid are clipped)
   if (active) {

@@ -35,7 +35,8 @@ Extra, optional config keys (all default to the reference's behaviour):
 
 Collective calls under config['distributed'] (every rank must make them, in the same order):
 define(), run() (each iteration), fire_op(), image(), pot().eval() / _State[..].eval(),
-var[r, c].eval(), masked_image_mean(), excitable_fraction(), close().  cl_observer callbacks run on
+var[r, c].eval(), masked_image_mean(), excitable_fraction(), watch_activation(), activation_maps(),
+stop_activation(), close().  cl_observer callbacks run on
 the rank that owns row 20 only and therefore must not call any of these.
 """
 import json
@@ -512,6 +513,42 @@ class IonicModel:
             dist.all_gather_object(parts, (below, total))
             below, total = sum(p[0] for p in parts), sum(p[1] for p in parts)
         return below / total if total else float('nan')
+
+    def watch_activation(self, up=None, down=None):
+        """Arms the device-side activation maps of the transmembrane variable (include/fib_b200.h,
+        fib_activation_watch): from now on, after every iteration, every cell records its up-crossings of
+        `up` and down-crossings of `down` (raw units of the potential; both default to min_v + 0.5 (max_v -
+        min_v), the reference's cycle-length probe level of 0.5 on the normalised image), linearly
+        interpolated between consecutive iterations.  Calling it again resets the maps."""
+        if not self.defined:
+            raise AssertionError('watch_activation should be called after calling define')
+        mid = float(self.min_v) + 0.5 * (float(self.max_v) - float(self.min_v))
+        self._ctx.activation_watch(mid if up is None else float(up), mid if down is None else float(down))
+
+    def activation_maps(self):
+        """{name: [height, width] float64} in ms since watch_activation():
+            first, last, previous  the first, the last and the one-before-last activation time
+            repol                  the last repolarisation time
+            count                  the number of activations
+            apd                    repol - last where repol > last (the last beat has repolarised), else NaN
+            cycle                  last - previous
+        Empty times are NaN.  Conduction velocity follows from differences of `last` (or `first`) between
+        cells; cycle-length and APD heterogeneity from `cycle` and `apd`."""
+        ms = self.dt_per_step * self.dt
+        c = self._ctx
+        raw = {k: self._gather(c.activation_get(m)).astype(np.float64)
+               for k, m in (('first', _capi.ACT_FIRST), ('last', _capi.ACT_LAST), ('previous', _capi.ACT_PREV),
+                            ('repol', _capi.ACT_REPOL), ('count', _capi.ACT_COUNT))}
+        out = {k: v * ms for k, v in raw.items() if k != 'count'}
+        out['count'] = raw['count']
+        with np.errstate(invalid='ignore'):
+            out['apd'] = np.where(out['repol'] > out['last'], out['repol'] - out['last'], np.nan)
+        out['cycle'] = out['last'] - out['previous']
+        return out
+
+    def stop_activation(self):
+        """Disarms the activation maps and frees their device memory."""
+        self._ctx.activation_stop()
 
     def nonfinite_cells(self):
         """{variable: count} of NaN/Inf cells in this shard (empty dict when the state is healthy):

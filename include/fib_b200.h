@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define FIB_ABI_VERSION 2
+#define FIB_ABI_VERSION 3
 
 typedef struct fib_ctx fib_ctx;
 
@@ -226,6 +226,39 @@ int fib_probe_fetch(fib_ctx *ctx, float *out, size_t max, size_t *n);
  * cutoff, *total = cells with weight > w_min (weight = phase field, 1 if none).  Synchronous. */
 int fib_count_below(fib_ctx *ctx, int var, float sub, float div, float cutoff, float w_min,
                     uint64_t *below, uint64_t *total);
+
+/* activation maps (SURVEY 8f1): the activation-time (LAT), repolarisation and cycle-length maps of the whole
+ * shard, recorded on the device while stepping, so that APD, cycle length and conduction velocity need no
+ * frame on the host.  A map watches the DIFFUSING variable (U of 4v, V of BR / Courtemanche).
+ *   samples  s[0] = the plane when fib_activation_watch is called; s[k] (k >= 1) = the plane at the end of
+ *            the k-th FIB_OP_ODE iteration enqueued since, taken before anything the caller does between
+ *            iterations (fib_stimulate, fib_set_*): a host write shows up in the next sample.  FIB_OP_SLOW
+ *            does not write the variable and takes no sample.
+ *   events   activation in iteration k:      s[k-1] < up <= s[k],   t = (k-1) + (up - s[k-1]) / (s[k] - s[k-1])
+ *            repolarisation in iteration k:  s[k-1] >= down > s[k], t = (k-1) + (s[k-1] - down) / (s[k-1] - s[k])
+ *            the event rule of tests/test_spiral_statistics.py events(), in fp32 with one rounding per
+ *            operation (no contraction); a NaN sample produces no event.
+ *   times    in iterations since arming, fp32.  Iteration indices are exact up to 2^24; the resolution of the
+ *            fraction shrinks with k (one ulp of t is ~0.008 iteration at k = 10^5).
+ *   maps     FIRST: first activation; LAST: last activation; PREV: the activation before LAST; REPOL: last
+ *            repolarisation -- NaN while empty; COUNT: number of activations, as a float.  On an activation
+ *            PREV := LAST, LAST := t, COUNT += 1 and FIRST := t if it is NaN; on a repolarisation REPOL := t.
+ * Cost: 12 bytes per cell per iteration (the plane and the last sample read, the sample written), plus the
+ * map planes at cells with an event.  An armed map keeps fib_set_rect_async blocks out of the pipelined
+ * upload (they are copied in order instead).
+ * fib_activation_watch arms the map, or re-arms it: everything is reset and s[0] re-taken; FIB_E_ARG if a
+ * level is not finite.  fib_activation_stop disarms it and frees the planes.  fib_activation_get copies map
+ * `map` (fib_act_map) of this shard, rows*width floats; synchronous; FIB_E_STATE without a watch. */
+typedef enum {
+  FIB_ACT_FIRST = 0,
+  FIB_ACT_LAST = 1,
+  FIB_ACT_PREV = 2,
+  FIB_ACT_REPOL = 3,
+  FIB_ACT_COUNT = 4
+} fib_act_map;
+int fib_activation_watch(fib_ctx *ctx, float up, float down);
+int fib_activation_stop(fib_ctx *ctx);
+int fib_activation_get(fib_ctx *ctx, int map, float *host, size_t n);
 
 /* ---- op-level entry points of IonicModel's helpers on dense host planes [h][w] (eager; used by the
  * drop-in IonicModel.enforce_boundary / laplace / phase_field / rush_larsen and by the parity tests that
