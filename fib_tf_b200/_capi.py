@@ -9,8 +9,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# FIB_B200_LIB selects another build of the same library (kernel tuning experiments)
-LIB_PATH = os.environ.get('FIB_B200_LIB') or os.path.join(_HERE, 'libfibb200.so')
+LIB_PATH = os.path.join(_HERE, 'libfibb200.so')
 
 # model ids / flags / ops / tables: keep in sync with include/fib_b200.h
 FENTON4V, BR, COURT, COURT_ULTRA = 0, 1, 2, 3

@@ -174,7 +174,6 @@ struct fib_ctx {
   long long pipeline_min_cells = 1ll << 22;   // smaller grids: not worth it (FIB_PIPELINE_MIN_CELLS)
   int pipeline_block_rows = 1024;             // rows per block of the skewed schedule, at least (FIB_PIPELINE_BLOCK_ROWS)
   int* perr = nullptr;                // page-locked, device-visible: raised by a timed-out neighbour wait
-  unsigned long long* ptimeline = nullptr;   // page-locked [16], FIB_PERSIST_TIMELINE=1 only
   CUtensorMap pmap_x[2], pmap_s[8];
   // NCCL
   void* comm = nullptr;
@@ -552,7 +551,6 @@ extern "C" int fib_destroy(fib_ctx* c) {
   cudaFree(c->act_iter);
   cudaFree(c->pmail);
   if (c->perr) cudaFreeHost(c->perr);
-  if (c->ptimeline) cudaFreeHost(c->ptimeline);
   for (int k = 0; k < 4; ++k) cudaFree(c->weights[k]);
   for (cudaEvent_t e : {c->ev_start, c->ev_stop, c->ev_bnd, c->ev_comm, c->ev_group})
     if (e) cudaEventDestroy(e);
@@ -960,9 +958,7 @@ extern "C" int fib_court_inter(fib_ctx* c, const float* v_host, size_t n, float*
 // the step schedule
 // ------------------------------------------------------------------------------------------
 static int substeps_of(const fib_ctx* c, int op) {
-  // FIB_DEBUG_SUBSTEPS=n: run only the first n time steps of an iteration (diagnostics only)
-  static const int dbg = getenv("FIB_DEBUG_SUBSTEPS") ? atoi(getenv("FIB_DEBUG_SUBSTEPS")) : 0;
-  if (op == FIB_OP_ODE) return (dbg > 0 && dbg < c->dt_per_step) ? dbg : c->dt_per_step;
+  if (op == FIB_OP_ODE) return c->dt_per_step;
   return c->cfg.model == FIB_COURT ? 1 : 0;   // 'slow' is an empty group elsewhere
 }
 
@@ -1179,16 +1175,14 @@ static cudaError_t launch_persist_t(fib_ctx* c, const PersistArgs<MS, MF>& a) {
   attr[0].id = cudaLaunchAttributeCooperative;       // all tiles co-resident, or the launch fails
   attr[0].val.cooperative = 1;
   cfg.attrs = attr;
-  // FIB_PERSIST_COOP=0 (experiments only): a plain launch; co-residency then rests on tiles <= SMs alone
-  static const bool coop = !(getenv("FIB_PERSIST_COOP") && atoi(getenv("FIB_PERSIST_COOP")) == 0);
-  cfg.numAttrs = coop ? 1 : 0;
+  cfg.numAttrs = 1;
   snprintf(last_kernel_name(), 160, "persist_kernel<%s,TH=%d,PHASE=%d%s>", MS::name(), TH, PHASE ? 1 : 0,
            ACT ? ",ACT=1" : "");
   return cudaLaunchKernelEx(&cfg, kern, maps, c->g, a);
 }
 
 template <class MS, class MF>
-static cudaError_t launch_persist_m(fib_ctx* c, PersistArgs<MS, MF>& a, int max_th, int iters) {
+static cudaError_t launch_persist_m(fib_ctx* c, PersistArgs<MS, MF>& a, int iters) {
   a.x[0] = c->x[0];
   a.x[1] = c->x[1];
   a.cur = c->cur;
@@ -1197,7 +1191,6 @@ static cudaError_t launch_persist_m(fib_ctx* c, PersistArgs<MS, MF>& a, int max_
   a.mail = c->pmail;
   a.base = c->pbase;
   a.err = c->perr;
-  a.timeline = c->ptimeline;
   a.phase = c->phase;
   a.pmask = c->pmask;
   a.pmask_pitch = c->pmask_pitch;
@@ -1215,7 +1208,6 @@ static cudaError_t launch_persist_m(fib_ctx* c, PersistArgs<MS, MF>& a, int max_
   a.act_up = c->act_up;
   a.act_down = c->act_down;
   const bool ph = c->phase != nullptr, act = c->act_maps != nullptr;
-  (void)max_th;
   auto go = [&](auto th) {
     constexpr int TH = decltype(th)::value;
     if (act) return ph ? launch_persist_t<MS, MF, TH, true, true>(c, a) : launch_persist_t<MS, MF, TH, false, true>(c, a);
@@ -1260,14 +1252,6 @@ static void decide_persist(fib_ctx* c) {
     cudaMemsetAsync(c->pmail, 0, fbytes, c->stream);       // step number 0 = "nothing published yet"
     if (cudaHostAlloc(&c->perr, sizeof(int), cudaHostAllocMapped) != cudaSuccess) { cudaGetLastError(); return; }
     *c->perr = 0;
-    if (getenv("FIB_PERSIST_TIMELINE") && atoi(getenv("FIB_PERSIST_TIMELINE"))) {
-      if (cudaHostAlloc(&c->ptimeline, 16 * sizeof(unsigned long long), cudaHostAllocMapped) != cudaSuccess) {
-        cudaGetLastError();
-        c->ptimeline = nullptr;
-      } else {
-        memset(c->ptimeline, 0, 16 * sizeof(unsigned long long));
-      }
-    }
   }
   c->persist_th = th;
   c->persist_tiles = tiles;
@@ -1285,7 +1269,7 @@ static int run_iteration_persist(fib_ctx* c, int iters) {
     a.slow_first_only = 0;
     a.ps.dt = a.pf.dt = (float)dt;
     a.ps.ddt = a.pf.ddt = (float)(c->cfg.diff * dt);
-    e = launch_persist_m<Fenton4v, Fenton4v>(c, a, 8, iters);
+    e = launch_persist_m<Fenton4v, Fenton4v>(c, a, iters);
   } else {
     const bool cheby = fl & FIB_F_CHEBY, strict = cheby && (fl & FIB_F_CHEBY_STRICT), skip = fl & FIB_F_SKIP;
     if (cheby && !c->have_cheb) return fail(FIB_E_STATE, "cheby=True but FIB_TABLE_BR_CHEBY has not been set");
@@ -1305,7 +1289,7 @@ static int run_iteration_persist(fib_ctx* c, int iters) {
       };
       fill(a.ps, skip ? 5 : 1);
       fill(a.pf, 0);
-      return launch_persist_m<MS, MF>(c, a, 4, iters);
+      return launch_persist_m<MS, MF>(c, a, iters);
     };
     if (strict)     e = go(BeelerReuter<2, true>(), BeelerReuter<2, false>());
     else if (cheby) e = go(BeelerReuter<1, true>(), BeelerReuter<1, false>());
@@ -1331,14 +1315,6 @@ static int run_iteration_persist(fib_ctx* c, int iters) {
   const int ns = substeps_of(c, FIB_OP_ODE) * iters;
   c->pbase += (unsigned)ns;
   if (ns & 1) c->cur ^= 1;
-  if (c->ptimeline) {          // diagnostics: print the middle tile's phase times of this launch
-    cudaStreamSynchronize(c->stream);
-    const unsigned long long* tl = c->ptimeline;
-    fprintf(stderr, "persist timeline (ns): load %llu |", tl[1] - tl[0]);
-    for (int k = 0; k < ns && k < 12; ++k) fprintf(stderr, " %llu", tl[2 + k] - tl[1 + k]);
-    if (ns <= 12) fprintf(stderr, " | store %llu | total %llu", tl[2 + ns] - tl[1 + ns], tl[2 + ns] - tl[0]);
-    fprintf(stderr, "\n");
-  }
   return 0;
 }
 
@@ -1454,7 +1430,7 @@ static int step_now(fib_ctx* c, int op, int n_iter) {
     // watched probe is recorded by the kernel itself after every iteration
     int i = 0;
     while (i < n_iter) {
-      const int batch = c->ptimeline ? 1 : min(n_iter - i, kPersistMaxIters);
+      const int batch = min(n_iter - i, kPersistMaxIters);
       int r = run_iteration_persist(c, batch);
       if (r > 0) break;                 // could not launch: plain path from here on
       if (r) return r;
@@ -1481,9 +1457,7 @@ static int step_now(fib_ctx* c, int op, int n_iter) {
       CU(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
       const uint64_t l0 = c->launches;
       const unsigned long long rt0 = c->ring_total, an0 = c->act_n;
-      pdl_enabled() = false;               // plain kernel nodes replay faster (see fib_kernels.cuh)
       int r = run_iteration_plain(c, op);
-      pdl_enabled() = true;
       cudaError_t ce = cudaStreamEndCapture(c->stream, &graph);
       c->launches = l0;
       c->ring_total = rt0;
@@ -1603,7 +1577,7 @@ extern "C" int fib_step(fib_ctx* c, int op, int n_iter) {
       return 0;
     }
   }
-  if (c->persist == 1 && op == FIB_OP_ODE && !c->ptimeline) {
+  if (c->persist == 1 && op == FIB_OP_ODE) {
     // persistent path: count now, launch later (see FLUSH); whatever can fail is checked here
     if (c->cfg.model == FIB_BR && (c->cfg.flags & FIB_F_CHEBY) && !c->have_cheb)
       return fail(FIB_E_STATE, "cheby=True but FIB_TABLE_BR_CHEBY has not been set");

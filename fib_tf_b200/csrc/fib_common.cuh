@@ -20,31 +20,20 @@ struct Geom {
   int pitch;        // floats per row
 };
 
-// FIB_NC_LOADS=1 (default) reads the planes through the non-coherent path (ld.global.nc).  An
-// in-place plane is read exactly once, by the thread that later overwrites the same address, and
-// L1 is invalidated at every kernel boundary, so no stale line can be observed AS LONG AS
-// consecutive step kernels do not overlap -- which is why programmatic dependent launch is compiled
-// out in this mode (fib_kernels.cuh).  It lets the scheduler interleave the state loads with the
-// phase-field / lookup-table reads: 4v + phase field 157 -> 169, Courtemanche LUT 28.5 -> 32.3
-// Gcell-steps/s; no effect on the other flavours.  FIB_NC_LOADS=0 + FIB_PDL=1 is the alternative
-// for launch-bound direct launches on tiny grids.
-#ifndef FIB_NC_LOADS
-#define FIB_NC_LOADS 1
-#endif
-#if FIB_NC_LOADS
-#define FIB_LD(p) __ldg(p)
-#else
-#define FIB_LD(p) (*(p))
-#endif
-
+// The planes are read through the non-coherent path (ld.global.nc, __ldg).  An in-place plane is
+// read exactly once, by the thread that later overwrites the same address, and L1 is invalidated at
+// every kernel boundary, so no stale line can be observed AS LONG AS consecutive step kernels do not
+// overlap (no programmatic dependent launch).  It lets the scheduler interleave the state loads with
+// the phase-field / lookup-table reads: 4v + phase field 157 -> 169, Courtemanche LUT 28.5 -> 32.3
+// Gcell-steps/s; no effect on the other flavours.
 template <int VEC> struct VecIO;
 template <> struct VecIO<1> {
-  static __device__ __forceinline__ void ld(const float* p, float* v) { v[0] = FIB_LD(p); }
+  static __device__ __forceinline__ void ld(const float* p, float* v) { v[0] = __ldg(p); }
   static __device__ __forceinline__ void st(float* p, const float* v) { *p = v[0]; }
 };
 template <> struct VecIO<2> {
   static __device__ __forceinline__ void ld(const float* p, float* v) {
-    float2 t = FIB_LD(reinterpret_cast<const float2*>(p)); v[0] = t.x; v[1] = t.y;
+    float2 t = __ldg(reinterpret_cast<const float2*>(p)); v[0] = t.x; v[1] = t.y;
   }
   static __device__ __forceinline__ void st(float* p, const float* v) {
     *reinterpret_cast<float2*>(p) = make_float2(v[0], v[1]);
@@ -52,7 +41,7 @@ template <> struct VecIO<2> {
 };
 template <> struct VecIO<4> {
   static __device__ __forceinline__ void ld(const float* p, float* v) {
-    float4 t = FIB_LD(reinterpret_cast<const float4*>(p)); v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+    float4 t = __ldg(reinterpret_cast<const float4*>(p)); v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
   }
   static __device__ __forceinline__ void st(float* p, const float* v) {
     *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);

@@ -26,14 +26,13 @@
 #pragma once
 #include "model_fenton.cuh"
 
-#ifndef FIB_FUSE_MINB
-#define FIB_FUSE_MINB 5
-#endif
-
 namespace fib {
 
 constexpr int kFuseHalo = 2;     // halo rows of every plane in the fused layout
 constexpr int kFuseCols = 120;   // output columns per warp: lanes 1..30 x 4 cells
+constexpr int kFuseBY = 4;       // warps (row blocks) per CTA
+constexpr int kFuseMinB = 5;     // resident CTAs per SM without the phase field
+constexpr int kFusePFD = 1;      // prefetch distance in rows
 
 struct Fused2Args {
   const float* in[4];   // U, V, W, S at time t   (halo layout, kFuseHalo rows above and below)
@@ -46,25 +45,13 @@ struct Fused2Args {
   Fenton4v::Params p;
 };
 
-#ifndef FIB_FUSE_PREFETCH
-#define FIB_FUSE_PREFETCH 1
-#endif
-#ifndef FIB_FUSE_UNROLL
-#define FIB_FUSE_UNROLL 1
-#endif
-#ifndef FIB_FUSE_BY
-#define FIB_FUSE_BY 4      // warps (row blocks) per CTA
-#endif
-#ifndef FIB_FUSE_PFD
-#define FIB_FUSE_PFD 1      // prefetch distance in rows
-#endif
 __device__ __forceinline__ float pick4(const float (&v)[4], int i) {
   return i == 0 ? v[0] : (i == 1 ? v[1] : (i == 2 ? v[2] : v[3]));
 }
 
 // the phase-field flavour needs ~20 more registers for the phi windows: one CTA per SM fewer
 template <bool PHASE>
-__global__ void __launch_bounds__(kBX * FIB_FUSE_BY, (FIB_FUSE_MINB - (PHASE ? 1 : 0)) * 4 / FIB_FUSE_BY)
+__global__ void __launch_bounds__(kBX * kFuseBY, (kFuseMinB - (PHASE ? 1 : 0)) * 4 / kFuseBY)
 fenton_fused2_kernel(const Geom g, const Fused2Args a) {
   const int lane = threadIdx.x;
   const int c = blockIdx.x * kFuseCols - 4 + lane * 4;        // first of my four columns
@@ -106,24 +93,18 @@ fenton_fused2_kernel(const Geom g, const Fused2Args a) {
   load_enforced_row<4>(a.in[0], xrow(j - 1), cw, W, xN);
   load_enforced_row<4>(a.in[0], xrow(j), cw, W, xC);
 
-#if FIB_FUSE_UNROLL == 2
-#pragma unroll 2
-#else
 #pragma unroll 1
-#endif
   for (; j <= g1; ++j) {
     // ---------------- step 1 on row j ----------------
     load_enforced_row<4>(a.in[0], xrow(j + 1), cw, W, xS);
-#if FIB_FUSE_PREFETCH
     // the next iteration's lines: an iteration is ~800 instructions of arithmetic behind five
     // loads, and only 20 warps per SM are resident to cover their latency
-    if (j + FIB_FUSE_PFD <= g1) {
-      prefetch_l1(a.in[0] + xrow(j + 1 + FIB_FUSE_PFD) + cs);
-      const int offn = rowoff(min(j + FIB_FUSE_PFD, H - 1)) + cs;
+    if (j + kFusePFD <= g1) {
+      prefetch_l1(a.in[0] + xrow(j + 1 + kFusePFD) + cs);
+      const int offn = rowoff(min(j + kFusePFD, H - 1)) + cs;
 #pragma unroll
       for (int k = 0; k < 3; ++k) prefetch_l1(a.in[k + 1] + offn);
     }
-#endif
     float u1[4] = {0.f, 0.f, 0.f, 0.f};
     if (j >= 0 && j < H) {                                    // warp-uniform
       const int off = rowoff(j) + cs;
@@ -228,27 +209,22 @@ fenton_fused2_kernel(const Geom g, const Fused2Args a) {
 }
 
 // Output rows per warp R.  A row block costs R + 2 first-step rows, so deep marches are cheaper per
-// output row, but the grid is only a few waves of 148 SMs x FIB_FUSE_MINB CTAs at 4096^2 and a
+// output row, but the grid is only a few waves of 148 SMs x kFuseMinB CTAs at 4096^2 and a
 // badly filled last wave costs more than the two extra rows: pick the R in [8, 48] that minimises
 // waves x (R + 2) (4096^2: R = 25, two full waves, instead of 1.5 waves at R = 32: 235 -> see
 // profiles/r1_tuning_log.md).  The result does not depend on R (same arithmetic per cell).
 inline cudaError_t launch_fused2(const Geom& g, Fused2Args a, cudaStream_t st, int sms) {
   if (a.nrows <= 0) return cudaSuccess;
   const long nseg = (g.W + kFuseCols - 1) / kFuseCols;
-  static const int force = getenv("FIB_FUSE_R") ? atoi(getenv("FIB_FUSE_R")) : 0;   // experiments
-  constexpr int BY = FIB_FUSE_BY;
+  constexpr int BY = kFuseBY;
   auto ctas = [&](int R) { return nseg * (((a.nrows + R - 1) / R + BY - 1) / BY); };
+  const long slots = (long)sms * ((kFuseMinB - (a.phase ? 1 : 0)) * 4 / BY);
   int R = 8;
-  if (force > 0) {
-    R = force;
-  } else {
-    const long slots = (long)sms * ((FIB_FUSE_MINB - (a.phase ? 1 : 0)) * 4 / BY);
-    long best = -1;
-    for (int r = 8; r <= 48; ++r) {
-      const long waves = (ctas(r) + slots - 1) / slots;
-      const long cost = waves * (r + 2);
-      if (best < 0 || cost < best || (cost == best && r > R)) { best = cost; R = r; }
-    }
+  long best = -1;
+  for (int r = 8; r <= 48; ++r) {
+    const long waves = (ctas(r) + slots - 1) / slots;
+    const long cost = waves * (r + 2);
+    if (best < 0 || cost < best || (cost == best && r > R)) { best = cost; R = r; }
   }
   a.R = R;
   dim3 block(kBX, BY), grid((unsigned)nseg, (unsigned)(((a.nrows + R - 1) / R + BY - 1) / BY));

@@ -44,9 +44,6 @@ struct StepArgs {
 };
 
 constexpr int kBX = 32;   // threads along columns (one warp)
-#ifndef FIB_STEP_PREFETCH
-#define FIB_STEP_PREFETCH 1
-#endif
 __device__ __forceinline__ void prefetch_l1(const float* p) {
   asm volatile("prefetch.global.L1 [%0];" ::"l"(p));
 }
@@ -54,14 +51,6 @@ __device__ __forceinline__ void prefetch_l1(const float* p) {
 // per thread 49 vs 43 Gcell-steps/s, 640^2 -> 2 cells per thread 59 vs 53)
 constexpr long kSmallGridCells = 320L * 1024;
 
-// Programmatic dependent launch (only in builds with FIB_NC_LOADS=0, see fib_common.cuh) is used
-// for DIRECT stream launches only (measured at 512^2, 4v: direct launches 63 -> 71 Gcell-steps/s
-// with it, CUDA-graph replay 85 -> 77, so the graph path keeps plain kernel nodes).  fib_step
-// clears this flag around stream capture.
-inline bool& pdl_enabled() {
-  static thread_local bool on = true;
-  return on;
-}
 // Set around a launch wrapper: do not launch, only make sure the kernel is LOADED (the runtime loads
 // kernels lazily on first use, and that load waits for copies in flight -- fatal for the pipelined
 // upload, whose whole point is to launch behind them; see preload_kernels in fib_capi.cu)
@@ -79,12 +68,6 @@ inline char* last_kernel_name() {
 template <class M, int VEC, int R, int BY, bool PHASE>
 __global__ void __launch_bounds__(kBX* BY, M::min_blocks(VEC, PHASE))
 step_kernel(const Geom g, const StepArgs<M> a) {
-  // Programmatic dependent launch: let the NEXT time step's kernel be scheduled while this one
-  // drains (its CTAs park at their own griddepcontrol.wait), and do not touch memory before the
-  // PREVIOUS step has completed and flushed.  Both are no-ops for a launch without the attribute.
-  asm volatile("griddepcontrol.launch_dependents;");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  M::prologue(a);   // e.g. stage the Courtemanche LUT in shared memory
   const int c = (blockIdx.x * kBX + threadIdx.x) * VEC;
   const int strip = blockIdx.y * BY + threadIdx.y;
   const int gr0 = g.row0 + a.lr0 + strip * R;                 // first global row of my strip
@@ -111,7 +94,7 @@ step_kernel(const Geom g, const StepArgs<M> a) {
       if (M::NEED_LAP) load_enforced_row<VEC>(a.xin, xrow(gr + 1), cw, g.W, xS);
       // next marching row: pull its lines towards L1 while this row computes (4v +2 %, BR +5 %;
       // off for Courtemanche: 21 planes of prefetches evict the L1-resident table, LUT flavour -31 %)
-      if (FIB_STEP_PREFETCH && M::PREFETCH && R > 1 && i + 1 < R && gr + 1 < gend) {
+      if (M::PREFETCH && R > 1 && i + 1 < R && gr + 1 < gend) {
 #pragma unroll
         for (int k = 0; k < M::NS; ++k) prefetch_l1(a.s[k] + (off + pitch));
         if (M::NEED_LAP) prefetch_l1(a.xin + (xrow(gr + 2) + c));
@@ -199,17 +182,10 @@ step_kernel(const Geom g, const StepArgs<M> a) {
 template <class M, int VEC, int R, int BY, bool PHASE>
 inline cudaError_t launch_step_r(const Geom& g, const StepArgs<M>& a, cudaStream_t st) {
   const int ncg = (g.W + VEC - 1) / VEC;
-  static const bool pdl = !(getenv("FIB_PDL") && atoi(getenv("FIB_PDL")) == 0);
   cudaLaunchConfig_t cfg = {};
   cfg.blockDim = dim3(kBX, BY);
   cfg.gridDim = dim3((ncg + kBX - 1) / kBX, ((a.nrows + R - 1) / R + BY - 1) / BY);
-  cfg.dynamicSmemBytes = M::smem_bytes();
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = (FIB_NC_LOADS == 0 && pdl && pdl_enabled()) ? 1 : 0;   // see fib_common.cuh
   if (preload_only()) {
     cudaFuncAttributes fa;
     return cudaFuncGetAttributes(&fa, step_kernel<M, VEC, R, BY, PHASE>);
@@ -227,11 +203,6 @@ inline cudaError_t launch_step_p(const Geom& g, const StepArgs<M>& a, cudaStream
   const long bx = (ncg + kBX - 1) / kBX;
   auto blocks = [&](int R) { return bx * (((a.nrows + R - 1) / R + BY - 1) / BY); };
   const long want = 4L * sms;
-  static const int force = getenv("FIB_FORCE_R") ? atoi(getenv("FIB_FORCE_R")) : 0;   // experiments
-  if (force == 8 && M::MAX_R >= 8) return launch_step_r<M, VEC, (M::MAX_R >= 8 ? 8 : 1), BY, PHASE>(g, a, st);
-  if (force == 4 && M::MAX_R >= 4) return launch_step_r<M, VEC, (M::MAX_R >= 4 ? 4 : 1), BY, PHASE>(g, a, st);
-  if (force == 2 && M::MAX_R >= 2) return launch_step_r<M, VEC, (M::MAX_R >= 2 ? 2 : 1), BY, PHASE>(g, a, st);
-  if (force == 1) return launch_step_r<M, VEC, 1, BY, PHASE>(g, a, st);
   if (M::MAX_R >= 8 && M::AUTO_R >= 8 && blocks(8) >= want) return launch_step_r<M, VEC, (M::MAX_R >= 8 ? 8 : 1), BY, PHASE>(g, a, st);
   if (M::MAX_R >= 4 && M::AUTO_R >= 4 && blocks(4) >= want) return launch_step_r<M, VEC, (M::MAX_R >= 4 ? 4 : 1), BY, PHASE>(g, a, st);
   if (M::MAX_R >= 2 && M::AUTO_R >= 2 && blocks(2) >= want) return launch_step_r<M, VEC, (M::MAX_R >= 2 ? 2 : 1), BY, PHASE>(g, a, st);

@@ -9,7 +9,6 @@
 //     tests/test_gpu_math_layer.py against float64) -- the same error class as swapping one fp32
 //     libm for another, which is what the parity bars are calibrated against
 //     (oracle/tfshim.ALT_LIBM, tests/test_gpu_parity.py).
-//     Build with -DFIB_ACCURATE_MATH=1 to get IEEE division and CUDA's libm instead (A/B checks).
 //
 //  2. Packed fp32 (sm_100: fma/mul/add.rn.f32x2 -> SASS FFMA2 / FMUL2 / FADD2): a thread that owns
 //     two cells carries every quantity as an `f2` pair and issues ONE instruction for both cells'
@@ -28,10 +27,6 @@
 #include <cuda_runtime.h>
 
 #include <type_traits>
-
-#ifndef FIB_ACCURATE_MATH
-#define FIB_ACCURATE_MATH 0
-#endif
 
 namespace fib {
 
@@ -154,26 +149,6 @@ __device__ __forceinline__ f2 sfu_ex2(f2 a) { return f2(sfu_ex2(a.x), sfu_ex2(a.
 __device__ __forceinline__ f2 sfu_lg2(f2 a) { return f2(sfu_lg2(a.x), sfu_lg2(a.y)); }
 __device__ __forceinline__ f2 sfu_sqrt(f2 a) { return f2(sfu_sqrt(a.x), sfu_sqrt(a.y)); }
 
-#if FIB_ACCURATE_MATH
-__device__ __forceinline__ float m_rcp(float x) { return 1.0f / x; }
-__device__ __forceinline__ float m_div(float a, float b) { return a / b; }
-__device__ __forceinline__ float m_exp(float x) { return expf(x); }
-__device__ __forceinline__ float m_expm1(float x) { return expm1f(x); }
-__device__ __forceinline__ float m_expm1_neg(float x) { return expm1f(x); }
-__device__ __forceinline__ float m_exp_affine(float x, float c, float add) { return c * expf(x) + add; }
-__device__ __forceinline__ float m_log(float x) { return logf(x); }
-__device__ __forceinline__ float m_sqrt(float x) { return sqrtf(x); }
-// 1 / (1 + e^{-2z}) == 0.5 (1 + tanh z)
-__device__ __forceinline__ float m_half_1p_tanh(float z) { return 0.5f * (1.f + tanhf(z)); }
-#define FIB_LANEWISE1(F) __device__ __forceinline__ f2 F(f2 a) { return f2(F(a.x), F(a.y)); }
-FIB_LANEWISE1(m_rcp) FIB_LANEWISE1(m_exp) FIB_LANEWISE1(m_expm1) FIB_LANEWISE1(m_expm1_neg)
-FIB_LANEWISE1(m_log) FIB_LANEWISE1(m_sqrt) FIB_LANEWISE1(m_half_1p_tanh)
-#undef FIB_LANEWISE1
-__device__ __forceinline__ f2 m_div(f2 a, f2 b) { return f2(a.x / b.x, a.y / b.y); }
-__device__ __forceinline__ f2 m_exp_affine(f2 x, float c, float add) {
-  return f2(m_exp_affine(x.x, c, add), m_exp_affine(x.y, c, add));
-}
-#else
 // < 1 ulp (measured 0.96) / < 2 ulp (1.95); subnormal inputs and results flush to zero
 template <class T> __device__ __forceinline__ T m_rcp(T x) { return sfu_rcp(x); }
 template <class T, class U> __device__ __forceinline__ T m_div(U a, T b) { return T(a) * sfu_rcp(b); }
@@ -250,7 +225,6 @@ template <class T> __device__ __forceinline__ T m_sqrt(T x) { return sfu_sqrt(x)
 template <class T> __device__ __forceinline__ T m_half_1p_tanh(T z) {
   return sfu_rcp(m_exp_affine(T(-2.0f) * z, 1.0f, 1.0f));
 }
-#endif
 
 // The Laplacian enters a cell function only in its last expression.  A cell function takes it either
 // as a value or as a callable evaluated at that point: the persistent kernel passes a callable that

@@ -112,8 +112,6 @@ struct PersistArgs {
   unsigned long long* mail;    // the mailbox (persist_mailbox_words), words {value, step number}
   unsigned base;               // step number of the state at the start of this launch (monotonic over the run)
   int* err;                    // set to 1 if a neighbour wait ran into the spin limit
-  unsigned long long* timeline;   // optional (FIB_PERSIST_TIMELINE=1): %globaltimer of the middle tile at kernel
-                                  // start, after the TMA loads, after every step, after the TMA stores (ns)
   const float* phase;          // halo layout (one row), or nullptr
   const unsigned char* pmask;  // [rows][pmask_pitch] as in StepArgs
   int pmask_pitch;
@@ -167,15 +165,6 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
   uint64_t* bar = reinterpret_cast<uint64_t*>(st + (NS + 1) * TH * 512);
 
   const int t = threadIdx.x, tile = blockIdx.x, ntiles = gridDim.x;
-  const bool stamp = a.timeline && t == 0 && tile == ntiles / 2;
-  auto now = [&](int slot) __attribute__((always_inline)) {
-    if (stamp) {
-      unsigned long long ns;
-      asm volatile("mov.u64 %0, %globaltimer;" : "=l"(ns));
-      a.timeline[slot] = ns;
-    }
-  };
-  now(0);
   const int W = g.W, H = g.H, pitch = g.pitch;
   const int r0 = tile * TH;
   const int nrows = min(TH, H - r0);
@@ -226,7 +215,6 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
   }
   const bool need_top = tile > 0, need_bot = tile + 1 < ntiles;
   while (!mbar_try_wait(bar, 0)) {}
-  now(1);
 
   float s[NS][TH], u[TH];
   {
@@ -483,7 +471,6 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
       }
     }
     __syncthreads();            // shared tile of the next step complete, the old one free for reuse
-    now(2 + step);
   }
   if (probe_me) *a.ring_count = probe_n;
   if constexpr (ACT) {
@@ -511,7 +498,6 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
     }
     tma_store_commit_wait();
   }
-  now(2 + a.nsteps);
 }
 
 template <int NS, int TH>

@@ -37,11 +37,11 @@ __device__ __forceinline__ void load_enforced_row(const float* __restrict__ x, i
   if (cw.interior_x) {
     const float* p = x + (row + cw.c);
     VecIO<VEC>::ld(p, &e[1]);
-    e[0] = FIB_LD(p - 1);
-    e[VEC + 1] = FIB_LD(p + VEC);
+    e[0] = __ldg(p - 1);
+    e[VEC + 1] = __ldg(p + VEC);
   } else {
 #pragma unroll
-    for (int j = 0; j < VEC + 2; ++j) e[j] = FIB_LD(x + (row + clampi(cw.c - 1 + j, 1, W - 2)));
+    for (int j = 0; j < VEC + 2; ++j) e[j] = __ldg(x + (row + clampi(cw.c - 1 + j, 1, W - 2)));
   }
 }
 
@@ -75,7 +75,7 @@ __device__ __forceinline__ float phase_term(float xN, float xS, float xW, float 
                                             float pS, float pW, float pE, float pC) {
   float a = __fmul_rn(__fsub_rn(xS, xN), __fsub_rn(pS, pN));
   float b = __fmul_rn(__fsub_rn(xE, xW), __fsub_rn(pE, pW));
-  return m_div(__fadd_rn(a, b), __fmul_rn(4.0f, pC));   // 2-ulp SFU division (IEEE with FIB_ACCURATE_MATH)
+  return m_div(__fadd_rn(a, b), __fmul_rn(4.0f, pC));   // 2-ulp SFU division
 }
 
 }  // namespace fib

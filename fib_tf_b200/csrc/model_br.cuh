@@ -16,36 +16,11 @@
 #pragma once
 #include "fib_kernels.cuh"
 
-// tuning knobs, chosen by measurement on B200 (cells per thread, resident CTAs per SM): the
-// kernels are issue/latency bound, so occupancy beats per-thread vector width.  The step that also
-// advances the four slow gates holds more live values than the fast-only step of the skip schedule.
-#ifndef FIB_BR_VEC_SLOW
-#define FIB_BR_VEC_SLOW 2
-#endif
-#ifndef FIB_BR_MINB_SLOW
-#define FIB_BR_MINB_SLOW 7
-#endif
-#ifndef FIB_BR_MINB_SLOW_EXACT
-#define FIB_BR_MINB_SLOW_EXACT 5   /* packed pairs want registers: 4 / 5 / 6 / 7 CTAs -> 77.9 / 79.3 / 77.1 / 60.8 */
-#endif
-#ifndef FIB_BR_VEC_FAST
-#define FIB_BR_VEC_FAST 2
-#endif
-#ifndef FIB_BR_MINB_FAST
-#define FIB_BR_MINB_FAST 8
-#endif
-#ifndef FIB_BR_PACKED            /* two cells per thread as one f2 pair; 0 = two scalar cells (A/B) */
-#define FIB_BR_PACKED 1
-#endif
-#ifndef FIB_BR_PACKED_EXACT
-#define FIB_BR_PACKED_EXACT FIB_BR_PACKED
-#endif
-
 namespace fib {
 
 // (c0 e^{c1(v+c2)} + c3 (v+c4)) / (e^{c5(v+c2)} + c6)  -- br.py:255-264.  Called with literal
 // coefficients only, so every `== 0` test below folds at compile time (exp(0) == 1 exactly).
-// Scalar: the readable statement of the exact gates, used by the FIB_ACCURATE_MATH build.
+// Scalar: the readable statement of the exact gates, checked against float64 by the math-layer tests.
 __device__ __forceinline__ float br_rate(float v, float c0, float c1, float c2, float c3, float c4,
                                          float c5, float c6) {
   const float e_num = (c1 == 0.f) ? 1.f : m_exp(c1 * (v + c2));
@@ -94,9 +69,9 @@ __device__ __forceinline__ T rush_larsen_frac(T g, T n1, T d1, T n2, T d2, float
 }
 
 // The exact gates of br.py:175-205 / 255-273 for one cell (or a pair), same formulas as
-// br_inf_rate_exact (which stays as the readable statement and is what the accurate-math build
-// uses), with the SFU work trimmed -- the exact-gate kernel is MUFU-bound (~47 SFU ops per cell):
-// exponentials that differ only by a constant factor are computed once
+// br_inf_rate_exact (which stays as the readable statement), with the SFU work trimmed -- the
+// exact-gate kernel is MUFU-bound (~47 SFU ops per cell): exponentials that differ only by a
+// constant factor are computed once
 //   e^{-0.25(v+78)} = e^{-0.25(v+77)} e^{-0.25}          (alpha_j <- alpha_h)
 //   e^{-0.2(v+30)}  = e^{-0.2(v+78)} e^{9.6}              (beta_f  <- alpha_j)
 //   e^{-0.1(v+32)}  = e^{-0.1(v+47)} e^{1.5}              (beta_j  <- alpha_m)
@@ -105,19 +80,6 @@ __device__ __forceinline__ T rush_larsen_frac(T g, T n1, T d1, T n2, T d2, float
 // structure, so V0 == -47.0f still yields the reference's 0/0 -> clip upper bound (fib_common.cuh).
 template <bool SLOW, class T>
 __device__ __forceinline__ void br_gates_exact(T v, T rk, T (&s)[7], float neg_dt, float neg_dt_slow) {
-#if FIB_ACCURATE_MATH
-  static_assert(Lanes<T>::N == 1, "the accurate-math build runs the scalar flavours only");
-  float inf, rate;
-  br_inf_rate_exact<1>(v, inf, rate); s[1] = rush_larsen_rate(s[1], inf, rate, neg_dt);
-  br_inf_rate_exact<2>(v, inf, rate); s[2] = rush_larsen_rate(s[2], inf, rate, neg_dt);
-  if (SLOW) {
-    br_inf_rate_exact<0>(v, inf, rate); s[6] = rush_larsen_rate(s[6], inf, rate, neg_dt_slow);
-    br_inf_rate_exact<3>(v, inf, rate); s[3] = rush_larsen_rate(s[3], inf, rate, neg_dt_slow);
-    br_inf_rate_exact<4>(v, inf, rate); s[4] = rush_larsen_rate(s[4], inf, rate, neg_dt_slow);
-    br_inf_rate_exact<5>(v, inf, rate); s[5] = rush_larsen_rate(s[5], inf, rate, neg_dt_slow);
-  }
-  (void)rk;
-#else
   // m: a = -(v+47)/expm1(-0.1(v+47)), b = 40 e^{-0.056(v+72)}
   const T v47 = v + T(47.f);
   const T zm = T(-0.1f) * v47;
@@ -161,7 +123,6 @@ __device__ __forceinline__ void br_gates_exact(T v, T rk, T (&s)[7], float neg_d
                             m_exp_affine(T(-0.06f) * (v + T(20.f)), 0.0013f, 0.f),
                             vfma(rk, T(0.44932896411722156f), T(1.f)), neg_dt_slow);
   }
-#endif
 }
 // rush_larsen with the argument-compensated expm1 (same result class, three instructions longer)
 template <class T> __device__ __forceinline__ T rush_larsen_comp(T g, T g_inf, T tau, float neg_dt) {
@@ -199,14 +160,17 @@ template <class T> __device__ __forceinline__ T br_strict_eval(const float* __re
 template <int CHEBY, bool SLOW>
 struct BeelerReuter {
   static constexpr int NS = 7;            // C, M, H, J, D, F, XI  (V is the diffusing variable)
-  static constexpr int VEC = SLOW ? FIB_BR_VEC_SLOW : FIB_BR_VEC_FAST;
+  // cells per thread and resident CTAs per SM, chosen by measurement on B200: the kernels are
+  // issue/latency bound, so occupancy beats per-thread vector width.  The step that also advances
+  // the four slow gates holds more live values than the fast-only step of the skip schedule; the
+  // exact slow step's packed pairs want registers (4 / 5 / 6 / 7 CTAs -> 77.9 / 79.3 / 77.1 / 60.8).
+  static constexpr int VEC = 2;
   static constexpr int VEC_SMALL = 1;   // cells per thread on small grids (kSmallGridCells)
-  static constexpr bool PACKED = !FIB_ACCURATE_MATH && (CHEBY == 0 ? FIB_BR_PACKED_EXACT : FIB_BR_PACKED);
+  static constexpr bool PACKED = true;  // two cells per thread as one f2 pair
   static constexpr int BY = 4;
   static constexpr int MAX_R = 4;
   static constexpr int AUTO_R = 2;   // marching depth picked by launch_step (measured best)
-  static constexpr int MIN_BLOCKS =
-      SLOW ? (CHEBY == 1 ? FIB_BR_MINB_SLOW : FIB_BR_MINB_SLOW_EXACT) : FIB_BR_MINB_FAST;
+  static constexpr int MIN_BLOCKS = SLOW ? (CHEBY == 1 ? 7 : 5) : 8;
   // the one-cell-per-thread flavour of small grids keeps 6 (512^2 + hole: 45.7 vs 44.2 at 7)
   static __host__ __device__ constexpr int min_blocks(int vec, bool /*phase*/) {
     return (SLOW && CHEBY == 1 && vec == 1) ? 6 : MIN_BLOCKS;
@@ -217,7 +181,6 @@ struct BeelerReuter {
   static constexpr bool STORE_X = true;
   // slow gates J, D, F, XI are frozen when n == 0 (br.py:199-203): not even written back
   static __host__ __device__ constexpr bool stores(int k) { return k <= 2 || SLOW; }
-  static size_t smem_bytes() { return 0; }
   static const char* name() {
     return CHEBY == 2 ? (SLOW ? "BeelerReuter<strict,slow>" : "BeelerReuter<strict,fast>")
          : CHEBY == 1 ? (SLOW ? "BeelerReuter<cheby,slow>" : "BeelerReuter<cheby,fast>")
@@ -231,7 +194,6 @@ struct BeelerReuter {
     float poly[12][9];   // FIB_TABLE_BR_CHEBY re-expressed as monomial coefficients c_i = d_i 2^(i-1)
                          // (CHEBY == 2: the table's own d_i, fp32)
   };
-  static __device__ __forceinline__ void prologue(const StepArgs<BeelerReuter>&) {}
 
   // A: anything with a member `p` of type Params (StepArgs<BeelerReuter>, or a reference wrapper)
   template <class A, class T, class L>

@@ -5,44 +5,6 @@
 #pragma once
 #include "fib_kernels.cuh"
 
-// cells per thread / resident CTAs per SM / packed pairs per kernel flavour, measured on B200 (4096^2,
-// Gcell-steps/s; profiles/r2_tuning_log.md):
-//   fast op   2 scalar cells @8 CTAs 78.3 (packed pair @6/8/10: 73.5 / 75.2 / 55.7: HBM-bound, packing only
-//             costs registers)
-//   all-state 1 cell @8 CTAs 28.0 -> packed pair @4 CTAs 32.7 -> @5 CTAs 34.8 (89 % of the 168-B roofline)
-//   LUT       packed pair @4/5/6 CTAs 32.2 / 33.1 / 31.1; 2 scalar cells @4 CTAs 34.1 -> @5 CTAs 36.6 (94 %):
-//             the table flavour is load-bound (60 table reads per pair), the pair registers do not pay
-#ifndef FIB_COURT_VEC_FAST
-#define FIB_COURT_VEC_FAST 2
-#endif
-#ifndef FIB_COURT_VEC_ALL
-#define FIB_COURT_VEC_ALL 2
-#endif
-#ifndef FIB_COURT_VEC_LUT
-#define FIB_COURT_VEC_LUT 2
-#endif
-#ifndef FIB_COURT_MINB_FAST
-#define FIB_COURT_MINB_FAST 8
-#endif
-#ifndef FIB_COURT_MINB_ALL
-#define FIB_COURT_MINB_ALL 5
-#endif
-#ifndef FIB_COURT_MINB_LUT
-#define FIB_COURT_MINB_LUT 5
-#endif
-#ifndef FIB_COURT_LUT_SMEM       /* 1: stage the transposed table in shared memory (A/B, see prologue) */
-#define FIB_COURT_LUT_SMEM 0
-#endif
-#ifndef FIB_COURT_PACKED_FAST    /* two cells per thread as one f2 pair; 0 = two scalar cells (A/B) */
-#define FIB_COURT_PACKED_FAST 0
-#endif
-#ifndef FIB_COURT_PACKED_LUT
-#define FIB_COURT_PACKED_LUT 0
-#endif
-#ifndef FIB_COURT_PACKED_ALL
-#define FIB_COURT_PACKED_ALL 1
-#endif
-
 namespace fib {
 
 constexpr int kLutRows = 150;   // ionic.h:47  TABLE_ROWS
@@ -116,12 +78,10 @@ __device__ __forceinline__ void court_inter_dev(T V, T (&q)[kInterCols]) {
     em1[k] = ey[k] - 1.0f;
     ymin = vmin(ymin, vabs(y[k]));
   }
-#if !FIB_ACCURATE_MATH
   if (__any_sync(__activemask(), any_lane(lt(ymin, T(0.03f))))) {
 #pragma unroll
     for (int k = 0; k < 6; ++k) em1[k] = sel(lt(vabs(y[k]), T(0.03f)), m_expm1(y[k]), em1[k]);
   }
-#endif
 
   q[Q_d_inf] = m_rcp(m_exp_affine((V + 10.0f) * -0.125f, 1.f, 1.0f));
   {
@@ -278,20 +238,24 @@ enum CourtMode {
 template <int MODE, bool LUT, bool US>
 struct Courtemanche {
   static constexpr int NS = S_COUNT;      // 21 slots; S_us only used when US
-  static constexpr int VEC =
-      MODE == COURT_FAST ? FIB_COURT_VEC_FAST : (LUT ? FIB_COURT_VEC_LUT : FIB_COURT_VEC_ALL);
+  // cells per thread / resident CTAs per SM / packed pairs per kernel flavour, measured on B200 (4096^2,
+  // Gcell-steps/s; profiles/r2_tuning_log.md):
+  //   fast op   2 scalar cells @8 CTAs 78.3 (packed pair @6/8/10: 73.5 / 75.2 / 55.7: HBM-bound, packing only
+  //             costs registers)
+  //   all-state 1 cell @8 CTAs 28.0 -> packed pair @4 CTAs 32.7 -> @5 CTAs 34.8 (89 % of the 168-B roofline)
+  //   LUT       packed pair @4/5/6 CTAs 32.2 / 33.1 / 31.1; 2 scalar cells @4 CTAs 34.1 -> @5 CTAs 36.6 (94 %):
+  //             the table flavour is load-bound (60 table reads per pair), the pair registers do not pay
+  static constexpr int VEC = 2;
   static constexpr int VEC_SMALL = 1;   // cells per thread on small grids (kSmallGridCells)
   static constexpr int BY = 4;
   static constexpr int MAX_R = LUT ? 2 : 1;
   static constexpr int AUTO_R = LUT ? 2 : 1;   // marching depth picked by launch_step (measured best)
-  static constexpr int MIN_BLOCKS =
-      MODE == COURT_FAST ? FIB_COURT_MINB_FAST : (LUT ? FIB_COURT_MINB_LUT : FIB_COURT_MINB_ALL);
+  static constexpr int MIN_BLOCKS = MODE == COURT_FAST ? 8 : 5;
   // the one-cell-per-thread flavour of the direct all-state kernel (small grids) keeps 8 CTAs per SM
   static __host__ __device__ constexpr int min_blocks(int vec, bool /*phase*/) {
     return (MODE == COURT_ALL && !LUT && vec == 1) ? 8 : MIN_BLOCKS;
   }
-  static constexpr bool PACKED = !FIB_ACCURATE_MATH &&
-      (MODE == COURT_FAST ? FIB_COURT_PACKED_FAST : (LUT ? FIB_COURT_PACKED_LUT : FIB_COURT_PACKED_ALL));
+  static constexpr bool PACKED = MODE != COURT_FAST && !LUT;
   static constexpr bool PREFETCH = false;
   static constexpr bool NEED_RAW = false; // V = enforce_boundary(V0) everywhere (court.py:126-127)
   static constexpr bool NEED_LAP = MODE != COURT_SLOW;
@@ -301,7 +265,6 @@ struct Courtemanche {
     return (k == S_us) ? (US && MODE != COURT_FAST)
                        : (MODE == COURT_ALL ? true : (MODE == COURT_FAST ? is_fast(k) : !is_fast(k)));
   }
-  static size_t smem_bytes() { return (LUT && FIB_COURT_LUT_SMEM) ? sizeof(float) * kLutCols * kLutTStride : 0; }
   static const char* name() {
     static const char* n[3][2][2] = {
         {{"Courtemanche<fast>", "Courtemanche<fast,us>"}, {"Courtemanche<fast,lut>", "Courtemanche<fast,lut,us>"}},
@@ -320,39 +283,6 @@ struct Courtemanche {
                                   // on the host like the reference's Python (court.py:193-194,218)
   };
 
-  // Where the table lives (north_star: "lookup tables held in shared/constant memory"): measured A/B on B200
-  // (profiles/r2_tuning_log.md).  Default: the transposed copy [30][160] (19 KB) in global memory, read
-  // through L1 with ld.global.nc -- it stays L1-resident (every CTA of every wave reads the same 19 KB)
-  // and costs no shared memory, so five CTAs per SM keep all of L1.  FIB_COURT_LUT_SMEM=1 stages it into
-  // dynamic shared memory in this prologue instead (one cooperative copy + barrier per CTA).
-  static __device__ __forceinline__ void prologue(const StepArgs<Courtemanche>& a) {
-#if FIB_COURT_LUT_SMEM
-    if (LUT) {
-      extern __shared__ float fib_lut_smem[];
-      const int n = kLutCols * kLutTStride, nt = blockDim.x * blockDim.y, t = threadIdx.y * blockDim.x + threadIdx.x;
-      for (int i = t; i < n; i += nt) fib_lut_smem[i] = __ldg(a.lut + i);
-      __syncthreads();
-    }
-#else
-    (void)a;
-#endif
-  }
-  static __device__ __forceinline__ const float* lut_base(const float* global_lut) {
-#if FIB_COURT_LUT_SMEM
-    extern __shared__ float fib_lut_smem[];
-    return fib_lut_smem;
-#else
-    return global_lut;
-#endif
-  }
-  static __device__ __forceinline__ float lut_read(const float* p) {
-#if FIB_COURT_LUT_SMEM
-    return *p;
-#else
-    return __ldg(p);
-#endif
-  }
-
   // rush_larsen_b with t = tau (table flavours) or t = 1/tau (direct flavours)
   template <class T>
   static __device__ __forceinline__ T gate(T g, T g_inf, T t, float neg_dt, const Params& p) {
@@ -365,16 +295,20 @@ struct Courtemanche {
     int i = static_cast<int>(V + 100.f);
     return i < 0 ? 0 : (i >= kLutRows ? kLutRows - 1 : i);
   }
+  // Where the table lives: the transposed copy [30][160] (19 KB) in global memory, read through L1
+  // with ld.global.nc -- it stays L1-resident (every CTA of every wave reads the same 19 KB) and costs
+  // no shared memory, so five CTAs per SM keep all of L1 (measured against a shared-memory copy on
+  // B200, profiles/r2_tuning_log.md).
   static __device__ __forceinline__ void lut_fetch(const float* lut, float V, float (&q)[kInterCols]) {
-    const float* col = lut_base(lut) + lut_row(V);
+    const float* col = lut + lut_row(V);
 #pragma unroll
-    for (int k = 0; k < kLutCols; ++k) q[k] = lut_read(col + k * kLutTStride);
+    for (int k = 0; k < kLutCols; ++k) q[k] = __ldg(col + k * kLutTStride);
   }
   static __device__ __forceinline__ void lut_fetch(const float* lut, f2 V, f2 (&q)[kInterCols]) {
-    const float* c0 = lut_base(lut) + lut_row(V.x);
-    const float* c1 = lut_base(lut) + lut_row(V.y);
+    const float* c0 = lut + lut_row(V.x);
+    const float* c1 = lut + lut_row(V.y);
 #pragma unroll
-    for (int k = 0; k < kLutCols; ++k) q[k] = f2(lut_read(c0 + k * kLutTStride), lut_read(c1 + k * kLutTStride));
+    for (int k = 0; k < kLutCols; ++k) q[k] = f2(__ldg(c0 + k * kLutTStride), __ldg(c1 + k * kLutTStride));
   }
 
   template <class T>

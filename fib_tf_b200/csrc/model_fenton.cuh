@@ -3,16 +3,6 @@
 #pragma once
 #include "fib_kernels.cuh"
 
-#ifndef FIB_4V_MINB
-#define FIB_4V_MINB 8
-#endif
-#ifndef FIB_4V_MINB_PHASE
-#define FIB_4V_MINB_PHASE 6
-#endif
-#ifndef FIB_4V_PACKED           /* the four cells of a thread as two f2 pairs (packed fp32) */
-#define FIB_4V_PACKED 1
-#endif
-
 namespace fib {
 
 struct Fenton4v {
@@ -22,25 +12,23 @@ struct Fenton4v {
   static constexpr int BY = 4;
   static constexpr int MAX_R = 4;
   static constexpr int AUTO_R = 4;   // marching depth picked by launch_step (measured best)
-  static constexpr int MIN_BLOCKS = FIB_4V_MINB;
+  static constexpr int MIN_BLOCKS = 8;
   // the phase-field flavour holds the phi window as well: at 8 CTAs per SM (64 registers) it spilled 33
   // values per thread (round-1 ncu); 6 CTAs (80 registers) keeps everything in registers
   static __host__ __device__ constexpr int min_blocks(int /*cells per thread*/, bool phase) {
-    return phase ? FIB_4V_MINB_PHASE : MIN_BLOCKS;
+    return phase ? 6 : MIN_BLOCKS;
   }
-  static constexpr bool PACKED = FIB_4V_PACKED != 0;   // the four cells of a thread as two f2 pairs
+  static constexpr bool PACKED = true;   // the four cells of a thread as two f2 pairs
   static constexpr bool PREFETCH = true;
   static constexpr bool NEED_RAW = true;  // reaction sees the raw U (fenton.py:101), SURVEY fact 3
   static constexpr bool NEED_LAP = true;
   static constexpr bool STORE_X = true;
   static __host__ __device__ constexpr bool stores(int) { return true; }
-  static size_t smem_bytes() { return 0; }
   static const char* name() { return "Fenton4v"; }
   struct Params {
     float dt;    // fp32(dt)
     float ddt;   // fp32(diff * dt), folded in double like the reference (fenton.py:103)
   };
-  static __device__ __forceinline__ void prologue(const StepArgs<Fenton4v>&) {}
 
   // Divisions by literals are multiplications by the correctly rounded reciprocal (<= 1 ulp from
   // the reference's fp32 division; budgeted in SURVEY.md Appendix B.2).
@@ -90,10 +78,9 @@ struct Fenton4v {
     Unew = add_rn(reaction, mul_rn(T(a.p.ddt), lap_value<T>(lap)));
   }
 
-  // four cells of a thread: two packed pairs (FIB_4V_PACKED, default) or four scalar cells
+  // four cells of a thread as two packed pairs
   static __device__ __forceinline__ void cell4(const StepArgs<Fenton4v>& a, const float (&raw)[4], const float* x0,
                                                const float (&lap)[4], float (&sv)[3][4], float (&unew)[4]) {
-#if FIB_4V_PACKED
 #pragma unroll
     for (int l = 0; l < 4; l += 2) {
       f2 sp[3] = {f2(sv[0][l], sv[0][l + 1]), f2(sv[1][l], sv[1][l + 1]), f2(sv[2][l], sv[2][l + 1])};
@@ -104,14 +91,6 @@ struct Fenton4v {
 #pragma unroll
       for (int k = 0; k < 3; ++k) { sv[k][l] = sp[k].x; sv[k][l + 1] = sp[k].y; }
     }
-#else
-#pragma unroll
-    for (int l = 0; l < 4; ++l) {
-      float sl[3] = {sv[0][l], sv[1][l], sv[2][l]};
-      cell(a, raw[l], x0[l], lap[l], sl, unew[l]);
-      sv[0][l] = sl[0]; sv[1][l] = sl[1]; sv[2][l] = sl[2];
-    }
-#endif
   }
 };
 
