@@ -20,7 +20,7 @@ PROBE_RING = 4096
 OP_ODE, OP_SLOW = 0, 1
 TABLE_BR_CHEBY, TABLE_COURT_LUT = 0, 1
 ACT_FIRST, ACT_LAST, ACT_PREV, ACT_REPOL, ACT_COUNT = 0, 1, 2, 3, 4
-ABI_VERSION = 3
+ABI_VERSION = 4
 INTER_COLS = 32
 
 # courtemanche.h:105-134 column order (+ the two court_ultra.py:445-450 extras)
@@ -71,6 +71,10 @@ _SIGNATURES = {
     'fib_activation_watch': (C.c_int, [_P, C.c_float, C.c_float]),
     'fib_activation_stop': (C.c_int, [_P]),
     'fib_activation_get': (C.c_int, [_P, C.c_int, _P, C.c_size_t]),
+    'fib_frames_watch': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    'fib_frames_stop': (C.c_int, [_P]),
+    'fib_frames_shape': (C.c_int, [_P, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    'fib_frames_fetch': (C.c_int, [_P, _P, C.POINTER(C.c_uint64), C.c_size_t, C.POINTER(C.c_size_t)]),
     'fib_count_below': (C.c_int, [_P, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float,
                                   C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     'fib_op_enforce_boundary': (C.c_int, [C.c_int, _P, C.c_int, C.c_int, _P]),
@@ -304,6 +308,30 @@ class Context:
         out = np.empty((self.rows, self.width), dtype=np.float32)
         check(lib().fib_activation_get(self._h, which, out.ctypes.data_as(_P), out.size))
         return out
+
+    def frames_watch(self, var, first, every, stride, capacity):
+        """Arm (or re-arm) the frame recorder: plane `var`[::stride, ::stride] at k = first + j * every."""
+        check(lib().fib_frames_watch(self._h, self.var(var), int(first), int(every), int(stride), int(capacity)))
+
+    def frames_stop(self):
+        check(lib().fib_frames_stop(self._h))
+
+    def frames_shape(self):
+        """(rows, cols) of this shard's frame."""
+        r, c = C.c_int(), C.c_int()
+        check(lib().fib_frames_shape(self._h, C.byref(r), C.byref(c)))
+        return r.value, c.value
+
+    def frames_fetch(self, max_frames):
+        """(iters, frames): the oldest unfetched frames, at most max_frames, as uint64 [n] and float32
+        [n, rows, cols]."""
+        rows, cols = self.frames_shape()
+        out = np.empty((max_frames, rows, cols), dtype=np.float32)
+        iters = np.empty(max_frames, dtype=np.uint64)
+        n = C.c_size_t()
+        check(lib().fib_frames_fetch(self._h, out.ctypes.data_as(_P), iters.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                     max_frames, C.byref(n)))
+        return iters[:n.value], out[:n.value]
 
     def count_below(self, var, sub, div, cutoff, w_min):
         a, b = C.c_uint64(), C.c_uint64()

@@ -150,6 +150,23 @@ struct fib_ctx {
   unsigned long long* act_iter = nullptr;   // device: samples taken since arming (= k - 1 of the next one)
   unsigned long long act_n = 0;       // host mirror of *act_iter (iterations enqueued since arming)
   float act_up = 0.f, act_down = 0.f;
+  // frame recorder (fib_frames_watch): armed iff frames != nullptr.  Frame j is the plane at k = fr_first +
+  // j * fr_every and lives in slot j % fr_cap; the host knows k, so only recording iterations launch anything.
+  float* frames = nullptr;            // [fr_cap][fr_rows][fr_cols]
+  int fr_var = 0, fr_first = 0, fr_every = 1, fr_stride = 1, fr_cap = 0;
+  int fr_rows = 0, fr_cols = 0, fr_lr0 = 0;   // this shard's frame; fr_lr0 = local row of its first row
+  unsigned long long fr_k = 0;        // ODE iterations enqueued since arming
+  unsigned long long fr_fetched = 0;  // frames handed out (or lost to overflow)
+  // {event after a launch that recorded frames, frames recorded up to it}: a fetch waits for the covering one
+  static constexpr int kFrameEvents = 256;
+  cudaEvent_t fr_ev[kFrameEvents] = {};
+  unsigned long long fr_ev_total[kFrameEvents] = {};
+  int fr_ev_next = 0;
+  size_t frame_floats() const { return (size_t)fr_rows * fr_cols; }
+  // frames recorded once k iterations have run
+  unsigned long long frames_upto(unsigned long long k) const {
+    return k < (unsigned long long)fr_first ? 0 : (k - fr_first) / fr_every + 1;
+  }
   float* weights[4] = {nullptr, nullptr, nullptr, nullptr};   // user masks, halo layout like phase
   // persistent on-chip kernel (fib_persist.cuh): small unsharded 4v / BR grids
   int persist = -1;                   // -1 not decided yet, 0 no, 1 yes
@@ -291,6 +308,16 @@ __global__ void probe_update_kernel(const float* __restrict__ src, float* __rest
                                     const unsigned long long* __restrict__ count) {
   const unsigned long long n = *count;
   if (n) ring[(n - 1) % FIB_PROBE_RING] = *src;
+}
+
+// fib_frames_watch: one frame, a strided gather of a plane's owned rows.  `src` = the first owned row whose
+// global index is a multiple of the stride, `src_step` = floats between two frame rows (stride * pitch).
+__global__ void frame_record_kernel(const float* __restrict__ src, size_t src_step, int stride, int rows, int cols,
+                                    float* __restrict__ dst) {
+  const int fc = blockIdx.x * blockDim.x + threadIdx.x;
+  if (fc >= cols) return;
+  for (int fr = blockIdx.y; fr < rows; fr += gridDim.y)
+    dst[(size_t)fr * cols + fc] = src[(size_t)fr * src_step + (size_t)fc * stride];
 }
 
 // court_ultra.py:504-509: cells with weight > w_min, and among them those whose normalised value
@@ -549,6 +576,9 @@ extern "C" int fib_destroy(fib_ctx* c) {
   cudaFree(c->act_prev);
   cudaFree(c->act_maps);
   cudaFree(c->act_iter);
+  cudaFree(c->frames);
+  for (auto& e : c->fr_ev)
+    if (e) cudaEventDestroy(e);
   cudaFree(c->pmail);
   if (c->perr) cudaFreeHost(c->perr);
   for (int k = 0; k < 4; ++k) cudaFree(c->weights[k]);
@@ -752,7 +782,7 @@ static int set_rect_impl(fib_ctx* c, int var, int r0, int r1, int c0, int c1, co
     // On an NCCL shard the block order may also run bottom to top (odd ranks do, so that both shards of a seam
     // either begin or end there: fib_step_behind_upload).
     const bool eligible = (c->comm ? c->pipeline_nccl : c->g.rows == c->g.H) && c0 == 0 && c1 == c->g.W &&
-                          c->watch_var < 0 && !c->act_maps && (long long)c->g.rows * c->g.W >= c->pipeline_min_cells;
+                          c->watch_var < 0 && !c->act_maps && !c->frames && (long long)c->g.rows * c->g.W >= c->pipeline_min_cells;
     const int row_end = c->g.row0 + c->g.rows;
     const int dir = c->up_session ? c->up_dir : (r0 == c->g.row0 ? +1 : (r1 == row_end && c->comm ? -1 : 0));
     const int dlo = dir > 0 ? r0 - c->g.row0 : row_end - r1, dhi = dir > 0 ? r1 - c->g.row0 : row_end - r0;
@@ -1152,13 +1182,13 @@ static bool make_tile_map(CUtensorMap* m, float* base, int W, int rows, int pitc
          CUDA_SUCCESS;
 }
 
-template <class MS, class MF, int TH, bool PHASE, bool ACT>
+template <class MS, class MF, int TH, bool PHASE, bool ACT, bool FRAMES>
 static cudaError_t launch_persist_t(fib_ctx* c, const PersistArgs<MS, MF>& a) {
   PersistMaps<MS::NS> maps;
   maps.x[0] = c->pmap_x[0];
   maps.x[1] = c->pmap_x[1];
   for (int k = 0; k < MS::NS; ++k) maps.s[k] = c->pmap_s[k];
-  auto kern = persist_kernel<MS, MF, TH, PHASE, ACT>;
+  auto kern = persist_kernel<MS, MF, TH, PHASE, ACT, FRAMES>;
   constexpr size_t smem = persist_smem_bytes<MS::NS, TH>();
   static bool attr_set = false;           // per instantiation
   if (!attr_set) {
@@ -1176,8 +1206,8 @@ static cudaError_t launch_persist_t(fib_ctx* c, const PersistArgs<MS, MF>& a) {
   attr[0].val.cooperative = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  snprintf(last_kernel_name(), 160, "persist_kernel<%s,TH=%d,PHASE=%d%s>", MS::name(), TH, PHASE ? 1 : 0,
-           ACT ? ",ACT=1" : "");
+  snprintf(last_kernel_name(), 160, "persist_kernel<%s,TH=%d,PHASE=%d%s%s>", MS::name(), TH, PHASE ? 1 : 0,
+           ACT ? ",ACT=1" : "", FRAMES ? ",FRAMES=1" : "");
   return cudaLaunchKernelEx(&cfg, kern, maps, c->g, a);
 }
 
@@ -1207,11 +1237,34 @@ static cudaError_t launch_persist_m(fib_ctx* c, PersistArgs<MS, MF>& a, int iter
   a.act_k0 = c->act_n;
   a.act_up = c->act_up;
   a.act_down = c->act_down;
-  const bool ph = c->phase != nullptr, act = c->act_maps != nullptr;
+  // frames: the first recording iteration of this launch (k = fr_k + 1 + it0), if there is one
+  a.frames = nullptr;
+  if (c->frames) {
+    const unsigned long long k1 = c->fr_k + 1, f0 = c->fr_first, ev = c->fr_every;
+    const unsigned long long kf = k1 <= f0 ? f0 : f0 + (k1 - f0 + ev - 1) / ev * ev;
+    if (kf < k1 + (unsigned)iters) {
+      a.frames = c->frames;
+      a.frame_step0 = (int)(kf - k1 + 1) * a.period;
+      a.frame_steps = (int)min(ev, (unsigned long long)kPersistMaxIters) * a.period;
+      a.frame_slot0 = (int)((c->frames_upto(kf) - 1) % (unsigned long long)c->fr_cap);
+      a.frame_cap = c->fr_cap;
+      a.frame_var = c->fr_var;
+      a.frame_stride = c->fr_stride;
+      a.frame_cols = c->fr_cols;
+      a.frame_floats = c->frame_floats();
+    }
+  }
+  const bool ph = c->phase != nullptr, act = c->act_maps != nullptr, fr = a.frames != nullptr;
+  auto flag = [](bool b, auto&& fn) { return b ? fn(std::true_type()) : fn(std::false_type()); };
   auto go = [&](auto th) {
-    constexpr int TH = decltype(th)::value;
-    if (act) return ph ? launch_persist_t<MS, MF, TH, true, true>(c, a) : launch_persist_t<MS, MF, TH, false, true>(c, a);
-    return ph ? launch_persist_t<MS, MF, TH, true, false>(c, a) : launch_persist_t<MS, MF, TH, false, false>(c, a);
+    return flag(ph, [&](auto P) {
+      return flag(act, [&](auto A) {
+        return flag(fr, [&](auto F) {
+          return launch_persist_t<MS, MF, decltype(th)::value, decltype(P)::value, decltype(A)::value,
+                                  decltype(F)::value>(c, a);
+        });
+      });
+    });
   };
   switch (c->persist_th) {
     case 2: return go(std::integral_constant<int, 2>());
@@ -1259,6 +1312,29 @@ static void decide_persist(fib_ctx* c) {
   c->persist = 1;
 }
 
+// fib_frames_watch: marks everything enqueued so far as the producer of the frames recorded so far
+static int record_frame_event(fib_ctx* c) {
+  const int k = c->fr_ev_next;
+  CU(cudaEventRecord(c->fr_ev[k], c->stream));
+  c->fr_ev_total[k] = c->frames_upto(c->fr_k);
+  c->fr_ev_next = (k + 1) % fib_ctx::kFrameEvents;
+  return 0;
+}
+
+// frame j of the current plane into its ring slot
+static int launch_frame(fib_ctx* c, unsigned long long j) {
+  if (c->fr_rows > 0) {
+    const float* src = owned_rows(c, c->fr_var) + (size_t)c->fr_lr0 * c->g.pitch;
+    float* dst = c->frames + (j % (unsigned long long)c->fr_cap) * c->frame_floats();
+    const dim3 grid((c->fr_cols + 127) / 128, min(c->fr_rows, 65535));
+    frame_record_kernel<<<grid, 128, 0, c->stream>>>(src, (size_t)c->fr_stride * c->g.pitch, c->fr_stride,
+                                                     c->fr_rows, c->fr_cols, dst);
+    CU(cudaGetLastError());
+    c->launches++;
+  }
+  return record_frame_event(c);
+}
+
 // `iters` ODE iterations (dt_per_step time steps each) as ONE launch
 static int run_iteration_persist(fib_ctx* c, int iters) {
   const double dt = c->cfg.dt;
@@ -1304,6 +1380,14 @@ static int run_iteration_persist(fib_ctx* c, int iters) {
   }
   c->launches++;
   if (c->act_maps) c->act_n += (unsigned)iters;
+  if (c->frames) {
+    const unsigned long long before = c->frames_upto(c->fr_k);
+    c->fr_k += (unsigned)iters;
+    if (c->frames_upto(c->fr_k) != before) {
+      const int r = record_frame_event(c);
+      if (r) return r;
+    }
+  }
   if (c->watch_var >= 0) {
     c->ring_total += (unsigned)iters;
     const int k = c->ring_ev_next;
@@ -1354,20 +1438,30 @@ static int record_activation(fib_ctx* c, int op) {
   return 0;
 }
 
-// the observers that sample the state at the end of an ODE iteration
-static int record_observers(fib_ctx* c, int op) {
-  const int r = record_activation(c, op);
-  return r ? r : record_probe(c, op);
+// fib_frames_watch: after an ODE iteration, count it and gather a frame if it is a recording one.  Never part
+// of an iteration graph: the graph path calls it after each replay.
+static int record_frame(fib_ctx* c, int op) {
+  if (!c->frames || op != FIB_OP_ODE) return 0;
+  const unsigned long long k = ++c->fr_k;
+  if (k < (unsigned long long)c->fr_first || (k - c->fr_first) % c->fr_every) return 0;
+  return launch_frame(c, c->frames_upto(k) - 1);
 }
 
-static int run_iteration_plain(fib_ctx* c, int op) {
+// the observers that sample the state at the end of an ODE iteration (`frames` = false while capturing a graph)
+static int record_observers(fib_ctx* c, int op, bool frames = true) {
+  int r = record_activation(c, op);
+  if (!r) r = record_probe(c, op);
+  return (r || !frames) ? r : record_frame(c, op);
+}
+
+static int run_iteration_plain(fib_ctx* c, int op, bool frames = true) {
   const int ns = substeps_of(c, op);
   for (int s = 0; s < ns; s += c->fuse) {
     int r = launch_substep(c, op, s, 0, c->g.rows);
     if (r) return r;
     if (op_writes_x(c, op)) c->cur ^= 1;
   }
-  return record_observers(c, op);
+  return record_observers(c, op, frames);
 }
 
 // boundary rows first, halo exchange on the side stream overlapped with the interior rows
@@ -1457,7 +1551,7 @@ static int step_now(fib_ctx* c, int op, int n_iter) {
       CU(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
       const uint64_t l0 = c->launches;
       const unsigned long long rt0 = c->ring_total, an0 = c->act_n;
-      int r = run_iteration_plain(c, op);
+      int r = run_iteration_plain(c, op, false);
       cudaError_t ce = cudaStreamEndCapture(c->stream, &graph);
       c->launches = l0;
       c->ring_total = rt0;
@@ -1477,6 +1571,8 @@ static int step_now(fib_ctx* c, int op, int n_iter) {
     c->ring_total += rec;
     c->act_n += act;
     if (op_writes_x(c, op) && (nl & 1)) c->cur ^= 1;
+    const int r = record_frame(c, op);
+    if (r) return r;
   }
   return 0;
 }
@@ -1958,6 +2054,111 @@ extern "C" int fib_activation_get(fib_ctx* c, int map, float* host, size_t n) {
                        c->g.pitch * sizeof(float), c->g.W * sizeof(float), c->g.rows, cudaMemcpyDeviceToHost,
                        c->stream));
   CU(cudaStreamSynchronize(c->stream));
+  return check_persist_error(c);
+}
+
+// Frame recorder: a ring of strided frames in device memory.  Nothing joins the iteration graphs: the host
+// counts iterations (fr_k) and gathers a frame after the recording ones (record_frame), or hands the persistent
+// kernel the first recording iteration of its launch (launch_persist_m).
+extern "C" int fib_frames_watch(fib_ctx* c, int var, int first, int every, int stride, int capacity) {
+  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
+  if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
+  if (first < 0 || every < 1 || stride < 1 || capacity < 1)
+    return fail(FIB_E_ARG, "fib_frames_watch: need first >= 0, every >= 1, stride >= 1 and capacity >= 1 "
+                "(got %d, %d, %d, %d)", first, every, stride, capacity);
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  CU(cudaStreamSynchronize(c->stream));         // the old ring may still be written
+  CU(cudaFree(c->frames));
+  c->frames = nullptr;
+  const int gr0 = (c->g.row0 + stride - 1) / stride * stride, row_end = c->g.row0 + c->g.rows;
+  c->fr_rows = gr0 < row_end ? (row_end - 1 - gr0) / stride + 1 : 0;
+  c->fr_cols = (c->g.W + stride - 1) / stride;
+  c->fr_lr0 = gr0 - c->g.row0;
+  c->fr_var = var;
+  c->fr_first = first;
+  c->fr_every = every;
+  c->fr_stride = stride;
+  c->fr_cap = capacity;
+  c->fr_k = 0;
+  c->fr_fetched = 0;
+  for (int k = 0; k < fib_ctx::kFrameEvents; ++k) {
+    if (!c->fr_ev[k]) CU(cudaEventCreateWithFlags(&c->fr_ev[k], cudaEventDisableTiming));
+    c->fr_ev_total[k] = 0;
+  }
+  c->fr_ev_next = 0;
+  const size_t bytes = max((size_t)capacity * c->frame_floats() * sizeof(float), sizeof(float));
+  if (cudaMalloc(&c->frames, bytes) != cudaSuccess) {
+    cudaGetLastError();
+    c->frames = nullptr;
+    return fail(FIB_E_CUDA, "fib_frames_watch: cannot allocate a ring of %d frames (%zu bytes)", capacity, bytes);
+  }                                              // armed from here
+  return first == 0 ? launch_frame(c, 0) : 0;
+}
+
+extern "C" int fib_frames_stop(fib_ctx* c) {
+  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  CU(cudaStreamSynchronize(c->stream));
+  CU(cudaFree(c->frames));
+  c->frames = nullptr;
+  return check_persist_error(c);
+}
+
+extern "C" int fib_frames_shape(const fib_ctx* c, int* rows, int* cols) {
+  if (!c || !rows || !cols) return fail(FIB_E_ARG, "NULL argument");
+  if (!c->frames) return fail(FIB_E_STATE, "no frame recorder is armed (fib_frames_watch)");
+  *rows = c->fr_rows;
+  *cols = c->fr_cols;
+  return 0;
+}
+
+extern "C" int fib_frames_fetch(fib_ctx* c, float* host, uint64_t* iters, size_t max, size_t* n) {
+  if (!c || !n || ((!host || !iters) && max)) return fail(FIB_E_ARG, "NULL argument");
+  *n = 0;
+  if (!c->frames) return fail(FIB_E_STATE, "no frame recorder is armed (fib_frames_watch)");
+  DevGuard dg(c->cfg.device);
+  // Iterations the persistent path has deferred are launched only when the frames already launched do not
+  // satisfy the request: a caller that fetches one batch behind never cuts a batch.
+  unsigned long long total = c->frames_upto(c->fr_k);
+  if (total - c->fr_fetched < max) {
+    FLUSH(c);
+    total = c->frames_upto(c->fr_k);
+  }
+  unsigned long long first = c->fr_fetched;
+  if (total - first > (unsigned long long)c->fr_cap) first = total - c->fr_cap;   // overwritten
+  const unsigned long long take = min(total - first, (unsigned long long)max);
+  if (take) {
+    // wait for the earliest launch that covers the last frame taken, not for the launches queued behind it
+    int best = -1;
+    for (int k = 0; k < fib_ctx::kFrameEvents; ++k)
+      if (c->fr_ev_total[k] >= first + take && c->fr_ev_total[k] <= total &&
+          (best < 0 || c->fr_ev_total[k] < c->fr_ev_total[best]))
+        best = k;
+    if (best < 0) {
+      const int r = record_frame_event(c);
+      if (r) return r;
+      best = (c->fr_ev_next + fib_ctx::kFrameEvents - 1) % fib_ctx::kFrameEvents;
+    }
+    CU(cudaStreamWaitEvent(c->copy_stream, c->fr_ev[best], 0));
+    // at most two contiguous pieces of the ring (the frames taken cannot be overwritten by work already enqueued:
+    // that only writes frames < total, and first >= total - capacity)
+    const size_t ff = c->frame_floats();
+    unsigned long long done = 0;
+    while (done < take) {
+      const unsigned long long pos = (first + done) % (unsigned long long)c->fr_cap;
+      const unsigned long long len = min((unsigned long long)c->fr_cap - pos, take - done);
+      if (ff)
+        CU(cudaMemcpyAsync(host + done * ff, c->frames + pos * ff, len * ff * sizeof(float), cudaMemcpyDeviceToHost,
+                           c->copy_stream));
+      done += len;
+    }
+    CU(cudaStreamSynchronize(c->copy_stream));
+    for (unsigned long long i = 0; i < take; ++i) iters[i] = c->fr_first + (first + i) * c->fr_every;
+  }
+  c->fr_fetched = first + take;
+  *n = (size_t)take;
   return check_persist_error(c);
 }
 

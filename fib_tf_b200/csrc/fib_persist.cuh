@@ -134,12 +134,21 @@ struct PersistArgs {
   unsigned long long* act_iter;
   unsigned long long act_k0;
   float act_up, act_down;
+  // fib_frames_watch (FRAMES instantiations only: launches that record at least one frame): at the end of the
+  // iteration whose last step is step frame_step0 + j * frame_steps of this launch (counted from 1), the thread owning a cell
+  // whose row and column are multiples of frame_stride writes plane frame_var (picked as probe_var is) into
+  // ring slot (frame_slot0 + j) % frame_cap -- exactly what frame_record_kernel gathers on the other paths
+  float* frames;
+  int frame_step0, frame_steps, frame_slot0, frame_cap;
+  int frame_var, frame_stride, frame_cols;
+  size_t frame_floats;
 };
 
 // ---- the kernel ----------------------------------------------------------------------------------
 // MS / MF: the cell types of the "slow" and "fast" steps of a schedule (Fenton4v twice; BeelerReuter<C,true>
 // and <C,false> for br.py's skip schedule).  TH: rows per tile.  PHASE: phase field present.  ACT: an
-// activation map is armed (fib_activation.cuh).
+// activation map is armed (fib_activation.cuh).  FRAMES: the launch records frames (fib_frames_watch); a
+// compile-time switch like ACT, so that the other instantiations keep their registers.
 //
 // Where the state lives between the steps of a launch:
 //   * a thread owns ONE column of its tile: its TH cells of every plane, the diffusing variable included
@@ -153,7 +162,7 @@ struct PersistArgs {
 //     and the rows of a column are read once per step (marching reuse in registers);
 //   * the rows of the neighbour tiles arrive through the mailbox and are written into the ring rows by
 //     the thread that will read them (each thread writes the three columns it reads: no barrier).
-template <class MS, class MF, int TH, bool PHASE, bool ACT>
+template <class MS, class MF, int TH, bool PHASE, bool ACT, bool FRAMES>
 __global__ void __launch_bounds__(kPersistThreads, 1)
 persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, const PersistArgs<MS, MF> a) {
   constexpr int NS = MS::NS;
@@ -454,6 +463,22 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
           }
         a.ring[probe_n % FIB_PROBE_RING] = v;
         ++probe_n;
+      }
+      if constexpr (FRAMES) {
+        const int d = step + 1 - a.frame_step0;
+        if (d >= 0 && d % a.frame_steps == 0 && active && c % a.frame_stride == 0) {
+          float* f = a.frames + (size_t)((a.frame_slot0 + d / a.frame_steps) % a.frame_cap) * a.frame_floats +
+                     c / a.frame_stride;
+#pragma unroll
+          for (int i = 0; i < TH; ++i)
+            if (i < nrows && (r0 + i) % a.frame_stride == 0) {
+              float v = u[i];
+#pragma unroll
+              for (int k = 0; k < NS; ++k)
+                if (a.frame_var == k + 1) v = s[k][i];
+              f[(size_t)((r0 + i) / a.frame_stride) * a.frame_cols] = v;
+            }
+        }
       }
       if constexpr (ACT) {
         if (active) {

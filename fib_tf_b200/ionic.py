@@ -36,7 +36,7 @@ Extra, optional config keys (all default to the reference's behaviour):
 Collective calls under config['distributed'] (every rank must make them, in the same order):
 define(), run() (each iteration), fire_op(), image(), pot().eval() / _State[..].eval(),
 var[r, c].eval(), masked_image_mean(), excitable_fraction(), watch_activation(), activation_maps(),
-stop_activation(), close().  cl_observer callbacks run on
+stop_activation(), frames(), close().  cl_observer callbacks run on
 the rank that owns row 20 only and therefore must not call any of these.
 """
 import json
@@ -378,6 +378,8 @@ class IonicModel:
                         self._ctx                            # noqa: B018 (the window is full: go)
                 else:
                     self._ctx.step(self.ode_op(i), 1)
+                if self.__dict__.get('_frames') is not None:
+                    self._drain_frames()
                 yield i
                 if ring:
                     unread.append(i)
@@ -549,6 +551,84 @@ class IonicModel:
     def stop_activation(self):
         """Disarms the activation maps and frees their device memory."""
         self._ctx.activation_stop()
+
+    # The persistent kernel launches 64 iterations at a time (csrc fib_step); run() fetches frames one such batch
+    # behind the stepping, so a fetch never waits for the launch in flight and never cuts a batch.
+    FRAME_BATCH = 64
+
+    @classmethod
+    def default_frame_capacity(cls, every):
+        """Ring frames that run()'s drain never overflows: it leaves at most two batches of iterations unfetched,
+        which hold at most 2 * (ceil(64 / every) + 1) frames."""
+        return 2 * (-(-cls.FRAME_BATCH // int(every)) + 1)
+
+    def record_frames(self, every, stride=1, first=1, name=None, capacity=None):
+        """Arms the device-side frame recorder (include/fib_b200.h, fib_frames_watch): plane `name` (default: the
+        potential) at every `stride`-th row and column, recorded on the device at the end of iterations k = first,
+        first + every, ... counted from this call (k = 0 is the plane now), into a ring of `capacity` frames.
+        run() drains the ring by itself; frames() returns the movie.  first = 1, every = 10 are the reference
+        drivers' cadence (`cube[i // 10]` grabbed after the iteration run() yields as i = 0, 10, ...).
+        Calling it again starts a new movie."""
+        if not self.defined:
+            raise AssertionError('record_frames should be called after calling define')
+        every, stride, first = int(every), int(stride), int(first)
+        if every < 1 or stride < 1 or first < 0:
+            raise ValueError('record_frames: need every >= 1, stride >= 1 and first >= 0')
+        capacity = self.default_frame_capacity(every) if capacity is None else int(capacity)
+        name = self._pot_name if name is None else name
+        self._ctx.frames_watch(name, first, every, stride, capacity)
+        self._frames = {'name': name, 'first': first, 'every': every, 'stride': stride, 'capacity': capacity,
+                        'k': 0, 'upto': 0, 'iters': [], 'cube': []}
+
+    def _drain_frames(self):
+        """After an ODE iteration of run(): every FRAME_BATCH iterations, fetch the frames of the batch before
+        the last one (they are in launched work, so the library neither flushes nor waits for the last launch)."""
+        f = self._frames
+        f['k'] += 1
+        B = self.FRAME_BATCH
+        if f['k'] % B or f['k'] < 2 * B:
+            return
+        limit = f['k'] - B
+        upto = 0 if limit < f['first'] else (limit - f['first']) // f['every'] + 1
+        if upto > f['upto']:
+            iters, cube = self._ctx.frames_fetch(upto - f['upto'])
+            f['iters'].append(iters)
+            f['cube'].append(cube)
+            f['upto'] = upto
+
+    def frames(self):
+        """(iters, cube): the frames recorded since record_frames() or the last frames() call.  iters[n] (int64)
+        are the k of the frames; cube is [n, ceil(height / stride), ceil(width / stride)] float32, the potential
+        normalised exactly like image() (raw U for 4v, (V - min_v) / (max_v - min_v) otherwise), any other
+        variable raw.  Frames lost to a ring overflow show as gaps in iters.  Collective when distributed: the
+        shards' rows are gathered in rank order."""
+        f = self.__dict__.get('_frames')
+        if f is None:
+            raise AssertionError('frames() needs record_frames() first')
+        rows, cols = self._ctx.frames_shape()
+        while True:
+            iters, cube = self._ctx.frames_fetch(self.FRAME_BATCH)
+            f['iters'].append(iters)
+            f['cube'].append(cube)
+            if len(iters) < self.FRAME_BATCH:
+                break
+        iters = np.concatenate(f['iters']).astype(np.int64)
+        cube = np.concatenate(f['cube']) if f['cube'] else np.empty((0, rows, cols), np.float32)
+        f['iters'], f['cube'] = [], []
+        f['upto'] = 0 if f['k'] < f['first'] else (f['k'] - f['first']) // f['every'] + 1
+        if self._nranks > 1:
+            import torch.distributed as dist
+            parts = [None] * self._nranks
+            dist.all_gather_object(parts, cube)
+            cube = np.concatenate(parts, axis=1)
+        if f['name'] == self._pot_name and self.MODEL_ID != _capi.FENTON4V:
+            cube = self._normalise(cube)
+        return iters, cube
+
+    def stop_frames(self):
+        """Disarms the frame recorder and frees its ring; frames not yet returned by frames() are dropped."""
+        self._ctx.frames_stop()
+        self._frames = None
 
     def nonfinite_cells(self):
         """{variable: count} of NaN/Inf cells in this shard (empty dict when the state is healthy):

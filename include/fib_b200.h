@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define FIB_ABI_VERSION 3
+#define FIB_ABI_VERSION 4
 
 typedef struct fib_ctx fib_ctx;
 
@@ -259,6 +259,33 @@ typedef enum {
 int fib_activation_watch(fib_ctx *ctx, float up, float down);
 int fib_activation_stop(fib_ctx *ctx);
 int fib_activation_get(fib_ctx *ctx, int map, float *host, size_t n);
+
+/* frame recorder (SURVEY 8f2): a strided movie of one state plane, recorded on the device while stepping into
+ * a ring in device memory and fetched in batches -- the cube.npy of fenton.py:179-187 / br.py without a full
+ * plane crossing to the host per frame and without cutting the persistent kernel's 64-iteration batches.
+ *   which    k counts as for the activation maps: k = 0 is the plane when fib_frames_watch is called, k >= 1
+ *            the plane at the end of the k-th FIB_OP_ODE iteration enqueued since, taken before anything the
+ *            caller does between iterations.  FIB_OP_SLOW records nothing.  A frame is recorded at
+ *            k = first + j * every, j = 0, 1, ...  (the reference's cadence is first = 1, every = 10: run()
+ *            yields i after iteration i + 1 and the drivers grab at i % 10 == 0).
+ *   frame    plane `var` (any state variable) at the cells whose GLOBAL row and column are both multiples of
+ *            `stride`, dense and row-major: fib_frames_shape rows x ceil(width / stride) columns per shard.
+ *            The rows are global multiples, so the shards' frames concatenated in rank order are the global
+ *            frame.  Exact copies: a frame equals fib_get_state(var)[::stride, ::stride] at its k, bit for bit.
+ *   storage  a ring of `capacity` frames in device memory, written by a gather kernel after a recording
+ *            iteration (or by the persistent kernel itself); nothing is added to the iteration graphs.
+ *   fetch    fib_frames_fetch copies the oldest unfetched frames, at most `max`, to `host` (max frames) with
+ *            their k in `iters`, and returns their number in *n.  It waits only for the launch that produced
+ *            the last frame it returns.  More than `capacity` unfetched frames: the oldest are lost, which
+ *            shows as a gap in `iters`.
+ * fib_frames_watch arms the recorder, or re-arms it: the ring is reset and k = 0 re-taken if first == 0.
+ * FIB_E_ARG for every, stride or capacity < 1, first < 0 or an unknown var; FIB_E_CUDA if the ring cannot be
+ * allocated.  fib_frames_stop disarms it and frees the ring.  fib_frames_shape / fib_frames_fetch: FIB_E_STATE
+ * without a watch.  An armed recorder keeps fib_set_rect_async blocks out of the pipelined upload. */
+int fib_frames_watch(fib_ctx *ctx, int var, int first, int every, int stride, int capacity);
+int fib_frames_stop(fib_ctx *ctx);
+int fib_frames_shape(const fib_ctx *ctx, int *rows, int *cols);
+int fib_frames_fetch(fib_ctx *ctx, float *host, uint64_t *iters, size_t max, size_t *n);
 
 /* ---- op-level entry points of IonicModel's helpers on dense host planes [h][w] (eager; used by the
  * drop-in IonicModel.enforce_boundary / laplace / phase_field / rush_larsen and by the parity tests that
