@@ -102,7 +102,40 @@ static const char* kCourtVars[] = {"V", "_Na_i_", "_m_", "_h_", "_j_", "_K_i_", 
                                    "_ua_", "_ui_", "_xr_", "_xs_", "_Ca_i_", "_d_", "_f_", "_f_Ca_",
                                    "_Ca_rel_", "_u_", "_v_", "_w_", "_Ca_up_", "_us_"};
 
-struct GraphKey { int op, cur; cudaGraphExec_t exec; };
+// one captured iteration of `op`: a replay launches `launches` kernels and moves the state from `cur` to `cur_end`
+struct GraphKey { int op, cur, cur_end; uint64_t launches; cudaGraphExec_t exec; };
+
+// "The records up to total[k] were produced by the work enqueued before event ev[k]": a fetch of older records
+// waits for the covering event only, not for the launches queued behind it.
+template <int N>
+struct Ledger {
+  cudaEvent_t ev[N] = {};
+  unsigned long long total[N] = {};
+  int next = 0;
+  int create() {
+    for (auto& e : ev)
+      if (!e) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    return 0;
+  }
+  void destroy() {
+    for (auto& e : ev)
+      if (e) cudaEventDestroy(e);
+  }
+  int mark(cudaStream_t st, unsigned long long t) {
+    CU(cudaEventRecord(ev[next], st));
+    total[next] = t;
+    next = (next + 1) % N;
+    return 0;
+  }
+  void clear() { for (auto& t : total) t = 0; }
+  // the earliest mark that covers the records up to `need`, among those not past `upto`; -1 if there is none
+  int covering(unsigned long long need, unsigned long long upto) const {
+    int best = -1;
+    for (int k = 0; k < N; ++k)
+      if (total[k] >= need && total[k] <= upto && (best < 0 || total[k] < total[best])) best = k;
+    return best;
+  }
+};
 
 struct fib_ctx {
   fib_config cfg;
@@ -132,41 +165,36 @@ struct fib_ctx {
   uint64_t launches = 0;
   std::vector<GraphKey> graphs;
   double* red = nullptr;              // 2 doubles for reductions
+  // ODE iterations enqueued on this context: each observer below counts its own from the value at its arming
+  unsigned long long ode_iters = 0;
+  unsigned long long since(unsigned long long armed_at) const { return ode_iters - armed_at; }
   // device-side cycle-length probe (fib_probe_watch): one watched cell, a ring of recorded values
   float* ring = nullptr;              // page-locked, device-visible: a fetch is a stream sync + host reads
   unsigned long long* ring_count = nullptr;   // device: the slot the next record goes to
-  unsigned long long ring_total = 0;  // host mirror of *ring_count once the stream has drained
+  unsigned long long probe_armed_at = 0;      // records made = since(probe_armed_at)
   unsigned long long ring_fetched = 0;
-  // the last few persistent launches that recorded probes: {event after the launch, ring_total after it};
-  // a fetch of older values waits for the covering event only, not for the launches queued behind it
-  static constexpr int kRingEvents = 4;
-  cudaEvent_t ring_ev[kRingEvents] = {nullptr, nullptr, nullptr, nullptr};
-  unsigned long long ring_ev_total[kRingEvents] = {0, 0, 0, 0};
-  int ring_ev_next = 0;
+  Ledger<4> probe_ledger;             // marked after the last few persistent launches (which record in-kernel)
   int watch_var = -1, watch_row = -1, watch_col = -1;
   // activation maps (fib_activation_watch, fib_activation.cuh): armed iff act_maps != nullptr
   float* act_prev = nullptr;          // the last sample of the diffusing variable, [rows][pitch]
   float* act_maps = nullptr;          // kActMaps planes [rows][pitch]
   unsigned long long* act_iter = nullptr;   // device: samples taken since arming (= k - 1 of the next one)
-  unsigned long long act_n = 0;       // host mirror of *act_iter (iterations enqueued since arming)
+  unsigned long long act_armed_at = 0;      // *act_iter = since(act_armed_at) once the stream has drained
   float act_up = 0.f, act_down = 0.f;
   // frame recorder (fib_frames_watch): armed iff frames != nullptr.  Frame j is the plane at k = fr_first +
   // j * fr_every and lives in slot j % fr_cap; the host knows k, so only recording iterations launch anything.
   float* frames = nullptr;            // [fr_cap][fr_rows][fr_cols]
   int fr_var = 0, fr_first = 0, fr_every = 1, fr_stride = 1, fr_cap = 0;
   int fr_rows = 0, fr_cols = 0, fr_lr0 = 0;   // this shard's frame; fr_lr0 = local row of its first row
-  unsigned long long fr_k = 0;        // ODE iterations enqueued since arming
+  unsigned long long fr_armed_at = 0; // k = since(fr_armed_at)
   unsigned long long fr_fetched = 0;  // frames handed out (or lost to overflow)
-  // {event after a launch that recorded frames, frames recorded up to it}: a fetch waits for the covering one
-  static constexpr int kFrameEvents = 256;
-  cudaEvent_t fr_ev[kFrameEvents] = {};
-  unsigned long long fr_ev_total[kFrameEvents] = {};
-  int fr_ev_next = 0;
+  Ledger<256> frame_ledger;           // marked after every launch that records frames
   size_t frame_floats() const { return (size_t)fr_rows * fr_cols; }
   // frames recorded once k iterations have run
   unsigned long long frames_upto(unsigned long long k) const {
     return k < (unsigned long long)fr_first ? 0 : (k - fr_first) / fr_every + 1;
   }
+  unsigned long long frames_recorded() const { return frames_upto(since(fr_armed_at)); }
   float* weights[4] = {nullptr, nullptr, nullptr, nullptr};   // user masks, halo layout like phase
   // persistent on-chip kernel (fib_persist.cuh): small unsharded 4v / BR grids
   int persist = -1;                   // -1 not decided yet, 0 no, 1 yes
@@ -200,7 +228,13 @@ struct fib_ctx {
   size_t fused_floats() const { return (size_t)(g.rows + 2 * kFuseHalo) * g.pitch; }
   bool top_is_border() const { return g.row0 == 0; }
   bool bottom_is_border() const { return g.row0 + g.rows == g.H; }
+  bool observing() const { return watch_var >= 0 || act_maps || frames; }
 };
+
+static void drop_graphs(fib_ctx* c) {
+  for (auto& gk : c->graphs) cudaGraphExecDestroy(gk.exec);
+  c->graphs.clear();
+}
 
 static int check_persist_error(fib_ctx* c);
 
@@ -570,15 +604,13 @@ extern "C" int fib_destroy(fib_ctx* c) {
   cudaFree(c->lut_t);
   cudaFree(c->red);
   cudaFreeHost(c->ring);
-  for (auto& e : c->ring_ev)
-    if (e) cudaEventDestroy(e);
+  c->probe_ledger.destroy();
   cudaFree(c->ring_count);
   cudaFree(c->act_prev);
   cudaFree(c->act_maps);
   cudaFree(c->act_iter);
   cudaFree(c->frames);
-  for (auto& e : c->fr_ev)
-    if (e) cudaEventDestroy(e);
+  c->frame_ledger.destroy();
   cudaFree(c->pmail);
   if (c->perr) cudaFreeHost(c->perr);
   for (int k = 0; k < 4; ++k) cudaFree(c->weights[k]);
@@ -615,9 +647,6 @@ static float* owned_rows(fib_ctx* c, int var) {
   const PlaneRef p = plane_of(c, var);
   return p.base + (size_t)p.halo * c->g.pitch;
 }
-__global__ void probe_update_kernel(const float* __restrict__ src, float* __restrict__ ring,
-                                    const unsigned long long* __restrict__ count);
-static PlaneRef plane_of(fib_ctx* c, int var);
 // a host write into `var` invalidates the neighbours' copies of the rows they hold as halo, and
 // the last value the cycle-length probe recorded if it watches this plane (enqueue-only)
 static void mark_written(fib_ctx* c, int var) {
@@ -627,7 +656,7 @@ static void mark_written(fib_ctx* c, int var) {
     const float* src = p.base + (size_t)(p.halo + c->watch_row - c->g.row0) * c->g.pitch + c->watch_col;
     probe_update_kernel<<<1, 1, 0, c->stream>>>(src, c->ring, c->ring_count);
     c->launches++;
-    for (auto& t : c->ring_ev_total) t = 0;     // a recorded value changes after its launch's event
+    c->probe_ledger.clear();                    // a recorded value changes after its launch's event
   }
 }
 // a halo exchange still running on the side stream must land before anything else touches the
@@ -737,9 +766,7 @@ static int ensure_ring(fib_ctx* c) {
     CU(cudaHostAlloc(&c->ring, FIB_PROBE_RING * sizeof(float), cudaHostAllocMapped | cudaHostAllocPortable));
     CU(cudaMalloc(&c->ring_count, sizeof(unsigned long long)));
   }
-  for (int k = 0; k < fib_ctx::kRingEvents; ++k)
-    if (!c->ring_ev[k]) CU(cudaEventCreateWithFlags(&c->ring_ev[k], cudaEventDisableTiming));
-  return 0;
+  return c->probe_ledger.create();
 }
 
 static int launch_substep(fib_ctx* c, int op, int sub, int lr0, int nrows);
@@ -782,7 +809,7 @@ static int set_rect_impl(fib_ctx* c, int var, int r0, int r1, int c0, int c1, co
     // On an NCCL shard the block order may also run bottom to top (odd ranks do, so that both shards of a seam
     // either begin or end there: fib_step_behind_upload).
     const bool eligible = (c->comm ? c->pipeline_nccl : c->g.rows == c->g.H) && c0 == 0 && c1 == c->g.W &&
-                          c->watch_var < 0 && !c->act_maps && !c->frames && (long long)c->g.rows * c->g.W >= c->pipeline_min_cells;
+                          !c->observing() && (long long)c->g.rows * c->g.W >= c->pipeline_min_cells;
     const int row_end = c->g.row0 + c->g.rows;
     const int dir = c->up_session ? c->up_dir : (r0 == c->g.row0 ? +1 : (r1 == row_end && c->comm ? -1 : 0));
     const int dlo = dir > 0 ? r0 - c->g.row0 : row_end - r1, dhi = dir > 0 ? r1 - c->g.row0 : row_end - r0;
@@ -841,8 +868,7 @@ extern "C" int fib_set_phase(fib_ctx* c, const float* rows_host, int first_row, 
   DevGuard dg(c->cfg.device);
   FLUSH(c);
   CU(cudaStreamSynchronize(c->stream));
-  for (auto& gk : c->graphs) cudaGraphExecDestroy(gk.exec);   // graphs bake the phase pointer in
-  c->graphs.clear();
+  drop_graphs(c);                       // graphs bake the phase pointer in
   if (!rows_host) {
     CU(cudaFree(c->phase));
     CU(cudaFree(c->pmask));
@@ -911,8 +937,7 @@ extern "C" int fib_set_table(fib_ctx* c, int table, const float* data, size_t n)
     CU(cudaStreamSynchronize(c->stream));
     memcpy(c->cheb, data, sizeof c->cheb);
     c->have_cheb = true;
-    for (auto& gk : c->graphs) cudaGraphExecDestroy(gk.exec);
-    c->graphs.clear();
+    drop_graphs(c);
     return 0;
   }
   if (table == FIB_TABLE_COURT_LUT) {
@@ -1029,10 +1054,54 @@ static cudaError_t launch_court(fib_ctx* c, int lr0, int nrows) {
   return launch_step<M>(c->g, a, c->stream, c->sms);
 }
 
+// The tables the model's flags ask for have been set: checked before any step launch, and by fib_step before it
+// defers iterations (so that the error reaches the caller that asked for them).
+static int check_tables(const fib_ctx* c) {
+  const uint32_t fl = c->cfg.flags;
+  if (c->cfg.model == FIB_BR && (fl & FIB_F_CHEBY) && !c->have_cheb)
+    return fail(FIB_E_STATE, "cheby=True but FIB_TABLE_BR_CHEBY has not been set");
+  if (c->cfg.model >= FIB_COURT && (fl & FIB_F_LUT) && !c->have_lut)
+    return fail(FIB_E_STATE, "lut=True but no table was set/built");
+  return 0;
+}
+
+static Fenton4v::Params fenton_params(const fib_ctx* c) {
+  return {(float)c->cfg.dt, (float)(c->cfg.diff * c->cfg.dt)};     // dt, ddt
+}
+
+// A Beeler-Reuter time step that advances the slow gates by n * dt (n = 0: they stay frozen), br.py:96-107.
+template <class P>
+static P br_params(const fib_ctx* c, int n) {
+  const double dt = c->cfg.dt;
+  const bool strict = (c->cfg.flags & FIB_F_CHEBY) && (c->cfg.flags & FIB_F_CHEBY_STRICT);
+  P p;
+  p.dt = (float)dt;
+  p.neg_dt = (float)(-dt);
+  p.neg_dt_slow = (float)(-(dt * n));
+  p.ddt = (float)(c->cfg.diff * dt);
+  // S_i = 2^(i-1) x^i (br.py:289-301): hand the kernel plain monomial coefficients (the strict
+  // flavour evaluates the S-basis sum itself and takes the table as it is)
+  for (int g = 0; g < 12; ++g)
+    for (int i = 0; i < 9; ++i)
+      p.poly[g][i] = (i < 2 || strict) ? c->cheb[g][i] : ldexpf(c->cheb[g][i], i - 1);
+  return p;
+}
+
+// fn(slow, fast): the Beeler-Reuter model types of the flavour the flags select (strict Chebyshev, Chebyshev or
+// exact gates), for a time step that advances the slow gates and for one that freezes them
+template <class F>
+static cudaError_t with_br_flavour(const fib_ctx* c, F&& fn) {
+  const uint32_t fl = c->cfg.flags;
+  if (!(fl & FIB_F_CHEBY)) return fn(BeelerReuter<0, true>(), BeelerReuter<0, false>());
+  if (fl & FIB_F_CHEBY_STRICT) return fn(BeelerReuter<2, true>(), BeelerReuter<2, false>());
+  return fn(BeelerReuter<1, true>(), BeelerReuter<1, false>());
+}
+
 // One time step `sub` of op over local rows [lr0, lr0+nrows).  Does NOT flip the ping-pong.
 static int launch_substep(fib_ctx* c, int op, int sub, int lr0, int nrows) {
   if (nrows <= 0) return 0;
-  const double dt = c->cfg.dt;
+  const int tr = check_tables(c);
+  if (tr) return tr;
   const uint32_t fl = c->cfg.flags;
   cudaError_t e = cudaSuccess;
   switch (c->cfg.model) {
@@ -1046,48 +1115,31 @@ static int launch_substep(fib_ctx* c, int op, int sub, int lr0, int nrows) {
         f.lr0 = lr0;
         f.nrows = nrows;
         f.R = 0;
-        f.p.dt = (float)dt;
-        f.p.ddt = (float)(c->cfg.diff * dt);
+        f.p = fenton_params(c);
         e = launch_fused2(c->g, f, c->stream, c->sms);
         break;
       }
       StepArgs<Fenton4v> a;
       fill_common<Fenton4v>(c, a, lr0, nrows);
-      a.p.dt = (float)dt;
-      a.p.ddt = (float)(c->cfg.diff * dt);
+      a.p = fenton_params(c);
       e = launch_step<Fenton4v>(c->g, a, c->stream, c->sms);
       break;
     }
     case FIB_BR: {
       // br.py:96-107: skip -> solve(n=5) then 4x solve(n=0); else 5x solve(n=1)
       const int n = (fl & FIB_F_SKIP) ? (sub == 0 ? 5 : 0) : 1;
-      const bool cheby = fl & FIB_F_CHEBY;
-      const bool strict = cheby && (fl & FIB_F_CHEBY_STRICT);
-      if (cheby && !c->have_cheb)
-        return fail(FIB_E_STATE, "cheby=True but FIB_TABLE_BR_CHEBY has not been set");
       auto go = [&](auto tag) {
         using M = decltype(tag);
         StepArgs<M> a;
         fill_common<M>(c, a, lr0, nrows);
-        a.p.dt = (float)dt;
-        a.p.neg_dt = (float)(-dt);
-        a.p.neg_dt_slow = (float)(-(dt * n));
-        a.p.ddt = (float)(c->cfg.diff * dt);
-        // S_i = 2^(i-1) x^i (br.py:289-301): hand the kernel plain monomial coefficients (the strict
-        // flavour evaluates the S-basis sum itself and takes the table as it is)
-        for (int g = 0; g < 12; ++g)
-          for (int i = 0; i < 9; ++i)
-            a.p.poly[g][i] = (i < 2 || strict) ? c->cheb[g][i] : ldexpf(c->cheb[g][i], i - 1);
+        a.p = br_params<typename M::Params>(c, n);
         return launch_step<M>(c->g, a, c->stream, c->sms);
       };
-      if (strict)     e = n > 0 ? go(BeelerReuter<2, true>()) : go(BeelerReuter<2, false>());
-      else if (cheby) e = n > 0 ? go(BeelerReuter<1, true>()) : go(BeelerReuter<1, false>());
-      else            e = n > 0 ? go(BeelerReuter<0, true>()) : go(BeelerReuter<0, false>());
+      e = with_br_flavour(c, [&](auto slow, auto fast) { return n > 0 ? go(slow) : go(fast); });
       break;
     }
     case FIB_COURT: {
       const bool lut = fl & FIB_F_LUT;
-      if (lut && !c->have_lut) return fail(FIB_E_STATE, "lut=True but no table was set/built");
       if (op == FIB_OP_ODE) e = lut ? launch_court<COURT_FAST, true, false>(c, lr0, nrows)
                                     : launch_court<COURT_FAST, false, false>(c, lr0, nrows);
       else                  e = lut ? launch_court<COURT_SLOW, true, false>(c, lr0, nrows)
@@ -1096,7 +1148,6 @@ static int launch_substep(fib_ctx* c, int op, int sub, int lr0, int nrows) {
     }
     default: {
       const bool lut = fl & FIB_F_LUT, us = fl & FIB_F_ULTRA_SLOW;
-      if (lut && !c->have_lut) return fail(FIB_E_STATE, "lut=True but no table was set/built");
       if (us) e = lut ? launch_court<COURT_ALL, true, true>(c, lr0, nrows)
                       : launch_court<COURT_ALL, false, true>(c, lr0, nrows);
       else    e = lut ? launch_court<COURT_ALL, true, false>(c, lr0, nrows)
@@ -1234,13 +1285,13 @@ static cudaError_t launch_persist_m(fib_ctx* c, PersistArgs<MS, MF>& a, int iter
   a.act_maps = c->act_maps;
   a.act_plane = c->plane_floats();
   a.act_iter = c->act_iter;
-  a.act_k0 = c->act_n;
+  a.act_k0 = c->since(c->act_armed_at);
   a.act_up = c->act_up;
   a.act_down = c->act_down;
-  // frames: the first recording iteration of this launch (k = fr_k + 1 + it0), if there is one
+  // frames: the first recording iteration of this launch (k = k1 + it0), if there is one
   a.frames = nullptr;
   if (c->frames) {
-    const unsigned long long k1 = c->fr_k + 1, f0 = c->fr_first, ev = c->fr_every;
+    const unsigned long long k1 = c->since(c->fr_armed_at) + 1, f0 = c->fr_first, ev = c->fr_every;
     const unsigned long long kf = k1 <= f0 ? f0 : f0 + (k1 - f0 + ev - 1) / ev * ev;
     if (kf < k1 + (unsigned)iters) {
       a.frames = c->frames;
@@ -1312,16 +1363,12 @@ static void decide_persist(fib_ctx* c) {
   c->persist = 1;
 }
 
-// fib_frames_watch: marks everything enqueued so far as the producer of the frames recorded so far
-static int record_frame_event(fib_ctx* c) {
-  const int k = c->fr_ev_next;
-  CU(cudaEventRecord(c->fr_ev[k], c->stream));
-  c->fr_ev_total[k] = c->frames_upto(c->fr_k);
-  c->fr_ev_next = (k + 1) % fib_ctx::kFrameEvents;
-  return 0;
-}
-
-// frame j of the current plane into its ring slot
+// ------------------------------------------------------------------------------------------
+// observers: the probe ring, the activation maps and the frame recorder sample the state at the end of every ODE
+// iteration.  Every stepping route calls the two halves of one hook: record_observers inside the iteration (the
+// graphs capture it) and end_iterations on the host once the route has enqueued iterations.
+// ------------------------------------------------------------------------------------------
+// frame j of the current plane into its ring slot, and a ledger mark behind it
 static int launch_frame(fib_ctx* c, unsigned long long j) {
   if (c->fr_rows > 0) {
     const float* src = owned_rows(c, c->fr_var) + (size_t)c->fr_lr0 * c->g.pitch;
@@ -1332,74 +1379,87 @@ static int launch_frame(fib_ctx* c, unsigned long long j) {
     CU(cudaGetLastError());
     c->launches++;
   }
-  return record_frame_event(c);
+  return c->frame_ledger.mark(c->stream, c->frames_recorded());
+}
+
+// Local rows [lo, hi) of the CURRENT buffers have finished an ODE iteration: the probe records its cell if it lies
+// there.  The upload session finishes iterations in row blocks; only the probe can be armed while it is open.
+static int observe_rows(fib_ctx* c, int lo, int hi) {
+  const int lr = c->watch_row - c->g.row0;
+  if (c->watch_var < 0 || lr < lo || lr >= hi) return 0;
+  const float* src = owned_rows(c, c->watch_var) + (size_t)lr * c->g.pitch + c->watch_col;
+  probe_record_kernel<<<1, 1, 0, c->stream>>>(src, c->ring, c->ring_count);
+  CU(cudaGetLastError());
+  c->launches++;
+  return 0;
+}
+
+// The graph-capturable half of the hook, after an iteration of `op` on the CURRENT buffers: the activation update
+// and the advance of its device iteration index, then the probe record.
+static int record_observers(fib_ctx* c, int op) {
+  if (op != FIB_OP_ODE) return 0;
+  if (c->act_maps) {
+    const size_t n4 = c->plane_floats() / 4;
+    const int grid = (int)min((n4 + 255) / 256, (size_t)c->sms * 32);
+    activation_update_kernel<<<grid, 256, 0, c->stream>>>(reinterpret_cast<const float4*>(owned_rows(c, 0)),
+                                                          reinterpret_cast<float4*>(c->act_prev), c->act_maps, n4,
+                                                          c->plane_floats(), c->act_iter, c->act_up, c->act_down);
+    activation_advance_kernel<<<1, 1, 0, c->stream>>>(c->act_iter);
+    CU(cudaGetLastError());
+    c->launches += 2;
+  }
+  return observe_rows(c, 0, c->g.rows);
+}
+
+// The host half of the hook: the route has enqueued `n` iterations of `op`, after their record_observers nodes or,
+// `persistent`, as one persistent launch that recorded its probe values and frames itself.  Counts them; gathers
+// the frame of a recording iteration (the other routes end one iteration at a time; no recorder is armed behind
+// an upload) or marks the frame ledger behind the launch; marks the probe ledger behind a persistent launch.
+static int end_iterations(fib_ctx* c, int op, int n, bool persistent = false) {
+  if (op != FIB_OP_ODE) return 0;
+  const unsigned long long frames0 = c->frames_recorded();
+  c->ode_iters += (unsigned)n;
+  int r = 0;
+  if (c->frames && c->frames_recorded() != frames0)
+    r = persistent ? c->frame_ledger.mark(c->stream, c->frames_recorded()) : launch_frame(c, c->frames_recorded() - 1);
+  if (!r && persistent && c->watch_var >= 0) r = c->probe_ledger.mark(c->stream, c->since(c->probe_armed_at));
+  return r;
 }
 
 // `iters` ODE iterations (dt_per_step time steps each) as ONE launch
 static int run_iteration_persist(fib_ctx* c, int iters) {
-  const double dt = c->cfg.dt;
-  const uint32_t fl = c->cfg.flags;
+  const int tr = check_tables(c);
+  if (tr) return tr;
   cudaError_t e;
   if (c->cfg.model == FIB_FENTON4V) {
     PersistArgs<Fenton4v, Fenton4v> a;
     a.slow_first_only = 0;
-    a.ps.dt = a.pf.dt = (float)dt;
-    a.ps.ddt = a.pf.ddt = (float)(c->cfg.diff * dt);
+    a.ps = a.pf = fenton_params(c);
     e = launch_persist_m<Fenton4v, Fenton4v>(c, a, iters);
   } else {
-    const bool cheby = fl & FIB_F_CHEBY, strict = cheby && (fl & FIB_F_CHEBY_STRICT), skip = fl & FIB_F_SKIP;
-    if (cheby && !c->have_cheb) return fail(FIB_E_STATE, "cheby=True but FIB_TABLE_BR_CHEBY has not been set");
-    auto go = [&](auto ts, auto tf) {
-      using MS = decltype(ts);
-      using MF = decltype(tf);
+    const bool skip = c->cfg.flags & FIB_F_SKIP;
+    e = with_br_flavour(c, [&](auto slow, auto fast) {
+      using MS = decltype(slow);
+      using MF = decltype(fast);
       PersistArgs<MS, MF> a;
       a.slow_first_only = skip ? 1 : 0;                                               // br.py:96-107
-      auto fill = [&](auto& p, int n) {
-        p.dt = (float)dt;
-        p.neg_dt = (float)(-dt);
-        p.neg_dt_slow = (float)(-(dt * n));
-        p.ddt = (float)(c->cfg.diff * dt);
-        for (int g = 0; g < 12; ++g)
-          for (int i = 0; i < 9; ++i)
-            p.poly[g][i] = (i < 2 || strict) ? c->cheb[g][i] : ldexpf(c->cheb[g][i], i - 1);
-      };
-      fill(a.ps, skip ? 5 : 1);
-      fill(a.pf, 0);
+      a.ps = br_params<typename MS::Params>(c, skip ? 5 : 1);
+      a.pf = br_params<typename MF::Params>(c, 0);
       return launch_persist_m<MS, MF>(c, a, iters);
-    };
-    if (strict)     e = go(BeelerReuter<2, true>(), BeelerReuter<2, false>());
-    else if (cheby) e = go(BeelerReuter<1, true>(), BeelerReuter<1, false>());
-    else            e = go(BeelerReuter<0, true>(), BeelerReuter<0, false>());
+    });
   }
   if (e != cudaSuccess) {
     // e.g. the tiles cannot all be resident (another context holds SMs): never a partial launch.
     // Fall back to one launch per step for the rest of this context's life.
     cudaGetLastError();
     c->persist = 0;
-    return 1;           // caller retries on the plain path
+    return 1;           // caller retries on the plain path; these iterations were not counted
   }
   c->launches++;
-  if (c->act_maps) c->act_n += (unsigned)iters;
-  if (c->frames) {
-    const unsigned long long before = c->frames_upto(c->fr_k);
-    c->fr_k += (unsigned)iters;
-    if (c->frames_upto(c->fr_k) != before) {
-      const int r = record_frame_event(c);
-      if (r) return r;
-    }
-  }
-  if (c->watch_var >= 0) {
-    c->ring_total += (unsigned)iters;
-    const int k = c->ring_ev_next;
-    if (c->ring_ev[k] && cudaEventRecord(c->ring_ev[k], c->stream) == cudaSuccess) {
-      c->ring_ev_total[k] = c->ring_total;
-      c->ring_ev_next = (k + 1) % fib_ctx::kRingEvents;
-    }
-  }
   const int ns = substeps_of(c, FIB_OP_ODE) * iters;
   c->pbase += (unsigned)ns;
   if (ns & 1) c->cur ^= 1;
-  return 0;
+  return end_iterations(c, FIB_OP_ODE, iters, true);
 }
 
 static int check_persist_error(fib_ctx* c) {
@@ -1411,57 +1471,15 @@ static int check_persist_error(fib_ctx* c) {
   return 0;
 }
 
-// fib_probe_watch: after an ODE iteration, append the watched cell of the CURRENT buffers to the ring
-static int record_probe(fib_ctx* c, int op) {
-  if (c->watch_var < 0 || op != FIB_OP_ODE) return 0;
-  const float* src = owned_rows(c, c->watch_var) + (size_t)(c->watch_row - c->g.row0) * c->g.pitch + c->watch_col;
-  probe_record_kernel<<<1, 1, 0, c->stream>>>(src, c->ring, c->ring_count);
-  CU(cudaGetLastError());
-  c->launches++;
-  c->ring_total++;
-  return 0;
-}
-
-// fib_activation_watch: after an ODE iteration, sample the diffusing variable of the CURRENT buffers into
-// the maps, then advance the iteration index (two nodes of the iteration graph)
-static int record_activation(fib_ctx* c, int op) {
-  if (!c->act_maps || op != FIB_OP_ODE) return 0;
-  const size_t n4 = c->plane_floats() / 4;
-  const int grid = (int)min((n4 + 255) / 256, (size_t)c->sms * 32);
-  activation_update_kernel<<<grid, 256, 0, c->stream>>>(reinterpret_cast<const float4*>(owned_rows(c, 0)),
-                                                        reinterpret_cast<float4*>(c->act_prev), c->act_maps, n4,
-                                                        c->plane_floats(), c->act_iter, c->act_up, c->act_down);
-  activation_advance_kernel<<<1, 1, 0, c->stream>>>(c->act_iter);
-  CU(cudaGetLastError());
-  c->launches += 2;
-  c->act_n++;
-  return 0;
-}
-
-// fib_frames_watch: after an ODE iteration, count it and gather a frame if it is a recording one.  Never part
-// of an iteration graph: the graph path calls it after each replay.
-static int record_frame(fib_ctx* c, int op) {
-  if (!c->frames || op != FIB_OP_ODE) return 0;
-  const unsigned long long k = ++c->fr_k;
-  if (k < (unsigned long long)c->fr_first || (k - c->fr_first) % c->fr_every) return 0;
-  return launch_frame(c, c->frames_upto(k) - 1);
-}
-
-// the observers that sample the state at the end of an ODE iteration (`frames` = false while capturing a graph)
-static int record_observers(fib_ctx* c, int op, bool frames = true) {
-  int r = record_activation(c, op);
-  if (!r) r = record_probe(c, op);
-  return (r || !frames) ? r : record_frame(c, op);
-}
-
-static int run_iteration_plain(fib_ctx* c, int op, bool frames = true) {
+// one iteration as direct launches: what the iteration graphs capture
+static int run_iteration_plain(fib_ctx* c, int op) {
   const int ns = substeps_of(c, op);
   for (int s = 0; s < ns; s += c->fuse) {
     int r = launch_substep(c, op, s, 0, c->g.rows);
     if (r) return r;
     if (op_writes_x(c, op)) c->cur ^= 1;
   }
-  return record_observers(c, op, frames);
+  return record_observers(c, op);
 }
 
 // boundary rows first, halo exchange on the side stream overlapped with the interior rows
@@ -1514,10 +1532,9 @@ static int refresh_halos_nccl(fib_ctx* c) {
 static int step_now(fib_ctx* c, int op, int n_iter) {
   if (c->comm) {
     int r = refresh_halos_nccl(c);
-    if (r) return r;
-    for (int i = 0; i < n_iter; ++i)
-      if ((r = run_iteration_nccl(c, op))) return r;
-    return 0;
+    for (int i = 0; i < n_iter && !r; ++i)
+      if (!(r = run_iteration_nccl(c, op))) r = end_iterations(c, op, 1);
+    return r;
   }
   if (c->persist == 1 && op == FIB_OP_ODE) {
     // up to kPersistMaxIters iterations per launch (no launch gap, no tile reload between them); a
@@ -1534,44 +1551,39 @@ static int step_now(fib_ctx* c, int op, int n_iter) {
     n_iter -= i;
   }
   if (c->cfg.flags & FIB_F_NO_GRAPH) {
-    for (int i = 0; i < n_iter; ++i) {
-      int r = run_iteration_plain(c, op);
-      if (r) return r;
-    }
-    return 0;
+    int r = 0;
+    for (int i = 0; i < n_iter && !r; ++i)
+      if (!(r = run_iteration_plain(c, op))) r = end_iterations(c, op, 1);
+    return r;
   }
   // CUDA graph of one iteration, cached per (op, ping-pong parity)
   for (int i = 0; i < n_iter; ++i) {
-    cudaGraphExec_t exec = nullptr;
-    for (auto& gk : c->graphs)
-      if (gk.op == op && gk.cur == c->cur) exec = gk.exec;
-    const int cur0 = c->cur;
-    if (!exec) {
+    const GraphKey* gk = nullptr;
+    for (auto& k : c->graphs)
+      if (k.op == op && k.cur == c->cur) gk = &k;
+    if (!gk) {
+      // capture one iteration and measure what it launches and where it leaves the state; nothing runs yet
+      GraphKey k = {op, c->cur, 0, 0, nullptr};
+      const uint64_t l0 = c->launches;
       cudaGraph_t graph = nullptr;
       CU(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-      const uint64_t l0 = c->launches;
-      const unsigned long long rt0 = c->ring_total, an0 = c->act_n;
-      int r = run_iteration_plain(c, op, false);
+      int r = run_iteration_plain(c, op);
       cudaError_t ce = cudaStreamEndCapture(c->stream, &graph);
+      k.cur_end = c->cur;
+      k.launches = c->launches - l0;
       c->launches = l0;
-      c->ring_total = rt0;
-      c->act_n = an0;
-      c->cur = cur0;
+      c->cur = k.cur;
       if (r) { if (graph) cudaGraphDestroy(graph); return r; }
       if (ce != cudaSuccess) return fail(FIB_E_CUDA, "graph capture failed: %s", cudaGetErrorString(ce));
-      CU(cudaGraphInstantiate(&exec, graph, 0));
+      CU(cudaGraphInstantiate(&k.exec, graph, 0));
       CU(cudaGraphDestroy(graph));
-      c->graphs.push_back({op, cur0, exec});
+      c->graphs.push_back(k);
+      gk = &c->graphs.back();
     }
-    CU(cudaGraphLaunch(exec, c->stream));
-    const int nl = substeps_of(c, op) / c->fuse;      // step launches per iteration
-    const int rec = (c->watch_var >= 0 && op == FIB_OP_ODE) ? 1 : 0;
-    const int act = (c->act_maps && op == FIB_OP_ODE) ? 1 : 0;
-    c->launches += nl + rec + 2 * act;
-    c->ring_total += rec;
-    c->act_n += act;
-    if (op_writes_x(c, op) && (nl & 1)) c->cur ^= 1;
-    const int r = record_frame(c, op);
+    CU(cudaGraphLaunch(gk->exec, c->stream));
+    c->launches += gk->launches;
+    c->cur = gk->cur_end;
+    const int r = end_iterations(c, op, 1);
     if (r) return r;
   }
   return 0;
@@ -1637,16 +1649,16 @@ static int finish_upload_session(fib_ctx* c, int n, bool comm_skew = false) {
       r = launch_substep(c, op, (l % nl) * c->fuse, lo, hi - lo);
       if (!r && flips && first && seam_start) r = nccl_exchange(c, c->cur ^ 1, c->stream, side_start);
       if (!r && flips && last && seam_end) r = nccl_exchange(c, c->cur ^ 1, c->stream, side_end);
-      if (!r && (l + 1) % nl == 0 && c->watch_var >= 0 && c->watch_row - c->g.row0 >= lo && c->watch_row - c->g.row0 < hi) {
+      if (!r && (l + 1) % nl == 0) {    // rows [lo, hi) have finished an iteration, in the buffer just written
         if (flips) c->cur ^= 1;
-        r = record_probe(c, op);        // the watched cell's row has finished this iteration
+        r = observe_rows(c, lo, hi);
       }
     }
   }
   c->cur = cur0 ^ ((flips && (L & 1)) ? 1 : 0);
   if (sharded && !r) c->halo_dirty = false;
   release();
-  return r;
+  return r ? r : end_iterations(c, op, n);
 }
 
 static int flush_pending(fib_ctx* c) {
@@ -1675,8 +1687,8 @@ extern "C" int fib_step(fib_ctx* c, int op, int n_iter) {
   }
   if (c->persist == 1 && op == FIB_OP_ODE) {
     // persistent path: count now, launch later (see FLUSH); whatever can fail is checked here
-    if (c->cfg.model == FIB_BR && (c->cfg.flags & FIB_F_CHEBY) && !c->have_cheb)
-      return fail(FIB_E_STATE, "cheby=True but FIB_TABLE_BR_CHEBY has not been set");
+    const int tr = check_tables(c);
+    if (tr) return tr;
     while (n_iter > 0) {
       const int take = min(n_iter, kPersistMaxIters - c->pending);
       c->pending += take;
@@ -1818,7 +1830,7 @@ extern "C" int fib_step_group(fib_ctx** cs, int n, int op, int n_iter) {
     }
     for (int i = 0; i < n; ++i) {
       DevGuard dg(cs[i]->cfg.device);
-      if ((r = record_observers(cs[i], op))) return r;
+      if ((r = record_observers(cs[i], op)) || (r = end_iterations(cs[i], op, 1))) return r;
     }
   }
   return 0;
@@ -1924,11 +1936,6 @@ extern "C" int fib_masked_sum(fib_ctx* c, int var, int slot, double* sum_wx, dou
   return reduce_weighted(c, var, c->weights[slot], sum_wx, sum_w);
 }
 
-static void drop_graphs(fib_ctx* c) {
-  for (auto& gk : c->graphs) cudaGraphExecDestroy(gk.exec);
-  c->graphs.clear();
-}
-
 extern "C" int fib_probe_watch(fib_ctx* c, int var, int row, int col) {
   if (!c) return fail(FIB_E_ARG, "ctx is NULL");
   DevGuard dg(c->cfg.device);
@@ -1948,12 +1955,25 @@ extern "C" int fib_probe_watch(fib_ctx* c, int var, int row, int col) {
   }
   CU(cudaMemsetAsync(c->ring_count, 0, sizeof(unsigned long long), c->stream));
   CU(cudaStreamSynchronize(c->stream));
-  for (int k = 0; k < fib_ctx::kRingEvents; ++k) c->ring_ev_total[k] = 0;
-  c->ring_total = 0;
+  c->probe_ledger.clear();
+  c->probe_armed_at = c->ode_iters;
   c->ring_fetched = 0;
   c->watch_var = var;
   c->watch_row = row;
   c->watch_col = col;
+  return 0;
+}
+
+// records [first, first + n) of a ring of `cap` slots as at most two contiguous pieces: copy(done, slot, len)
+// copies `len` records from `slot` on to position `done` of the output
+template <class Copy>
+static int copy_ring(unsigned long long first, unsigned long long n, unsigned long long cap, Copy&& copy) {
+  for (unsigned long long done = 0; done < n;) {
+    const unsigned long long pos = (first + done) % cap, len = min(cap - pos, n - done);
+    const int r = copy(done, pos, len);
+    if (r) return r;
+    done += len;
+  }
   return 0;
 }
 
@@ -1965,43 +1985,29 @@ extern "C" int fib_probe_fetch(fib_ctx* c, float* out, size_t max, size_t* n) {
   FLUSH(c);
   // The records land in page-locked host memory.  Asked for fewer values than were recorded, wait only
   // for the launch that produced the last of them (the later ones keep the GPU busy meanwhile).
-  unsigned long long count = c->ring_total;
-  if (count - c->ring_fetched > max) {
-    const unsigned long long need = c->ring_fetched + max;
-    int best = -1;
-    for (int k = 0; k < fib_ctx::kRingEvents; ++k)
-      if (c->ring_ev_total[k] >= need && c->ring_ev_total[k] <= c->ring_total &&
-          (best < 0 || c->ring_ev_total[k] < c->ring_ev_total[best]))
-        best = k;
-    if (best >= 0) {
-      CU(cudaEventSynchronize(c->ring_ev[best]));
-      count = c->ring_ev_total[best];
-    } else {
-      CU(cudaStreamSynchronize(c->stream));
-    }
+  const unsigned long long total = c->since(c->probe_armed_at);
+  unsigned long long count = total;
+  const int k = total - c->ring_fetched > max ? c->probe_ledger.covering(c->ring_fetched + max, total) : -1;
+  if (k >= 0) {
+    CU(cudaEventSynchronize(c->probe_ledger.ev[k]));
+    count = c->probe_ledger.total[k];
   } else {
     CU(cudaStreamSynchronize(c->stream));
   }
   unsigned long long first = c->ring_fetched;
   if (count - first > FIB_PROBE_RING) first = count - FIB_PROBE_RING;      // the oldest were overwritten
-  unsigned long long take = count - first;
-  if (take > max) take = max;
-  // at most two contiguous pieces of the ring
-  unsigned long long done = 0;
-  while (done < take) {
-    const unsigned long long pos = (first + done) % FIB_PROBE_RING;
-    unsigned long long len = FIB_PROBE_RING - pos;
-    if (len > take - done) len = take - done;
+  const unsigned long long take = min(count - first, (unsigned long long)max);
+  copy_ring(first, take, FIB_PROBE_RING, [&](unsigned long long done, unsigned long long pos, unsigned long long len) {
     memcpy(out + done, c->ring + pos, len * sizeof(float));
-    done += len;
-  }
+    return 0;
+  });
   c->ring_fetched = first + take;
   *n = (size_t)take;
   return 0;
 }
 
 // Activation maps: the sample s[0] is the current plane; the update runs after every ODE iteration from
-// here on (record_activation, or inside the persistent kernel).  The iteration graphs are rebuilt with or
+// here on (record_observers, or inside the persistent kernel).  The iteration graphs are rebuilt with or
 // without the update nodes.
 extern "C" int fib_activation_watch(fib_ctx* c, float up, float down) {
   if (!c) return fail(FIB_E_ARG, "ctx is NULL");
@@ -2021,7 +2027,7 @@ extern "C" int fib_activation_watch(fib_ctx* c, float up, float down) {
   c->launches++;
   CU(cudaMemsetAsync(c->act_iter, 0, sizeof(unsigned long long), c->stream));
   CU(cudaStreamSynchronize(c->stream));
-  c->act_n = 0;
+  c->act_armed_at = c->ode_iters;
   c->act_up = up;
   c->act_down = down;
   return 0;
@@ -2038,7 +2044,6 @@ extern "C" int fib_activation_stop(fib_ctx* c) {
   CU(cudaFree(c->act_iter));
   c->act_maps = c->act_prev = nullptr;
   c->act_iter = nullptr;
-  c->act_n = 0;
   return check_persist_error(c);
 }
 
@@ -2058,8 +2063,8 @@ extern "C" int fib_activation_get(fib_ctx* c, int map, float* host, size_t n) {
 }
 
 // Frame recorder: a ring of strided frames in device memory.  Nothing joins the iteration graphs: the host
-// counts iterations (fr_k) and gathers a frame after the recording ones (record_frame), or hands the persistent
-// kernel the first recording iteration of its launch (launch_persist_m).
+// counts iterations and gathers a frame after the recording ones (end_iterations), or hands the persistent kernel
+// the first recording iteration of its launch (launch_persist_m).
 extern "C" int fib_frames_watch(fib_ctx* c, int var, int first, int every, int stride, int capacity) {
   if (!c) return fail(FIB_E_ARG, "ctx is NULL");
   if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
@@ -2080,13 +2085,11 @@ extern "C" int fib_frames_watch(fib_ctx* c, int var, int first, int every, int s
   c->fr_every = every;
   c->fr_stride = stride;
   c->fr_cap = capacity;
-  c->fr_k = 0;
+  c->fr_armed_at = c->ode_iters;
   c->fr_fetched = 0;
-  for (int k = 0; k < fib_ctx::kFrameEvents; ++k) {
-    if (!c->fr_ev[k]) CU(cudaEventCreateWithFlags(&c->fr_ev[k], cudaEventDisableTiming));
-    c->fr_ev_total[k] = 0;
-  }
-  c->fr_ev_next = 0;
+  const int er = c->frame_ledger.create();
+  if (er) return er;
+  c->frame_ledger.clear();
   const size_t bytes = max((size_t)capacity * c->frame_floats() * sizeof(float), sizeof(float));
   if (cudaMalloc(&c->frames, bytes) != cudaSuccess) {
     cudaGetLastError();
@@ -2121,39 +2124,34 @@ extern "C" int fib_frames_fetch(fib_ctx* c, float* host, uint64_t* iters, size_t
   DevGuard dg(c->cfg.device);
   // Iterations the persistent path has deferred are launched only when the frames already launched do not
   // satisfy the request: a caller that fetches one batch behind never cuts a batch.
-  unsigned long long total = c->frames_upto(c->fr_k);
+  unsigned long long total = c->frames_recorded();
   if (total - c->fr_fetched < max) {
     FLUSH(c);
-    total = c->frames_upto(c->fr_k);
+    total = c->frames_recorded();
   }
   unsigned long long first = c->fr_fetched;
   if (total - first > (unsigned long long)c->fr_cap) first = total - c->fr_cap;   // overwritten
   const unsigned long long take = min(total - first, (unsigned long long)max);
   if (take) {
     // wait for the earliest launch that covers the last frame taken, not for the launches queued behind it
-    int best = -1;
-    for (int k = 0; k < fib_ctx::kFrameEvents; ++k)
-      if (c->fr_ev_total[k] >= first + take && c->fr_ev_total[k] <= total &&
-          (best < 0 || c->fr_ev_total[k] < c->fr_ev_total[best]))
-        best = k;
-    if (best < 0) {
-      const int r = record_frame_event(c);
+    int k = c->frame_ledger.covering(first + take, total);
+    if (k < 0) {                                 // no mark yet behind the launch that recorded them: one now
+      const int r = c->frame_ledger.mark(c->stream, total);
       if (r) return r;
-      best = (c->fr_ev_next + fib_ctx::kFrameEvents - 1) % fib_ctx::kFrameEvents;
+      k = c->frame_ledger.covering(first + take, total);
     }
-    CU(cudaStreamWaitEvent(c->copy_stream, c->fr_ev[best], 0));
-    // at most two contiguous pieces of the ring (the frames taken cannot be overwritten by work already enqueued:
-    // that only writes frames < total, and first >= total - capacity)
+    CU(cudaStreamWaitEvent(c->copy_stream, c->frame_ledger.ev[k], 0));
+    // the frames taken cannot be overwritten by work already enqueued: that only writes frames < total, and
+    // first >= total - capacity
     const size_t ff = c->frame_floats();
-    unsigned long long done = 0;
-    while (done < take) {
-      const unsigned long long pos = (first + done) % (unsigned long long)c->fr_cap;
-      const unsigned long long len = min((unsigned long long)c->fr_cap - pos, take - done);
+    const int r = copy_ring(first, take, c->fr_cap, [&](unsigned long long done, unsigned long long pos,
+                                                        unsigned long long len) {
       if (ff)
         CU(cudaMemcpyAsync(host + done * ff, c->frames + pos * ff, len * ff * sizeof(float), cudaMemcpyDeviceToHost,
                            c->copy_stream));
-      done += len;
-    }
+      return 0;
+    });
+    if (r) return r;
     CU(cudaStreamSynchronize(c->copy_stream));
     for (unsigned long long i = 0; i < take; ++i) iters[i] = c->fr_first + (first + i) * c->fr_every;
   }
