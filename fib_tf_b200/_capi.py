@@ -19,8 +19,8 @@ F_CHEBY_STRICT, F_NO_PERSIST = 0x80, 0x100
 PROBE_RING = 4096
 OP_ODE, OP_SLOW = 0, 1
 TABLE_BR_CHEBY, TABLE_COURT_LUT = 0, 1
-ACT_FIRST, ACT_LAST, ACT_PREV, ACT_REPOL, ACT_COUNT = 0, 1, 2, 3, 4
-ABI_VERSION = 4
+ACT_FIRST, ACT_LAST, ACT_PREV, ACT_REPOL, ACT_COUNT, ACT_SAMPLE = 0, 1, 2, 3, 4, 16
+ABI_VERSION = 5
 INTER_COLS = 32
 
 # courtemanche.h:105-134 column order (+ the two court_ultra.py:445-450 extras)
@@ -43,6 +43,16 @@ class FibConfig(C.Structure):
         ('flags', C.c_uint32), ('device', C.c_int32),
         ('row0', C.c_int32), ('rows', C.c_int32),
         ('steps_per_launch', C.c_int32), ('reserved', C.c_int32 * 6),
+    ]
+
+
+class CheckpointInfo(C.Structure):
+    _fields_ = [
+        ('struct_size', C.c_uint32), ('nparts', C.c_int32), ('iterations', C.c_uint64),
+        ('act_armed', C.c_int32), ('act_up', C.c_float), ('act_down', C.c_float), ('fr_armed', C.c_int32),
+        ('act_k', C.c_uint64),
+        ('fr_var', C.c_int32), ('fr_first', C.c_int32), ('fr_every', C.c_int32), ('fr_stride', C.c_int32),
+        ('fr_capacity', C.c_int32), ('reserved0', C.c_int32), ('fr_k', C.c_uint64), ('reserved', C.c_int32 * 6),
     ]
 
 
@@ -69,12 +79,18 @@ _SIGNATURES = {
     'fib_probe_watch': (C.c_int, [_P, C.c_int, C.c_int, C.c_int]),
     'fib_probe_fetch': (C.c_int, [_P, _P, C.c_size_t, C.POINTER(C.c_size_t)]),
     'fib_activation_watch': (C.c_int, [_P, C.c_float, C.c_float]),
+    'fib_activation_resume': (C.c_int, [_P, C.c_float, C.c_float, C.c_uint64]),
     'fib_activation_stop': (C.c_int, [_P]),
     'fib_activation_get': (C.c_int, [_P, C.c_int, _P, C.c_size_t]),
+    'fib_activation_set': (C.c_int, [_P, C.c_int, _P, C.c_size_t]),
     'fib_frames_watch': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    'fib_frames_resume': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint64]),
     'fib_frames_stop': (C.c_int, [_P]),
     'fib_frames_shape': (C.c_int, [_P, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     'fib_frames_fetch': (C.c_int, [_P, _P, C.POINTER(C.c_uint64), C.c_size_t, C.POINTER(C.c_size_t)]),
+    'fib_checkpoint_begin': (C.c_int, [_P, C.POINTER(CheckpointInfo)]),
+    'fib_checkpoint_read': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P]),
+    'fib_checkpoint_end': (C.c_int, [_P]),
     'fib_count_below': (C.c_int, [_P, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float,
                                   C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     'fib_op_enforce_boundary': (C.c_int, [C.c_int, _P, C.c_int, C.c_int, _P]),
@@ -176,6 +192,7 @@ class Context:
         h = _P()
         check(L.fib_create(C.byref(cfg), C.byref(h)))
         self._h = h
+        self.model, self.dt, self.diff, self.flags = int(model), float(dt), float(diff), int(flags)
         self.height, self.width = int(height), int(width)
         self.row0 = int(row0) if rows else 0
         self.rows = int(rows) if rows else int(height)
@@ -309,9 +326,25 @@ class Context:
         check(lib().fib_activation_get(self._h, which, out.ctypes.data_as(_P), out.size))
         return out
 
+    def activation_resume(self, up, down, k):
+        """Arm the activation maps with their counter at k and no sample taken (activation_set fills them)."""
+        check(lib().fib_activation_resume(self._h, up, down, int(k)))
+
+    def activation_set(self, which, plane):
+        """Upload map ACT_* (or the last sample, ACT_SAMPLE) of this shard, [rows, W]."""
+        a, p = _f32c(plane)
+        if a.shape != (self.rows, self.width):
+            raise FibError('activation_set: array shape %r != shard shape %r' % (a.shape, (self.rows, self.width)))
+        check(lib().fib_activation_set(self._h, which, p, a.size))
+
     def frames_watch(self, var, first, every, stride, capacity):
         """Arm (or re-arm) the frame recorder: plane `var`[::stride, ::stride] at k = first + j * every."""
         check(lib().fib_frames_watch(self._h, self.var(var), int(first), int(every), int(stride), int(capacity)))
+
+    def frames_resume(self, var, first, every, stride, capacity, k):
+        """Arm the frame recorder with its count at k: frames up to k count as fetched, none is taken now."""
+        check(lib().fib_frames_resume(self._h, self.var(var), int(first), int(every), int(stride), int(capacity),
+                                      int(k)))
 
     def frames_stop(self):
         check(lib().fib_frames_stop(self._h))
@@ -332,6 +365,26 @@ class Context:
         check(lib().fib_frames_fetch(self._h, out.ctypes.data_as(_P), iters.ctypes.data_as(C.POINTER(C.c_uint64)),
                                      max_frames, C.byref(n)))
         return iters[:n.value], out[:n.value]
+
+    def checkpoint_begin(self):
+        """Stage a copy of this shard's state (and armed activation map) behind everything stepped so far and
+        return its info as a dict at once; checkpoint_read() reads it out (from any thread), checkpoint_end()
+        releases it."""
+        info = CheckpointInfo()
+        info.struct_size = C.sizeof(CheckpointInfo)
+        check(lib().fib_checkpoint_begin(self._h, C.byref(info)))
+        return {name: getattr(info, name) for name, _ in CheckpointInfo._fields_
+                if name not in ('struct_size', 'reserved0', 'reserved')}
+
+    def checkpoint_read(self, part, r0, out):
+        """Global rows [r0, r0 + len(out)) of staged part `part` into `out`, a C-contiguous float32 [n, W] array
+        (page-locked is fastest); returns when the copy is done."""
+        if (out.dtype != np.float32 or not out.flags['C_CONTIGUOUS'] or out.ndim != 2 or out.shape[1] != self.width):
+            raise FibError('checkpoint_read: `out` must be a C-contiguous float32 [n, %d] array' % self.width)
+        check(lib().fib_checkpoint_read(self._h, int(part), int(r0), int(r0) + out.shape[0], out.ctypes.data_as(_P)))
+
+    def checkpoint_end(self):
+        check(lib().fib_checkpoint_end(self._h))
 
     def count_below(self, var, sub, div, cutoff, w_min):
         a, b = C.c_uint64(), C.c_uint64()

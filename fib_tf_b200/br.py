@@ -44,14 +44,7 @@ class BeelerReuter(IonicModel):
 
     def define(self, s1=True):
         """Initial state br.py:71-82; S1 = column 1 of V set to 10 mV."""
-        super().define()
-        flags = (_capi.F_CHEBY if self.cheby else 0) | (_capi.F_SKIP if self.skip else 0)
-        # config['cheby_strict'] (optional, default False): evaluate the polynomial gates in the
-        # reference's own fp32 operation order (br.py:215,289-301,327-331) instead of Horner's scheme;
-        # slower, used to show how closely the reference's result is defined (DESIGN.md section 4)
-        if self.cheby and self.__dict__.get('cheby_strict'):
-            flags |= _capi.F_CHEBY_STRICT
-        ctx = self._make_context(flags)
+        ctx = self._create()
         init = {'V': -84.624, 'C': 1e-4, 'M': 0.01, 'H': 0.988, 'J': 0.975, 'D': 0.003,
                 'F': 0.994, 'XI': 0.0001}
         for name, val in init.items():
@@ -59,12 +52,24 @@ class BeelerReuter(IonicModel):
             if s1 and name == 'V':
                 a[:, 1] = 10.0
             ctx.set_state(name, a)
+
+    def _create(self):
+        """The context, table and handles of define(), without the initial state (define() and restore())."""
+        IonicModel.define(self)
+        flags = (_capi.F_CHEBY if self.cheby else 0) | (_capi.F_SKIP if self.skip else 0)
+        # config['cheby_strict'] (optional, default False): evaluate the polynomial gates in the
+        # reference's own fp32 operation order (br.py:215,289-301,327-331) instead of Horner's scheme;
+        # slower, used to show how closely the reference's result is defined (DESIGN.md section 4)
+        if self.cheby and self.__dict__.get('cheby_strict'):
+            flags |= _capi.F_CHEBY_STRICT
+        ctx = self._make_context(flags)
         if self.cheby:
             ctx.set_table(_capi.TABLE_BR_CHEBY, self.chebyshev_table())
         self.dt_per_step = ctx.dt_per_step      # 5 in both schedules (br.py:101,105)
         self._ode_op = _capi.OP_ODE
         self._State = {n: DeviceVar(self, n) for n in ctx.var_names}
         self._V = self._State['V']
+        return ctx
 
     # ---- define()-time NumPy set-up, as in the reference -------------------------------------
     def calc_alpha_beta_np(self):

@@ -63,11 +63,7 @@ class Courtemanche(IonicModel):
     def define(self, s1=True, state=None):
         """Resting state (court.py:57-78) or a saved `state` dict (court.py:49-56, 623-626);
         S1 = columns 0..24 of V set to 20 mV."""
-        IonicModel.define(self)
-        if list(self.fast_states) != ['V', '_Na_i_', '_m_', '_h_']:
-            raise NotImplementedError('the fast/slow split is compiled into the kernels: '
-                                      "fast_states must stay ['V', '_Na_i_', '_m_', '_h_']")
-        ctx = self._make_context(self._flags())
+        ctx = self._create()
         if state is None:
             state = {}
             for name, val in self._initial_names():
@@ -82,6 +78,14 @@ class Courtemanche(IonicModel):
             raise KeyError('state is missing %s' % missing)
         for name in ctx.var_names:
             ctx.set_state(name, state[name])
+
+    def _create(self):
+        """The context, LUT, ops and handles of define(), without the initial state (define() and restore())."""
+        IonicModel.define(self)
+        if list(self.fast_states) != ['V', '_Na_i_', '_m_', '_h_']:
+            raise NotImplementedError('the fast/slow split is compiled into the kernels: '
+                                      "fast_states must stay ['V', '_Na_i_', '_m_', '_h_']")
+        ctx = self._make_context(self._flags())
         if self.__dict__.get('lut'):
             ctx.build_lut()
         self.dt_per_step = 1
@@ -91,6 +95,7 @@ class Courtemanche(IonicModel):
         self._State = {n: DeviceVar(self, n) for n in ctx.var_names}
         self._V = self._State['V']
         self._Trend = _HostValue(2)
+        return ctx
 
     def _update_trend(self):
         """court.py:107-112: Trend := (V, _Na_i_) at [width//2, 20] (row index from `width`)."""

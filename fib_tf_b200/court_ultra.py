@@ -36,10 +36,11 @@ class Courtemanche(_MultiRate):
     def _flags(self):
         return _MultiRate._flags(self) | (_capi.F_ULTRA_SLOW if self.ultra_slow else 0)
 
-    def define(self, s1=True, state=None):
-        _MultiRate.define(self, s1, state)
+    def _create(self):
+        ctx = _MultiRate._create(self)
         self._ops['slow'] = ('call', lambda: None)      # court_ultra.py:108: empty group
         self._Inter = {name: _InterVar(self, k) for k, name in enumerate(_capi.INTER_NAMES)}
+        return ctx
 
     def _update_trend(self):
         """court_ultra.py:117-120: only Trend[0] := V[width//2, height//8]."""

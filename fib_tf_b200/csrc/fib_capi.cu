@@ -195,6 +195,11 @@ struct fib_ctx {
     return k < (unsigned long long)fr_first ? 0 : (k - fr_first) / fr_every + 1;
   }
   unsigned long long frames_recorded() const { return frames_upto(since(fr_armed_at)); }
+  // checkpoint in flight (fib_checkpoint_begin): ck_parts dense [rows][W] planes, complete at ev_ck on `stream`
+  float* ck = nullptr;
+  int ck_parts = 0;
+  cudaStream_t ck_stream = nullptr;   // fib_checkpoint_read's copies (possibly from another thread)
+  cudaEvent_t ev_ck = nullptr;
   float* weights[4] = {nullptr, nullptr, nullptr, nullptr};   // user masks, halo layout like phase
   // persistent on-chip kernel (fib_persist.cuh): small unsharded 4v / BR grids
   int persist = -1;                   // -1 not decided yet, 0 no, 1 yes
@@ -533,7 +538,9 @@ static int create_resources(fib_ctx* c) {
   CU(cudaStreamCreateWithFlags(&c->comm_stream, cudaStreamNonBlocking));
   CU(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
   CU(cudaStreamCreateWithFlags(&c->up_stream, cudaStreamNonBlocking));
+  CU(cudaStreamCreateWithFlags(&c->ck_stream, cudaStreamNonBlocking));
   CU(cudaEventCreateWithFlags(&c->ev_up_begin, cudaEventDisableTiming));
+  CU(cudaEventCreateWithFlags(&c->ev_ck, cudaEventDisableTiming));
   if (const char* e = getenv("FIB_PIPELINE_MIN_CELLS")) c->pipeline_min_cells = atoll(e);
   if (const char* e = getenv("FIB_PIPELINE_BLOCK_ROWS")) c->pipeline_block_rows = max(atoi(e), 1);
   if (const char* e = getenv("FIB_PIPELINE_NCCL")) c->pipeline_nccl = atoi(e) != 0;
@@ -579,6 +586,15 @@ extern "C" int fib_destroy(fib_ctx* c) {
   if (c->stream) cudaStreamSynchronize(c->stream);
   if (c->comm_stream) cudaStreamSynchronize(c->comm_stream);
   if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
+  if (c->ck) {
+    cudaFreeAsync(c->ck, c->stream);
+    cudaStreamSynchronize(c->stream);
+  }
+  if (c->ck_stream) {
+    cudaStreamSynchronize(c->ck_stream);
+    cudaStreamDestroy(c->ck_stream);
+  }
+  if (c->ev_ck) cudaEventDestroy(c->ev_ck);
   if (c->up_stream) {
     cudaStreamSynchronize(c->up_stream);
     cudaStreamDestroy(c->up_stream);
@@ -2008,8 +2024,9 @@ extern "C" int fib_probe_fetch(fib_ctx* c, float* out, size_t max, size_t* n) {
 
 // Activation maps: the sample s[0] is the current plane; the update runs after every ODE iteration from
 // here on (record_observers, or inside the persistent kernel).  The iteration graphs are rebuilt with or
-// without the update nodes.
-extern "C" int fib_activation_watch(fib_ctx* c, float up, float down) {
+// without the update nodes.  A resume (`resume`) starts the counter at k and leaves the sample NaN for
+// fib_activation_set to fill.
+static int activation_arm(fib_ctx* c, float up, float down, bool resume, unsigned long long k) {
   if (!c) return fail(FIB_E_ARG, "ctx is NULL");
   if (!isfinite(up) || !isfinite(down)) return fail(FIB_E_ARG, "activation levels must be finite (up %g, down %g)", up, down);
   DevGuard dg(c->cfg.device);
@@ -2021,16 +2038,45 @@ extern "C" int fib_activation_watch(fib_ctx* c, float up, float down) {
   if (!c->act_iter) CU(cudaMalloc(&c->act_iter, sizeof(unsigned long long)));
   if (!c->act_prev) CU(cudaMalloc(&c->act_prev, plane * sizeof(float)));
   if (!c->act_maps) CU(cudaMalloc(&c->act_maps, kActMaps * plane * sizeof(float)));   // last: armed from here
-  CU(cudaMemcpyAsync(c->act_prev, owned_rows(c, 0), plane * sizeof(float), cudaMemcpyDeviceToDevice, c->stream));
+  if (resume)
+    CU(cudaMemsetAsync(c->act_prev, 0xff, plane * sizeof(float), c->stream));         // all-ones bits: NaN
+  else
+    CU(cudaMemcpyAsync(c->act_prev, owned_rows(c, 0), plane * sizeof(float), cudaMemcpyDeviceToDevice, c->stream));
   activation_reset_kernel<<<c->sms * 4, 256, 0, c->stream>>>(c->act_maps, plane);
   CU(cudaGetLastError());
   c->launches++;
-  CU(cudaMemsetAsync(c->act_iter, 0, sizeof(unsigned long long), c->stream));
+  CU(cudaMemcpyAsync(c->act_iter, &k, sizeof k, cudaMemcpyHostToDevice, c->stream));
   CU(cudaStreamSynchronize(c->stream));
-  c->act_armed_at = c->ode_iters;
+  c->act_armed_at = c->ode_iters - k;     // since(act_armed_at) == k (modulo 2^64)
   c->act_up = up;
   c->act_down = down;
   return 0;
+}
+extern "C" int fib_activation_watch(fib_ctx* c, float up, float down) {
+  return activation_arm(c, up, down, false, 0);
+}
+extern "C" int fib_activation_resume(fib_ctx* c, float up, float down, uint64_t k) {
+  return activation_arm(c, up, down, true, k);
+}
+
+// map `map` (fib_act_map) of an armed context: a plane of the shard's row layout
+static bool act_map_valid(int map) { return (map >= 0 && map < kActMaps) || map == FIB_ACT_SAMPLE; }
+static float* act_plane(fib_ctx* c, int map) {
+  return map == FIB_ACT_SAMPLE ? c->act_prev : c->act_maps + (size_t)map * c->plane_floats();
+}
+
+extern "C" int fib_activation_set(fib_ctx* c, int map, const float* host, size_t n) {
+  if (!c || !host) return fail(FIB_E_ARG, "ctx/host is NULL");
+  if (!act_map_valid(map)) return fail(FIB_E_ARG, "unknown activation map %d", map);
+  if (n != (size_t)c->g.rows * c->g.W)
+    return fail(FIB_E_ARG, "fib_activation_set: n=%zu, expected rows*width=%zu", n, (size_t)c->g.rows * c->g.W);
+  if (!c->act_maps) return fail(FIB_E_STATE, "no activation map is armed (fib_activation_resume)");
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  CU(cudaMemcpy2DAsync(act_plane(c, map), c->g.pitch * sizeof(float), host, c->g.W * sizeof(float),
+                       c->g.W * sizeof(float), c->g.rows, cudaMemcpyHostToDevice, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return check_persist_error(c);
 }
 
 extern "C" int fib_activation_stop(fib_ctx* c) {
@@ -2049,13 +2095,13 @@ extern "C" int fib_activation_stop(fib_ctx* c) {
 
 extern "C" int fib_activation_get(fib_ctx* c, int map, float* host, size_t n) {
   if (!c || !host) return fail(FIB_E_ARG, "ctx/host is NULL");
-  if (map < 0 || map >= kActMaps) return fail(FIB_E_ARG, "unknown activation map %d", map);
+  if (!act_map_valid(map)) return fail(FIB_E_ARG, "unknown activation map %d", map);
   if (n != (size_t)c->g.rows * c->g.W)
     return fail(FIB_E_ARG, "fib_activation_get: n=%zu, expected rows*width=%zu", n, (size_t)c->g.rows * c->g.W);
   if (!c->act_maps) return fail(FIB_E_STATE, "no activation map is armed (fib_activation_watch)");
   DevGuard dg(c->cfg.device);
   FLUSH(c);
-  CU(cudaMemcpy2DAsync(host, c->g.W * sizeof(float), c->act_maps + (size_t)map * c->plane_floats(),
+  CU(cudaMemcpy2DAsync(host, c->g.W * sizeof(float), act_plane(c, map),
                        c->g.pitch * sizeof(float), c->g.W * sizeof(float), c->g.rows, cudaMemcpyDeviceToHost,
                        c->stream));
   CU(cudaStreamSynchronize(c->stream));
@@ -2064,8 +2110,10 @@ extern "C" int fib_activation_get(fib_ctx* c, int map, float* host, size_t n) {
 
 // Frame recorder: a ring of strided frames in device memory.  Nothing joins the iteration graphs: the host
 // counts iterations and gathers a frame after the recording ones (end_iterations), or hands the persistent kernel
-// the first recording iteration of its launch (launch_persist_m).
-extern "C" int fib_frames_watch(fib_ctx* c, int var, int first, int every, int stride, int capacity) {
+// the first recording iteration of its launch (launch_persist_m).  A resume (`resume`) starts k at `k`, with the
+// frames up to k counted as fetched and none taken now.
+static int frames_arm(fib_ctx* c, int var, int first, int every, int stride, int capacity, bool resume,
+                      unsigned long long k) {
   if (!c) return fail(FIB_E_ARG, "ctx is NULL");
   if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
   if (first < 0 || every < 1 || stride < 1 || capacity < 1)
@@ -2085,8 +2133,8 @@ extern "C" int fib_frames_watch(fib_ctx* c, int var, int first, int every, int s
   c->fr_every = every;
   c->fr_stride = stride;
   c->fr_cap = capacity;
-  c->fr_armed_at = c->ode_iters;
-  c->fr_fetched = 0;
+  c->fr_armed_at = c->ode_iters - k;      // since(fr_armed_at) == k (modulo 2^64)
+  c->fr_fetched = resume ? c->frames_upto(k) : 0;
   const int er = c->frame_ledger.create();
   if (er) return er;
   c->frame_ledger.clear();
@@ -2096,7 +2144,13 @@ extern "C" int fib_frames_watch(fib_ctx* c, int var, int first, int every, int s
     c->frames = nullptr;
     return fail(FIB_E_CUDA, "fib_frames_watch: cannot allocate a ring of %d frames (%zu bytes)", capacity, bytes);
   }                                              // armed from here
-  return first == 0 ? launch_frame(c, 0) : 0;
+  return first == 0 && !resume ? launch_frame(c, 0) : 0;
+}
+extern "C" int fib_frames_watch(fib_ctx* c, int var, int first, int every, int stride, int capacity) {
+  return frames_arm(c, var, first, every, stride, capacity, false, 0);
+}
+extern "C" int fib_frames_resume(fib_ctx* c, int var, int first, int every, int stride, int capacity, uint64_t k) {
+  return frames_arm(c, var, first, every, stride, capacity, true, k);
 }
 
 extern "C" int fib_frames_stop(fib_ctx* c) {
@@ -2158,6 +2212,90 @@ extern "C" int fib_frames_fetch(fib_ctx* c, float* host, uint64_t* iters, size_t
   c->fr_fetched = first + take;
   *n = (size_t)take;
   return check_persist_error(c);
+}
+
+// ------------------------------------------------------------------------------------------
+// checkpoints: a stream-ordered staging copy of the owned rows, read out on ck_stream
+// ------------------------------------------------------------------------------------------
+extern "C" int fib_checkpoint_begin(fib_ctx* c, fib_checkpoint_info* info) {
+  if (!c || !info) return fail(FIB_E_ARG, "ctx/info is NULL");
+  if (info->struct_size != sizeof(fib_checkpoint_info))
+    return fail(FIB_E_ARG, "fib_checkpoint_info.struct_size %u != %zu (ABI mismatch)", info->struct_size,
+                sizeof(fib_checkpoint_info));
+  if (c->ck) return fail(FIB_E_STATE, "a checkpoint is already in flight on this context (fib_checkpoint_end)");
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  const size_t plane = (size_t)c->g.rows * c->g.W;
+  const int parts = c->nvars + (c->act_maps ? 1 + kActMaps : 0);
+  // stream-ordered: neither this allocation nor fib_checkpoint_end's release waits for the stepping
+  cudaError_t e = cudaMallocAsync((void**)&c->ck, parts * plane * sizeof(float), c->stream);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    c->ck = nullptr;
+    return fail(FIB_E_CUDA, "fib_checkpoint_begin: cannot allocate the staging copy of %d planes (%zu bytes): %s",
+                parts, parts * plane * sizeof(float), cudaGetErrorString(e));
+  }
+  c->ck_parts = parts;
+  for (int p = 0; p < parts && e == cudaSuccess; ++p) {
+    const float* src = p < c->nvars ? owned_rows(c, p) : act_plane(c, p == c->nvars ? FIB_ACT_SAMPLE : p - c->nvars - 1);
+    e = cudaMemcpy2DAsync(c->ck + p * plane, c->g.W * sizeof(float), src, c->g.pitch * sizeof(float),
+                          c->g.W * sizeof(float), c->g.rows, cudaMemcpyDeviceToDevice, c->stream);
+  }
+  if (e == cudaSuccess) e = cudaEventRecord(c->ev_ck, c->stream);
+  if (e != cudaSuccess) {
+    cudaFreeAsync(c->ck, c->stream);
+    c->ck = nullptr;
+    return fail(FIB_E_CUDA, "fib_checkpoint_begin: staging copy failed: %s", cudaGetErrorString(e));
+  }
+  const fib_checkpoint_info z = {};
+  *info = z;
+  info->struct_size = sizeof(fib_checkpoint_info);
+  info->nparts = parts;
+  info->iterations = c->ode_iters;
+  if (c->act_maps) {
+    info->act_armed = 1;
+    info->act_up = c->act_up;
+    info->act_down = c->act_down;
+    info->act_k = c->since(c->act_armed_at);
+  }
+  if (c->frames) {
+    info->fr_armed = 1;
+    info->fr_var = c->fr_var;
+    info->fr_first = c->fr_first;
+    info->fr_every = c->fr_every;
+    info->fr_stride = c->fr_stride;
+    info->fr_capacity = c->fr_cap;
+    info->fr_k = c->since(c->fr_armed_at);
+  }
+  return 0;
+}
+
+// May run on another thread than the owner's: it touches only the staged copy, ck_stream and ev_ck, which the
+// owner changes only in fib_checkpoint_begin / fib_checkpoint_end.
+extern "C" int fib_checkpoint_read(fib_ctx* c, int part, int r0, int r1, float* host) {
+  if (!c || !host) return fail(FIB_E_ARG, "ctx/host is NULL");
+  if (!c->ck) return fail(FIB_E_STATE, "no checkpoint is in flight (fib_checkpoint_begin)");
+  if (part < 0 || part >= c->ck_parts) return fail(FIB_E_ARG, "checkpoint part %d out of range (%d parts)", part, c->ck_parts);
+  if (r0 < c->g.row0 || r1 > c->g.row0 + c->g.rows || r0 >= r1)
+    return fail(FIB_E_ARG, "rows [%d,%d) not inside this shard [%d,%d)", r0, r1, c->g.row0, c->g.row0 + c->g.rows);
+  DevGuard dg(c->cfg.device);
+  const size_t W = c->g.W;
+  CU(cudaStreamWaitEvent(c->ck_stream, c->ev_ck, 0));
+  CU(cudaMemcpyAsync(host, c->ck + (size_t)part * c->g.rows * W + (size_t)(r0 - c->g.row0) * W,
+                     (size_t)(r1 - r0) * W * sizeof(float), cudaMemcpyDeviceToHost, c->ck_stream));
+  CU(cudaStreamSynchronize(c->ck_stream));
+  return 0;
+}
+
+extern "C" int fib_checkpoint_end(fib_ctx* c) {
+  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
+  if (!c->ck) return 0;
+  DevGuard dg(c->cfg.device);
+  // after the staging copy on `stream`; every read of it has returned
+  CU(cudaFreeAsync(c->ck, c->stream));
+  c->ck = nullptr;
+  c->ck_parts = 0;
+  return 0;
 }
 
 extern "C" int fib_count_below(fib_ctx* c, int var, float sub, float div, float cutoff, float w_min,

@@ -27,19 +27,24 @@ class Fenton4v(IonicModel):
 
     def define(self, s1=True):
         """Initial state U=0, V=W=1, S=0; S1 = column 1 of U set to 1 (fenton.py:116-123)."""
-        super().define()
-        self.steps_per_launch_used = self._steps_per_launch()
-        ctx = self._make_context(steps_per_launch=self.steps_per_launch_used)
+        ctx = self._create()
         init = {'U': 0.0, 'V': 1.0, 'W': 1.0, 'S': 0.0}
         for name, val in init.items():
             a = self._local_full(val)
             if s1 and name == 'U':
                 a[:, 1] = 1.0
             ctx.set_state(name, a)
+
+    def _create(self):
+        """The context and handles of define(), without the initial state (define() and restore())."""
+        IonicModel.define(self)
+        self.steps_per_launch_used = self._steps_per_launch()
+        ctx = self._make_context(steps_per_launch=self.steps_per_launch_used)
         self.dt_per_step = ctx.dt_per_step      # 10
         self._ode_op = _capi.OP_ODE
         self._State = {n: DeviceVar(self, n) for n in ctx.var_names}
         self._U = self._State['U']
+        return ctx
 
     # grids from this many cells up run two time steps per launch by default: below it the state
     # (4 planes) is L2-resident and the one-step kernel is faster (2048^2: 242 vs 209 Gcell-steps/s);

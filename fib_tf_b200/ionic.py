@@ -36,16 +36,18 @@ Extra, optional config keys (all default to the reference's behaviour):
 Collective calls under config['distributed'] (every rank must make them, in the same order):
 define(), run() (each iteration), fire_op(), image(), pot().eval() / _State[..].eval(),
 var[r, c].eval(), masked_image_mean(), excitable_fraction(), watch_activation(), activation_maps(),
-stop_activation(), frames(), close().  cl_observer callbacks run on
+stop_activation(), frames(), checkpoint(), Checkpoint.wait(), restore(), close().  cl_observer callbacks run on
 the rank that owns row 20 only and therefore must not call any of these.
 """
 import json
 import os
+import shutil
 import time
 
 import numpy as np
 
 from . import _capi
+from . import checkpoint as _ckpt
 from .sharding import owner_of_row, partition_rows
 
 
@@ -378,6 +380,7 @@ class IonicModel:
                         self._ctx                            # noqa: B018 (the window is full: go)
                 else:
                     self._ctx.step(self.ode_op(i), 1)
+                self.iterations += 1
                 if self.__dict__.get('_frames') is not None:
                     self._drain_frames()
                 yield i
@@ -405,6 +408,7 @@ class IonicModel:
         if getattr(self, 'timeline', False):
             self._write_timeline()
         self._ctx.sync()
+        self._release_restore_buffers()
         print('elapsed: %f sec' % (time.time() - then))
         if block and im:
             im.wait()
@@ -431,6 +435,7 @@ class IonicModel:
         n0 = c.launch_count()
         c.timer_start()
         c.step(self.ode_op(self.samples), 1)
+        self.iterations += 1
         c.timer_stop()
         ms = c.timer_ms()
         ev = [{'name': 'ode_op (%d fused step kernels)' % (c.launch_count() - n0), 'ph': 'X',
@@ -446,6 +451,7 @@ class IonicModel:
     def define(self, s1=True):
         """Placeholder replaced in subclasses: builds the initial state and the device context."""
         self.defined = True
+        self.iterations = 0         # ODE iterations since define(), continued by restore()
 
     def image(self):
         """[height x width] float ndarray in 0..1 encoding the transmembrane potential."""
@@ -606,16 +612,10 @@ class IonicModel:
         if f is None:
             raise AssertionError('frames() needs record_frames() first')
         rows, cols = self._ctx.frames_shape()
-        while True:
-            iters, cube = self._ctx.frames_fetch(self.FRAME_BATCH)
-            f['iters'].append(iters)
-            f['cube'].append(cube)
-            if len(iters) < self.FRAME_BATCH:
-                break
+        self._fetch_frames()
         iters = np.concatenate(f['iters']).astype(np.int64)
         cube = np.concatenate(f['cube']) if f['cube'] else np.empty((0, rows, cols), np.float32)
         f['iters'], f['cube'] = [], []
-        f['upto'] = 0 if f['k'] < f['first'] else (f['k'] - f['first']) // f['every'] + 1
         if self._nranks > 1:
             import torch.distributed as dist
             parts = [None] * self._nranks
@@ -624,6 +624,17 @@ class IonicModel:
         if f['name'] == self._pot_name and self.MODEL_ID != _capi.FENTON4V:
             cube = self._normalise(cube)
         return iters, cube
+
+    def _fetch_frames(self):
+        """Moves every frame recorded so far from the ring into the host list."""
+        f = self._frames
+        while True:
+            iters, cube = self._ctx.frames_fetch(self.FRAME_BATCH)
+            f['iters'].append(iters)
+            f['cube'].append(cube)
+            if len(iters) < self.FRAME_BATCH:
+                break
+        f['upto'] = 0 if f['k'] < f['first'] else (f['k'] - f['first']) // f['every'] + 1
 
     def stop_frames(self):
         """Disarms the frame recorder and frees its ring; frames not yet returned by frames() are dropped."""
@@ -656,10 +667,133 @@ class IonicModel:
             raise RuntimeError('image_wait() without a preceding image_async()')
         return a if self.MODEL_ID == _capi.FENTON4V else self._normalise(a)
 
+    # ---- checkpoint and restart (fib_tf_b200/checkpoint.py) -----------------------------------
+    def checkpoint(self, path):
+        """Saves the state after the iterations stepped so far, and the armed activation map and frame recorder,
+        to the directory `path` while stepping continues: stages a device copy of every shard behind the work
+        already enqueued and returns a Checkpoint at once; writer threads fill the files meanwhile.  Frames
+        recorded so far move to the host list first (frames() returns them; they are not saved).  The previous
+        checkpoint at `path` stays readable until Checkpoint.wait() replaces it, atomically where the file
+        system allows.  Collective when distributed."""
+        if not self.defined:
+            raise AssertionError('checkpoint should be called after calling define')
+        self._finish_checkpoint()
+        if self.__dict__.get('_frames') is not None:
+            self._fetch_frames()
+        path = os.path.abspath(path)
+        partial = path + '.partial'
+        if self._rank == 0 and os.path.exists(partial):
+            shutil.rmtree(partial)
+        if self._rank == 0:
+            os.makedirs(partial)
+        if self._nranks > 1:
+            import torch.distributed as dist
+            dist.barrier()
+        ck = Checkpoint(self, path, partial, _ckpt.save_shard(self._ctx, partial, self._own_phase_rows()),
+                        self.iterations)
+        self._ckpt = ck
+        return ck
+
+    def _own_phase_rows(self):
+        """This shard's rows of the phase field, or None."""
+        if self._phase_rows is None:
+            return None
+        lo = self._row0 - self._phase_row0
+        return self._phase_rows[lo:lo + self._rows]
+
+    def _finish_checkpoint(self):
+        ck = self.__dict__.get('_ckpt')
+        if ck is not None:
+            ck.wait()
+
+    def restore(self, path):
+        """Instead of define(): builds the device context exactly as define() does, then loads the checkpoint
+        at `path` -- saved on any number of ranks -- with the armed observers resumed, and continues
+        `iterations` from it.  ValueError if this model's config or phase field would compute differently.
+        A large grid with no observer steps its first iterations behind its own upload.  Collective when
+        distributed."""
+        man = _ckpt.load_manifest(path)
+        ctx = self._create()
+        own = self._own_phase_rows()
+        try:
+            _ckpt.check_compatible(man, ctx, own)
+            _ckpt.check_phase(path, man, ctx, own)
+            self._restore_pinned = _ckpt.restore_context(ctx, path, bottom_up=self._rank % 2 == 1, man=man)
+        except BaseException:
+            self.close()
+            self.defined = False
+            raise
+        self.iterations = man['iterations']
+        fr = man['frames']
+        if fr['armed']:
+            k = fr['k']
+            self._frames = {'name': fr['var'], 'first': fr['first'], 'every': fr['every'], 'stride': fr['stride'],
+                            'capacity': fr['capacity'], 'k': k, 'iters': [], 'cube': [],
+                            'upto': 0 if k < fr['first'] else (k - fr['first']) // fr['every'] + 1}
+        return man
+
+    def _release_restore_buffers(self):
+        """The host copies of a restore, once a synchronous call has consumed them."""
+        _ckpt.release(self.__dict__.get('_restore_pinned') or [])
+
     def sync(self):
         self._ctx.sync()
+        self._release_restore_buffers()
 
     def close(self):
-        if self._ctx is not None:
-            self._ctx.close()
-            self._ctx = None
+        try:
+            self._finish_checkpoint()
+        finally:
+            if self._ctx is not None:
+                self._ctx.close()
+                self._ctx = None
+            self._release_restore_buffers()
+
+
+class Checkpoint:
+    """A save started by IonicModel.checkpoint(); wait() completes it."""
+
+    def __init__(self, model, path, partial, writer, iterations):
+        self.model, self.path, self.partial, self.writer = model, path, partial, writer
+        self.iterations = iterations
+        self.done = False
+
+    def wait(self):
+        """Joins the writers, agrees with the other ranks that every shard was saved, then rank 0 writes the
+        manifest and puts the checkpoint at `path`.  RuntimeError if any rank failed; the previous checkpoint
+        at `path` is then left as it was.  Collective when distributed."""
+        if self.done:
+            return self
+        self.done = True
+        m = self.model
+        if m.__dict__.get('_ckpt') is self:
+            m._ckpt = None
+        ok = self.writer.join()
+        mine = (ok, None if ok else repr(self.writer.error), self.writer.record, self.writer.info)
+        parts = [mine]
+        if m._nranks > 1:
+            import torch.distributed as dist
+            parts = [None] * m._nranks
+            dist.all_gather_object(parts, mine)
+        failed = ['rank %d: %s' % (r, p[1]) for r, p in enumerate(parts) if not p[0]]
+        err = None
+        if m._rank == 0:
+            try:
+                if failed:
+                    shutil.rmtree(self.partial, ignore_errors=True)
+                else:
+                    man = _ckpt.manifest(self.writer.ctx, parts[0][3], [p[2] for p in parts], self.iterations)
+                    _ckpt.write_manifest(self.partial, man)
+                    _ckpt.publish(self.partial, self.path)
+            except Exception as e:
+                err = repr(e)
+        if m._nranks > 1:
+            import torch.distributed as dist
+            box = [err]
+            dist.broadcast_object_list(box, src=0)
+            err = box[0]
+        if failed:
+            raise RuntimeError('checkpoint %s was not saved: %s' % (self.path, '; '.join(failed)))
+        if err is not None:
+            raise RuntimeError('checkpoint %s was not published: %s' % (self.path, err))
+        return self

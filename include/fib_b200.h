@@ -16,7 +16,8 @@
  *   - all device work is ENQUEUE-ONLY on the context's stream unless stated "synchronous"
  *     (the reference's run() generator hands control back to user code between iterations,
  *     ionic.py:202-204, so the only sync points are state reads, probes and fib_sync);
- *   - one context is not thread-safe (single caller); different contexts are independent;
+ *   - one context is not thread-safe (single caller); different contexts are independent; the one exception
+ *     is fib_checkpoint_read, which another thread may call while the owner keeps stepping;
  *   - there is no CPU fallback: without a CUDA device fib_create fails with FIB_E_CUDA.
  */
 #ifndef FIB_B200_H_
@@ -29,7 +30,7 @@
 extern "C" {
 #endif
 
-#define FIB_ABI_VERSION 4
+#define FIB_ABI_VERSION 5
 
 typedef struct fib_ctx fib_ctx;
 
@@ -248,17 +249,28 @@ int fib_count_below(fib_ctx *ctx, int var, float sub, float div, float cutoff, f
  * upload (they are copied in order instead).
  * fib_activation_watch arms the map, or re-arms it: everything is reset and s[0] re-taken; FIB_E_ARG if a
  * level is not finite.  fib_activation_stop disarms it and frees the planes.  fib_activation_get copies map
- * `map` (fib_act_map) of this shard, rows*width floats; synchronous; FIB_E_STATE without a watch. */
+ * `map` (fib_act_map) of this shard, rows*width floats; synchronous; FIB_E_STATE without a watch.
+ * FIB_ACT_SAMPLE is the last sample s[k] itself, the plane the next iteration's events are measured from (not a
+ * map: its id lies outside FIB_ACT_FIRST..FIB_ACT_COUNT, which stay the five maps).
+ * Resuming a map saved by fib_checkpoint_begin: fib_activation_resume arms it with its counter at `k` (the next
+ * iteration takes s[k+1] and its events have times k + fraction) and WITHOUT taking a sample -- the five maps
+ * are reset (NaN, COUNT 0) and the sample is NaN (no event) until fib_activation_set fills them; synchronous.
+ * fib_activation_set uploads map `map` (FIB_ACT_FIRST..FIB_ACT_COUNT or FIB_ACT_SAMPLE), rows*width floats; synchronous;
+ * FIB_E_STATE without a watch.  After a resume and a set of all six planes, every later iteration produces
+ * exactly the events and times of the context that was saved. */
 typedef enum {
   FIB_ACT_FIRST = 0,
   FIB_ACT_LAST = 1,
   FIB_ACT_PREV = 2,
   FIB_ACT_REPOL = 3,
-  FIB_ACT_COUNT = 4
+  FIB_ACT_COUNT = 4,
+  FIB_ACT_SAMPLE = 16
 } fib_act_map;
 int fib_activation_watch(fib_ctx *ctx, float up, float down);
+int fib_activation_resume(fib_ctx *ctx, float up, float down, uint64_t k);
 int fib_activation_stop(fib_ctx *ctx);
 int fib_activation_get(fib_ctx *ctx, int map, float *host, size_t n);
+int fib_activation_set(fib_ctx *ctx, int map, const float *host, size_t n);
 
 /* frame recorder (SURVEY 8f2): a strided movie of one state plane, recorded on the device while stepping into
  * a ring in device memory and fetched in batches -- the cube.npy of fenton.py:179-187 / br.py without a full
@@ -281,11 +293,55 @@ int fib_activation_get(fib_ctx *ctx, int map, float *host, size_t n);
  * fib_frames_watch arms the recorder, or re-arms it: the ring is reset and k = 0 re-taken if first == 0.
  * FIB_E_ARG for every, stride or capacity < 1, first < 0 or an unknown var; FIB_E_CUDA if the ring cannot be
  * allocated.  fib_frames_stop disarms it and frees the ring.  fib_frames_shape / fib_frames_fetch: FIB_E_STATE
- * without a watch.  An armed recorder keeps fib_set_rect_async blocks out of the pipelined upload. */
+ * without a watch.  An armed recorder keeps fib_set_rect_async blocks out of the pipelined upload.
+ * fib_frames_resume continues a recorder saved by fib_checkpoint_begin: it arms like fib_frames_watch, but k
+ * starts at `k` (the next iteration is k + 1), no frame is taken at arming, and the frames of k' <= k count as
+ * already fetched -- the first frame fetched is the one at the first recording k' > k, with the k' the saved
+ * context would have given it. */
 int fib_frames_watch(fib_ctx *ctx, int var, int first, int every, int stride, int capacity);
+int fib_frames_resume(fib_ctx *ctx, int var, int first, int every, int stride, int capacity, uint64_t k);
 int fib_frames_stop(fib_ctx *ctx);
 int fib_frames_shape(const fib_ctx *ctx, int *rows, int *cols);
 int fib_frames_fetch(fib_ctx *ctx, float *host, uint64_t *iters, size_t max, size_t *n);
+
+/* checkpoints (SURVEY 8f3): a copy of this shard's state, and of its observers, taken while stepping continues,
+ * from which a new context -- on any partition of the grid -- continues bit for bit as this one would.
+ *   begin    fib_checkpoint_begin launches the deferred iterations, then enqueues on the context's stream a
+ *            device-to-device copy of the shard's OWNED rows into a staging buffer, dense [rows][width] per part,
+ *            ordered after everything stepped so far, and returns without waiting: later fib_step calls run
+ *            while the copy is read out.  The copy holds the state after fib_checkpoint_info.iterations ODE
+ *            iterations (and after whatever the caller wrote since the last of them).
+ *   parts    0 .. nvars-1: the state planes (fib_var_name order); then, with an armed activation map,
+ *            nvars: its last sample (FIB_ACT_SAMPLE) and nvars+1 .. nvars+5: FIB_ACT_FIRST .. FIB_ACT_COUNT.
+ *            Not saved, because a context rebuilds them: halo rows, the two-steps-per-launch ping-pong copies,
+ *            the persistent kernel's mailbox, the graphs, the phase field and the tables (set them again; the
+ *            Courtemanche LUT with fib_build_lut).  Frames recorded before the checkpoint stay with this context.
+ *   read     fib_checkpoint_read copies global rows [r0, r1) of staged part `part` to `host` (dense, (r1-r0)*width
+ *            floats; page-locked memory is fastest) on a stream of its own, after the staging copy, and returns
+ *            when it is done.  It reads only the staged copy, so it is the ONE entry point that may be called
+ *            from another thread while the owning thread keeps calling fib_step and the other entry points.
+ *   end      fib_checkpoint_end releases the staging buffer (stream-ordered: it does not wait for the stepping);
+ *            no fib_checkpoint_read may be in progress.  A no-op without a checkpoint.  fib_destroy releases it too.
+ *   restore  a new context of the same model, grid and arithmetic flags: set the phase field and tables, upload
+ *            the planes (fib_set_state / fib_set_rect / fib_set_rect_async), re-arm the observers with
+ *            fib_activation_resume + fib_activation_set and fib_frames_resume from the info, and step.
+ * One checkpoint may be in flight per context: a second begin is FIB_E_STATE.  The staging buffer is one more
+ * copy of the shard (plus six planes with an armed map); FIB_E_CUDA if it cannot be allocated. */
+typedef struct {
+  uint32_t struct_size;      /* = sizeof(fib_checkpoint_info), set by the caller                       */
+  int32_t  nparts;           /* staged parts: nvars, or nvars + 6 with an armed activation map          */
+  uint64_t iterations;       /* ODE iterations enqueued on this context since fib_create                */
+  int32_t  act_armed;        /* activation map: armed (1) or not (0); then its levels and counter k     */
+  float    act_up, act_down;
+  int32_t  fr_armed;         /* frame recorder: armed (1) or not (0); then its arguments and counter k  */
+  uint64_t act_k;
+  int32_t  fr_var, fr_first, fr_every, fr_stride, fr_capacity, reserved0;
+  uint64_t fr_k;
+  int32_t  reserved[6];
+} fib_checkpoint_info;
+int fib_checkpoint_begin(fib_ctx *ctx, fib_checkpoint_info *info);
+int fib_checkpoint_read(fib_ctx *ctx, int part, int r0, int r1, float *host);
+int fib_checkpoint_end(fib_ctx *ctx);
 
 /* ---- op-level entry points of IonicModel's helpers on dense host planes [h][w] (eager; used by the
  * drop-in IonicModel.enforce_boundary / laplace / phase_field / rush_larsen and by the parity tests that
