@@ -20,7 +20,8 @@ PROBE_RING = 4096
 OP_ODE, OP_SLOW = 0, 1
 TABLE_BR_CHEBY, TABLE_COURT_LUT = 0, 1
 ACT_FIRST, ACT_LAST, ACT_PREV, ACT_REPOL, ACT_COUNT, ACT_SAMPLE = 0, 1, 2, 3, 4, 16
-ABI_VERSION = 5
+ABI_VERSION = 6
+PACE_MAX = 4
 INTER_COLS = 32
 
 # courtemanche.h:105-134 column order (+ the two court_ultra.py:445-450 extras)
@@ -104,6 +105,9 @@ _SIGNATURES = {
     'fib_step': (C.c_int, [_P, C.c_int, C.c_int]),
     'fib_step_group': (C.c_int, [C.POINTER(_P), C.c_int, C.c_int, C.c_int]),
     'fib_stimulate': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float]),
+    'fib_pace_add': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_int, C.c_int,
+                               C.c_int, C.POINTER(C.c_int)]),
+    'fib_pace_remove': (C.c_int, [_P, C.c_int]),
     'fib_probe': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _FP]),
     'fib_weighted_sum': (C.c_int, [_P, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     'fib_count_nonfinite': (C.c_int, [_P, C.c_int, C.POINTER(C.c_uint64)]),
@@ -297,6 +301,18 @@ class Context:
 
     def stimulate(self, var, r0, r1, c0, c1, value, floor_v):
         check(lib().fib_stimulate(self._h, self.var(var), r0, r1, c0, c1, value, floor_v))
+
+    def pace_add(self, r0, r1, c0, c1, value, floor_v, first, every=0, count=1):
+        """Schedule stimulate(diffusing variable, r0, r1, c0, c1, value, floor_v) after the ODE iterations
+        k = first + j * every (j < count; count 0: until removed) counted from now, k = 1 the next; returns the id."""
+        i = C.c_int()
+        check(lib().fib_pace_add(self._h, int(r0), int(r1), int(c0), int(c1), float(value), float(floor_v),
+                                 int(first), int(every), int(count), C.byref(i)))
+        return i.value
+
+    def pace_remove(self, pace_id=-1):
+        """Remove pacing entry `pace_id`, or every entry (pace_id < 0)."""
+        check(lib().fib_pace_remove(self._h, int(pace_id)))
 
     def probe(self, var, row, col):
         v = C.c_float()

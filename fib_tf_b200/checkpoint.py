@@ -5,7 +5,8 @@ restored bit for bit into a context on any number of GPUs.
 Format: a directory.
     manifest.json                written last (a directory without it is not a checkpoint): the format version,
                                  the model and the config that changes arithmetic, `iterations`, the observers'
-                                 info and the shard files with their global row ranges
+                                 info, the pacing entries still to fire and the shard files with their global row
+                                 ranges
     <part>.rows<r0>-<r1>.npy     one [r1 - r0, width] float32 array per (shard, part); parts are the state
                                  planes by their reference names, the activation map's last sample and five maps
                                  (act_*) when one was armed, and `phase` when the model has a phase field
@@ -140,8 +141,39 @@ def save_shard(ctx, directory, phase_rows=None):
     return ShardWriter(ctx, directory, phase_rows)
 
 
-def manifest(ctx, info, shards, iterations=None):
-    """The manifest dict of a checkpoint of `ctx`'s model: `shards` = the ShardWriter records of every shard."""
+def pacing_state(entries, iterations):
+    """The pacing entries (IonicModel.pace) that still fire after absolute ODE iteration `iterations`, as manifest
+    records: name, rect [r0, r1, c0, c1], value, floor, `next` (the absolute iteration its next beat follows),
+    `every` and `count` (the beats left; 0: until removed).  An entry fires after iterations next + j * every."""
+    out = []
+    for e in entries:
+        step = max(int(e['every']), 1)
+        done = 0 if iterations < e['next'] else (iterations - e['next']) // step + 1
+        if e['count'] and done >= e['count']:
+            continue
+        out.append({'name': e['name'], 'rect': [int(x) for x in e['rect']], 'value': float(e['value']),
+                    'floor': float(e['floor']), 'next': int(e['next'] + done * step), 'every': int(e['every']),
+                    'count': int(e['count'] - done) if e['count'] else 0})
+    return out
+
+
+def resume_pacing(ctx, entries, iterations):
+    """Adds the manifest's pacing records `entries` to `ctx`, a context that continues absolute ODE iteration
+    `iterations`, so that every beat follows the same absolute iteration as in the saved run; returns the records
+    with their entry ids (key `id`)."""
+    out = []
+    for e in entries:
+        if e['next'] <= iterations:
+            raise CheckpointError('pacing entry %r: next beat after iteration %d, but the run continues from %d'
+                                  % (e['name'], e['next'], iterations))
+        pid = ctx.pace_add(*e['rect'], e['value'], e['floor'], e['next'] - iterations, e['every'], e['count'])
+        out.append(dict(e, id=pid))
+    return out
+
+
+def manifest(ctx, info, shards, iterations=None, pacing=()):
+    """The manifest dict of a checkpoint of `ctx`'s model: `shards` = the ShardWriter records of every shard,
+    `pacing` = pacing_state() of the run at the checkpoint."""
     act = {'armed': bool(info['act_armed'])}
     if act['armed']:
         act.update(up=float(info['act_up']), down=float(info['act_down']), k=int(info['act_k']))
@@ -153,7 +185,7 @@ def manifest(ctx, info, shards, iterations=None):
     return {'format': FORMAT, 'version': VERSION, 'config': arithmetic_config(ctx),
             'iterations': int(info['iterations'] if iterations is None else iterations),
             'parts': part_names(ctx, info), 'phase': 'phase' in shards[0]['files'],
-            'activation': act, 'frames': frames, 'shards': shards}
+            'activation': act, 'frames': frames, 'pacing': list(pacing), 'shards': shards}
 
 
 def write_manifest(directory, man):

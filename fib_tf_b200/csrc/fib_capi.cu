@@ -8,6 +8,7 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <type_traits>
 #include <vector>
@@ -201,6 +202,19 @@ struct fib_ctx {
   cudaStream_t ck_stream = nullptr;   // fib_checkpoint_read's copies (possibly from another thread)
   cudaEvent_t ev_ck = nullptr;
   float* weights[4] = {nullptr, nullptr, nullptr, nullptr};   // user masks, halo layout like phase
+  // pacing (fib_pace_add): entry p stimulates the diffusing variable right after the ODE iterations whose ode_iters
+  // is p.at + j * p.every, j < p.count (count 0: every such iteration); dropped once its last beat is enqueued
+  struct Pace {
+    int id, r0, r1, c0, c1;
+    float value, floor_v;
+    unsigned long long at, every, count;
+    bool fires(unsigned long long n) const {
+      return n >= at && (n - at) % every == 0 && (count == 0 || (n - at) / every < count);
+    }
+    bool done(unsigned long long n) const { return count != 0 && n >= at + (count - 1) * every; }
+  };
+  std::vector<Pace> paces;
+  int pace_ids = 0;                   // ids handed out so far
   // persistent on-chip kernel (fib_persist.cuh): small unsharded 4v / BR grids
   int persist = -1;                   // -1 not decided yet, 0 no, 1 yes
   int persist_th = 0, persist_tiles = 0, persist_bw = 0;
@@ -233,7 +247,7 @@ struct fib_ctx {
   size_t fused_floats() const { return (size_t)(g.rows + 2 * kFuseHalo) * g.pitch; }
   bool top_is_border() const { return g.row0 == 0; }
   bool bottom_is_border() const { return g.row0 + g.rows == g.H; }
-  bool observing() const { return watch_var >= 0 || act_maps || frames; }
+  bool observing() const { return watch_var >= 0 || act_maps || frames || !paces.empty(); }
 };
 
 static void drop_graphs(fib_ctx* c) {
@@ -681,6 +695,17 @@ static cudaError_t wait_comm(fib_ctx* c) {
   if (!c->comm_pending) return cudaSuccess;
   c->comm_pending = false;
   return cudaStreamWaitEvent(c->stream, c->ev_comm, 0);
+}
+
+// the stimulus of fib_stimulate on the CURRENT plane `var` (enqueue-only; the caller marks the plane written)
+static int launch_stim(fib_ctx* c, int var, int r0, int r1, int c0, int c1, float value, float floor_v) {
+  CU(wait_comm(c));
+  dim3 block(128), grid((c->g.W + 127) / 128, min(c->g.rows, 65535));
+  const PlaneRef pl = plane_of(c, var);
+  stim_kernel<<<grid, block, 0, c->stream>>>(pl.base, c->g, pl.halo, r0, r1, c0, c1, value, floor_v);
+  CU(cudaGetLastError());
+  c->launches++;
+  return 0;
 }
 
 // The persistent path DEFERS iterations: fib_step only counts them, and they are launched -- up to
@@ -1249,13 +1274,13 @@ static bool make_tile_map(CUtensorMap* m, float* base, int W, int rows, int pitc
          CUDA_SUCCESS;
 }
 
-template <class MS, class MF, int TH, bool PHASE, bool ACT, bool FRAMES>
+template <class MS, class MF, int TH, bool PHASE, bool ACT, bool EVENTS>
 static cudaError_t launch_persist_t(fib_ctx* c, const PersistArgs<MS, MF>& a) {
   PersistMaps<MS::NS> maps;
   maps.x[0] = c->pmap_x[0];
   maps.x[1] = c->pmap_x[1];
   for (int k = 0; k < MS::NS; ++k) maps.s[k] = c->pmap_s[k];
-  auto kern = persist_kernel<MS, MF, TH, PHASE, ACT, FRAMES>;
+  auto kern = persist_kernel<MS, MF, TH, PHASE, ACT, EVENTS>;
   constexpr size_t smem = persist_smem_bytes<MS::NS, TH>();
   static bool attr_set = false;           // per instantiation
   if (!attr_set) {
@@ -1273,8 +1298,8 @@ static cudaError_t launch_persist_t(fib_ctx* c, const PersistArgs<MS, MF>& a) {
   attr[0].val.cooperative = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  snprintf(last_kernel_name(), 160, "persist_kernel<%s,TH=%d,PHASE=%d%s%s>", MS::name(), TH, PHASE ? 1 : 0,
-           ACT ? ",ACT=1" : "", FRAMES ? ",FRAMES=1" : "");
+  snprintf(last_kernel_name(), 160, "persist_kernel<%s,TH=%d,PHASE=%d%s%s%s>", MS::name(), TH, PHASE ? 1 : 0,
+           ACT ? ",ACT=1" : "", a.frames ? ",FRAMES=1" : "", a.pace_n ? ",PACE=1" : "");
   return cudaLaunchKernelEx(&cfg, kern, maps, c->g, a);
 }
 
@@ -1306,6 +1331,8 @@ static cudaError_t launch_persist_m(fib_ctx* c, PersistArgs<MS, MF>& a, int iter
   a.act_down = c->act_down;
   // frames: the first recording iteration of this launch (k = k1 + it0), if there is one
   a.frames = nullptr;
+  a.frame_step0 = a.nsteps + 1;
+  a.frame_steps = 1;
   if (c->frames) {
     const unsigned long long k1 = c->since(c->fr_armed_at) + 1, f0 = c->fr_first, ev = c->fr_every;
     const unsigned long long kf = k1 <= f0 ? f0 : f0 + (k1 - f0 + ev - 1) / ev * ev;
@@ -1321,7 +1348,24 @@ static cudaError_t launch_persist_m(fib_ctx* c, PersistArgs<MS, MF>& a, int iter
       a.frame_floats = c->frame_floats();
     }
   }
-  const bool ph = c->phase != nullptr, act = c->act_maps != nullptr, fr = a.frames != nullptr;
+  // pacing: the entries that fire in this launch, with one bit per iteration (the iteration's ode_iters is
+  // ode_iters + 1 + it)
+  a.pace_n = 0;
+  for (const auto& p : c->paces) {
+    unsigned long long mask = 0;
+    for (int it = 0; it < iters; ++it)
+      if (p.fires(c->ode_iters + 1 + it)) mask |= 1ull << it;
+    if (!mask) continue;
+    const int e = a.pace_n++;
+    a.pace_rect[e][0] = p.r0;
+    a.pace_rect[e][1] = p.r1;
+    a.pace_rect[e][2] = p.c0;
+    a.pace_rect[e][3] = p.c1;
+    a.pace_value[e] = p.value;
+    a.pace_floor[e] = p.floor_v;
+    a.pace_mask[e] = mask;
+  }
+  const bool ph = c->phase != nullptr, act = c->act_maps != nullptr, fr = a.frames != nullptr || a.pace_n > 0;
   auto flag = [](bool b, auto&& fn) { return b ? fn(std::true_type()) : fn(std::false_type()); };
   auto go = [&](auto th) {
     return flag(ph, [&](auto P) {
@@ -1427,10 +1471,27 @@ static int record_observers(fib_ctx* c, int op) {
   return observe_rows(c, 0, c->g.rows);
 }
 
+// The pacing entries that fire after the iteration just counted, in the order they were added: the stimulus of
+// each, then the probe's value of this iteration taken again (mark_written), as after a fib_stimulate.
+static int fire_paces(fib_ctx* c) {
+  bool fired = false;
+  for (const auto& p : c->paces)
+    if (p.fires(c->ode_iters)) {
+      const int r = launch_stim(c, 0, p.r0, p.r1, p.c0, p.c1, p.value, p.floor_v);
+      if (r) return r;
+      fired = true;
+    }
+  if (fired) mark_written(c, 0);
+  return 0;
+}
+
 // The host half of the hook: the route has enqueued `n` iterations of `op`, after their record_observers nodes or,
-// `persistent`, as one persistent launch that recorded its probe values and frames itself.  Counts them; gathers
-// the frame of a recording iteration (the other routes end one iteration at a time; no recorder is armed behind
-// an upload) or marks the frame ledger behind the launch; marks the probe ledger behind a persistent launch.
+// `persistent`, as one persistent launch that recorded its probe values and frames and applied its pacing itself.
+// Counts them; gathers the frame of a recording iteration (the other routes end one iteration at a time; no recorder
+// or pacing is armed behind an upload) or marks the frame ledger behind the launch; then fires the pacing entries
+// of the iteration, so that the frame and the activation sample precede the stimulus and the probe follows it;
+// marks the probe ledger behind a persistent launch.  A stimulus marks the halos dirty: a sharded route that goes
+// on stepping refreshes them first.
 static int end_iterations(fib_ctx* c, int op, int n, bool persistent = false) {
   if (op != FIB_OP_ODE) return 0;
   const unsigned long long frames0 = c->frames_recorded();
@@ -1438,7 +1499,11 @@ static int end_iterations(fib_ctx* c, int op, int n, bool persistent = false) {
   int r = 0;
   if (c->frames && c->frames_recorded() != frames0)
     r = persistent ? c->frame_ledger.mark(c->stream, c->frames_recorded()) : launch_frame(c, c->frames_recorded() - 1);
+  if (!r && !persistent) r = fire_paces(c);
   if (!r && persistent && c->watch_var >= 0) r = c->probe_ledger.mark(c->stream, c->since(c->probe_armed_at));
+  c->paces.erase(std::remove_if(c->paces.begin(), c->paces.end(),
+                                [&](const fib_ctx::Pace& p) { return p.done(c->ode_iters); }),
+                 c->paces.end());
   return r;
 }
 
@@ -1547,9 +1612,13 @@ static int refresh_halos_nccl(fib_ctx* c) {
 // n_iter iterations of `op`, enqueued now
 static int step_now(fib_ctx* c, int op, int n_iter) {
   if (c->comm) {
+    // a pacing stimulus inside this call (halo_dirty) changed edge rows the neighbours hold as halo: every rank
+    // registered the same entries, so all of them take the same refresh
     int r = refresh_halos_nccl(c);
-    for (int i = 0; i < n_iter && !r; ++i)
+    for (int i = 0; i < n_iter && !r; ++i) {
       if (!(r = run_iteration_nccl(c, op))) r = end_iterations(c, op, 1);
+      if (!r && c->halo_dirty && i + 1 < n_iter) r = refresh_halos_nccl(c);
+    }
     return r;
   }
   if (c->persist == 1 && op == FIB_OP_ODE) {
@@ -1844,9 +1913,16 @@ extern "C" int fib_step_group(fib_ctx** cs, int n, int op, int n_iter) {
         for (int i = 0; i < n; ++i) cs[i]->cur ^= 1;
       }
     }
+    dirty = false;
     for (int i = 0; i < n; ++i) {
       DevGuard dg(cs[i]->cfg.device);
       if ((r = record_observers(cs[i], op)) || (r = end_iterations(cs[i], op, 1))) return r;
+      dirty |= cs[i]->halo_dirty;
+    }
+    if (dirty && it + 1 < n_iter) {   // a pacing stimulus changed edge rows the neighbours hold as halo
+      if ((r = group_copy_halos(cs, n, false))) return r;
+      if ((r = group_wait_neighbours(cs, n))) return r;
+      for (int i = 0; i < n; ++i) cs[i]->halo_dirty = false;
     }
   }
   return 0;
@@ -1861,13 +1937,46 @@ extern "C" int fib_stimulate(fib_ctx* c, int var, int r0, int r1, int c0, int c1
   if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
   DevGuard dg(c->cfg.device);
   FLUSH(c);
-  CU(wait_comm(c));
-  dim3 block(128), grid((c->g.W + 127) / 128, min(c->g.rows, 65535));
-  const PlaneRef pl = plane_of(c, var);
-  stim_kernel<<<grid, block, 0, c->stream>>>(pl.base, c->g, pl.halo, r0, r1, c0, c1, value, floor_v);
-  CU(cudaGetLastError());
-  c->launches++;
+  const int r = launch_stim(c, var, r0, r1, c0, c1, value, floor_v);
+  if (r) return r;
   mark_written(c, var);
+  return 0;
+}
+
+extern "C" int fib_pace_add(fib_ctx* c, int r0, int r1, int c0, int c1, float value, float floor_v, int first,
+                            int every, int count, int* id) {
+  if (!c || !id) return fail(FIB_E_ARG, "ctx/id is NULL");
+  if (first < 1 || count < 0 || (count != 1 && every < 1))
+    return fail(FIB_E_ARG, "fib_pace_add: need first >= 1, count >= 0 and every >= 1 unless count == 1 (got first %d, "
+                "every %d, count %d)", first, every, count);
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  if ((int)c->paces.size() >= kPaceMax)
+    return fail(FIB_E_STATE, "fib_pace_add: at most %d pacing entries per context", kPaceMax);
+  fib_ctx::Pace p;
+  p.id = c->pace_ids++;
+  p.r0 = r0;
+  p.r1 = r1;
+  p.c0 = c0;
+  p.c1 = c1;
+  p.value = value;
+  p.floor_v = floor_v;
+  p.at = c->ode_iters + (unsigned)first;
+  p.every = count == 1 ? 1 : (unsigned)every;
+  p.count = (unsigned)count;
+  c->paces.push_back(p);
+  *id = p.id;
+  return 0;
+}
+
+extern "C" int fib_pace_remove(fib_ctx* c, int id) {
+  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
+  if (id >= c->pace_ids) return fail(FIB_E_ARG, "fib_pace_remove: no pacing entry %d was added", id);
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  c->paces.erase(std::remove_if(c->paces.begin(), c->paces.end(),
+                                [&](const fib_ctx::Pace& p) { return id < 0 || p.id == id; }),
+                 c->paces.end());
   return 0;
 }
 

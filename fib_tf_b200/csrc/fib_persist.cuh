@@ -95,6 +95,8 @@ __device__ __forceinline__ void ll_load(const unsigned long long* p, float& v, u
 }
 // ---- arguments --------------------------------------------------------------------------------
 constexpr int kPersistMaxIters = 64;      // run() iterations one launch may cover (fib_step with n_iter > 1)
+constexpr int kPaceMax = 4;               // pacing entries per context (fib_pace_add); a launch's mask has one bit per iteration
+static_assert(kPersistMaxIters <= 64, "pace_mask holds one bit per iteration of a launch");
 
 template <int NS>
 struct PersistMaps {
@@ -134,21 +136,30 @@ struct PersistArgs {
   unsigned long long* act_iter;
   unsigned long long act_k0;
   float act_up, act_down;
-  // fib_frames_watch (FRAMES instantiations only: launches that record at least one frame): at the end of the
+  // fib_frames_watch (EVENTS instantiations only; frame_step0 > nsteps when the launch records none): at the end of the
   // iteration whose last step is step frame_step0 + j * frame_steps of this launch (counted from 1), the thread owning a cell
   // whose row and column are multiples of frame_stride writes plane frame_var (picked as probe_var is) into
-  // ring slot (frame_slot0 + j) % frame_cap -- exactly what frame_record_kernel gathers on the other paths
+  // ring slot (frame_slot0 + j) % frame_cap -- exactly what frame_record_kernel gathers on the other paths.  Frames
+  // and activation samples are taken before a stimulus of the same iteration, the probe value after it.
   float* frames;
   int frame_step0, frame_steps, frame_slot0, frame_cap;
   int frame_var, frame_stride, frame_cols;
   size_t frame_floats;
+  // fib_pace_add (EVENTS instantiations only): entry e < pace_n fires at the end of iteration `it` of this launch
+  // (counted from 0) when bit `it` of pace_mask[e] is set, as u := fmaxf(u, rows [r0, r1) x columns [c0, c1) of
+  // pace_rect[e] ? pace_value[e] : pace_floor[e]) -- exactly what stim_kernel does between the other paths' launches
+  int pace_n;
+  int pace_rect[kPaceMax][4];
+  float pace_value[kPaceMax], pace_floor[kPaceMax];
+  unsigned long long pace_mask[kPaceMax];
 };
 
 // ---- the kernel ----------------------------------------------------------------------------------
 // MS / MF: the cell types of the "slow" and "fast" steps of a schedule (Fenton4v twice; BeelerReuter<C,true>
 // and <C,false> for br.py's skip schedule).  TH: rows per tile.  PHASE: phase field present.  ACT: an
-// activation map is armed (fib_activation.cuh).  FRAMES: the launch records frames (fib_frames_watch); a
-// compile-time switch like ACT, so that the other instantiations keep their registers.
+// activation map is armed (fib_activation.cuh).  EVENTS: the launch records frames (fib_frames_watch) or paces
+// (fib_pace_add) at the end of some of its iterations; a compile-time switch like ACT, so that the other
+// instantiations keep their registers.
 //
 // Where the state lives between the steps of a launch:
 //   * a thread owns ONE column of its tile: its TH cells of every plane, the diffusing variable included
@@ -162,7 +173,7 @@ struct PersistArgs {
 //     and the rows of a column are read once per step (marching reuse in registers);
 //   * the rows of the neighbour tiles arrive through the mailbox and are written into the ring rows by
 //     the thread that will read them (each thread writes the three columns it reads: no barrier).
-template <class MS, class MF, int TH, bool PHASE, bool ACT, bool FRAMES>
+template <class MS, class MF, int TH, bool PHASE, bool ACT, bool EVENTS>
 __global__ void __launch_bounds__(kPersistThreads, 1)
 persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, const PersistArgs<MS, MF> a) {
   constexpr int NS = MS::NS;
@@ -421,6 +432,7 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
     // are all shown by themselves (`lazy`: every tile but a one-row last tile) the wait sits INSIDE the
     // cell function at that point -- gates, currents and the reaction term of the edge rows are computed
     // while the mailbox words are in flight, and receive -> publish is ring write, Laplacian, two adds.
+    float pre[TH];              // EVENTS: my cells before a stimulus
     if (active) {
       if (poll && !lazy) wait_ring();
       if (!plain_tile && !lazy) {     // the ring write may have refreshed rows loaded earlier
@@ -444,6 +456,26 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
         });
         if (TH - 1 < nrows) do_row(TH - 1, lap_row(TH - 1));
       }
+      // A firing iteration's stimulus goes into the values the neighbours and the next step read (the mailbox
+      // words and the shared tile below); the frame and activation samples keep the values before it (pre[]).
+      if constexpr (EVENTS) {
+#pragma unroll
+        for (int i = 0; i < TH; ++i) pre[i] = u[i];
+        if (sub + 1 == a.period) {
+          const int it = step / a.period;
+          for (int e = 0; e < a.pace_n; ++e)
+            if ((a.pace_mask[e] >> it) & 1ull) {
+              const bool in_c = c >= a.pace_rect[e][2] && c < a.pace_rect[e][3];
+#pragma unroll
+              for (int i = 0; i < TH; ++i) {
+                const int gr = r0 + i;
+                const float m = (gr >= a.pace_rect[e][0] && gr < a.pace_rect[e][1] && in_c) ? a.pace_value[e]
+                                                                                             : a.pace_floor[e];
+                u[i] = fmaxf(u[i], m);
+              }
+            }
+        }
+      }
       // (the last step's rows are not consumed through the mailbox: the next launch starts from the plane)
       if (need_top) ll_store(box(want + 1, tile, 0) + c, u[0], want + 1);
       if (need_bot) ll_store(box(want + 1, tile, 1) + c, u[TH - 1], want + 1);
@@ -464,7 +496,7 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
         a.ring[probe_n % FIB_PROBE_RING] = v;
         ++probe_n;
       }
-      if constexpr (FRAMES) {
+      if constexpr (EVENTS) {
         const int d = step + 1 - a.frame_step0;
         if (d >= 0 && d % a.frame_steps == 0 && active && c % a.frame_stride == 0) {
           float* f = a.frames + (size_t)((a.frame_slot0 + d / a.frame_steps) % a.frame_cap) * a.frame_floats +
@@ -472,7 +504,7 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
 #pragma unroll
           for (int i = 0; i < TH; ++i)
             if (i < nrows && (r0 + i) % a.frame_stride == 0) {
-              float v = u[i];
+              float v = pre[i];
 #pragma unroll
               for (int k = 0; k < NS; ++k)
                 if (a.frame_var == k + 1) v = s[k][i];
@@ -487,9 +519,11 @@ persist_kernel(const __grid_constant__ PersistMaps<MS::NS> maps, const Geom g, c
           for (int i = 0; i < TH; ++i)
             if (i < nrows) {
               const size_t idx = (size_t)(r0 + i) * pitch + c;
+              float x = u[i];
+              if constexpr (EVENTS) x = pre[i];
               const float pv = a.act_prev[idx];
-              a.act_prev[idx] = u[i];
-              act_cell(pv, u[i], k1, a.act_up, a.act_down, a.act_maps + idx, a.act_plane);
+              a.act_prev[idx] = x;
+              act_cell(pv, x, k1, a.act_up, a.act_down, a.act_maps + idx, a.act_plane);
             }
         }
         ++act_k;

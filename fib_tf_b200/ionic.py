@@ -34,7 +34,7 @@ Extra, optional config keys (all default to the reference's behaviour):
                  0 = never; the ranks agree on the number at the start of run())
 
 Collective calls under config['distributed'] (every rank must make them, in the same order):
-define(), run() (each iteration), fire_op(), image(), pot().eval() / _State[..].eval(),
+define(), run() (each iteration), fire_op(), pace(), stop_pacing(), image(), pot().eval() / _State[..].eval(),
 var[r, c].eval(), masked_image_mean(), excitable_fraction(), watch_activation(), activation_maps(),
 stop_activation(), frames(), checkpoint(), Checkpoint.wait(), restore(), close().  cl_observer callbacks run on
 the rank that owns row 20 only and therefore must not call any of these.
@@ -321,6 +321,44 @@ class IonicModel:
         elif op[0] == 'call':
             op[1]()
 
+    def pace(self, name, at, every=0, count=1):
+        """Schedules the op `name` registered with add_pace_op on the device: it fires after the absolute ODE
+        iterations n = at + 1 + j * every (n counts `iterations`), j = 0 .. count - 1, or until stop_pacing() with
+        count = 0.  That is the iteration after which a driver's `for i in run(): if i == at: fire_op(name)` fires,
+        in the first run() after define(); `at` usually comes from millisecond_to_step(t).  The stimulus is applied
+        while stepping (include/fib_b200.h fib_pace_add): a train needs no call per beat and keeps the persistent
+        kernel's batches.  Frames and activation maps see an iteration before its stimulus, the probe after it.
+        checkpoint() saves the schedules and restore() continues them.  At most 4 schedules are active at once.
+        ValueError if iteration at + 1 has already been stepped.  Collective when distributed."""
+        if not self.defined:
+            raise AssertionError('pace should be called after calling define')
+        op = self._ops.get(name)
+        if op is None or op[0] != 'pace':
+            raise ValueError('pace: %r is not an op registered with add_pace_op' % (name,))
+        at, every, count = int(at), int(every), int(count)
+        if count < 0 or (count != 1 and every < 1):
+            raise ValueError('pace: need count >= 0 and every >= 1 unless count == 1 (got every %d, count %d)'
+                             % (every, count))
+        if at + 1 <= self.iterations:
+            raise ValueError('pace: iteration %d (at = %d) has already been stepped (iterations = %d)'
+                             % (at + 1, at, self.iterations))
+        (r0, r1, c0, c1), v = op[1], op[2]
+        entry = {'name': name, 'rect': [max(r0, 0), r1, max(c0, 0), c1], 'value': v, 'floor': float(self.min_v),
+                 'next': at + 1, 'every': every, 'count': count}
+        entry['id'] = self._ctx.pace_add(*entry['rect'], v, entry['floor'], at + 1 - self.iterations, every, count)
+        self._pacing = self._active_pacing() + [entry]
+
+    def _active_pacing(self):
+        """The schedules whose last beat is still to come (the library drops the others by itself)."""
+        return [e for e in self.__dict__.get('_pacing') or [] if _ckpt.pacing_state([e], self.iterations)]
+
+    def stop_pacing(self, name=None):
+        """Removes the schedules of the op `name`, or every schedule.  Collective when distributed."""
+        for e in self.__dict__.get('_pacing') or []:
+            if name is None or e['name'] == name:
+                self._ctx.pace_remove(e['id'])
+        self._pacing = [e for e in self._active_pacing() if name is not None and e['name'] != name]
+
     # ---- the run() generator (ionic.py:171-245) ----------------------------------------------
     def run(self, im=None, keep_state=False, block=True):
         """Generator: advances the model one iteration (= dt_per_step time steps) per yield.
@@ -452,6 +490,7 @@ class IonicModel:
         """Placeholder replaced in subclasses: builds the initial state and the device context."""
         self.defined = True
         self.iterations = 0         # ODE iterations since define(), continued by restore()
+        self._pacing = []           # the pace() schedules: name, rect, value, floor, next, every, count, entry id
 
     def image(self):
         """[height x width] float ndarray in 0..1 encoding the transmembrane potential."""
@@ -669,8 +708,8 @@ class IonicModel:
 
     # ---- checkpoint and restart (fib_tf_b200/checkpoint.py) -----------------------------------
     def checkpoint(self, path):
-        """Saves the state after the iterations stepped so far, and the armed activation map and frame recorder,
-        to the directory `path` while stepping continues: stages a device copy of every shard behind the work
+        """Saves the state after the iterations stepped so far, the armed activation map and frame recorder, and
+        the pacing schedules still to fire, to the directory `path` while stepping continues: stages a device copy of every shard behind the work
         already enqueued and returns a Checkpoint at once; writer threads fill the files meanwhile.  Frames
         recorded so far move to the host list first (frames() returns them; they are not saved).  The previous
         checkpoint at `path` stays readable until Checkpoint.wait() replaces it, atomically where the file
@@ -690,7 +729,7 @@ class IonicModel:
             import torch.distributed as dist
             dist.barrier()
         ck = Checkpoint(self, path, partial, _ckpt.save_shard(self._ctx, partial, self._own_phase_rows()),
-                        self.iterations)
+                        self.iterations, _ckpt.pacing_state(self.__dict__.get('_pacing') or [], self.iterations))
         self._ckpt = ck
         return ck
 
@@ -708,7 +747,7 @@ class IonicModel:
 
     def restore(self, path):
         """Instead of define(): builds the device context exactly as define() does, then loads the checkpoint
-        at `path` -- saved on any number of ranks -- with the armed observers resumed, and continues
+        at `path` -- saved on any number of ranks -- with the armed observers and the pacing schedules resumed, and continues
         `iterations` from it.  ValueError if this model's config or phase field would compute differently.
         A large grid with no observer steps its first iterations behind its own upload.  Collective when
         distributed."""
@@ -718,6 +757,7 @@ class IonicModel:
         try:
             _ckpt.check_compatible(man, ctx, own)
             _ckpt.check_phase(path, man, ctx, own)
+            self._pacing = _ckpt.resume_pacing(ctx, man.get('pacing', []), man['iterations'])
             self._restore_pinned = _ckpt.restore_context(ctx, path, bottom_up=self._rank % 2 == 1, man=man)
         except BaseException:
             self.close()
@@ -753,9 +793,9 @@ class IonicModel:
 class Checkpoint:
     """A save started by IonicModel.checkpoint(); wait() completes it."""
 
-    def __init__(self, model, path, partial, writer, iterations):
+    def __init__(self, model, path, partial, writer, iterations, pacing=()):
         self.model, self.path, self.partial, self.writer = model, path, partial, writer
-        self.iterations = iterations
+        self.iterations, self.pacing = iterations, list(pacing)
         self.done = False
 
     def wait(self):
@@ -782,7 +822,8 @@ class Checkpoint:
                 if failed:
                     shutil.rmtree(self.partial, ignore_errors=True)
                 else:
-                    man = _ckpt.manifest(self.writer.ctx, parts[0][3], [p[2] for p in parts], self.iterations)
+                    man = _ckpt.manifest(self.writer.ctx, parts[0][3], [p[2] for p in parts], self.iterations,
+                                         self.pacing)
                     _ckpt.write_manifest(self.partial, man)
                     _ckpt.publish(self.partial, self.path)
             except Exception as e:

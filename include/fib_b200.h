@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define FIB_ABI_VERSION 5
+#define FIB_ABI_VERSION 6
 
 typedef struct fib_ctx fib_ctx;
 
@@ -196,6 +196,32 @@ int fib_last_kernel(char *buf, size_t n);
  * X := max(X, inside [r0,r1)x[c0,c1) ? value : floor_v) over the whole plane, GLOBAL coords. */
 int fib_stimulate(fib_ctx *ctx, int var, int r0, int r1, int c0, int c1, float value,
                   float floor_v);
+
+/* pacing: stimulus trains scheduled once and applied on the device while stepping (S1 trains at a basic cycle
+ * length, burst pacing, S1-S2 protocols), so that a train neither needs the host every beat nor cuts the
+ * persistent kernel's 64-iteration batches.
+ *   when     k counts the FIB_OP_ODE iterations enqueued since fib_pace_add (k = 1 is the first iteration after
+ *            the call; FIB_OP_SLOW does not count).  The entry fires at the end of iterations k = first + j * every,
+ *            j = 0 .. count - 1; count = 0 fires until the entry is removed.  FIB_E_ARG unless first >= 1,
+ *            count >= 0 and every >= 1 (every is ignored when count == 1).
+ *   effect   exactly fib_stimulate(ctx, 0, r0, r1, c0, c1, value, floor_v) -- the diffusing variable, the rectangle
+ *            in GLOBAL coordinates, any rectangle fib_stimulate accepts -- issued right after iteration k is
+ *            enqueued and before anything else.  So the activation sample and the frame of iteration k are taken
+ *            BEFORE the stimulus (observers sample before the caller acts), the probe ring's value of iteration k
+ *            AFTER it (as after a fib_stimulate), and iteration k + 1 steps from the stimulated state.  Entries
+ *            that fire at the same k are all applied (each is an fmaxf with the plane, so their order does not
+ *            matter).  The persistent kernel applies them inside its launch; the other routes launch the stimulus
+ *            after the iteration.  Row shards apply their own rows; every rank (every context of a
+ *            fib_step_group) must add the same entries in the same order.  A stimulus on a shard's edge rows
+ *            reaches the neighbour before its next iteration, inside one fib_step call too.
+ *   limits   at most 4 entries per context: a fifth is FIB_E_STATE.  An entry is dropped by itself once its
+ *            last beat has been enqueued.  An armed entry keeps fib_set_rect_async blocks out of the pipelined
+ *            upload.  Both calls launch the deferred iterations first.
+ * fib_pace_add returns the entry's id in *id (ids count up from 0 per context).  fib_pace_remove removes entry
+ * `id` (a no-op when it has finished), or every entry when id < 0; FIB_E_ARG for an id that was never handed out. */
+int fib_pace_add(fib_ctx *ctx, int r0, int r1, int c0, int c1, float value, float floor_v,
+                 int first, int every, int count, int *id);
+int fib_pace_remove(fib_ctx *ctx, int id);
 
 /* ---- probes: replaces Variable[r,c] reads (ionic.py:216, court.py:109-110) --------------
  * Synchronous.  FIB_E_ARG if (row,col) is not in this shard. */
