@@ -63,11 +63,17 @@ __device__ __forceinline__ void load_reflect_row(const float* __restrict__ ph, i
 
 // ionic.py:51-53, same association order as the reference, no FMA contraction: given identical
 // inputs this is bit-identical to the NumPy oracle.
+// lap9_combine: its last three operations, edges + 0.5 corners - 6 C, on the two sums.  T = float, or
+// f2 for two neighbouring cells (FADD2 / FFMA2; each lane rounds like the scalar form, fib_math.cuh).
+template <class T>
+__device__ __forceinline__ T lap9_combine(T edges, T corners, T C) {
+  return sub_rn(add_rn(edges, mul_rn(T(0.5f), corners)), mul_rn(T(6.0f), C));
+}
 __device__ __forceinline__ float lap9(float N, float S, float Wv, float E, float NW, float SW,
                                       float NE, float SE, float C) {
   float edges = __fadd_rn(__fadd_rn(__fadd_rn(N, S), Wv), E);
   float corners = __fadd_rn(__fadd_rn(__fadd_rn(NW, SW), NE), SE);
-  return __fsub_rn(__fadd_rn(edges, __fmul_rn(0.5f, corners)), __fmul_rn(6.0f, C));
+  return lap9_combine(edges, corners, C);
 }
 
 // ionic.py:78-80: ((X_S-X_N)(phi_S-phi_N) + (X_E-X_W)(phi_E-phi_W)) / (4 phi_C)
