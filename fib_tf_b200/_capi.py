@@ -43,7 +43,7 @@ class FibConfig(C.Structure):
         ('dt', C.c_double), ('diff', C.c_double),
         ('flags', C.c_uint32), ('device', C.c_int32),
         ('row0', C.c_int32), ('rows', C.c_int32),
-        ('steps_per_launch', C.c_int32), ('reserved', C.c_int32 * 6),
+        ('steps_per_launch', C.c_int32), ('replicas', C.c_int32), ('reserved', C.c_int32 * 5),
     ]
 
 
@@ -105,8 +105,13 @@ _SIGNATURES = {
     'fib_step': (C.c_int, [_P, C.c_int, C.c_int]),
     'fib_step_group': (C.c_int, [C.POINTER(_P), C.c_int, C.c_int, C.c_int]),
     'fib_stimulate': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float]),
+    'fib_stimulate_replica': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float,
+                                        C.c_float]),
+    'fib_set_replica_diff': (C.c_int, [_P, C.POINTER(C.c_double), C.c_size_t]),
     'fib_pace_add': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_int, C.c_int,
                                C.c_int, C.POINTER(C.c_int)]),
+    'fib_pace_add_replica': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float,
+                                       C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int)]),
     'fib_pace_remove': (C.c_int, [_P, C.c_int]),
     'fib_probe': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _FP]),
     'fib_weighted_sum': (C.c_int, [_P, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
@@ -186,20 +191,25 @@ class Context:
     """One shard of one model on one GPU (fib_ctx*)."""
 
     def __init__(self, model, height, width, dt, diff, flags=0, device=0, row0=0, rows=0,
-                 steps_per_launch=0):
+                 steps_per_launch=0, replicas=1):
+        """`replicas` > 1: a batched context of that many grids of height x width (include/fib_b200.h, Replicas),
+        addressed as one grid of replicas * height rows; `rows` and `height` stay those of one replica."""
         L = lib()
         cfg = FibConfig()
         cfg.struct_size = C.sizeof(FibConfig)
         cfg.model, cfg.height, cfg.width = int(model), int(height), int(width)
         cfg.dt, cfg.diff, cfg.flags, cfg.device = float(dt), float(diff), int(flags), int(device)
         cfg.row0, cfg.rows, cfg.steps_per_launch = int(row0), int(rows), int(steps_per_launch)
+        cfg.replicas = int(replicas)
         h = _P()
         check(L.fib_create(C.byref(cfg), C.byref(h)))
         self._h = h
         self.model, self.dt, self.diff, self.flags = int(model), float(dt), float(diff), int(flags)
+        self.replicas = max(int(replicas), 1)
+        self.replica_diff = [self.diff] * self.replicas      # diff of every replica (set_replica_diff)
         self.height, self.width = int(height), int(width)
         self.row0 = int(row0) if rows else 0
-        self.rows = int(rows) if rows else int(height)
+        self.rows = int(rows) if rows else int(height) * self.replicas
         self.nvars = L.fib_num_vars(h)
         self.var_names = [L.fib_var_name(h, i).decode() for i in range(self.nvars)]
         self.dt_per_step = L.fib_dt_per_step(h)
@@ -299,15 +309,22 @@ class Context:
     def step(self, op=OP_ODE, n_iter=1):
         check(lib().fib_step(self._h, op, n_iter))
 
-    def stimulate(self, var, r0, r1, c0, c1, value, floor_v):
-        check(lib().fib_stimulate(self._h, self.var(var), r0, r1, c0, c1, value, floor_v))
+    def set_replica_diff(self, diff):
+        """diff of every replica of a batched context, from the next iteration on."""
+        a = np.ascontiguousarray(diff, dtype=np.float64)
+        check(lib().fib_set_replica_diff(self._h, a.ctypes.data_as(C.POINTER(C.c_double)), a.size))
+        self.replica_diff = [float(x) for x in a]
 
-    def pace_add(self, r0, r1, c0, c1, value, floor_v, first, every=0, count=1):
-        """Schedule stimulate(diffusing variable, r0, r1, c0, c1, value, floor_v) after the ODE iterations
+    def stimulate(self, var, r0, r1, c0, c1, value, floor_v, replica=-1):
+        """replica -1: the rectangle in every replica (rows local to a replica), else in that replica only."""
+        check(lib().fib_stimulate_replica(self._h, int(replica), self.var(var), r0, r1, c0, c1, value, floor_v))
+
+    def pace_add(self, r0, r1, c0, c1, value, floor_v, first, every=0, count=1, replica=-1):
+        """Schedule stimulate(diffusing variable, r0, r1, c0, c1, value, floor_v, replica) after the ODE iterations
         k = first + j * every (j < count; count 0: until removed) counted from now, k = 1 the next; returns the id."""
         i = C.c_int()
-        check(lib().fib_pace_add(self._h, int(r0), int(r1), int(c0), int(c1), float(value), float(floor_v),
-                                 int(first), int(every), int(count), C.byref(i)))
+        check(lib().fib_pace_add_replica(self._h, int(replica), int(r0), int(r1), int(c0), int(c1), float(value),
+                                         float(floor_v), int(first), int(every), int(count), C.byref(i)))
         return i.value
 
     def pace_remove(self, pace_id=-1):

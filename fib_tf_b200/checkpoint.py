@@ -50,6 +50,9 @@ def arithmetic_config(ctx):
     """The model and the config keys of a context that change what it computes."""
     cfg = {'model': MODEL_NAMES[ctx.model], 'height': int(ctx.height), 'width': int(ctx.width),
            'dt': float(ctx.dt), 'diff': float(ctx.diff)}
+    replicas = getattr(ctx, 'replicas', 1)
+    if replicas > 1:        # the parts are then [replicas * height, width]: replica b is rows b * height ..
+        cfg.update(replicas=int(replicas), diff=[float(d) for d in ctx.replica_diff])
     for key, bit in ARITH_FLAGS:
         cfg[key] = bool(ctx.flags & bit)
     return cfg
@@ -154,6 +157,8 @@ def pacing_state(entries, iterations):
         out.append({'name': e['name'], 'rect': [int(x) for x in e['rect']], 'value': float(e['value']),
                     'floor': float(e['floor']), 'next': int(e['next'] + done * step), 'every': int(e['every']),
                     'count': int(e['count'] - done) if e['count'] else 0})
+        if e.get('replica') is not None:                # a batched model's entry of one replica
+            out[-1]['replica'] = int(e['replica'])
     return out
 
 
@@ -166,7 +171,8 @@ def resume_pacing(ctx, entries, iterations):
         if e['next'] <= iterations:
             raise CheckpointError('pacing entry %r: next beat after iteration %d, but the run continues from %d'
                                   % (e['name'], e['next'], iterations))
-        pid = ctx.pace_add(*e['rect'], e['value'], e['floor'], e['next'] - iterations, e['every'], e['count'])
+        where = {'replica': e['replica']} if e.get('replica') is not None else {}
+        pid = ctx.pace_add(*e['rect'], e['value'], e['floor'], e['next'] - iterations, e['every'], e['count'], **where)
         out.append(dict(e, id=pid))
     return out
 
@@ -265,8 +271,9 @@ def read_rows(path, part, r0, r1, man=None):
     array, assembled from whichever shard files cover them (memory-mapped: only these rows are read)."""
     man = load_manifest(path) if man is None else man
     width = man['config']['width']
-    if not 0 <= r0 < r1 <= man['config']['height']:
-        raise ValueError('rows [%d, %d) outside the grid of height %d' % (r0, r1, man['config']['height']))
+    height = man['config']['height'] * man['config'].get('replicas', 1)
+    if not 0 <= r0 < r1 <= height:
+        raise ValueError('rows [%d, %d) outside the grid of height %d' % (r0, r1, height))
     out = np.empty((r1 - r0, width), np.float32)
     covered = 0
     for sh in man['shards']:
@@ -291,7 +298,9 @@ def check_compatible(man, ctx, phase_rows=None):
     """ValueError naming the first key in which `ctx` (and `phase_rows`, its shard's rows of the phase field or
     None) would compute differently from the run that was saved."""
     mine = arithmetic_config(ctx)
-    for key, saved in man['config'].items():
+    saved_cfg = dict({'replicas': 1}, **man['config'])
+    mine.setdefault('replicas', 1)
+    for key, saved in saved_cfg.items():
         if mine.get(key) != saved:
             raise ValueError('checkpoint was saved with %s=%r, this model has %s=%r' % (key, saved, key, mine.get(key)))
     if man['phase'] != (phase_rows is not None):

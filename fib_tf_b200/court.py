@@ -70,9 +70,9 @@ class Courtemanche(IonicModel):
                 self.init_state_variable(state, name, val)
             if s1:
                 state['V'][:, :25] = 20.0
-        else:   # a full-grid dict saved by run(keep_state=True): take this shard's rows
-            state = {k: np.asarray(v, dtype=np.float32)[self._row0:self._row0 + self._rows]
-                     for k, v in state.items()}
+        else:   # a full-grid dict saved by run(keep_state=True): take this shard's rows ([H, W] for every
+            # replica of a batched model, or [replicas, H, W])
+            state = {k: self._own_rows(v) for k, v in state.items()}
         missing = [n for n in ctx.var_names if n not in state]
         if missing:
             raise KeyError('state is missing %s' % missing)
@@ -128,7 +128,7 @@ class Courtemanche(IonicModel):
         if self._ctx is not None:
             return self._ctx
         if getattr(self, '_aux_ctx', None) is None:     # calc_inter before define()
-            self._aux_ctx = _capi.Context(self.MODEL_ID, 3, 3, self.dt, self.diff)
+            self._aux_ctx = _capi.Context(self.MODEL_ID, 3, 3, self.dt, self.replica_diff[0])
         return self._aux_ctx
 
     def pot(self):

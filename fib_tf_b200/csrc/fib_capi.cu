@@ -140,7 +140,9 @@ struct Ledger {
 
 struct fib_ctx {
   fib_config cfg;
-  Geom g;
+  Geom g;                             // this shard; a batched context: all replicas as one grid of nrep * height rows
+  int nrep = 1;                       // replicas (fib_config.replicas)
+  float* zddt = nullptr;              // nrep > 1: fp32(diff_b * dt) of every replica (the kernels' StepArgs::zddt)
   int nvars = 0, dt_per_step = 1, sms = 148;
   const char** names = nullptr;
   cudaStream_t stream = nullptr, comm_stream = nullptr, copy_stream = nullptr;
@@ -205,7 +207,7 @@ struct fib_ctx {
   // pacing (fib_pace_add): entry p stimulates the diffusing variable right after the ODE iterations whose ode_iters
   // is p.at + j * p.every, j < p.count (count 0: every such iteration); dropped once its last beat is enqueued
   struct Pace {
-    int id, r0, r1, c0, c1;
+    int id, replica, r0, r1, c0, c1;
     float value, floor_v;
     unsigned long long at, every, count;
     bool fires(unsigned long long n) const {
@@ -248,6 +250,8 @@ struct fib_ctx {
   bool top_is_border() const { return g.row0 == 0; }
   bool bottom_is_border() const { return g.row0 + g.rows == g.H; }
   bool observing() const { return watch_var >= 0 || act_maps || frames || !paces.empty(); }
+  // what the step kernels see: ONE replica (the whole shard when nrep == 1), launched nrep times along blockIdx.z
+  Geom step_geom() const { return nrep == 1 ? g : Geom{g.H / nrep, g.W, 0, g.H / nrep, g.pitch}; }
 };
 
 static void drop_graphs(fib_ctx* c) {
@@ -268,12 +272,13 @@ struct DevGuard {
 // ------------------------------------------------------------------------------------------
 // ionic.py:144-163: X := max(X, s) with s = value inside the rectangle and floor_v elsewhere.
 // fmaxf: tf.maximum on the reference's GPU target returns the non-NaN operand (see clip_tf).
-__global__ void stim_kernel(float* __restrict__ x, Geom g, int halo, int r0, int r1, int c0, int c1,
-                            float value, float floor_v) {
+// Over local rows [lr0, lr0 + nrows); the rectangle's rows count within a replica of rh rows (rh = H: the grid).
+__global__ void stim_kernel(float* __restrict__ x, Geom g, int halo, int rh, int lr0, int nrows, int r0, int r1,
+                            int c0, int c1, float value, float floor_v) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= g.W) return;
-  for (int lr = blockIdx.y; lr < g.rows; lr += gridDim.y) {
-    const int gr = g.row0 + lr;
+  for (int lr = lr0 + (int)blockIdx.y; lr < lr0 + nrows; lr += gridDim.y) {
+    const int gr = (g.row0 + lr) % rh;
     const float m = (gr >= r0 && gr < r1 && c >= c0 && c < c1) ? value : floor_v;
     float* p = x + (size_t)(lr + halo) * g.pitch + c;
     const float v = *p;
@@ -283,11 +288,14 @@ __global__ void stim_kernel(float* __restrict__ x, Geom g, int halo, int r0, int
 
 // fib_set_phase: flag the 32-column blocks of each row whose phase term can be non-zero, i.e.
 // where phi is not constant over rows r-1..r+1 (REFLECT) x columns c0-1..c0+32 (clipped: the
-// reflected columns -1 -> 1 and W -> W-2 lie inside that range).
+// reflected columns -1 -> 1 and W -> W-2 lie inside that range).  g: one replica (blockIdx.z), as the step
+// kernels see it, so the REFLECT stays inside the replica.
 __global__ void phase_mask_kernel(const float* __restrict__ phase, Geom g, unsigned char* __restrict__ mask,
                                   int mpitch) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= mpitch) return;
+  phase += (size_t)blockIdx.z * g.rows * g.pitch;
+  mask += (size_t)blockIdx.z * g.rows * mpitch;
   const int c0 = max(b * 32 - 1, 0), c1 = min(b * 32 + 32, g.W - 1);
   for (int lr = blockIdx.y; lr < g.rows; lr += gridDim.y) {
     const int gr = g.row0 + lr;
@@ -307,8 +315,12 @@ __global__ void phase_mask2_kernel(const float* __restrict__ phase, Geom g, unsi
                                    int mpitch) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= mpitch) return;
+  phase += (size_t)blockIdx.z * g.rows * g.pitch;
+  mask += (size_t)blockIdx.z * g.rows * mpitch;
   const int c0 = max(b * 32 - 1, 0), c1 = min(b * 32 + 32, g.W - 1);
   for (int lr = (int)blockIdx.y - 1; lr <= g.rows; lr += gridDim.y) {
+    // the rows just outside a replica are its neighbours' first / last rows: theirs to flag
+    if ((lr < 0 && blockIdx.z > 0) || (lr == g.rows && blockIdx.z + 1 < gridDim.z)) continue;
     const int gr = g.row0 + lr;
     bool same = true;
     if (gr >= 0 && gr < g.H) {
@@ -482,6 +494,14 @@ extern "C" int fib_host_free(void* p) {
 }
 
 static int create_resources(fib_ctx* c);
+// fp32(diff_b * dt) of every replica, folded in double as fenton_params / br_params / launch_court fold cfg.diff
+static int upload_replica_diff(fib_ctx* c, const double* diff) {
+  std::vector<float> ddt(c->nrep);
+  for (int b = 0; b < c->nrep; ++b) ddt[b] = (float)(diff[b] * c->cfg.dt);
+  CU(cudaMemcpyAsync(c->zddt, ddt.data(), c->nrep * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return 0;
+}
 extern "C" int fib_create(const fib_config* cfg, fib_ctx** out) {
   if (!cfg || !out) return fail(FIB_E_ARG, "cfg/out is NULL");
   if (cfg->struct_size != sizeof(fib_config))
@@ -498,6 +518,11 @@ extern "C" int fib_create(const fib_config* cfg, fib_ctx** out) {
   if (cfg->steps_per_launch == 2 && (cfg->model != FIB_FENTON4V || cfg->width % 4 != 0))
     return fail(FIB_E_ARG, "steps_per_launch=2 needs the Fenton 4v model and a width that is a multiple "
                 "of 4 (got model %d, width %d)", cfg->model, cfg->width);
+  const int nrep = cfg->replicas < 1 ? 1 : cfg->replicas;
+  if (cfg->replicas < 0 || nrep > 65535)
+    return fail(FIB_E_ARG, "replicas=%d: 0 or 1 (one grid) up to 65535", cfg->replicas);
+  if (nrep > 1 && cfg->rows != 0)
+    return fail(FIB_E_ARG, "replicas=%d: a batched context cannot be a row shard (rows must be 0)", nrep);
   int rows = cfg->rows == 0 ? cfg->height : cfg->rows;
   int row0 = cfg->rows == 0 ? 0 : cfg->row0;
   if (row0 < 0 || rows < 1 || row0 + rows > cfg->height)
@@ -505,10 +530,10 @@ extern "C" int fib_create(const fib_config* cfg, fib_ctx** out) {
                 cfg->height);
   if (cfg->steps_per_launch == 2 && rows != cfg->height && rows < kFuseHalo)
     return fail(FIB_E_ARG, "steps_per_launch=2: a shard must own at least %d rows (got %d)", kFuseHalo, rows);
-  if ((long long)(rows + 2 * kFuseHalo) * ((cfg->width + 31) / 32 * 32) >= (1LL << 31))
-    return fail(FIB_E_ARG, "shard of %d rows x %d columns exceeds 2^31 cells per plane: the kernels "
-                "index planes with 32-bit element offsets; shard the grid over more GPUs", rows,
-                cfg->width);
+  if ((long long)((long long)rows * nrep + 2 * kFuseHalo) * ((cfg->width + 31) / 32 * 32) >= (1LL << 31))
+    return fail(FIB_E_ARG, "shard of %lld rows x %d columns exceeds 2^31 cells per plane: the kernels "
+                "index planes with 32-bit element offsets; shard the grid over more GPUs, or use fewer replicas",
+                (long long)rows * nrep, cfg->width);
   int ndev = 0;
   CU(cudaGetDeviceCount(&ndev));
   if (cfg->device < 0 || cfg->device >= ndev)
@@ -517,10 +542,11 @@ extern "C" int fib_create(const fib_config* cfg, fib_ctx** out) {
 
   fib_ctx* c = new fib_ctx();
   c->cfg = *cfg;
-  c->g.H = cfg->height;
+  c->nrep = nrep;
+  c->g.H = cfg->height * nrep;
   c->g.W = cfg->width;
   c->g.row0 = row0;
-  c->g.rows = rows;
+  c->g.rows = rows * nrep;
   c->g.pitch = (cfg->width + 31) / 32 * 32;
   // a failure half way (e.g. out of memory at 32768^2 on a busy GPU) must release what exists
   const int rc = create_resources(c);
@@ -583,6 +609,12 @@ static int create_resources(fib_ctx* c) {
     }
   }
   CU(cudaMalloc(&c->red, 2 * sizeof(double)));
+  if (c->nrep > 1) {
+    CU(cudaMalloc(&c->zddt, c->nrep * sizeof(float)));
+    const std::vector<double> diff(c->nrep, cfg->diff);
+    const int r = upload_replica_diff(c, diff.data());
+    if (r) return r;
+  }
   if (cfg->model >= FIB_COURT) {
     CU(cudaMalloc(&c->lut, sizeof(float) * kLutRows * kLutCols));
     CU(cudaMalloc(&c->lut_t, sizeof(float) * kLutCols * kLutTStride));
@@ -633,6 +665,7 @@ extern "C" int fib_destroy(fib_ctx* c) {
   cudaFree(c->lut);
   cudaFree(c->lut_t);
   cudaFree(c->red);
+  cudaFree(c->zddt);
   cudaFreeHost(c->ring);
   c->probe_ledger.destroy();
   cudaFree(c->ring_count);
@@ -697,12 +730,17 @@ static cudaError_t wait_comm(fib_ctx* c) {
   return cudaStreamWaitEvent(c->stream, c->ev_comm, 0);
 }
 
-// the stimulus of fib_stimulate on the CURRENT plane `var` (enqueue-only; the caller marks the plane written)
-static int launch_stim(fib_ctx* c, int var, int r0, int r1, int c0, int c1, float value, float floor_v) {
+// the stimulus of fib_stimulate_replica on the CURRENT plane `var` (enqueue-only; the caller marks the plane
+// written): rows local to a replica, in replica `replica` only or (-1) in every replica
+static int launch_stim(fib_ctx* c, int var, int replica, int r0, int r1, int c0, int c1, float value,
+                       float floor_v) {
   CU(wait_comm(c));
-  dim3 block(128), grid((c->g.W + 127) / 128, min(c->g.rows, 65535));
+  const int rh = c->g.H / c->nrep;
+  const int lr0 = replica < 0 ? 0 : replica * rh, nrows = replica < 0 ? c->g.rows : rh;
+  dim3 block(128), grid((c->g.W + 127) / 128, min(nrows, 65535));
   const PlaneRef pl = plane_of(c, var);
-  stim_kernel<<<grid, block, 0, c->stream>>>(pl.base, c->g, pl.halo, r0, r1, c0, c1, value, floor_v);
+  stim_kernel<<<grid, block, 0, c->stream>>>(pl.base, c->g, pl.halo, rh, lr0, nrows, r0, r1, c0, c1, value,
+                                             floor_v);
   CU(cudaGetLastError());
   c->launches++;
   return 0;
@@ -849,7 +887,8 @@ static int set_rect_impl(fib_ctx* c, int var, int r0, int r1, int c0, int c1, co
     // result then run block by block BEHIND the copies instead of after them (finish_upload_session).
     // On an NCCL shard the block order may also run bottom to top (odd ranks do, so that both shards of a seam
     // either begin or end there: fib_step_behind_upload).
-    const bool eligible = (c->comm ? c->pipeline_nccl : c->g.rows == c->g.H) && c0 == 0 && c1 == c->g.W &&
+    // (a batched context steps whole replicas only: not the row blocks of the skewed schedule)
+    const bool eligible = (c->comm ? c->pipeline_nccl : c->g.rows == c->g.H) && c->nrep == 1 && c0 == 0 && c1 == c->g.W &&
                           !c->observing() && (long long)c->g.rows * c->g.W >= c->pipeline_min_cells;
     const int row_end = c->g.row0 + c->g.rows;
     const int dir = c->up_session ? c->up_dir : (r0 == c->g.row0 ? +1 : (r1 == row_end && c->comm ? -1 : 0));
@@ -953,15 +992,17 @@ extern "C" int fib_set_phase(fib_ctx* c, const float* rows_host, int first_row, 
   c->pmask_pitch = (c->g.W + 31) / 32;
   if (!c->pmask) CU(cudaMalloc(&c->pmask, (size_t)c->g.rows * c->pmask_pitch));
   {
-    dim3 block(64), grid((c->pmask_pitch + 63) / 64, min(c->g.rows, 65535));
-    phase_mask_kernel<<<grid, block, 0, c->stream>>>(c->phase, c->g, c->pmask, c->pmask_pitch);
+    const Geom sg = c->step_geom();
+    dim3 block(64), grid((c->pmask_pitch + 63) / 64, min(sg.rows, 65535), c->nrep);
+    phase_mask_kernel<<<grid, block, 0, c->stream>>>(c->phase, sg, c->pmask, c->pmask_pitch);
     CU(cudaGetLastError());
     c->launches++;
   }
   if (c->fuse == 2) {
     if (!c->pmask2) CU(cudaMalloc(&c->pmask2, (size_t)(c->g.rows + 2) * c->pmask_pitch));
-    dim3 block(64), grid((c->pmask_pitch + 63) / 64, min(c->g.rows + 2, 65535));
-    phase_mask2_kernel<<<grid, block, 0, c->stream>>>(c->phase2, c->g, c->pmask2, c->pmask_pitch);
+    const Geom sg = c->step_geom();
+    dim3 block(64), grid((c->pmask_pitch + 63) / 64, min(sg.rows + 2, 65535), c->nrep);
+    phase_mask2_kernel<<<grid, block, 0, c->stream>>>(c->phase2, sg, c->pmask2, c->pmask_pitch);
     CU(cudaGetLastError());
     c->launches++;
   }
@@ -1069,6 +1110,8 @@ static void fill_common(fib_ctx* c, StepArgs<M>& a, int lr0, int nrows) {
   a.lut = c->lut_t;
   a.lr0 = lr0;
   a.nrows = nrows;
+  a.nz = c->nrep;
+  a.zddt = c->zddt;
 }
 
 template <int MODE, bool LUT, bool US>
@@ -1092,7 +1135,7 @@ static cudaError_t launch_court(fib_ctx* c, int lr0, int nrows) {
   a.p.k_to = (float)((1.0 - 0.5 * chron) * 100 * 0.1652);
   a.p.k_Kur = (float)((1.0 - 0.5 * chron) * 100);
   a.p.k_CaL = (float)((1.0 - 0.7 * chron) * 100 * 0.12375);
-  return launch_step<M>(c->g, a, c->stream, c->sms);
+  return launch_step<M>(c->step_geom(), a, c->stream, c->sms);
 }
 
 // The tables the model's flags ask for have been set: checked before any step launch, and by fib_step before it
@@ -1141,6 +1184,10 @@ static cudaError_t with_br_flavour(const fib_ctx* c, F&& fn) {
 // One time step `sub` of op over local rows [lr0, lr0+nrows).  Does NOT flip the ping-pong.
 static int launch_substep(fib_ctx* c, int op, int sub, int lr0, int nrows) {
   if (nrows <= 0) return 0;
+  // a batched context launches whole replicas only (no upload session, no shards): local rows = replica rows
+  if (c->nrep > 1 && (lr0 != 0 || nrows != c->g.rows))
+    return fail(FIB_E_STATE, "internal: a row range [%d,%d) of a batched context", lr0, lr0 + nrows);
+  if (c->nrep > 1) nrows = c->g.rows / c->nrep;
   const int tr = check_tables(c);
   if (tr) return tr;
   const uint32_t fl = c->cfg.flags;
@@ -1156,14 +1203,16 @@ static int launch_substep(fib_ctx* c, int op, int sub, int lr0, int nrows) {
         f.lr0 = lr0;
         f.nrows = nrows;
         f.R = 0;
+        f.nz = c->nrep;
+        f.zddt = c->zddt;
         f.p = fenton_params(c);
-        e = launch_fused2(c->g, f, c->stream, c->sms);
+        e = launch_fused2(c->step_geom(), f, c->stream, c->sms);
         break;
       }
       StepArgs<Fenton4v> a;
       fill_common<Fenton4v>(c, a, lr0, nrows);
       a.p = fenton_params(c);
-      e = launch_step<Fenton4v>(c->g, a, c->stream, c->sms);
+      e = launch_step<Fenton4v>(c->step_geom(), a, c->stream, c->sms);
       break;
     }
     case FIB_BR: {
@@ -1174,7 +1223,7 @@ static int launch_substep(fib_ctx* c, int op, int sub, int lr0, int nrows) {
         StepArgs<M> a;
         fill_common<M>(c, a, lr0, nrows);
         a.p = br_params<typename M::Params>(c, n);
-        return launch_step<M>(c->g, a, c->stream, c->sms);
+        return launch_step<M>(c->step_geom(), a, c->stream, c->sms);
       };
       e = with_br_flavour(c, [&](auto slow, auto fast) { return n > 0 ? go(slow) : go(fast); });
       break;
@@ -1395,7 +1444,8 @@ static void decide_persist(fib_ctx* c) {
   if (!env_on || (c->cfg.flags & FIB_F_NO_PERSIST)) return;
   const int model = c->cfg.model;
   if (!(model == FIB_FENTON4V || model == FIB_BR) || c->fuse != 1) return;
-  if (c->comm || c->g.rows != c->g.H || c->g.W > kPersistThreads) return;
+  // one CTA per SM for one grid: a batched context exists to leave that regime
+  if (c->comm || c->nrep > 1 || c->g.rows != c->g.H || c->g.W > kPersistThreads) return;
   int coop = 0;
   if (cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, c->cfg.device) != cudaSuccess || !coop) return;
   const int max_th = model == FIB_FENTON4V ? 8 : 4;
@@ -1477,7 +1527,7 @@ static int fire_paces(fib_ctx* c) {
   bool fired = false;
   for (const auto& p : c->paces)
     if (p.fires(c->ode_iters)) {
-      const int r = launch_stim(c, 0, p.r0, p.r1, p.c0, p.c1, p.value, p.floor_v);
+      const int r = launch_stim(c, 0, p.replica, p.r0, p.r1, p.c0, p.c1, p.value, p.floor_v);
       if (r) return r;
       fired = true;
     }
@@ -1866,6 +1916,7 @@ extern "C" int fib_step_group(fib_ctx** cs, int n, int op, int n_iter) {
   int row = 0;
   for (int i = 0; i < n; ++i) {
     if (!cs[i]) return fail(FIB_E_ARG, "shard %d is NULL", i);
+    if (cs[i]->nrep > 1) return fail(FIB_E_ARG, "fib_step_group: shard %d is a batched context", i);
     if (cs[i]->g.row0 != row || cs[i]->g.H != cs[0]->g.H || cs[i]->g.W != cs[0]->g.W ||
         cs[i]->cfg.model != cs[0]->cfg.model || cs[i]->cfg.flags != cs[0]->cfg.flags ||
         cs[i]->fuse != cs[0]->fuse)
@@ -1931,21 +1982,45 @@ extern "C" int fib_step_group(fib_ctx** cs, int n, int op, int n_iter) {
 // ------------------------------------------------------------------------------------------
 // stimulus, probes, reductions
 // ------------------------------------------------------------------------------------------
-extern "C" int fib_stimulate(fib_ctx* c, int var, int r0, int r1, int c0, int c1, float value,
-                             float floor_v) {
-  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
-  if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
+extern "C" int fib_set_replica_diff(fib_ctx* c, const double* diff, size_t n) {
+  if (!c || !diff) return fail(FIB_E_ARG, "ctx/diff is NULL");
+  if (n != (size_t)c->nrep) return fail(FIB_E_ARG, "fib_set_replica_diff: n=%zu, the context has %d replicas", n, c->nrep);
+  if (c->nrep == 1) return fail(FIB_E_STATE, "fib_set_replica_diff: not a batched context (set fib_config.diff)");
   DevGuard dg(c->cfg.device);
   FLUSH(c);
-  const int r = launch_stim(c, var, r0, r1, c0, c1, value, floor_v);
+  drop_graphs(c);
+  return upload_replica_diff(c, diff);
+}
+
+extern "C" int fib_stimulate_replica(fib_ctx* c, int replica, int var, int r0, int r1, int c0, int c1, float value,
+                                     float floor_v) {
+  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
+  if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
+  if (replica < -1 || replica >= c->nrep)
+    return fail(FIB_E_ARG, "replica %d out of range -1..%d", replica, c->nrep - 1);
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  const int r = launch_stim(c, var, replica, r0, r1, c0, c1, value, floor_v);
   if (r) return r;
   mark_written(c, var);
   return 0;
 }
 
+extern "C" int fib_stimulate(fib_ctx* c, int var, int r0, int r1, int c0, int c1, float value,
+                             float floor_v) {
+  return fib_stimulate_replica(c, -1, var, r0, r1, c0, c1, value, floor_v);
+}
+
 extern "C" int fib_pace_add(fib_ctx* c, int r0, int r1, int c0, int c1, float value, float floor_v, int first,
                             int every, int count, int* id) {
+  return fib_pace_add_replica(c, -1, r0, r1, c0, c1, value, floor_v, first, every, count, id);
+}
+
+extern "C" int fib_pace_add_replica(fib_ctx* c, int replica, int r0, int r1, int c0, int c1, float value,
+                                    float floor_v, int first, int every, int count, int* id) {
   if (!c || !id) return fail(FIB_E_ARG, "ctx/id is NULL");
+  if (replica < -1 || replica >= c->nrep)
+    return fail(FIB_E_ARG, "replica %d out of range -1..%d", replica, c->nrep - 1);
   if (first < 1 || count < 0 || (count != 1 && every < 1))
     return fail(FIB_E_ARG, "fib_pace_add: need first >= 1, count >= 0 and every >= 1 unless count == 1 (got first %d, "
                 "every %d, count %d)", first, every, count);
@@ -1955,6 +2030,7 @@ extern "C" int fib_pace_add(fib_ctx* c, int r0, int r1, int c0, int c1, float va
     return fail(FIB_E_STATE, "fib_pace_add: at most %d pacing entries per context", kPaceMax);
   fib_ctx::Pace p;
   p.id = c->pace_ids++;
+  p.replica = replica;
   p.r0 = r0;
   p.r1 = r1;
   p.c0 = c0;
@@ -1994,8 +2070,14 @@ extern "C" int fib_probe(fib_ctx* c, int var, int row, int col, float* out) {
 }
 
 static int reduce_weighted(fib_ctx* c, int var, const float* w, double* sum_wx, double* sum_w);
+// a sum over a batched context would mix its replicas: a silently wrong mean, rho or electrogram
+static int refuse_batched_sum(const fib_ctx* c, const char* what) {
+  return fail(FIB_E_STATE, "%s sums over the whole context, which holds %d replicas", what, c->nrep);
+}
+
 extern "C" int fib_weighted_sum(fib_ctx* c, int var, double* sum_wx, double* sum_w) {
   if (!c || !sum_wx || !sum_w) return fail(FIB_E_ARG, "NULL argument");
+  if (c->nrep > 1) return refuse_batched_sum(c, "fib_weighted_sum");
   if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
   DevGuard dg(c->cfg.device);
   FLUSH(c);
@@ -2054,6 +2136,7 @@ extern "C" int fib_set_weights(fib_ctx* c, int slot, const float* rows_host, int
 
 extern "C" int fib_masked_sum(fib_ctx* c, int var, int slot, double* sum_wx, double* sum_w) {
   if (!c || !sum_wx || !sum_w) return fail(FIB_E_ARG, "NULL argument");
+  if (c->nrep > 1) return refuse_batched_sum(c, "fib_masked_sum");
   if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
   if (slot < 0 || slot >= 4 || !c->weights[slot]) return fail(FIB_E_STATE, "weight slot %d is empty", slot);
   DevGuard dg(c->cfg.device);
@@ -2228,6 +2311,9 @@ static int frames_arm(fib_ctx* c, int var, int first, int every, int stride, int
   if (first < 0 || every < 1 || stride < 1 || capacity < 1)
     return fail(FIB_E_ARG, "fib_frames_watch: need first >= 0, every >= 1, stride >= 1 and capacity >= 1 "
                 "(got %d, %d, %d, %d)", first, every, stride, capacity);
+  if (c->nrep > 1 && (c->g.H / c->nrep) % stride != 0)
+    return fail(FIB_E_ARG, "fib_frames_watch: stride %d does not divide the replicas' height %d (each replica's "
+                "frame rows start at its row 0)", stride, c->g.H / c->nrep);
   DevGuard dg(c->cfg.device);
   FLUSH(c);
   CU(cudaStreamSynchronize(c->stream));         // the old ring may still be written
@@ -2410,6 +2496,7 @@ extern "C" int fib_checkpoint_end(fib_ctx* c) {
 extern "C" int fib_count_below(fib_ctx* c, int var, float sub, float div, float cutoff, float w_min,
                                uint64_t* below, uint64_t* total) {
   if (!c || !below || !total) return fail(FIB_E_ARG, "NULL argument");
+  if (c->nrep > 1) return refuse_batched_sum(c, "fib_count_below");
   if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
   DevGuard dg(c->cfg.device);
   FLUSH(c);
@@ -2571,6 +2658,7 @@ extern "C" int fib_comm_unique_id(void* out128) {
 extern "C" int fib_comm_init(fib_ctx* c, int nranks, int rank, const void* id128) {
   if (!c || !id128) return fail(FIB_E_ARG, "ctx/id is NULL");
   if (nranks < 1 || rank < 0 || rank >= nranks) return fail(FIB_E_ARG, "bad rank %d of %d", rank, nranks);
+  if (c->nrep > 1) return fail(FIB_E_ARG, "fib_comm_init: a batched context (%d replicas) cannot be sharded", c->nrep);
   if (c->comm) return fail(FIB_E_STATE, "communicator already initialised");
   if (nranks == 1) return 0;   // a single shard needs no communicator
   if ((rank == 0) != c->top_is_border() || (rank == nranks - 1) != c->bottom_is_border())

@@ -46,6 +46,8 @@ struct Fused2Args {
   int pmask_pitch;              //   of a 32-column block can be non-zero (fib_set_phase)
   int lr0, nrows;       // local OUTPUT row range of this launch
   int R;                // output rows per warp
+  int nz;               // replicas, blockIdx.z (fib_kernels.cuh StepArgs)
+  const float* zddt;    // per-replica p.ddt, or nullptr
   Fenton4v::Params p;
 };
 
@@ -65,17 +67,17 @@ __device__ __forceinline__ float pick4(const float (&v)[4], int i) {
 // in rotated order, so the rows' roles never move between registers; the remainder of the trip
 // count modulo 3 runs through the EDGE body before them.  Both bodies make the same loads, the same
 // cell4 calls with the same operands and hence the same results.
-template <bool PHASE, bool IX>
+template <bool PHASE, bool IX, bool Z>
 struct Fused2March {
   const Geom& g;
   const Fused2Args& a;
-  StepArgs<Fenton4v> sa;
-  int lane, c, cs, g0, g1;
+  StepArgsOf<Fenton4v, Z> sa;
+  int lane, c, cs, g0, g1, row0;
   bool emit_lane;
   ColWindow<4> cw;
 
   __device__ __forceinline__ Fused2March(const Geom& g_, const Fused2Args& a_, int c0, int g0_, int g1_)
-      : g(g_), a(a_), lane(threadIdx.x), c(c0 + (int)threadIdx.x * 4), g0(g0_), g1(g1_), cw(0, 0) {
+      : g(g_), a(a_), lane(threadIdx.x), c(c0 + (int)threadIdx.x * 4), g0(g0_), g1(g1_), row0(zrow0<Z>(g_)), cw(0, 0) {
     const int W = g.W;
     const bool valid = IX || (c >= 0 && c < W);                // W % 4 == 0: all four cells or none
     cs = valid ? c : (c < 0 ? 0 : W - 4);                      // in-bounds column for addressing
@@ -83,9 +85,10 @@ struct Fused2March {
     cw = ColWindow<4>(cs, W);
     if (IX) cw.interior_x = cw.interior_p = true;              // what it computes, known at compile time
     sa.p = a.p;
+    if (Z) sa.zddt = a.zddt;
   }
 
-  __device__ __forceinline__ int rowoff(int gr) const { return (gr - g.row0 + kFuseHalo) * g.pitch; }
+  __device__ __forceinline__ int rowoff(int gr) const { return (gr - row0 + kFuseHalo) * g.pitch; }
   __device__ __forceinline__ int xrow(int gr) const { return rowoff(clampi(gr, 1, g.H - 2)); }
   __device__ __forceinline__ int prow(int gr) const { return rowoff(reflecti(gr, g.H)); }
 
@@ -93,7 +96,7 @@ struct Fused2March {
   // demand, only where fib_set_phase flagged the 32-column block.  o*: offsets of my columns of the
   // (reflected) rows gr - 1, gr, gr + 1
   __device__ __forceinline__ bool phase_flag(int gr) const {
-    return a.pmask[(gr - g.row0 + 1) * a.pmask_pitch + (cs >> 5)] != 0;
+    return a.pmask[(gr - row0 + 1) * a.pmask_pitch + (cs >> 5)] != 0;
   }
   __device__ __forceinline__ void add_phase(int oN, int oC, int oS, const float (&n)[6], const float (&x)[6],
                                             const float (&s)[6], float (&lapv)[4]) const {
@@ -270,7 +273,7 @@ struct Fused2March {
 };
 
 // the phase-field flavour needs ~20 more registers for the phi windows: one CTA per SM fewer
-template <bool PHASE>
+template <bool PHASE, bool Z>
 __global__ void __launch_bounds__(kBX * kFuseBY, (kFuseMinB - (PHASE ? 1 : 0)) * 4 / kFuseBY)
 fenton_fused2_kernel(const Geom g, const Fused2Args a) {
   const int c0 = blockIdx.x * kFuseCols - 4;                  // first column of lane 0
@@ -279,8 +282,8 @@ fenton_fused2_kernel(const Geom g, const Fused2Args a) {
   const int g1 = min(g0 + a.R, g.row0 + a.lr0 + a.nrows);
   if (g0 >= g1) return;                                       // warp-uniform
   // lane 0 reads from column c0 - 1 >= 1, lane 31 up to c0 + 128 <= W - 2: no lane clamps
-  if (c0 >= 2 && c0 + 128 <= g.W - 2) Fused2March<PHASE, true>(g, a, c0, g0, g1).run();
-  else Fused2March<PHASE, false>(g, a, c0, g0, g1).run();
+  if (c0 >= 2 && c0 + 128 <= g.W - 2) Fused2March<PHASE, true, Z>(g, a, c0, g0, g1).run();
+  else Fused2March<PHASE, false, Z>(g, a, c0, g0, g1).run();
 }
 
 // Output rows per warp R.  A row block costs R + 2 first-step rows, so deep marches are cheaper per
@@ -292,7 +295,7 @@ inline cudaError_t launch_fused2(const Geom& g, Fused2Args a, cudaStream_t st, i
   if (a.nrows <= 0) return cudaSuccess;
   const long nseg = (g.W + kFuseCols - 1) / kFuseCols;
   constexpr int BY = kFuseBY;
-  auto ctas = [&](int R) { return nseg * (((a.nrows + R - 1) / R + BY - 1) / BY); };
+  auto ctas = [&](int R) { return nseg * (((a.nrows + R - 1) / R + BY - 1) / BY) * a.nz; };
   const long slots = (long)sms * ((kFuseMinB - (a.phase ? 1 : 0)) * 4 / BY);
   int R = 8;
   long best = -1;
@@ -302,15 +305,22 @@ inline cudaError_t launch_fused2(const Geom& g, Fused2Args a, cudaStream_t st, i
     if (best < 0 || cost < best || (cost == best && r > R)) { best = cost; R = r; }
   }
   a.R = R;
-  dim3 block(kBX, BY), grid((unsigned)nseg, (unsigned)(((a.nrows + R - 1) / R + BY - 1) / BY));
+  dim3 block(kBX, BY), grid((unsigned)nseg, (unsigned)(((a.nrows + R - 1) / R + BY - 1) / BY), (unsigned)a.nz);
   if (preload_only()) {
     cudaFuncAttributes fa;
-    return a.phase ? cudaFuncGetAttributes(&fa, fenton_fused2_kernel<true>)
-                   : cudaFuncGetAttributes(&fa, fenton_fused2_kernel<false>);
+    return a.phase ? cudaFuncGetAttributes(&fa, fenton_fused2_kernel<true, false>)
+                   : cudaFuncGetAttributes(&fa, fenton_fused2_kernel<false, false>);
   }
-  snprintf(last_kernel_name(), 160, "fenton_fused2_kernel<PHASE=%d>,R=%d", a.phase ? 1 : 0, R);
-  if (a.phase) fenton_fused2_kernel<true><<<grid, block, 0, st>>>(g, a);
-  else fenton_fused2_kernel<false><<<grid, block, 0, st>>>(g, a);
+  const int n = snprintf(last_kernel_name(), 160, "fenton_fused2_kernel<PHASE=%d>,R=%d", a.phase ? 1 : 0, R);
+  if (a.nz > 1) snprintf(last_kernel_name() + n, 160 - n, ",Z=%d", a.nz);
+  if (a.nz > 1) {
+    if (a.phase) fenton_fused2_kernel<true, true><<<grid, block, 0, st>>>(g, a);
+    else fenton_fused2_kernel<false, true><<<grid, block, 0, st>>>(g, a);
+  } else if (a.phase) {
+    fenton_fused2_kernel<true, false><<<grid, block, 0, st>>>(g, a);
+  } else {
+    fenton_fused2_kernel<false, false><<<grid, block, 0, st>>>(g, a);
+  }
   return cudaGetLastError();
 }
 

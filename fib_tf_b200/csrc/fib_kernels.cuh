@@ -14,6 +14,8 @@
 #include <stdio.h>
 #include <stdlib.h>
 
+#include <type_traits>
+
 #include "fib_stencil.cuh"
 
 namespace fib {
@@ -40,8 +42,32 @@ struct StepArgs {
   int pmask_pitch;               //   can be non-zero (fib_set_phase), 0 where phi is locally constant
   const float* lut;              // Courtemanche table, transposed [30][160] (global), or nullptr
   int lr0, nrows;                // local row range [lr0, lr0+nrows) processed by this launch
+  // Replicas (fib_config.replicas): the launch steps nz independent grids of g.H rows, stacked in every
+  // plane as one grid of nz * g.H rows; blockIdx.z = the replica.  zddt: per-replica p.ddt, or nullptr
+  int nz;
+  const float* zddt;
   typename M::Params p;
 };
+
+// The kernels' batched flavour (Z = true) takes its arguments as StepArgsZ: the same fields, but the cell
+// functions read replica blockIdx.z's diffusion factor from zddt.  The unbatched flavour is the kernel as it
+// was before replicas, instruction for instruction.
+template <class M>
+struct StepArgsZ : StepArgs<M> {};
+template <class M, bool Z>
+using StepArgsOf = typename std::conditional<Z, StepArgsZ<M>, StepArgs<M>>::type;
+
+// The state rows of replica blockIdx.z start at local row blockIdx.z * g.H of every plane: a block addresses
+// row gr of its replica as local row gr - zrow0(g), and never leaves it (the stencil clamps within the
+// replica), so a seam needs no halo rows
+template <bool Z>
+__device__ __forceinline__ int zrow0(const Geom& g) { return Z ? g.row0 - (int)blockIdx.z * g.H : g.row0; }
+// the diffusion factor p.ddt = fp32(diff * dt) the cell functions use: replica blockIdx.z's own, folded in double
+// on the host, in the batched flavour; A = StepArgs, StepArgsZ or a wrapper with a member `p` only
+template <class A>
+__device__ __forceinline__ float ddt_of(const A& a) { return a.p.ddt; }
+template <class M>
+__device__ __forceinline__ float ddt_of(const StepArgsZ<M>& a) { return __ldg(a.zddt + blockIdx.z); }
 
 constexpr int kBX = 32;   // threads along columns (one warp)
 __device__ __forceinline__ void prefetch_l1(const float* p) {
@@ -65,9 +91,10 @@ inline char* last_kernel_name() {
   return name;
 }
 
-template <class M, int VEC, int R, int BY, bool PHASE>
+template <class M, int VEC, int R, int BY, bool PHASE, bool Z>
 __global__ void __launch_bounds__(kBX* BY, M::min_blocks(VEC, PHASE))
-step_kernel(const Geom g, const StepArgs<M> a) {
+step_kernel(const Geom g, const StepArgsOf<M, Z> a) {
+  const int row0 = zrow0<Z>(g);                                 // g.row0, in this replica's rows
   const int c = (blockIdx.x * kBX + threadIdx.x) * VEC;
   const int strip = blockIdx.y * BY + threadIdx.y;
   const int gr0 = g.row0 + a.lr0 + strip * R;                 // first global row of my strip
@@ -79,14 +106,14 @@ step_kernel(const Geom g, const StepArgs<M> a) {
   const int pitch = g.pitch;
   const ColWindow<VEC> cw(c, g.W);
   // element index of the start of (clamped / reflected) global row `gr` in a halo-layout plane
-  auto xrow = [&](int gr) { return (clampi(gr, 1, g.H - 2) - g.row0 + 1) * pitch; };
-  auto prow = [&](int gr) { return (reflecti(gr, g.H) - g.row0 + 1) * pitch; };
+  auto xrow = [&](int gr) { return (clampi(gr, 1, g.H - 2) - row0 + 1) * pitch; };
+  auto prow = [&](int gr) { return (reflecti(gr, g.H) - row0 + 1) * pitch; };
 
   float xN[VEC + 2], xC[VEC + 2], xS[VEC + 2];
   if (M::NEED_LAP) load_enforced_row<VEC>(a.xin, xrow(gr0 - 1), cw, g.W, xN);
   load_enforced_row<VEC>(a.xin, xrow(gr0), cw, g.W, xC);
 
-  int off = (gr0 - g.row0) * pitch + c;          // my cell in a non-halo plane; += pitch per row
+  int off = (gr0 - row0) * pitch + c;            // my cell in a non-halo plane; += pitch per row
 #pragma unroll
   for (int i = 0; i < R; ++i, off += pitch) {
     const int gr = gr0 + i;
@@ -105,7 +132,7 @@ step_kernel(const Geom g, const StepArgs<M> a) {
       float pN[VEC], pS[VEC], pC[VEC + 2];
       bool ph = false;
       if (PHASE && M::NEED_LAP) {
-        ph = a.pmask[(gr - g.row0) * a.pmask_pitch + (c >> 5)] != 0;
+        ph = a.pmask[(gr - row0) * a.pmask_pitch + (c >> 5)] != 0;
         if (ph) {
           VecIO<VEC>::ld(a.phase + (prow(gr - 1) + c), pN);
           VecIO<VEC>::ld(a.phase + (prow(gr + 1) + c), pS);
@@ -179,34 +206,37 @@ step_kernel(const Geom g, const StepArgs<M> a) {
   }
 }
 
-template <class M, int VEC, int R, int BY, bool PHASE>
+template <class M, int VEC, int R, int BY, bool PHASE, bool Z>
 inline cudaError_t launch_step_r(const Geom& g, const StepArgs<M>& a, cudaStream_t st) {
   const int ncg = (g.W + VEC - 1) / VEC;
   cudaLaunchConfig_t cfg = {};
   cfg.blockDim = dim3(kBX, BY);
-  cfg.gridDim = dim3((ncg + kBX - 1) / kBX, ((a.nrows + R - 1) / R + BY - 1) / BY);
+  cfg.gridDim = dim3((ncg + kBX - 1) / kBX, ((a.nrows + R - 1) / R + BY - 1) / BY, a.nz);
   cfg.stream = st;
   if (preload_only()) {
     cudaFuncAttributes fa;
-    return cudaFuncGetAttributes(&fa, step_kernel<M, VEC, R, BY, PHASE>);
+    return cudaFuncGetAttributes(&fa, step_kernel<M, VEC, R, BY, PHASE, Z>);
   }
-  snprintf(last_kernel_name(), 160, "step_kernel<%s,VEC=%d,R=%d,BY=%d,PHASE=%d>", M::name(), VEC, R, BY,
-           PHASE ? 1 : 0);
-  return cudaLaunchKernelEx(&cfg, step_kernel<M, VEC, R, BY, PHASE>, g, a);
+  const int n = snprintf(last_kernel_name(), 160, "step_kernel<%s,VEC=%d,R=%d,BY=%d,PHASE=%d>", M::name(), VEC, R,
+                         BY, PHASE ? 1 : 0);
+  if (a.nz > 1) snprintf(last_kernel_name() + n, 160 - n, ",Z=%d", a.nz);
+  StepArgsOf<M, Z> az;
+  static_cast<StepArgs<M>&>(az) = a;
+  return cudaLaunchKernelEx(&cfg, step_kernel<M, VEC, R, BY, PHASE, Z>, g, az);
 }
 
-// Picks the marching depth R: as deep as possible while the grid still has >= 4 CTAs per SM
+// Picks the marching depth R: as deep as possible while the grid (all replicas) still has >= 4 CTAs per SM
 // (148 SMs); small grids (512^2) fall back to R = 1 and are launch-latency bound anyway.
-template <class M, int VEC, int BY, bool PHASE>
+template <class M, int VEC, int BY, bool PHASE, bool Z>
 inline cudaError_t launch_step_p(const Geom& g, const StepArgs<M>& a, cudaStream_t st, int sms) {
   const int ncg = (g.W + VEC - 1) / VEC;
   const long bx = (ncg + kBX - 1) / kBX;
-  auto blocks = [&](int R) { return bx * (((a.nrows + R - 1) / R + BY - 1) / BY); };
+  auto blocks = [&](int R) { return bx * (((a.nrows + R - 1) / R + BY - 1) / BY) * a.nz; };
   const long want = 4L * sms;
-  if (M::MAX_R >= 8 && M::AUTO_R >= 8 && blocks(8) >= want) return launch_step_r<M, VEC, (M::MAX_R >= 8 ? 8 : 1), BY, PHASE>(g, a, st);
-  if (M::MAX_R >= 4 && M::AUTO_R >= 4 && blocks(4) >= want) return launch_step_r<M, VEC, (M::MAX_R >= 4 ? 4 : 1), BY, PHASE>(g, a, st);
-  if (M::MAX_R >= 2 && M::AUTO_R >= 2 && blocks(2) >= want) return launch_step_r<M, VEC, (M::MAX_R >= 2 ? 2 : 1), BY, PHASE>(g, a, st);
-  return launch_step_r<M, VEC, 1, BY, PHASE>(g, a, st);
+  if (M::MAX_R >= 8 && M::AUTO_R >= 8 && blocks(8) >= want) return launch_step_r<M, VEC, (M::MAX_R >= 8 ? 8 : 1), BY, PHASE, Z>(g, a, st);
+  if (M::MAX_R >= 4 && M::AUTO_R >= 4 && blocks(4) >= want) return launch_step_r<M, VEC, (M::MAX_R >= 4 ? 4 : 1), BY, PHASE, Z>(g, a, st);
+  if (M::MAX_R >= 2 && M::AUTO_R >= 2 && blocks(2) >= want) return launch_step_r<M, VEC, (M::MAX_R >= 2 ? 2 : 1), BY, PHASE, Z>(g, a, st);
+  return launch_step_r<M, VEC, 1, BY, PHASE, Z>(g, a, st);
 }
 
 template <class M>
@@ -215,15 +245,20 @@ inline cudaError_t launch_step(const Geom& g, const StepArgs<M>& a, cudaStream_t
   const bool ph = a.phase && M::NEED_LAP;
   // Small grids (e.g. the reference's 512^2 configs) cannot fill 148 SMs with the
   // wide flavour: fall back to one cell per thread there (twice the CTAs, no tail wave).  The
-  // choice depends on the GLOBAL grid only, so every shard and every row-range launch of a run
+  // choice depends on the GLOBAL grid only (all replicas), so every shard and every row-range launch of a run
   // uses the same flavour as the unsharded run.
   static const long small_cells = getenv("FIB_SMALL_CELLS") ? atol(getenv("FIB_SMALL_CELLS")) : kSmallGridCells;
-  if (M::VEC > 1 && M::VEC_SMALL != M::VEC && (long)g.H * g.W <= small_cells) {
-    if (ph) return launch_step_p<M, M::VEC_SMALL, M::BY, true>(g, a, st, sms);
-    return launch_step_p<M, M::VEC_SMALL, M::BY, false>(g, a, st, sms);
-  }
-  if (ph) return launch_step_p<M, M::VEC, M::BY, true>(g, a, st, sms);
-  return launch_step_p<M, M::VEC, M::BY, false>(g, a, st, sms);
+  const bool small = M::VEC > 1 && M::VEC_SMALL != M::VEC && (long)g.H * g.W * a.nz <= small_cells;
+  auto go = [&](auto z) {
+    constexpr bool Z = decltype(z)::value;
+    if (small) {
+      if (ph) return launch_step_p<M, M::VEC_SMALL, M::BY, true, Z>(g, a, st, sms);
+      return launch_step_p<M, M::VEC_SMALL, M::BY, false, Z>(g, a, st, sms);
+    }
+    if (ph) return launch_step_p<M, M::VEC, M::BY, true, Z>(g, a, st, sms);
+    return launch_step_p<M, M::VEC, M::BY, false, Z>(g, a, st, sms);
+  };
+  return a.nz > 1 ? go(std::true_type()) : go(std::false_type());
 }
 
 }  // namespace fib

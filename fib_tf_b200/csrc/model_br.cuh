@@ -282,7 +282,7 @@ struct BeelerReuter {
     const T dC = vfma(T(-1.0e-7f), iCa, T(0.07f) * (T(1.0e-7f) - C));
     s[0] = vfma(T(p.dt), dC, C);
     const T reaction = mul_rn(T(p.dt), I_sum);
-    Vnew = clip_tf(sub_rn(add_rn(V0, mul_rn(T(p.ddt), lap_value<T>(lap))), reaction), -85.0f, 25.0f);
+    Vnew = clip_tf(sub_rn(add_rn(V0, mul_rn(T(ddt_of(a)), lap_value<T>(lap))), reaction), -85.0f, 25.0f);
   }
 };
 

@@ -311,8 +311,9 @@ struct Courtemanche {
     for (int k = 0; k < kLutCols; ++k) q[k] = f2(__ldg(c0 + k * kLutTStride), __ldg(c1 + k * kLutTStride));
   }
 
-  template <class T>
-  static __device__ __forceinline__ void cell(const StepArgs<Courtemanche>& a, T /*raw*/, T V, T lap,
+  // A: StepArgs<Courtemanche> or StepArgsZ<Courtemanche> (fib_kernels.cuh)
+  template <class A, class T>
+  static __device__ __forceinline__ void cell(const A& a, T /*raw*/, T V, T lap,
                                               T (&s)[NS], T& Vnew) {
     using namespace cc;
     const Params& p = a.p;
@@ -391,7 +392,7 @@ struct Courtemanche {
     const T I_tot = i_Na + i_K1 + i_to + i_Kur + i_Kr + i_Ks + i_B_Na + i_B_Ca + i_NaK + i_CaP + i_NaCa + i_Ca_L;
     // reference rounding sequence, no FMA contraction (V crosses 0 mV with ~80 mV operands)
     const T DV = add_rn(V, mul_rn(div_rn(-I_tot, T((float)Cm)), T(dtf)));       // court.py:223-227
-    Vnew = add_rn(DV, mul_rn(T(p.ddt), lap));                                    // court.py:229
+    Vnew = add_rn(DV, mul_rn(T(ddt_of(a)), lap));                                    // court.py:229
 
     // Ca handling (court.py:232-265)
     const T i_rel = (u * u) * (float)K_rel * v * w * (Ca_rel - Ca_i);

@@ -75,11 +75,12 @@ struct Fenton4v {
     s[1] = vfma(dt, dW, W);
     s[2] = vfma(dt, dS, S);
     const T reaction = add_rn(U0, mul_rn(dt, dU));
-    Unew = add_rn(reaction, mul_rn(T(a.p.ddt), lap_value<T>(lap)));
+    Unew = add_rn(reaction, mul_rn(T(ddt_of(a)), lap_value<T>(lap)));
   }
 
   // four cells of a thread as two packed pairs
-  static __device__ __forceinline__ void cell4(const StepArgs<Fenton4v>& a, const float (&raw)[4], const float* x0,
+  template <class A>
+  static __device__ __forceinline__ void cell4(const A& a, const float (&raw)[4], const float* x0,
                                                const float (&lap)[4], float (&sv)[3][4], float (&unew)[4]) {
 #pragma unroll
     for (int l = 0; l < 4; l += 2) {

@@ -58,14 +58,14 @@ class Fenton4v(IonicModel):
         """Temporal blocking: two time steps per kernel launch (csrc/fib_fused.cuh), BIT-IDENTICAL
         to one step per launch.  Config key 'steps_per_launch' (1 or 2) or FIB_STEPS_PER_LAUNCH
         override the size-based default; it needs width % 4 == 0, otherwise one step per launch
-        is used.  The choice depends on the global grid only, so every rank
+        is used.  The choice depends on the global grid only (all replicas of a batched model), so every rank
         of a sharded run makes the same one."""
         want = self.__dict__.get('steps_per_launch')
         if want is None:
             want = os.environ.get('FIB_STEPS_PER_LAUNCH')
         if want is None:
             floor = self.FUSE_MIN_CELLS if self._phase_rows is None else self.FUSE_MIN_CELLS_PHASE
-            want = 2 if self.height * self.width >= floor else 1
+            want = 2 if self.height * self.width * self.replicas >= floor else 1
         able = self.width % 4 == 0 and \
             (self._nranks == 1 or self.height // self._nranks >= 2)
         return 2 if int(want) == 2 and able else 1

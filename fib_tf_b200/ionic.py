@@ -29,6 +29,13 @@ Extra, optional config keys (all default to the reference's behaviour):
                  to twice that many iterations late, with the reference's arguments; 1 = read it
                  back every iteration like the reference)
 
+    replicas     B > 1: step B independent grids of height x width together, one launch per time step for all
+                 of them (include/fib_b200.h, Replicas; default 1).  Each replica has its own state, holes
+                 (add_hole_to_phase_field(replica=)), stimuli (fire_op / pace with replica=) and `diff`: config
+                 'diff' may be a sequence of B floats.  Reads (image(), pot().eval(), _State[n].eval(),
+                 activation_maps(), frames()) gain a leading replica axis; assign() takes [H, W] or [B, H, W].
+                 Not with `distributed`, run(im), a cl_observer, masked_image_mean() or excitable_fraction().
+
     upload_window  distributed runs: how many of run()'s first iterations may run behind a pipelined upload
                  (fib_set_rect_async blocks, even ranks top to bottom, odd ranks bottom to top; default 10,
                  0 = never; the ranks agree on the number at the start of run())
@@ -53,7 +60,8 @@ from .sharding import owner_of_row, partition_rows
 
 class DeviceVar:
     """Stand-in for a tf.Variable holding one state plane: .eval() reads it back
-    (fenton.py:152-153, court.py:619), .assign(a) uploads, var[r, c].eval() probes one cell."""
+    (fenton.py:152-153, court.py:619), .assign(a) uploads, var[r, c].eval() probes one cell (on a batched model
+    the row counts through the replicas: replica b's row r is row b * height + r)."""
 
     def __init__(self, model, name):
         self._model = model
@@ -67,8 +75,7 @@ class DeviceVar:
 
     def assign(self, value):
         m = self._model
-        a = np.broadcast_to(np.asarray(value, dtype=np.float32), (m.height, m.width))
-        m._ctx.set_state(self.name, a[m._row0:m._row0 + m._rows])
+        m._ctx.set_state(self.name, m._own_rows(value))
         return self
 
     def __getitem__(self, idx):
@@ -94,6 +101,18 @@ class IonicModel:
         for key, val in config.items():     # ionic.py:35-37
             if key != 'phase':
                 setattr(self, key, val)
+        self.replicas = int(config.get('replicas', 1))
+        if self.replicas < 1:
+            raise ValueError('replicas must be >= 1 (got %d)' % self.replicas)
+        if self.replicas > 1 and config.get('distributed'):
+            raise ValueError('replicas > 1 cannot be combined with distributed: a batched model runs on one GPU')
+        diff = config.get('diff')
+        if np.ndim(diff) == 1:
+            if len(diff) != self.replicas:
+                raise ValueError('diff holds %d values for %d replicas' % (len(diff), self.replicas))
+            self.replica_diff = [float(d) for d in diff]
+        elif diff is not None:
+            self.replica_diff = [float(diff)] * self.replicas
         self._ops = {}
         self.defined = False
         self.dt_per_step = 1
@@ -107,10 +126,11 @@ class IonicModel:
             self._rank, self._nranks = dist.get_rank(), dist.get_world_size()
         parts = partition_rows(self.height, self._nranks)
         self._row0, self._rows = parts[self._rank]
+        self._rows *= self.replicas             # a batched model: its replicas' rows one after another
         # host copy of the phase field covers these global rows (everything when not sharded)
         # (two halo rows: what the two-steps-per-launch kernel needs; one would do otherwise)
         self._phase_row0 = max(self._row0 - 2, 0)
-        self._phase_row1 = min(self._row0 + self._rows + 2, self.height)
+        self._phase_row1 = min(self._row0 + self._rows + 2, self.height * self.replicas)
         if config.get('phase') is not None:
             self.phase = config['phase']
 
@@ -164,6 +184,8 @@ class IonicModel:
         rows = self.__dict__.get('_phase_rows')
         if rows is None:
             return None
+        if self.replicas > 1:
+            return rows.reshape(self.replicas, self.height, self.width)
         if self._nranks == 1:
             return rows
         if self.__dict__.get('_phase_full') is None:
@@ -179,7 +201,12 @@ class IonicModel:
             self._phase_rows, self._phase_full, self._holes = None, None, []
             return
         a = np.asarray(value, dtype=np.float32)
-        if a.shape != (self.height, self.width):
+        if self.replicas > 1:
+            if a.shape not in ((self.height, self.width), (self.replicas, self.height, self.width)):
+                raise ValueError('phase must be [height, width] or [replicas, height, width] = %r'
+                                 % ((self.replicas, self.height, self.width),))
+            a = self._own_rows(a)
+        elif a.shape != (self.height, self.width):
             raise ValueError('phase must be [height, width] = %r' % ((self.height, self.width),))
         if self.__dict__.get('defined'):
             raise AssertionError('the phase field must be set before calling define')
@@ -201,13 +228,25 @@ class IonicModel:
         return np.maximum(phase, 1e-5)
 
     # ---- geometry (ionic.py:83-105) ----------------------------------------------------------
-    def add_hole_to_phase_field(self, x, y, radius, neg=False):
+    def add_hole_to_phase_field(self, x, y, radius, neg=False, replica=None):
         """Adds a circular hole centred at (x, y) = (column, row) to the phase field; with
-        neg=True the inside is kept and the outside excluded.  Must precede define()."""
+        neg=True the inside is kept and the outside excluded.  Must precede define().  A batched model:
+        in replica `replica` only, or in every replica (None)."""
         if self.defined:
             raise AssertionError('add_hole_to_phase_field should be called before calling define')
         if self._holes is None:
             raise AssertionError('the phase field was assigned directly; holes cannot be added to it')
+        if replica is not None or self.replicas > 1:
+            B, H = self.replicas, self.height
+            if replica is not None and not 0 <= int(replica) < B:
+                raise ValueError('replica %r out of range 0..%d' % (replica, B - 1))
+            if self._phase_rows is None:
+                self._phase_rows = np.ones([B * H, self.width], dtype=np.float32)
+            for b in range(B) if replica is None else [int(replica)]:
+                self._phase_rows[b * H:(b + 1) * H] = self._apply_hole(self._phase_rows[b * H:(b + 1) * H], 0, H,
+                                                                       x, y, radius, neg)
+            self._holes.append((x, y, radius, neg))
+            return
         self._phase_rows = self._apply_hole(self._phase_rows, self._phase_row0, self._phase_row1,
                                             x, y, radius, neg)
         self._holes.append((x, y, radius, neg))
@@ -224,9 +263,12 @@ class IonicModel:
         if not cfgd.get('persist', True):
             flags |= _capi.F_NO_PERSIST
         sharded = self._nranks > 1
-        ctx = _capi.Context(self.MODEL_ID, self.height, self.width, self.dt, self.diff, flags=flags,
+        batched = {'replicas': self.replicas} if self.replicas > 1 else {}
+        ctx = _capi.Context(self.MODEL_ID, self.height, self.width, self.dt, self.replica_diff[0], flags=flags,
                             device=device, row0=self._row0 if sharded else 0,
-                            rows=self._rows if sharded else 0, steps_per_launch=steps_per_launch)
+                            rows=self._rows if sharded else 0, steps_per_launch=steps_per_launch, **batched)
+        if batched and len(set(self.replica_diff)) > 1:
+            ctx.set_replica_diff(self.replica_diff)
         if self._phase_rows is not None:
             ctx.set_phase(np.asarray(self._phase_rows, dtype=np.float32), self._phase_row0)
         if sharded:
@@ -274,7 +316,16 @@ class IonicModel:
         """[rows, W] fp32 array filled with `value` for this shard's rows."""
         return np.full([self._rows, self.width], value, dtype=np.float32)
 
+    def _own_rows(self, value):
+        """This context's rows of a full-grid array: [height, width] (every replica), or [replicas, height, width]."""
+        a = np.asarray(value, dtype=np.float32)
+        if self.replicas > 1:
+            return np.broadcast_to(a, (self.replicas, self.height, self.width)).reshape(self._rows, self.width)
+        return np.broadcast_to(a, (self.height, self.width))[self._row0:self._row0 + self._rows]
+
     def _gather(self, local):
+        if self.replicas > 1:
+            return local.reshape(self.replicas, self.height, -1)
         if self._nranks == 1:
             return local
         import torch.distributed as dist
@@ -312,16 +363,23 @@ class IonicModel:
             rect = (0, 0, 0, 0)
         self._ops[name] = ('pace', rect, float(v))
 
-    def fire_op(self, name):
-        """Executes an op registered by add_pace_op (or a model op such as 'slow')."""
+    def fire_op(self, name, replica=None):
+        """Executes an op registered by add_pace_op (or a model op such as 'slow').  A batched model: a
+        stimulus in replica `replica` only, or in every replica (None)."""
         op = self._ops[name]
         if op[0] == 'pace':
             (r0, r1, c0, c1), v = op[1], op[2]
-            self._ctx.stimulate(self._pot_name, max(r0, 0), r1, max(c0, 0), c1, v, float(self.min_v))
+            where = {} if replica is None else {'replica': self._check_replica(replica)}
+            self._ctx.stimulate(self._pot_name, max(r0, 0), r1, max(c0, 0), c1, v, float(self.min_v), **where)
         elif op[0] == 'call':
             op[1]()
 
-    def pace(self, name, at, every=0, count=1):
+    def _check_replica(self, replica):
+        if not 0 <= int(replica) < self.replicas:
+            raise ValueError('replica %r out of range 0..%d' % (replica, self.replicas - 1))
+        return int(replica)
+
+    def pace(self, name, at, every=0, count=1, replica=None):
         """Schedules the op `name` registered with add_pace_op on the device: it fires after the absolute ODE
         iterations n = at + 1 + j * every (n counts `iterations`), j = 0 .. count - 1, or until stop_pacing() with
         count = 0.  That is the iteration after which a driver's `for i in run(): if i == at: fire_op(name)` fires,
@@ -329,7 +387,8 @@ class IonicModel:
         while stepping (include/fib_b200.h fib_pace_add): a train needs no call per beat and keeps the persistent
         kernel's batches.  Frames and activation maps see an iteration before its stimulus, the probe after it.
         checkpoint() saves the schedules and restore() continues them.  At most 4 schedules are active at once.
-        ValueError if iteration at + 1 has already been stepped.  Collective when distributed."""
+        ValueError if iteration at + 1 has already been stepped.  Collective when distributed.  A batched model:
+        the stimulus in replica `replica` only, or in every replica (None)."""
         if not self.defined:
             raise AssertionError('pace should be called after calling define')
         op = self._ops.get(name)
@@ -345,7 +404,11 @@ class IonicModel:
         (r0, r1, c0, c1), v = op[1], op[2]
         entry = {'name': name, 'rect': [max(r0, 0), r1, max(c0, 0), c1], 'value': v, 'floor': float(self.min_v),
                  'next': at + 1, 'every': every, 'count': count}
-        entry['id'] = self._ctx.pace_add(*entry['rect'], v, entry['floor'], at + 1 - self.iterations, every, count)
+        where = {}
+        if replica is not None:
+            entry['replica'] = where['replica'] = self._check_replica(replica)
+        entry['id'] = self._ctx.pace_add(*entry['rect'], v, entry['floor'], at + 1 - self.iterations, every, count,
+                                         **where)
         self._pacing = self._active_pacing() + [entry]
 
     def _active_pacing(self):
@@ -368,6 +431,9 @@ class IonicModel:
         """
         if not self.defined:
             raise AssertionError('define() must be called before run()')
+        if self.replicas > 1 and (im or self.cl_observer is not None):
+            raise ValueError('run(im) and cl_observer watch one cell of one grid: a batched model (replicas = %d) '
+                             'has activation maps (watch_activation) instead' % self.replicas)
         then = time.time()
         v0 = self.min_v
         last_spike = 0
@@ -534,6 +600,7 @@ class IonicModel:
     def masked_image_mean(self, slot):
         """np.mean(self.image() * mask) (egm.py:44-47) without moving the frame to the host:
         one weighted reduction on the device (summed over ranks when sharded)."""
+        self._refuse_batched_sum('masked_image_mean')
         swx, sw = self._ctx.masked_sum(self._pot_name, slot)
         if self._nranks > 1:
             import torch.distributed as dist
@@ -549,6 +616,7 @@ class IonicModel:
         """rho of court_ultra.py:504-509: np.sum(image[phase > phase_min] < cutoff) /
         np.sum(phase > phase_min) with image = self.image(), as one threshold-count reduction on the
         device (summed over ranks when sharded) -- no frame leaves the GPU."""
+        self._refuse_batched_sum('excitable_fraction')
         if self.MODEL_ID == _capi.FENTON4V:
             sub, div = 0.0, 1.0
         else:
@@ -560,6 +628,11 @@ class IonicModel:
             dist.all_gather_object(parts, (below, total))
             below, total = sum(p[0] for p in parts), sum(p[1] for p in parts)
         return below / total if total else float('nan')
+
+    def _refuse_batched_sum(self, what):
+        if self.replicas > 1:
+            raise ValueError('%s sums over the whole grid, and this model holds %d replicas: per-replica sums are not '
+                             'implemented yet (use image() or activation_maps() per replica)' % (what, self.replicas))
 
     def watch_activation(self, up=None, down=None):
         """Arms the device-side activation maps of the transmembrane variable (include/fib_b200.h,
@@ -660,6 +733,8 @@ class IonicModel:
             parts = [None] * self._nranks
             dist.all_gather_object(parts, cube)
             cube = np.concatenate(parts, axis=1)
+        if self.replicas > 1:
+            cube = cube.reshape(len(cube), self.replicas, rows // self.replicas, cols)
         if f['name'] == self._pot_name and self.MODEL_ID != _capi.FENTON4V:
             cube = self._normalise(cube)
         return iters, cube

@@ -81,8 +81,28 @@ typedef struct {
                                 (Fenton 4v only, width % 4 == 0; results are
                                 bit-identical to one step per launch; shards exchange two halo rows
                                 of every plane per launch).  Must divide dt_per_step (SURVEY fact 4) */
-  int32_t  reserved[6];
+  int32_t  replicas;         /* 0 or 1: one grid.  B > 1 (up to 65535): a BATCHED context of B independent grids of
+                                height x width, stepped together in every launch (see "Replicas" below)   */
+  int32_t  reserved[5];
 } fib_config;
+
+/* ---- Replicas: many independent simulations of one grid (ensembles, parameter sweeps) -------------------
+ * A context with replicas = B holds B grids of height x width, each with its own state, phase field, stimuli
+ * and diffusion coefficient; replica b of a batched context computes bit for bit what an unbatched context
+ * of the same config, with diff = diff_b, computes on replica b's inputs.  One launch per time step steps all
+ * of them (blockIdx.z = the replica), so small grids add up to a grid the GPU can fill.
+ * Addressing: state I/O (fib_set_state, fib_get_state, fib_*_rect, snapshots), fib_set_phase, probes, the
+ * activation maps, the frame recorder and the checkpoint parts address a batched context as ONE grid of
+ * B * height rows: replica b is rows [b * height, (b + 1) * height).  Stimuli and pacing
+ * (fib_stimulate_replica, fib_pace_add_replica) take a replica and rows local to it.
+ * Refused on a batched context: row shards (rows != 0), fib_comm_init and fib_step_group (FIB_E_ARG); the
+ * whole-context sums fib_weighted_sum, fib_masked_sum and fib_count_below (FIB_E_STATE: they would mix the
+ * replicas); fib_frames_watch / fib_frames_resume with a stride that does not divide height (FIB_E_ARG).
+ * fib_set_rect_async blocks are copied in order and never start a pipelined upload.  The persistent on-chip
+ * kernel is never used.
+ * fib_set_replica_diff sets diff of every replica (n == replicas; FIB_E_STATE on an unbatched context); it
+ * takes effect from the next iteration.  Until it is called every replica uses fib_config.diff. */
+int fib_set_replica_diff(fib_ctx *ctx, const double *diff, size_t n);
 
 /* ops of fib_step -- the reference's session ops */
 typedef enum {
@@ -188,14 +208,19 @@ int fib_step_behind_upload(fib_ctx *ctx, int n_iter);
  * multi-GPU decomposition on one device and for single-process multi-GPU. */
 int fib_step_group(fib_ctx **ctxs, int n, int op, int n_iter);
 
-/* name of the step-kernel flavour (model, cells per thread, marching depth, phase flag) launched last
- * by fib_step / fib_step_group on this thread: lets tests prove which instantiation they compared. */
+/* name of the step-kernel flavour (model, cells per thread, marching depth, phase flag; ",Z=B" for a launch of B
+ * replicas) launched last by fib_step / fib_step_group on this thread: lets tests prove which instantiation
+ * they compared. */
 int fib_last_kernel(char *buf, size_t n);
 
 /* ---- stimulus: replaces pot().assign(tf.maximum(pot(), s)) (ionic.py:144-163) -----------
  * X := max(X, inside [r0,r1)x[c0,c1) ? value : floor_v) over the whole plane, GLOBAL coords. */
 int fib_stimulate(fib_ctx *ctx, int var, int r0, int r1, int c0, int c1, float value,
                   float floor_v);
+/* the same on a batched context: rows local to a replica; replica -1 applies the rectangle (and the floor) in
+ * every replica, replica b in replica b only.  fib_stimulate is replica -1. */
+int fib_stimulate_replica(fib_ctx *ctx, int replica, int var, int r0, int r1, int c0, int c1, float value,
+                          float floor_v);
 
 /* pacing: stimulus trains scheduled once and applied on the device while stepping (S1 trains at a basic cycle
  * length, burst pacing, S1-S2 protocols), so that a train neither needs the host every beat nor cuts the
@@ -221,6 +246,9 @@ int fib_stimulate(fib_ctx *ctx, int var, int r0, int r1, int c0, int c1, float v
  * `id` (a no-op when it has finished), or every entry when id < 0; FIB_E_ARG for an id that was never handed out. */
 int fib_pace_add(fib_ctx *ctx, int r0, int r1, int c0, int c1, float value, float floor_v,
                  int first, int every, int count, int *id);
+/* the same with a replica selector and rows local to it, as fib_stimulate_replica; fib_pace_add is replica -1 */
+int fib_pace_add_replica(fib_ctx *ctx, int replica, int r0, int r1, int c0, int c1, float value, float floor_v,
+                         int first, int every, int count, int *id);
 int fib_pace_remove(fib_ctx *ctx, int id);
 
 /* ---- probes: replaces Variable[r,c] reads (ionic.py:216, court.py:109-110) --------------
