@@ -118,6 +118,11 @@ _SIGNATURES = {
     'fib_count_nonfinite': (C.c_int, [_P, C.c_int, C.POINTER(C.c_uint64)]),
     'fib_set_weights': (C.c_int, [_P, C.c_int, _P, C.c_int, C.c_int]),
     'fib_masked_sum': (C.c_int, [_P, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
+    'fib_replica_sums': (C.c_int, [_P, C.c_int, C.c_int, _P, _P, C.c_size_t]),
+    'fib_replica_count_below': (C.c_int, [_P, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, _P, _P,
+                                          C.c_size_t]),
+    'fib_replica_probe_watch': (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    'fib_replica_probe_fetch': (C.c_int, [_P, _P, C.c_size_t, C.POINTER(C.c_size_t)]),
     'fib_sync': (C.c_int, [_P]),
     'fib_flush': (C.c_int, [_P]),
     'fib_upload_state': (C.c_int, [_P, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
@@ -207,6 +212,7 @@ class Context:
         self.model, self.dt, self.diff, self.flags = int(model), float(dt), float(diff), int(flags)
         self.replicas = max(int(replicas), 1)
         self.replica_diff = [self.diff] * self.replicas      # diff of every replica (set_replica_diff)
+        self.replica_ring = PROBE_RING                       # records of the replica probe ring (replica_probe_watch)
         self.height, self.width = int(height), int(width)
         self.row0 = int(row0) if rows else 0
         self.rows = int(rows) if rows else int(height) * self.replicas
@@ -346,6 +352,22 @@ class Context:
         check(lib().fib_probe_fetch(self._h, out.ctypes.data_as(_P), max_values, C.byref(n)))
         return out[:n.value]
 
+    def replica_probe_watch(self, var, row, col):
+        """Record cell (row, col) of every replica (row local to a replica) after every iteration, one record of
+        `replicas` floats each (row < 0: stop); returns the ring's capacity in records."""
+        cap = C.c_size_t()
+        check(lib().fib_replica_probe_watch(self._h, self.var(var) if row >= 0 else 0, row, col, C.byref(cap)))
+        self.replica_ring = cap.value
+        return cap.value
+
+    def replica_probe_fetch(self, max_records=None):
+        """[n, replicas] float32: the oldest unfetched records, at most max_records (default: the capacity)."""
+        max_records = self.replica_ring if max_records is None else int(max_records)
+        out = np.empty((max_records, self.replicas), dtype=np.float32)
+        n = C.c_size_t()
+        check(lib().fib_replica_probe_fetch(self._h, out.ctypes.data_as(_P), max_records, C.byref(n)))
+        return out[:n.value]
+
     def activation_watch(self, up, down):
         """Arm (or re-arm) the activation maps of the diffusing variable at levels up / down."""
         check(lib().fib_activation_watch(self._h, up, down))
@@ -428,6 +450,20 @@ class Context:
         a, b = C.c_double(), C.c_double()
         check(lib().fib_weighted_sum(self._h, self.var(var), C.byref(a), C.byref(b)))
         return a.value, b.value
+
+    def replica_sums(self, var, slot=-1):
+        """(sum_wx, sum_w), float64 [replicas] each: weighted by the phase field (slot -1) or by weight slot 0..3."""
+        wx, w = np.empty(self.replicas), np.empty(self.replicas)
+        check(lib().fib_replica_sums(self._h, self.var(var), int(slot), wx.ctypes.data_as(_P), w.ctypes.data_as(_P),
+                                     self.replicas))
+        return wx, w
+
+    def replica_count_below(self, var, sub, div, cutoff, w_min):
+        """(below, total), int64 [replicas] each: count_below per replica."""
+        below, total = np.empty(self.replicas, np.uint64), np.empty(self.replicas, np.uint64)
+        check(lib().fib_replica_count_below(self._h, self.var(var), sub, div, cutoff, w_min,
+                                            below.ctypes.data_as(_P), total.ctypes.data_as(_P), self.replicas))
+        return below.astype(np.int64), total.astype(np.int64)
 
     def count_nonfinite(self, var):
         v = C.c_uint64()

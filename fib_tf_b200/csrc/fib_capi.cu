@@ -167,12 +167,17 @@ struct fib_ctx {
   float cheb[12][9];
   uint64_t launches = 0;
   std::vector<GraphKey> graphs;
-  double* red = nullptr;              // 2 doubles for reductions
+  double* red = nullptr;              // 2 doubles per replica for reductions
   // ODE iterations enqueued on this context: each observer below counts its own from the value at its arming
   unsigned long long ode_iters = 0;
   unsigned long long since(unsigned long long armed_at) const { return ode_iters - armed_at; }
-  // device-side cycle-length probe (fib_probe_watch): one watched cell, a ring of recorded values
+  // device-side cycle-length probe (fib_probe_watch): one watched cell, a ring of recorded values;
+  // fib_replica_probe_watch: the same local cell of every replica, one record of nrep values per iteration
   float* ring = nullptr;              // page-locked, device-visible: a fetch is a stream sync + host reads
+  size_t ring_floats = 0;             // allocated
+  unsigned long long ring_cap = FIB_PROBE_RING;   // records of the armed watch
+  int watch_n = 1;                    // floats per record: 1, or nrep for a replica watch
+  bool watch_replicas = false;        // the armed watch is fib_replica_probe_watch's
   unsigned long long* ring_count = nullptr;   // device: the slot the next record goes to
   unsigned long long probe_armed_at = 0;      // records made = since(probe_armed_at)
   unsigned long long ring_fetched = 0;
@@ -334,10 +339,14 @@ __global__ void phase_mask2_kernel(const float* __restrict__ phase, Geom g, unsi
   }
 }
 
+// Sums over row blocks of `rows` rows: block row blockIdx.y = z covers local rows [z * rows, (z + 1) * rows) and
+// adds into out[2z], out[2z + 1] (one block row over the shard: the whole-context sum; nrep: one per replica).
 __global__ void wsum_kernel(const float* __restrict__ x, const float* __restrict__ w, Geom g,
-                            int xhalo, double* out) {
+                            int xhalo, int rows, double* out) {
   double sx = 0.0, sw = 0.0;
-  for (int lr = blockIdx.x; lr < g.rows; lr += gridDim.x)
+  const int r0 = (int)blockIdx.y * rows;
+  out += 2 * blockIdx.y;
+  for (int lr = r0 + (int)blockIdx.x; lr < r0 + rows; lr += gridDim.x)
     for (int c = threadIdx.x; c < g.W; c += blockDim.x) {
       const double wv = w ? (double)w[(size_t)(lr + 1) * g.pitch + c] : 1.0;
       sx += wv * (double)x[(size_t)(lr + xhalo) * g.pitch + c];
@@ -359,20 +368,28 @@ __global__ void nonfinite_kernel(const float* __restrict__ x, Geom g, int xhalo,
   if ((threadIdx.x & 31) == 0 && n) atomicAdd(out, n);
 }
 
-// fib_probe_watch: append the watched cell to the ring (one thread; a node of the iteration graph)
-__global__ void probe_record_kernel(const float* __restrict__ src, float* __restrict__ ring,
+// fib_probe_watch / fib_replica_probe_watch: append one record, the `ncells` watched cells `rep_step` floats apart
+// (one per replica), to the ring of `cap` records (a node of the iteration graph).  ONE block: every thread has read
+// *count before thread 0 advances it.
+__global__ void probe_record_kernel(const float* __restrict__ src, size_t rep_step, int ncells,
+                                    float* __restrict__ ring, unsigned long long cap,
                                     unsigned long long* __restrict__ count) {
   const unsigned long long n = *count;
-  ring[n % FIB_PROBE_RING] = *src;
-  *count = n + 1;
+  float* rec = ring + (n % cap) * ncells;
+  for (int b = threadIdx.x; b < ncells; b += blockDim.x) rec[b] = src[(size_t)b * rep_step];
+  __syncthreads();
+  if (threadIdx.x == 0) *count = n + 1;
 }
 
 // a host-side write (stimulus, assign) after the iteration: the reference evaluates its probe AFTER
 // the driver's loop body (ionic.py:202-216), so the last recorded value follows the write
-__global__ void probe_update_kernel(const float* __restrict__ src, float* __restrict__ ring,
+__global__ void probe_update_kernel(const float* __restrict__ src, size_t rep_step, int ncells,
+                                    float* __restrict__ ring, unsigned long long cap,
                                     const unsigned long long* __restrict__ count) {
   const unsigned long long n = *count;
-  if (n) ring[(n - 1) % FIB_PROBE_RING] = *src;
+  if (!n) return;
+  float* rec = ring + ((n - 1) % cap) * ncells;
+  for (int b = threadIdx.x; b < ncells; b += blockDim.x) rec[b] = src[(size_t)b * rep_step];
 }
 
 // fib_frames_watch: one frame, a strided gather of a plane's owned rows.  `src` = the first owned row whose
@@ -387,11 +404,14 @@ __global__ void frame_record_kernel(const float* __restrict__ src, size_t src_st
 
 // court_ultra.py:504-509: cells with weight > w_min, and among them those whose normalised value
 // (x - sub) / div (the image() of br.py:337-343 / court.py:574-580, same fp32 operations) < cutoff
+// (row blocks as in wsum_kernel)
 __global__ void count_below_kernel(const float* __restrict__ x, const float* __restrict__ w, Geom g,
-                                   int xhalo, float sub, float div, float cutoff, float w_min,
+                                   int xhalo, int rows, float sub, float div, float cutoff, float w_min,
                                    unsigned long long* out) {
   unsigned long long below = 0, total = 0;
-  for (int lr = blockIdx.x; lr < g.rows; lr += gridDim.x)
+  const int r0 = (int)blockIdx.y * rows;
+  out += 2 * blockIdx.y;
+  for (int lr = r0 + (int)blockIdx.x; lr < r0 + rows; lr += gridDim.x)
     for (int c = threadIdx.x; c < g.W; c += blockDim.x) {
       const float wv = w ? w[(size_t)(lr + 1) * g.pitch + c] : 1.0f;
       if (wv > w_min) {
@@ -608,7 +628,7 @@ static int create_resources(fib_ctx* c) {
       CU(cudaMemsetAsync(c->s[k], 0, c->plane_floats() * sizeof(float), c->stream));
     }
   }
-  CU(cudaMalloc(&c->red, 2 * sizeof(double)));
+  CU(cudaMalloc(&c->red, 2 * c->nrep * sizeof(double)));
   if (c->nrep > 1) {
     CU(cudaMalloc(&c->zddt, c->nrep * sizeof(float)));
     const std::vector<double> diff(c->nrep, cfg->diff);
@@ -710,14 +730,20 @@ static float* owned_rows(fib_ctx* c, int var) {
   const PlaneRef p = plane_of(c, var);
   return p.base + (size_t)p.halo * c->g.pitch;
 }
+// the watched cell of the probe (of replica 0 for a replica watch), and the floats between two replicas' cells
+static const float* watch_src(fib_ctx* c) {
+  return owned_rows(c, c->watch_var) + (size_t)(c->watch_row - c->g.row0) * c->g.pitch + c->watch_col;
+}
+static size_t replica_step(const fib_ctx* c) { return (size_t)(c->g.H / c->nrep) * c->g.pitch; }
+static int probe_threads(const fib_ctx* c) { return min(c->watch_n, 1024); }
+
 // a host write into `var` invalidates the neighbours' copies of the rows they hold as halo, and
-// the last value the cycle-length probe recorded if it watches this plane (enqueue-only)
+// the last record the cycle-length probe made if it watches this plane (enqueue-only)
 static void mark_written(fib_ctx* c, int var) {
   if (var == 0 || c->fuse == 2) c->halo_dirty = true;
   if (var == c->watch_var) {
-    const PlaneRef p = plane_of(c, var);
-    const float* src = p.base + (size_t)(p.halo + c->watch_row - c->g.row0) * c->g.pitch + c->watch_col;
-    probe_update_kernel<<<1, 1, 0, c->stream>>>(src, c->ring, c->ring_count);
+    probe_update_kernel<<<1, probe_threads(c), 0, c->stream>>>(watch_src(c), replica_step(c), c->watch_n, c->ring,
+                                                               c->ring_cap, c->ring_count);
     c->launches++;
     c->probe_ledger.clear();                    // a recorded value changes after its launch's event
   }
@@ -838,13 +864,17 @@ extern "C" int fib_snapshot_wait(fib_ctx* c) {
   return 0;
 }
 
-// the probe ring's storage (allocations may synchronise with copies in flight: never between the
-// blocks of a pipelined upload and the steps behind it)
-static int ensure_ring(fib_ctx* c) {
-  if (!c->ring) {
-    CU(cudaHostAlloc(&c->ring, FIB_PROBE_RING * sizeof(float), cudaHostAllocMapped | cudaHostAllocPortable));
-    CU(cudaMalloc(&c->ring_count, sizeof(unsigned long long)));
+// the probe ring's storage, at least `floats` (allocations may synchronise with copies in flight: never between
+// the blocks of a pipelined upload and the steps behind it; the ring only grows, when no watch is armed)
+static int ensure_ring(fib_ctx* c, size_t floats) {
+  if (c->ring_floats < floats) {
+    cudaFreeHost(c->ring);
+    c->ring = nullptr;
+    c->ring_floats = 0;
+    CU(cudaHostAlloc(&c->ring, floats * sizeof(float), cudaHostAllocMapped | cudaHostAllocPortable));
+    c->ring_floats = floats;
   }
+  if (!c->ring_count) CU(cudaMalloc(&c->ring_count, sizeof(unsigned long long)));
   return c->probe_ledger.create();
 }
 
@@ -853,7 +883,7 @@ static int substeps_of(const fib_ctx* c, int op);
 // Everything an ODE iteration and its probe record can launch is loaded NOW (lazy loading would do it at
 // the first launch and wait for the copies in flight).  Called when a pipelined upload begins.
 static int preload_kernels(fib_ctx* c) {
-  int r = ensure_ring(c);
+  int r = ensure_ring(c, FIB_PROBE_RING);
   if (r) return r;
   cudaFuncAttributes fa;
   CU(cudaFuncGetAttributes(&fa, probe_record_kernel));
@@ -1497,8 +1527,8 @@ static int launch_frame(fib_ctx* c, unsigned long long j) {
 static int observe_rows(fib_ctx* c, int lo, int hi) {
   const int lr = c->watch_row - c->g.row0;
   if (c->watch_var < 0 || lr < lo || lr >= hi) return 0;
-  const float* src = owned_rows(c, c->watch_var) + (size_t)lr * c->g.pitch + c->watch_col;
-  probe_record_kernel<<<1, 1, 0, c->stream>>>(src, c->ring, c->ring_count);
+  probe_record_kernel<<<1, probe_threads(c), 0, c->stream>>>(watch_src(c), replica_step(c), c->watch_n, c->ring,
+                                                             c->ring_cap, c->ring_count);
   CU(cudaGetLastError());
   c->launches++;
   return 0;
@@ -2069,7 +2099,7 @@ extern "C" int fib_probe(fib_ctx* c, int var, int row, int col, float* out) {
   return 0;
 }
 
-static int reduce_weighted(fib_ctx* c, int var, const float* w, double* sum_wx, double* sum_w);
+static int reduce_weighted(fib_ctx* c, int var, const float* w, int parts, double* sum_wx, double* sum_w);
 // a sum over a batched context would mix its replicas: a silently wrong mean, rho or electrogram
 static int refuse_batched_sum(const fib_ctx* c, const char* what) {
   return fail(FIB_E_STATE, "%s sums over the whole context, which holds %d replicas", what, c->nrep);
@@ -2081,20 +2111,28 @@ extern "C" int fib_weighted_sum(fib_ctx* c, int var, double* sum_wx, double* sum
   if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
   DevGuard dg(c->cfg.device);
   FLUSH(c);
-  return reduce_weighted(c, var, c->phase, sum_wx, sum_w);
+  return reduce_weighted(c, var, c->phase, 1, sum_wx, sum_w);
 }
 
-static int reduce_weighted(fib_ctx* c, int var, const float* w, double* sum_wx, double* sum_w) {
-  CU(cudaMemsetAsync(c->red, 0, 2 * sizeof(double), c->stream));
+// the reductions' grid: `parts` row blocks of the shard (1, or one per replica), about 4 blocks per SM in all
+static dim3 reduce_grid(const fib_ctx* c, int parts) {
+  return dim3(min(c->g.rows / parts, max(4 * c->sms / parts, 1)), parts);
+}
+
+// sum(w * x) and sum(w) over each of `parts` row blocks of the shard into sum_wx[p], sum_w[p]
+static int reduce_weighted(fib_ctx* c, int var, const float* w, int parts, double* sum_wx, double* sum_w) {
+  CU(cudaMemsetAsync(c->red, 0, 2 * parts * sizeof(double), c->stream));
   const PlaneRef pl = plane_of(c, var);
-  wsum_kernel<<<min(c->g.rows, 4 * c->sms), 256, 0, c->stream>>>(pl.base, w, c->g, pl.halo, c->red);
+  wsum_kernel<<<reduce_grid(c, parts), 256, 0, c->stream>>>(pl.base, w, c->g, pl.halo, c->g.rows / parts, c->red);
   CU(cudaGetLastError());
   c->launches++;
-  double h[2];
-  CU(cudaMemcpyAsync(h, c->red, sizeof h, cudaMemcpyDeviceToHost, c->stream));
+  std::vector<double> h(2 * parts);
+  CU(cudaMemcpyAsync(h.data(), c->red, h.size() * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
-  *sum_wx = h[0];
-  *sum_w = h[1];
+  for (int p = 0; p < parts; ++p) {
+    sum_wx[p] = h[2 * p];
+    sum_w[p] = h[2 * p + 1];
+  }
   return 0;
 }
 
@@ -2141,11 +2179,23 @@ extern "C" int fib_masked_sum(fib_ctx* c, int var, int slot, double* sum_wx, dou
   if (slot < 0 || slot >= 4 || !c->weights[slot]) return fail(FIB_E_STATE, "weight slot %d is empty", slot);
   DevGuard dg(c->cfg.device);
   FLUSH(c);
-  return reduce_weighted(c, var, c->weights[slot], sum_wx, sum_w);
+  return reduce_weighted(c, var, c->weights[slot], 1, sum_wx, sum_w);
 }
 
-extern "C" int fib_probe_watch(fib_ctx* c, int var, int row, int col) {
-  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
+extern "C" int fib_replica_sums(fib_ctx* c, int var, int slot, double* sum_wx, double* sum_w, size_t n) {
+  if (!c || !sum_wx || !sum_w) return fail(FIB_E_ARG, "NULL argument");
+  if (n != (size_t)c->nrep) return fail(FIB_E_ARG, "fib_replica_sums: n=%zu, the context has %d replicas", n, c->nrep);
+  if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
+  if (slot < -1 || slot >= 4) return fail(FIB_E_ARG, "weight slot %d out of range -1..3", slot);
+  if (slot >= 0 && !c->weights[slot]) return fail(FIB_E_STATE, "weight slot %d is empty", slot);
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  return reduce_weighted(c, var, slot < 0 ? c->phase : c->weights[slot], c->nrep, sum_wx, sum_w);
+}
+
+// The probe ring's records: `ncells` cells per record (1, or one per replica), `cap` records.  Arming either kind
+// replaces the other; row < 0 disarms whichever is armed.
+static int probe_watch(fib_ctx* c, int var, int row, int col, bool replicas, int ncells, unsigned long long cap) {
   DevGuard dg(c->cfg.device);
   if (c->pending) FLUSH(c);             // (an upload still in flight stays in flight: nothing is read here)
   CU(cudaStreamSynchronize(c->stream));
@@ -2155,10 +2205,13 @@ extern "C" int fib_probe_watch(fib_ctx* c, int var, int row, int col) {
     return 0;
   }
   if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
-  if (row < c->g.row0 || row >= c->g.row0 + c->g.rows || col < 0 || col >= c->g.W)
-    return fail(FIB_E_ARG, "probe (%d,%d) is not in this shard", row, col);
+  // a replica watch: `row` local to a replica (the shard's own rows when unbatched: the replica is the grid)
+  const int rh = replicas ? c->g.H / c->nrep : c->g.H;
+  if (row >= rh || row < c->g.row0 || row >= c->g.row0 + c->g.rows || col < 0 || col >= c->g.W)
+    return fail(FIB_E_ARG, "probe (%d,%d) is not in this shard%s", row, col, replicas ? " or replica" : "");
+  c->watch_var = -1;
   {
-    const int er = ensure_ring(c);
+    const int er = ensure_ring(c, (size_t)cap * ncells);
     if (er) return er;
   }
   CU(cudaMemsetAsync(c->ring_count, 0, sizeof(unsigned long long), c->stream));
@@ -2166,10 +2219,29 @@ extern "C" int fib_probe_watch(fib_ctx* c, int var, int row, int col) {
   c->probe_ledger.clear();
   c->probe_armed_at = c->ode_iters;
   c->ring_fetched = 0;
+  c->ring_cap = cap;
+  c->watch_n = ncells;
+  c->watch_replicas = replicas;
   c->watch_var = var;
   c->watch_row = row;
   c->watch_col = col;
   return 0;
+}
+
+extern "C" int fib_probe_watch(fib_ctx* c, int var, int row, int col) {
+  if (!c) return fail(FIB_E_ARG, "ctx is NULL");
+  return probe_watch(c, var, row, col, false, 1, FIB_PROBE_RING);
+}
+
+// FIB_PROBE_RING records when unbatched: the layout the persistent kernel records into.  Batched: about 16 MiB of
+// page-locked memory, at least 256 records.
+extern "C" int fib_replica_probe_watch(fib_ctx* c, int var, int row, int col, size_t* capacity) {
+  if (!c || !capacity) return fail(FIB_E_ARG, "ctx/capacity is NULL");
+  const unsigned long long cap =
+      c->nrep == 1 ? FIB_PROBE_RING : min((unsigned long long)FIB_PROBE_RING, max(256ull, (1ull << 22) / c->nrep));
+  const int r = probe_watch(c, var, row, col, true, c->nrep, cap);
+  if (!r) *capacity = (size_t)cap;
+  return r;
 }
 
 // records [first, first + n) of a ring of `cap` slots as at most two contiguous pieces: copy(done, slot, len)
@@ -2185,13 +2257,14 @@ static int copy_ring(unsigned long long first, unsigned long long n, unsigned lo
   return 0;
 }
 
-extern "C" int fib_probe_fetch(fib_ctx* c, float* out, size_t max, size_t* n) {
+static int probe_fetch(fib_ctx* c, bool replicas, float* out, size_t max, size_t* n) {
   if (!c || !n || (!out && max)) return fail(FIB_E_ARG, "NULL argument");
   *n = 0;
-  if (c->watch_var < 0) return fail(FIB_E_STATE, "no probe is being watched (fib_probe_watch)");
+  if (c->watch_var < 0 || c->watch_replicas != replicas)
+    return fail(FIB_E_STATE, "no probe is being watched (%s)", replicas ? "fib_replica_probe_watch" : "fib_probe_watch");
   DevGuard dg(c->cfg.device);
   FLUSH(c);
-  // The records land in page-locked host memory.  Asked for fewer values than were recorded, wait only
+  // The records land in page-locked host memory.  Asked for fewer records than were made, wait only
   // for the launch that produced the last of them (the later ones keep the GPU busy meanwhile).
   const unsigned long long total = c->since(c->probe_armed_at);
   unsigned long long count = total;
@@ -2203,15 +2276,24 @@ extern "C" int fib_probe_fetch(fib_ctx* c, float* out, size_t max, size_t* n) {
     CU(cudaStreamSynchronize(c->stream));
   }
   unsigned long long first = c->ring_fetched;
-  if (count - first > FIB_PROBE_RING) first = count - FIB_PROBE_RING;      // the oldest were overwritten
+  if (count - first > c->ring_cap) first = count - c->ring_cap;      // the oldest were overwritten
   const unsigned long long take = min(count - first, (unsigned long long)max);
-  copy_ring(first, take, FIB_PROBE_RING, [&](unsigned long long done, unsigned long long pos, unsigned long long len) {
-    memcpy(out + done, c->ring + pos, len * sizeof(float));
+  const size_t rec = c->watch_n;
+  copy_ring(first, take, c->ring_cap, [&](unsigned long long done, unsigned long long pos, unsigned long long len) {
+    memcpy(out + done * rec, c->ring + pos * rec, len * rec * sizeof(float));
     return 0;
   });
   c->ring_fetched = first + take;
   *n = (size_t)take;
   return 0;
+}
+
+extern "C" int fib_probe_fetch(fib_ctx* c, float* out, size_t max, size_t* n) {
+  return probe_fetch(c, false, out, max, n);
+}
+
+extern "C" int fib_replica_probe_fetch(fib_ctx* c, float* out, size_t max_records, size_t* n) {
+  return probe_fetch(c, true, out, max_records, n);
 }
 
 // Activation maps: the sample s[0] is the current plane; the update runs after every ODE iteration from
@@ -2493,6 +2575,26 @@ extern "C" int fib_checkpoint_end(fib_ctx* c) {
   return 0;
 }
 
+// count_below_kernel over each of `parts` row blocks of the shard (as reduce_weighted) into below[p], total[p]
+static int reduce_count_below(fib_ctx* c, int var, float sub, float div, float cutoff, float w_min, int parts,
+                              uint64_t* below, uint64_t* total) {
+  CU(cudaMemsetAsync(c->red, 0, 2 * parts * sizeof(double), c->stream));
+  const PlaneRef pl = plane_of(c, var);
+  count_below_kernel<<<reduce_grid(c, parts), 256, 0, c->stream>>>(
+      pl.base, c->phase, c->g, pl.halo, c->g.rows / parts, sub, div, cutoff, w_min,
+      reinterpret_cast<unsigned long long*>(c->red));
+  CU(cudaGetLastError());
+  c->launches++;
+  std::vector<unsigned long long> h(2 * parts);
+  CU(cudaMemcpyAsync(h.data(), c->red, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  for (int p = 0; p < parts; ++p) {
+    below[p] = h[2 * p];
+    total[p] = h[2 * p + 1];
+  }
+  return 0;
+}
+
 extern "C" int fib_count_below(fib_ctx* c, int var, float sub, float div, float cutoff, float w_min,
                                uint64_t* below, uint64_t* total) {
   if (!c || !below || !total) return fail(FIB_E_ARG, "NULL argument");
@@ -2500,18 +2602,18 @@ extern "C" int fib_count_below(fib_ctx* c, int var, float sub, float div, float 
   if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
   DevGuard dg(c->cfg.device);
   FLUSH(c);
-  CU(cudaMemsetAsync(c->red, 0, 2 * sizeof(double), c->stream));
-  const PlaneRef pl = plane_of(c, var);
-  count_below_kernel<<<min(c->g.rows, 4 * c->sms), 256, 0, c->stream>>>(
-      pl.base, c->phase, c->g, pl.halo, sub, div, cutoff, w_min, reinterpret_cast<unsigned long long*>(c->red));
-  CU(cudaGetLastError());
-  c->launches++;
-  unsigned long long h[2] = {0, 0};
-  CU(cudaMemcpyAsync(h, c->red, sizeof h, cudaMemcpyDeviceToHost, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
-  *below = h[0];
-  *total = h[1];
-  return 0;
+  return reduce_count_below(c, var, sub, div, cutoff, w_min, 1, below, total);
+}
+
+extern "C" int fib_replica_count_below(fib_ctx* c, int var, float sub, float div, float cutoff, float w_min,
+                                       uint64_t* below, uint64_t* total, size_t n) {
+  if (!c || !below || !total) return fail(FIB_E_ARG, "NULL argument");
+  if (n != (size_t)c->nrep)
+    return fail(FIB_E_ARG, "fib_replica_count_below: n=%zu, the context has %d replicas", n, c->nrep);
+  if (var < 0 || var >= c->nvars) return fail(FIB_E_ARG, "state variable %d out of range", var);
+  DevGuard dg(c->cfg.device);
+  FLUSH(c);
+  return reduce_count_below(c, var, sub, div, cutoff, w_min, c->nrep, below, total);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -34,7 +34,9 @@ Extra, optional config keys (all default to the reference's behaviour):
                  (add_hole_to_phase_field(replica=)), stimuli (fire_op / pace with replica=) and `diff`: config
                  'diff' may be a sequence of B floats.  Reads (image(), pot().eval(), _State[n].eval(),
                  activation_maps(), frames()) gain a leading replica axis; assign() takes [H, W] or [B, H, W].
-                 Not with `distributed`, run(im), a cl_observer, masked_image_mean() or excitable_fraction().
+                 Not with `distributed`, run(im), a cl_observer, masked_image_mean() or excitable_fraction(): their
+                 per-replica forms are replica_cl_observer, masked_image_means(), excitable_fractions() and
+                 weighted_means(), computed on the device.
 
     upload_window  distributed runs: how many of run()'s first iterations may run behind a pipelined upload
                  (fib_set_rect_async blocks, even ranks top to bottom, odd ranks bottom to top; default 10,
@@ -117,6 +119,7 @@ class IonicModel:
         self.defined = False
         self.dt_per_step = 1
         self.cl_observer = None
+        self.replica_cl_observer = None
         self._ctx = None
         self._rank, self._nranks = 0, 1
         if config.get('distributed'):
@@ -428,18 +431,26 @@ class IonicModel:
 
             for i in model.run(im):
                 if i == s2: model.fire_op('s2')
+
+        replica_cl_observer(i, replica, cl), when set, is cl_observer for every replica: each replica's probe cell
+        image[20, W//2] is recorded on the device (include/fib_b200.h, fib_replica_probe_watch), and the observer is
+        called in order of i, then replica.  Headless, unsharded, and not together with cl_observer.
         """
         if not self.defined:
             raise AssertionError('define() must be called before run()')
         if self.replicas > 1 and (im or self.cl_observer is not None):
             raise ValueError('run(im) and cl_observer watch one cell of one grid: a batched model (replicas = %d) '
-                             'has activation maps (watch_activation) instead' % self.replicas)
+                             'has replica_cl_observer and activation maps (watch_activation) instead' % self.replicas)
+        rep_obs = self.replica_cl_observer
+        if rep_obs is not None and (self.cl_observer is not None or im or self._nranks > 1):
+            raise ValueError('replica_cl_observer: a headless run of an unsharded model, without cl_observer')
         then = time.time()
-        v0 = self.min_v
-        last_spike = 0
+        nrep = self.replicas if rep_obs is not None else 1
+        v0 = [self.min_v] * nrep
+        last_spike = [0] * nrep
         self.samples = int(self.duration / (self.dt_per_step * self.dt))
         plot_every = max(int(self.dt_per_plot / self.dt_per_step), 1)
-        watch = bool(im) or self.cl_observer is not None
+        watch = bool(im) or self.cl_observer is not None or rep_obs is not None
         prow, pcol = 20, self.width // 2                         # ionic.py:216
         # Headless watching: the owner rank of row 20 records the probe cell on the device after every
         # iteration (fib_probe_watch: a node of the iteration's CUDA graph) and reads the ring back once
@@ -449,32 +460,39 @@ class IonicModel:
         batch = max(1, min(int(self.__dict__.get('probe_batch', 64)), _capi.PROBE_RING // 2))
         unread = []                                              # iterations recorded, not yet read
 
-        def crossing(i, v1):
-            nonlocal v0, last_spike
-            if v1 >= 0.5 and v0 < 0.5:
-                cl = (i - last_spike) * self.dt_per_step * self.dt
-                if self.cl_observer is None:
+        def crossing(i, v1, b=0):
+            if v1 >= 0.5 and v0[b] < 0.5:
+                cl = (i - last_spike[b]) * self.dt_per_step * self.dt
+                if rep_obs is not None:
+                    rep_obs(i, b, cl)
+                elif self.cl_observer is None:
                     print('wavefront reaches the middle top point at %d, cycle length is %d' % (i, cl))
                 else:
                     self.cl_observer(i, cl)
-                last_spike = i
-            v0 = v1
+                last_spike[b] = i
+            v0[b] = v1
 
         def drain(n):
             # the oldest n recorded iterations; the library waits only for the launch that produced
             # them, so the iterations stepped since keep the device busy meanwhile
-            vals = self._ctx.probe_fetch(n) if n else []
+            fetch = self._ctx.probe_fetch if rep_obs is None else self._ctx.replica_probe_fetch
+            vals = fetch(n) if n else []
             if len(vals) != n:
                 raise RuntimeError('probe ring returned %d values for %d iterations' % (len(vals), n))
-            w = self._probe_weight(prow, pcol)
-            for k, raw in zip(unread[:n], vals):
+            # replica b's probe cell is row b * height + prow of the model's rows
+            w = [self._probe_weight(b * self.height + prow, pcol) for b in range(nrep)]
+            for k, rec in zip(unread[:n], vals):
                 if k % plot_every == 0:
-                    crossing(k, self._normalise(float(raw)) * w)
+                    for b, raw in enumerate(np.reshape(rec, nrep)):
+                        crossing(k, self._normalise(float(raw)) * w[b], b)
             del unread[:n]
 
         self._behind, self._behind_limit = 0, self._agree_on_upload_window(im, batch)
         self._upload_window_used = self._behind_limit
-        if ring:
+        if ring and rep_obs is not None:
+            # a batched ring may hold fewer records than run() leaves unread (two batches)
+            batch = max(1, min(batch, self._ctx.replica_probe_watch(self._pot_name, prow, pcol) // 2))
+        elif ring:
             self._ctx.probe_watch(self._pot_name, prow, pcol)
         try:
             for i in range(self.samples):
@@ -504,7 +522,7 @@ class IonicModel:
                 drain(len(unread))
         finally:
             if ring and self._ctx is not None:
-                self._ctx.probe_watch(self._pot_name, -1, -1)
+                (self._ctx.probe_watch if rep_obs is None else self._ctx.replica_probe_watch)(self._pot_name, -1, -1)
         if keep_state:                                           # ionic.py:226-229
             self.state = {}
             for s in self._State:
@@ -588,12 +606,12 @@ class IonicModel:
     # ---- extras ---------------------------------------------------------------------------------
     def add_probe_mask(self, mask):
         """Registers an [H, W] weight plane on the device (at most 4) and returns its slot; use
-        with masked_image_mean().  Backs the pseudo-electrograms of the reference's egm.py."""
+        with masked_image_mean().  Backs the pseudo-electrograms of the reference's egm.py.  A batched
+        model takes [H, W] (the same mask in every replica) or [B, H, W]; use with masked_image_means()."""
         if not self.defined:
             raise AssertionError('add_probe_mask should be called after calling define')
         slot = len(self.__dict__.setdefault('_mask_slots', []))
-        m = np.asarray(mask, dtype=np.float32)
-        self._ctx.set_weights(slot, m[self._row0:self._row0 + self._rows], self._row0)
+        self._ctx.set_weights(slot, self._own_rows(mask), self._row0)
         self._mask_slots.append(slot)
         return slot
 
@@ -631,8 +649,41 @@ class IonicModel:
 
     def _refuse_batched_sum(self, what):
         if self.replicas > 1:
-            raise ValueError('%s sums over the whole grid, and this model holds %d replicas: per-replica sums are not '
-                             'implemented yet (use image() or activation_maps() per replica)' % (what, self.replicas))
+            raise ValueError('%s sums over the whole grid, and this model holds %d replicas: use its per-replica form '
+                             '(masked_image_means, excitable_fractions, weighted_means)' % (what, self.replicas))
+
+    # ---- per-replica observers: one value per replica, [B] (B = 1 on an unbatched model) ------------------------
+    def _refuse_distributed(self, what):
+        if self._nranks > 1:
+            raise ValueError('%s: per-replica observers need an unsharded model (the scalar forms cover sharded '
+                             'runs)' % what)
+
+    def masked_image_means(self, slot):
+        """float64 [B]: masked_image_mean(slot) of every replica, np.mean(image()[b] * mask[b]), from one
+        reduction per replica on the device (include/fib_b200.h, fib_replica_sums)."""
+        self._refuse_distributed('masked_image_means')
+        swx, sw = self._ctx.replica_sums(self._pot_name, slot)
+        if self.MODEL_ID != _capi.FENTON4V:
+            swx = (swx - self.min_v * sw) / (self.max_v - self.min_v)
+        return swx / (self.height * self.width)
+
+    def excitable_fractions(self, cutoff=0.2, phase_min=1e-3):
+        """float64 [B]: excitable_fraction(cutoff, phase_min) of every replica (NaN where no cell has phase >
+        phase_min), from one threshold count per replica on the device (fib_replica_count_below)."""
+        self._refuse_distributed('excitable_fractions')
+        if self.MODEL_ID == _capi.FENTON4V:
+            sub, div = 0.0, 1.0
+        else:
+            sub, div = float(self.min_v), float(self.max_v - self.min_v)
+        below, total = self._ctx.replica_count_below(self._pot_name, sub, div, cutoff, phase_min)
+        return np.where(total > 0, below / np.maximum(total, 1), np.nan)
+
+    def weighted_means(self, name):
+        """float64 [B]: the phase-weighted mean of state `name` in every replica, np.average(x[b],
+        weights=phase[b]) (the plain mean without a phase field) -- the means of court_ultra.py's cl_observer."""
+        self._refuse_distributed('weighted_means')
+        swx, sw = self._ctx.replica_sums(name, -1)
+        return swx / sw
 
     def watch_activation(self, up=None, down=None):
         """Arms the device-side activation maps of the transmembrane variable (include/fib_b200.h,

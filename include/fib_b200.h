@@ -97,7 +97,9 @@ typedef struct {
  * (fib_stimulate_replica, fib_pace_add_replica) take a replica and rows local to it.
  * Refused on a batched context: row shards (rows != 0), fib_comm_init and fib_step_group (FIB_E_ARG); the
  * whole-context sums fib_weighted_sum, fib_masked_sum and fib_count_below (FIB_E_STATE: they would mix the
- * replicas); fib_frames_watch / fib_frames_resume with a stride that does not divide height (FIB_E_ARG).
+ * replicas; fib_replica_sums and fib_replica_count_below give one per replica, and fib_replica_probe_watch records
+ * one cell of every replica); fib_frames_watch / fib_frames_resume with a stride that does not divide height
+ * (FIB_E_ARG).
  * fib_set_rect_async blocks are copied in order and never start a pipelined upload.  The persistent on-chip
  * kernel is never used.
  * fib_set_replica_diff sets diff of every replica (n == replicas; FIB_E_STATE on an unbatched context); it
@@ -281,6 +283,31 @@ int fib_probe_fetch(fib_ctx *ctx, float *out, size_t max, size_t *n);
  * cutoff, *total = cells with weight > w_min (weight = phase field, 1 if none).  Synchronous. */
 int fib_count_below(fib_ctx *ctx, int var, float sub, float div, float cutoff, float w_min,
                     uint64_t *below, uint64_t *total);
+
+/* Per-replica observers: what the calls above give for one grid, for every replica of a batched context (and for
+ * the one grid of an unbatched context, replica 0 = this shard).  `n` must equal the number of replicas (1 when
+ * unbatched; FIB_E_ARG otherwise).  Each launches the deferred iterations first.
+ * fib_replica_sums: sum_wx[b] = sum(w * x) and sum_w[b] = sum(w) over replica b's rows, with w = the phase field
+ * (1 if none) for slot = -1, as fib_weighted_sum, or the weight plane of slot 0..3, as fib_masked_sum (FIB_E_STATE
+ * if the slot is empty).  The weight planes of a batched context hold replicas * height rows (fib_set_weights).
+ * fib_replica_count_below: fib_count_below per replica.  Synchronous.  Sums are accumulated in double in an order
+ * that varies from call to call: the last bits of sum_wx may differ between calls and from the unbatched sum. */
+int fib_replica_sums(fib_ctx *ctx, int var, int slot, double *sum_wx, double *sum_w, size_t n);
+int fib_replica_count_below(fib_ctx *ctx, int var, float sub, float div, float cutoff, float w_min,
+                            uint64_t *below, uint64_t *total, size_t n);
+/* fib_replica_probe_watch: the probe ring of fib_probe_watch for cell (row, col) of EVERY replica, `row` local to
+ * a replica (0 <= row < height; on an unbatched context it must lie in this shard).  After every FIB_OP_ODE
+ * iteration one record of `replicas` floats -- cell (b * height + row, col) for b = 0 .. replicas - 1 -- is
+ * appended, with the ordering rules of fib_probe_watch per replica: a fib_stimulate_replica, a fib_set_state or a
+ * pacing beat after iteration k re-takes record k for every replica.  *capacity returns the records the ring holds:
+ * FIB_PROBE_RING on an unbatched context (the persistent kernel keeps its batches), else
+ * min(FIB_PROBE_RING, max(256, 2^22 / replicas)) (16 MiB of page-locked memory up to 16384 replicas).  FIB_E_CUDA if
+ * the ring cannot be allocated.  row < 0 removes the watch.  One watch of either kind is armed at a time: arming one
+ * replaces the other, and the fetch of the kind not armed is FIB_E_STATE.
+ * fib_replica_probe_fetch: as fib_probe_fetch, in records: out[*n][replicas], oldest first, at most max_records;
+ * more than *capacity unfetched records lose the oldest. */
+int fib_replica_probe_watch(fib_ctx *ctx, int var, int row, int col, size_t *capacity);
+int fib_replica_probe_fetch(fib_ctx *ctx, float *out, size_t max_records, size_t *n);
 
 /* activation maps (SURVEY 8f1): the activation-time (LAT), repolarisation and cycle-length maps of the whole
  * shard, recorded on the device while stepping, so that APD, cycle length and conduction velocity need no
